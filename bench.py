@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- 33-bus env-steps/s (incl. power flow) of the fused flex_provision step.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs-per-gpu E] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs-per-gpu E] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one fused env step (action application, injections, DistFlow power flow,
 constraint masks, reward/penalty, ESS update, bookkeeping: flexibility_provision_env.py:241-356)
@@ -24,6 +24,12 @@ solves, both kernel variants, 776 B/solve), `config3` (65 536 envs), `config4` (
 ring, 262 144 envs), `config5_strong` (every N: 2^20 envs IN TOTAL split over the N GPUs -- strong
 scaling of config 5), `step_plus_get_obs` (fused step + observation push into the env-minor ring,
 the rollout loop's env cost), `roofline_fp64` (the step kernel against the fp64 pipe).
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what the last timed step returned to its caller
+(reward, terminated, the eight info fields; one value per env) as DIR/<name>.npy in float64 (terminated in
+float32), at most 64 MB in all: above that, the same fixed seeded sample of envs from every array, with its
+env indices in DIR/env_index.npy.  Inputs are seeded, so two builds run with the same arguments can be
+compared output for output.
 
 --impl reference: the CPU arm.  The reference's own implementation (Pyomo + IPOPT) is probed for
 (`import pyomo`, `which ipopt`: utils/pf.py:101) but is not installable here (SURVEY 8c), so this
@@ -183,6 +189,27 @@ def make_config(args, world, auto_reset):
     return c
 
 
+DUMP_MAX_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, reward, done, info):
+    """What one env.step(..., want_info=True) returned, as DIR/<name>.npy (see --dump-outputs)."""
+    import numpy as np
+    import torch
+    arrays = {"reward": reward.double(), "terminated": done.float()}
+    arrays.update({f"info_{k}": v.double() for k, v in info.items()})
+    n = reward.shape[0]
+    per_env = sum(t.element_size() for t in arrays.values())
+    if n * per_env > DUMP_MAX_BYTES:
+        k = (DUMP_MAX_BYTES - 4096) // (per_env + 8)               # + 8: the float64 env index; 4096: the .npy headers
+        sel = torch.from_numpy(np.sort(np.random.default_rng(0).choice(n, k, replace=False))).to(reward.device)
+        arrays = {name: t.index_select(0, sel) for name, t in arrays.items()}
+        arrays["env_index"] = sel.double()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 def probe_reference_solver():
     """BASELINE.md 4.1: is the reference's own power flow (Pyomo + the ipopt binary, utils/pf.py:101) runnable here?"""
     try:
@@ -265,7 +292,13 @@ def main():
     ap.add_argument("--no-strong", action="store_true", help="skip the extra strong-scaling (2^20 envs in total) measurement")
     ap.add_argument("--no-rollout", action="store_true", help="skip the extra device-rollout measurement (policy + step + get_obs [+ Transition writes])")
     ap.add_argument("--variant", default="thread", choices=["thread", "warp"], help="kernel variant (see include/flexgpu.h)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy "
+                    "(rank 0's envs only when several GPUs run)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of the GPU path; it does not apply to --impl reference")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -309,8 +342,9 @@ def main():
             env.reset(return_obs=False)                       # Philox auto-reset, one launch
             state["t"] = 0
             state["timed_resets"] += 1 if timed else 0
-        env.step(acts[k % n_act], want_info=True)
+        out = env.step(acts[k % n_act], want_info=True)
         state["t"] += 1
+        return out
 
     for k in range(W):
         if not args.no_flush:
@@ -330,7 +364,7 @@ def main():
         if not args.no_flush:
             flush.zero_()
         ev[k][0].record(stream)
-        one_step(W + k, True)
+        last = one_step(W + k, True)
         ev[k][1].record(stream)
     barrier()
     t_wall = time.perf_counter() - t_wall0
@@ -340,6 +374,8 @@ def main():
     step_ms = sorted(a.elapsed_time(b) for a, b in ev)
     kern_ms = statistics.median(step_ms)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)        # before the measurements below step or reset this env again
 
     # ---- e2e: through fp_step_host with pinned HOST buffers (copies + sync inside)
     h_act = torch.rand(4, E, 20, dtype=torch.float32).pin_memory()

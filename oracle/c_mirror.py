@@ -5,9 +5,12 @@ arrays and advances them with the C restatement of reset/step; `mirror_power_flo
 batched power flow.  Used by the GPU parity tests (bit-exact masks, ulp-level floats) and as
 bench.py's CPU baseline.
 """
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 from math import acos, tan
 
 import numpy as np
@@ -18,9 +21,18 @@ NL = 32
 
 
 def build(force=False):
+    """Compiles the mirror into oracle/_build/ if it is missing or older than its source.  A tree that cannot be
+    written (a read-only checkout) gets it compiled into a temporary directory instead, removed at exit."""
+    global LIB
     src = os.path.join(_HERE, "c", "flex_oracle.c")
     if force or not os.path.exists(LIB) or os.path.getmtime(LIB) < os.path.getmtime(src):
-        subprocess.run(["make", "-C", os.path.join(_HERE, "c")], check=True, capture_output=True)
+        out_dir = os.path.dirname(LIB)
+        if not os.access(out_dir if os.path.isdir(out_dir) else _HERE, os.W_OK):
+            out_dir = tempfile.mkdtemp(prefix="flex_oracle_")
+            atexit.register(shutil.rmtree, out_dir, True)
+        out = os.path.join(out_dir, "libflex_oracle.so")
+        subprocess.run(["make", "-C", os.path.join(_HERE, "c"), f"OUT={out}"], check=True, capture_output=True)
+        LIB = out
     return LIB
 
 

@@ -183,7 +183,8 @@ def test_reference_fit_predictions(env, cuda):
     """k_predict with the REFERENCE'S regressor + scalers against sklearn's predictions of all 1000 scenarios the
     reference generated, and against the scaled predictions its training script computed on its test split."""
     from flexgpu.predictor import VoltagePredictor
-    g = np.load(os.path.join(os.path.dirname(__file__), "golden", "ref_predictor.npz"))
+    from _golden import load_ref_predictor
+    g = load_ref_predictor()
     p = VoltagePredictor.from_linear_model(env, g["coef"], g["intercept"], g["x_scale"], g["x_min"], g["y_scale"], g["y_min"])
     vhat, pen = p.predict(torch.from_numpy(g["X"].astype(np.float32)).to(cuda))
     V = vhat.cpu().numpy().astype(np.float64)

@@ -115,6 +115,17 @@ def test_bench_reference_arm_runs_on_cpu():
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["e2e"]["value"] == line["value"]
 
 
+@pytest.mark.parametrize("extra,message", [(["--steps", "0"], "--steps must be at least 1"),
+                                           (["--impl", "reference", "--dump-outputs", "out"], "does not apply to --impl reference")])
+def test_bench_rejects_arguments_it_cannot_honour(extra, message):
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py")] + extra, capture_output=True, text=True, timeout=60, cwd=root)
+    assert out.returncode == 2 and message in out.stderr, out.stderr[-2000:]
+
+
 # ---------------------------------------------------------------------------------------------------
 def test_load_csv_profiles_equals_the_reference_loaders(tmp_path):
     """flexgpu.load_csv_profiles against the output of the reference's own _load_*_data + resample_data

@@ -7,6 +7,7 @@ import numpy as np
 import pytest
 
 from oracle import predictor_ref, replay_ref
+from _golden import load_ref_predictor
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "predictor_golden.npz")
 
@@ -63,18 +64,18 @@ def test_replay_fifo_and_contiguous_window():
 # PIN on the reference's own scripts: tests/golden/ref_predictor.npz holds what safety_signal/data_generation.py
 # and train_safety_signal_model.py (executed unchanged, file I/O intercepted) produced -- the 1000 scenarios, the
 # fitted regressor, the scalers the script forgets to save, and its own predictions.
-REF = os.path.join(os.path.dirname(__file__), "golden", "ref_predictor.npz")
+# The scenarios X are redrawn by tests/_golden.py and checked against the SHA-256 of the reference's bytes.
 
 
 def test_oracle_scenarios_equal_the_reference_script():
-    g = np.load(REF)
+    g = load_ref_predictor()
     X, Y = predictor_ref.generate_scenarios(40, seed=2024)         # same stream: 33 P draws then 33 Q draws per scenario
     assert np.array_equal(X, g["X"][:40])
     assert np.max(np.abs(Y - g["Y"][:40])) < 1e-10                 # sweep vs Newton behind the reference's model
 
 
 def test_oracle_fit_equals_the_reference_fit():
-    g = np.load(REF)
+    g = load_ref_predictor()
     m, sx, sy = predictor_ref.fit_pipeline(g["X"], g["Y"])
     coef = np.array([e.coef_ for e in m.estimators_])
     # the slack-bus columns of X and Y are constant (scale 1, all-zero scaled column): their coefficients are
@@ -89,7 +90,7 @@ def test_folded_affine_map_equals_the_reference_predictions():
     """The host-side folding (VoltagePredictor.from_linear_model) applied to the reference's regressor and scalers
     reproduces (i) sklearn's predictions in p.u. for all 1000 scenarios and (ii) the scaled predictions the
     reference's script itself computed on its test split (train_safety_signal_model.py:76)."""
-    g = np.load(REF)
+    g = load_ref_predictor()
     A, c = fold(g)
     V = predictor_ref.affine_predict(A, c, g["X"])
     assert np.max(np.abs(V - g["V_pred"])) < 1e-12
