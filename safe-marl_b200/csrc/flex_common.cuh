@@ -158,6 +158,11 @@ __device__ __forceinline__ void stage_topo(DevTopo* s_topo, const DevTopo* __res
     __syncthreads();
 }
 
+// two int32 fields of one 64-bit record word: lo in the low half
+__device__ __forceinline__ uint64_t pack2(int32_t lo, int32_t hi) {
+    return (uint64_t)(uint32_t)lo | ((uint64_t)(uint32_t)hi << 32);
+}
+
 __device__ __forceinline__ double clipd(double x, double lo, double hi) {
     // numpy.clip == minimum(maximum(x, lo), hi)
     double t = (x > lo) ? x : lo;

@@ -20,10 +20,6 @@ namespace {
 constexpr int WARPS_PER_CTA = FP_CTA_THREADS / 32;
 constexpr int SCRATCH_DOUBLES = 32;   // per-warp shared scratch
 
-__device__ __forceinline__ uint64_t pack2(int32_t lo, int32_t hi) {
-    return (uint64_t)(uint32_t)lo | ((uint64_t)(uint32_t)hi << 32);
-}
-
 template <int MODE>
 __global__ void __launch_bounds__(FP_CTA_THREADS) k_env(const EnvParams prm) {
     __shared__ DevTopo s_topo;

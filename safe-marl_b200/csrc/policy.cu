@@ -39,6 +39,7 @@
 #include <vector>
 
 #include "flex_common.cuh"
+#include "sm100_ptx.cuh"
 
 namespace {
 
@@ -85,114 +86,14 @@ struct PolParams {
     float* st_out; int64_t st_pitch, st_row0, st_cap, st_n;
 };
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-// Bounded wait: a protocol mistake must surface as a trap, never as a hung GPU.
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t done = 0;
-    for (uint32_t spin = 0; !done; ++spin) {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.b32 %0, 1, 0, p;\n\t}"
-            : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-        if (!done && spin > (1u << 24)) __trap();
-    }
-}
-__device__ __forceinline__ void tma_load_1d(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-// One box of the 3-D ring view [24 slots][30 = agent x feature][n_pad envs]: 24 x 6 x 128 floats -> [144][128] in shared memory
-__device__ __forceinline__ void tma_load_box(uint32_t dst, const CUtensorMap* map, int32_t c_env, int32_t c_row, uint32_t bar) {
+// One box of the 3-D ring view [24 slots][30 = agent x feature][n_pad envs], starting at (c_env, c_row, c_slot): box_slots x 6
+// x 128 floats -> [6 box_slots][128] in shared memory (k_policy: all 24 slots, k_critic: 12)
+__device__ __forceinline__ void tma_load_box(uint32_t dst, const CUtensorMap* map, int32_t c_env, int32_t c_row, int32_t c_slot, uint32_t bar) {
     asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
-                 ::"r"(dst), "l"(map), "r"(c_env), "r"(c_row), "r"(0), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(smem_dst)), "l"(gsrc) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
-template <int ID, int THREADS>
-__device__ __forceinline__ void group_sync() { asm volatile("bar.sync %0, %1;" ::"n"(ID), "n"(THREADS) : "memory"); }
-__device__ __forceinline__ bool elect_one() {
-    uint32_t p;
-    asm volatile("{\n\t.reg .pred P1;\n\telect.sync _|P1, 0xffffffff;\n\tselp.b32 %0, 1, 0, P1;\n\t}" : "=r"(p));
-    return p != 0u;
+                 ::"r"(dst), "l"(map), "r"(c_env), "r"(c_row), "r"(c_slot), "r"(bar) : "memory");
 }
 
-// Shared-memory matrix descriptor, K-major, no swizzle: [k-chunk of 4 tf32][n][4]; LBO = bytes between the two
-// 16-byte K chunks of one MMA (= N * 16), SBO = bytes between 8-row groups (128); version 1 (sm_100).
-__device__ __forceinline__ uint64_t umma_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-    return (uint64_t)((saddr >> 4) & 0x3FFFu) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16) |
-           ((uint64_t)((sbo_bytes >> 4) & 0x3FFFu) << 32) | (1ull << 46);
-}
-// Instruction descriptor: D fp32, A/B tf32, both K-major, N >> 3 at bit 17, M >> 4 at bit 24.
-__host__ __device__ constexpr uint32_t idesc_n(uint32_t n) {
-    return (1u << 4) | (2u << 7) | (2u << 10) | ((n >> 3) << 17) | ((uint32_t)(POL_M >> 4) << 24);
-}
-// D[tmem] (+)= A[tmem: lane = row, one 32-bit column per k] * B[smem]
-__device__ __forceinline__ void umma_tf32_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tmem_st4(uint32_t taddr, float a, float b, float c, float d) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};"
-                 ::"r"(taddr), "r"(__float_as_uint(a)), "r"(__float_as_uint(b)), "r"(__float_as_uint(c)), "r"(__float_as_uint(d)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld4(uint32_t taddr, float (&r)[4]) {
-    uint32_t a, b, c, d;
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(a), "=r"(b), "=r"(c), "=r"(d) : "r"(taddr));
-    r[0] = __uint_as_float(a); r[1] = __uint_as_float(b); r[2] = __uint_as_float(c); r[3] = __uint_as_float(d);
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
-    uint32_t r[32];
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
-          "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]), "=r"(r[18]),
-          "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]),
-          "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-        : "r"(taddr));
-#pragma unroll
-    for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
-    uint32_t r[16];
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-        : "r"(taddr));
-#pragma unroll
-    for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
-}
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&v)[8]) {
-    uint32_t r[8];
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]) : "r"(taddr));
-#pragma unroll
-    for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
-}
-__device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+constexpr uint32_t IDESC_N64 = umma_idesc_tf32(POL_M, 64), IDESC_N32 = umma_idesc_tf32(POL_M, 32);
 
 __device__ __forceinline__ float tf32_hi(float x) { return __uint_as_float(__float_as_uint(x) & 0xFFFFE000u); }
 
@@ -323,7 +224,7 @@ __global__ void __launch_bounds__(POL_THREADS, 1) k_policy(const PolParams prm, 
     // One TMA box copy by the MMA warp (tma_request); rings narrower than a tile take coalesced LDGSTS by the workers.
     auto tma_request = [&](int64_t tile) {                                   // one thread
         mbar_expect_tx(bar_x, POL_OBS * POL_M * 4);
-        tma_load_box(smem_u32(stage), &tmap, (int32_t)((tile / POL_NA) * POL_M), (int32_t)(tile % POL_NA) * POL_F, bar_x);
+        tma_load_box(smem_u32(stage), &tmap, (int32_t)((tile / POL_NA) * POL_M), (int32_t)(tile % POL_NA) * POL_F, 0, bar_x);
     };
     auto request = [&](int64_t tile) {
         const int a = (int)(tile % POL_NA);
@@ -344,7 +245,7 @@ __global__ void __launch_bounds__(POL_THREADS, 1) k_policy(const PolParams prm, 
     if (tid == 0) {
         mbar_init(bar_a, N_WORKERS); mbar_init(bar_m, 1); mbar_init(bar_w, 1); mbar_init(bar_x, 1);
         mbar_init(bar_q0, 1); mbar_init(bar_q0 + 8, 1); mbar_init(bar_s, N_WRITERS);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
         if (prm.use_tma && (int64_t)blockIdx.x < n_tiles) tma_request(blockIdx.x);
         mbar_expect_tx(bar_w, W1_BYTES + WG_BYTES + V_FLOATS * 4);          // weights: three bulk copies, one barrier
         tma_load_1d(smem_u32(smem + OFF_W1), prm.W1rot + (size_t)prm.slot * (W1_BYTES / 4), W1_BYTES, bar_w);
@@ -352,8 +253,8 @@ __global__ void __launch_bounds__(POL_THREADS, 1) k_policy(const PolParams prm, 
         tma_load_1d(smem_u32(smem + OFF_VEC), prm.vec, V_FLOATS * 4, bar_w);
     }
     if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(512) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc<512>(smem_u32(tmem_slot));
+        tmem_relinquish();
     }
     if (!prm.use_tma && tid < N_WORKERS && (int64_t)blockIdx.x < n_tiles) request(blockIdx.x);
     tc_fence_before();
@@ -377,8 +278,8 @@ __global__ void __launch_bounds__(POL_THREADS, 1) k_policy(const PolParams prm, 
 #pragma unroll
                 for (int ks = 0; ks < POL_OBS / 8; ++ks) {
                     const uint64_t db = umma_desc(w1 + ks * 2 * (64 * 16), 64 * 16, 128);
-                    umma_tf32_ts(tmem_base + C_ACC1, tmem_base + C_XHI + 8 * ks, db, idesc_n(64), ks > 0 ? 1u : 0u);
-                    umma_tf32_ts(tmem_base + C_ACC1, tmem_base + C_XLO + 8 * ks, db, idesc_n(64), 1u);
+                    umma_tf32_ts(tmem_base + C_ACC1, tmem_base + C_XHI + 8 * ks, db, IDESC_N64, ks > 0 ? 1u : 0u);
+                    umma_tf32_ts(tmem_base + C_ACC1, tmem_base + C_XLO + 8 * ks, db, IDESC_N64, 1u);
                 }
                 umma_commit(bar_m);
             }
@@ -407,14 +308,14 @@ __global__ void __launch_bounds__(POL_THREADS, 1) k_policy(const PolParams prm, 
                         const uint64_t d_rz_h = umma_desc(b_rz_hh + ks * 2 * (128 * 16) + hf * 64 * 16, 128 * 16, 128);
                         const uint64_t d_n_i = umma_desc(b_n_ih + ks * 2 * (64 * 16) + hf * 32 * 16, 64 * 16, 128);
                         const uint64_t d_n_h = umma_desc(b_n_hh + ks * 2 * (64 * 16) + hf * 32 * 16, 64 * 16, 128);
-                        umma_tf32_ts(tmem_base + C_RZ + 64 * hf, tmem_base + C_A2HI + 8 * ks, d_rz_i, idesc_n(64), ks > 0 ? 1u : 0u);
-                        umma_tf32_ts(tmem_base + C_RZ + 64 * hf, tmem_base + C_A2LO + 8 * ks, d_rz_i, idesc_n(64), 1u);
-                        umma_tf32_ts(tmem_base + C_RZ + 64 * hf, tmem_base + C_A3HI + 8 * ks, d_rz_h, idesc_n(64), 1u);
-                        umma_tf32_ts(tmem_base + C_RZ + 64 * hf, tmem_base + C_A3LO + 8 * ks, d_rz_h, idesc_n(64), 1u);
-                        umma_tf32_ts(tmem_base + C_GIN + 32 * hf, tmem_base + C_A2HI + 8 * ks, d_n_i, idesc_n(32), ks > 0 ? 1u : 0u);
-                        umma_tf32_ts(tmem_base + C_GIN + 32 * hf, tmem_base + C_A2LO + 8 * ks, d_n_i, idesc_n(32), 1u);
-                        umma_tf32_ts(tmem_base + C_GHN + 32 * hf, tmem_base + C_A3HI + 8 * ks, d_n_h, idesc_n(32), ks > 0 ? 1u : 0u);
-                        umma_tf32_ts(tmem_base + C_GHN + 32 * hf, tmem_base + C_A3LO + 8 * ks, d_n_h, idesc_n(32), 1u);
+                        umma_tf32_ts(tmem_base + C_RZ + 64 * hf, tmem_base + C_A2HI + 8 * ks, d_rz_i, IDESC_N64, ks > 0 ? 1u : 0u);
+                        umma_tf32_ts(tmem_base + C_RZ + 64 * hf, tmem_base + C_A2LO + 8 * ks, d_rz_i, IDESC_N64, 1u);
+                        umma_tf32_ts(tmem_base + C_RZ + 64 * hf, tmem_base + C_A3HI + 8 * ks, d_rz_h, IDESC_N64, 1u);
+                        umma_tf32_ts(tmem_base + C_RZ + 64 * hf, tmem_base + C_A3LO + 8 * ks, d_rz_h, IDESC_N64, 1u);
+                        umma_tf32_ts(tmem_base + C_GIN + 32 * hf, tmem_base + C_A2HI + 8 * ks, d_n_i, IDESC_N32, ks > 0 ? 1u : 0u);
+                        umma_tf32_ts(tmem_base + C_GIN + 32 * hf, tmem_base + C_A2LO + 8 * ks, d_n_i, IDESC_N32, 1u);
+                        umma_tf32_ts(tmem_base + C_GHN + 32 * hf, tmem_base + C_A3HI + 8 * ks, d_n_h, IDESC_N32, ks > 0 ? 1u : 0u);
+                        umma_tf32_ts(tmem_base + C_GHN + 32 * hf, tmem_base + C_A3LO + 8 * ks, d_n_h, IDESC_N32, 1u);
                     }
                     umma_commit(bar_q0 + 8 * hf);
                 }
@@ -596,8 +497,7 @@ __global__ void __launch_bounds__(POL_THREADS, 1) k_policy(const PolParams prm, 
 
     tc_fence_before();
     __syncthreads();
-    if (warp == 0)
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(512) : "memory");
+    if (warp == 0) tmem_dealloc<512>(tmem_base);
 }
 
 // ---------------------------------------------------------------------------- critic: MADDPG.value on tcgen05
@@ -670,9 +570,8 @@ __global__ void __launch_bounds__(CRIT_THREADS, 1) k_critic(const CritParams prm
         const uint32_t bar = bar_x0 + 8 * (uint32_t)(g % CR_NST);
         const int a = (int)((g % CR_HB) >> 1), hf = (int)(g & 1);
         mbar_expect_tx(bar, CR_ST_BYTES);
-        asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
-                     ::"r"(smem_u32(smem + CO_ST + (g % CR_NST) * CR_ST_BYTES)), "l"(&tmap), "r"((int32_t)(tile_of(g) * POL_M)), "r"(a * POL_F),
-                       "r"(hf * (POL_H / 2)), "r"(bar) : "memory");
+        tma_load_box(smem_u32(smem + CO_ST + (g % CR_NST) * CR_ST_BYTES), &tmap, (int32_t)(tile_of(g) * POL_M), a * POL_F,
+                     hf * (POL_H / 2), bar);
     };
     auto load_wb = [&](int64_t g) {                                          // one thread: fc1 half-block weights -> buffer g % 4
         const uint32_t bar = bar_wb0 + 8 * (uint32_t)(g % CR_NWB);
@@ -701,7 +600,7 @@ __global__ void __launch_bounds__(CRIT_THREADS, 1) k_critic(const CritParams prm
         mbar_init(bar_w, 1);
         for (int i = 0; i < CR_NST; ++i) mbar_init(bar_x0 + 8 * i, 1);
         for (int i = 0; i < CR_NWB; ++i) mbar_init(bar_wb0 + 8 * i, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
         for (int64_t g = 0; g < CR_NST && g < n_hb; ++g) if (prm.use_tma) tma_request(g);
         for (int64_t g = 0; g < 2 && g < n_hb; ++g) load_wb(g);
         mbar_expect_tx(bar_w, CR_W2_BYTES + CR_WA_BYTES + CV_FLOATS * 4);    // fc2, action columns, small arrays: one barrier
@@ -710,8 +609,8 @@ __global__ void __launch_bounds__(CRIT_THREADS, 1) k_critic(const CritParams prm
         tma_load_1d(smem_u32(smem + CO_VEC), prm.vec, CV_FLOATS * 4, bar_w);
     }
     if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(512) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc<512>(smem_u32(tmem_slot));
+        tmem_relinquish();
     }
     tc_fence_before();
     __syncthreads();
@@ -739,15 +638,15 @@ __global__ void __launch_bounds__(CRIT_THREADS, 1) k_critic(const CritParams prm
 #pragma unroll
                 for (int ks = 0; ks < CR_KH / 8; ++ks) {
                     const uint64_t db = d0 + (uint64_t)((ks * 2 * (64 * 16)) >> 4);
-                    umma_tf32_ts(tmem_base + CC_ACC1, xb + 8 * ks, db, idesc_n(64), (hb > 0 || ks > 0) ? 1u : 0u);
-                    umma_tf32_ts(tmem_base + CC_ACC1, xb + CR_KH + 8 * ks, db, idesc_n(64), 1u);
+                    umma_tf32_ts(tmem_base + CC_ACC1, xb + 8 * ks, db, IDESC_N64, (hb > 0 || ks > 0) ? 1u : 0u);
+                    umma_tf32_ts(tmem_base + CC_ACC1, xb + CR_KH + 8 * ks, db, IDESC_N64, 1u);
                 }
                 if (hb == 0) {
 #pragma unroll
                     for (int ks = 0; ks < CR_KACT / 8; ++ks) {
                         const uint64_t db = umma_desc(wa + ks * 2 * (64 * 16), 64 * 16, 128);
-                        umma_tf32_ts(tmem_base + CC_ACC1, tmem_base + CC_ACTHI + 8 * ks, db, idesc_n(64), 1u);
-                        umma_tf32_ts(tmem_base + CC_ACC1, tmem_base + CC_ACTLO + 8 * ks, db, idesc_n(64), 1u);
+                        umma_tf32_ts(tmem_base + CC_ACC1, tmem_base + CC_ACTHI + 8 * ks, db, IDESC_N64, 1u);
+                        umma_tf32_ts(tmem_base + CC_ACC1, tmem_base + CC_ACTLO + 8 * ks, db, IDESC_N64, 1u);
                     }
                 }
                 umma_commit(bar_m0 + 8 * b);
@@ -770,8 +669,8 @@ __global__ void __launch_bounds__(CRIT_THREADS, 1) k_critic(const CritParams prm
 #pragma unroll
                     for (int ks = 0; ks < POL_HID / 8; ++ks) {
                         const uint64_t db = umma_desc(w2 + ks * 2 * (64 * 16), 64 * 16, 128);
-                        umma_tf32_ts(acc, a2 + 8 * ks, db, idesc_n(64), ks > 0 ? 1u : 0u);
-                        umma_tf32_ts(acc, a2 + 64 + 8 * ks, db, idesc_n(64), 1u);
+                        umma_tf32_ts(acc, a2 + 8 * ks, db, IDESC_N64, ks > 0 ? 1u : 0u);
+                        umma_tf32_ts(acc, a2 + 64 + 8 * ks, db, IDESC_N64, 1u);
                     }
                     umma_commit(bar_m0 + 8 * bi);
                 }
@@ -880,8 +779,7 @@ __global__ void __launch_bounds__(CRIT_THREADS, 1) k_critic(const CritParams prm
 
     tc_fence_before();
     __syncthreads();
-    if (warp == 0)
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(512) : "memory");
+    if (warp == 0) tmem_dealloc<512>(tmem_base);
 }
 
 // ---------------------------------------------------------------------------- transitions -> replay ring, learner feed

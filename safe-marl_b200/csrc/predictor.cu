@@ -42,6 +42,7 @@
 
 #include "flex_kernels.cuh"
 #include "predictor.cuh"
+#include "sm100_ptx.cuh"
 
 // implemented in flex_api.cu
 PredictorState* fp_internal_predictor(FpHandle* h);
@@ -78,88 +79,7 @@ struct PredParams {
     float lo_f, hi_f;                                        // smallest float >= v_min, largest float <= v_max
 };
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-// Bounded wait: a descriptor or protocol mistake must surface as a trap, never as a hung GPU.
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t done = 0;
-    for (uint32_t spin = 0; !done; ++spin) {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.b32 %0, 1, 0, p;\n\t}"
-            : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-        if (!done && spin > (1u << 24)) __trap();
-    }
-}
-__device__ __forceinline__ void tma_load_1d(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-
-// Shared-memory matrix descriptor, K-major, no swizzle: start address, LBO (between the two
-// 16-byte K chunks of one MMA), SBO (between 8-row groups), version 1 (sm_100).
-__device__ __forceinline__ uint64_t umma_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-    return (uint64_t)((saddr >> 4) & 0x3FFFu) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16) |
-           ((uint64_t)((sbo_bytes >> 4) & 0x3FFFu) << 32) | (1ull << 46);
-}
-// Instruction descriptor: D fp32, A/B tf32, both K-major, N >> 3 at bit 17, M >> 4 at bit 24.
-constexpr uint32_t IDESC = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(PRED_N >> 3) << 17) | ((uint32_t)(PRED_M >> 4) << 24);
-
-// A operand from TMEM (lane = row, one 32-bit column per k), B from shared memory
-__device__ __forceinline__ void umma_tf32_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(IDESC), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void tmem_st4(uint32_t taddr, float a, float b, float c, float d) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};"
-                 ::"r"(taddr), "r"(__float_as_uint(a)), "r"(__float_as_uint(b)), "r"(__float_as_uint(c)), "r"(__float_as_uint(d)) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tmem_ld1(uint32_t taddr, uint32_t& r) {
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x1.b32 {%0}, [%1];" : "=r"(r) : "r"(taddr));
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-        : "r"(taddr));
-}
-// Bulk shared -> global stores (TMA engine)
-__device__ __forceinline__ void bulk_s2g(void* gdst, const void* smem_src, uint32_t bytes) {
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;"
-                 ::"l"(gdst), "r"((unsigned)__cvta_generic_to_shared(smem_src)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-template <int ID, int THREADS>
-__device__ __forceinline__ void group_sync() {               // named barrier of one warp group
-    asm volatile("bar.sync %0, %1;" ::"n"(ID), "n"(THREADS) : "memory");
-}
-__device__ __forceinline__ bool elect_one() {                // one lane of a converged warp (lets ptxas keep the
-    uint32_t p;                                              // descriptors of the MMA on the uniform datapath)
-    asm volatile("{\n\t.reg .pred P1;\n\telect.sync _|P1, 0xffffffff;\n\tselp.b32 %0, 1, 0, P1;\n\t}" : "=r"(p));
-    return p != 0u;
-}
+constexpr uint32_t IDESC = umma_idesc_tf32(PRED_M, PRED_N);
 
 constexpr int PROD_THREADS = 2 * PRED_M;     // warps 0-7: TMA + split (two threads per row) + MMA issue (warp 0)
 constexpr int EPI_THREADS = 2 * PRED_M;      // warps 8-15: epilogue (two threads per row: column halves)
@@ -201,14 +121,14 @@ __global__ void __launch_bounds__(PRED_THREADS, 1) k_predict(const PredParams pr
         mbar_init(bar_free0, EPI_THREADS); mbar_init(bar_free0 + 8, EPI_THREADS);
         mbar_init(bar_w, 1);
         mbar_init(bar_a0, PROD_THREADS); mbar_init(bar_a0 + 8, PROD_THREADS);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
         mbar_expect_tx(bar_w, 2 * B_BYTES);                             // weights: one bulk copy, awaited before the first MMA
         tma_load_1d(smem_u32(Bsm), prm.B, 2 * B_BYTES, bar_w);
         for (int k = 0; k < N_STAGES && k < n_my; ++k) issue(k);        // the first X tiles travel during the rest of the setup
     }
     if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(TMEM_COLS) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc<TMEM_COLS>(smem_u32(tmem_slot));
+        tmem_relinquish();
     }
     if (tid < PRED_N) bias[tid] = prm.bias[tid];
     fence_proxy_async();
@@ -225,9 +145,9 @@ __global__ void __launch_bounds__(PRED_THREADS, 1) k_predict(const PredParams pr
         for (int ks = 0; ks < PRED_K / 8; ++ks) {
             const uint32_t bo = ks * 2 * (PRED_N * 16);
             const uint64_t dbh = umma_desc(b_hi + bo, PRED_N * 16, 128), dbl = umma_desc(b_lo + bo, PRED_N * 16, 128);
-            umma_tf32_ts(acc, t_hi + 8 * ks, dbh, ks > 0 ? 1u : 0u);
-            umma_tf32_ts(acc, t_lo + 8 * ks, dbh, 1u);
-            umma_tf32_ts(acc, t_hi + 8 * ks, dbl, 1u);
+            umma_tf32_ts(acc, t_hi + 8 * ks, dbh, IDESC, ks > 0 ? 1u : 0u);
+            umma_tf32_ts(acc, t_lo + 8 * ks, dbh, IDESC, 1u);
+            umma_tf32_ts(acc, t_hi + 8 * ks, dbl, IDESC, 1u);
         }
     };
 
@@ -282,7 +202,7 @@ __global__ void __launch_bounds__(PRED_THREADS, 1) k_predict(const PredParams pr
                 tmem_st4(t_hi + 4 * c, hx, hy, hz, hw);
                 tmem_st4(t_lo + 4 * c, x.x - hx, x.y - hy, y.x - hz, y.y - hw);
             }
-            asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+            tmem_wait_st();
             tc_fence_before();
             mbar_arrive(bar_a0 + 8 * b);
         }
@@ -300,10 +220,10 @@ __global__ void __launch_bounds__(PRED_THREADS, 1) k_predict(const PredParams pr
             // columns 0..16 of their quarter, warps 12-15 columns 17..32
             const int c0 = ehalf ? 17 : 0;
             const uint32_t taddr = tmem_base + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)b * ACC_COLS + (uint32_t)c0;
-            uint32_t r0[16], r1 = 0u;
+            float r0[16], r1 = 0.0f;
             tmem_ld16(taddr, r0);
             if (ehalf == 0) tmem_ld1(taddr + 16, r1);
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            tmem_wait_ld();
             tc_fence_before();
             mbar_arrive(bar_free0 + 8 * b);              // the accumulator may be overwritten (tile k + 2)
             if (etid == 0) bulk_wait_read();             // the previous tile's bulk stores have read `out`
@@ -315,7 +235,7 @@ __global__ void __launch_bounds__(PRED_THREADS, 1) k_predict(const PredParams pr
 #pragma unroll
                 for (int i = 0; i < 17; ++i) {
                     if (i < 16 || ehalf == 0) {
-                        V[i] = __uint_as_float(i < 16 ? r0[i < 16 ? i : 0] : r1) + bias[c0 + i];
+                        V[i] = (i < 16 ? r0[i < 16 ? i : 0] : r1) + bias[c0 + i];
                         out[row * N_OUT + c0 + i] = V[i];
                         vmn = fminf(vmn, V[i]); vmx = fmaxf(vmx, V[i]);
                     }
@@ -385,8 +305,7 @@ __global__ void __launch_bounds__(PRED_THREADS, 1) k_predict(const PredParams pr
 
     tc_fence_before();
     __syncthreads();
-    if (warp == 0)
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(TMEM_COLS) : "memory");
+    if (warp == 0) tmem_dealloc<TMEM_COLS>(tmem_base);
 }
 
 // ---------------------------------------------------------------------------- replay ring

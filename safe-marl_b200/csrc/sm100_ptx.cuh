@@ -1,0 +1,139 @@
+// sm100_ptx.cuh -- inline-PTX wrappers of the sm_100a kernels: mbarriers, bulk / TMA and cp.async copies,
+// tcgen05 (tensor memory and the UMMA tensor-core instructions) and warp-group synchronisation.
+#pragma once
+#include <cstdint>
+
+#include <cuda_runtime.h>
+
+__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
+
+// ---------------------------------------------------------------------------- mbarrier
+__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
+}
+// makes the initialised barriers visible to the other threads and to the async proxy
+__device__ __forceinline__ void mbar_init_fence() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
+__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
+}
+// Bounded wait: a descriptor or protocol mistake must surface as a trap, never as a hung GPU.
+__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
+    uint32_t done = 0;
+    for (uint32_t spin = 0; !done; ++spin) {
+        asm volatile(
+            "{\n\t.reg .pred p;\n\t"
+            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
+            "selp.b32 %0, 1, 0, p;\n\t}"
+            : "=r"(done) : "r"(bar), "r"(parity) : "memory");
+        if (!done && spin > (1u << 24)) __trap();
+    }
+}
+
+// ---------------------------------------------------------------------------- bulk copies (TMA engine)
+__device__ __forceinline__ void tma_load_1d(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
+}
+// shared -> global: one instruction per contiguous block; bulk_wait_read frees the source, bulk_wait_all the destination
+__device__ __forceinline__ void bulk_s2g(void* gdst, const void* smem_src, uint32_t bytes) {
+    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;"
+                 ::"l"(gdst), "r"(smem_u32(smem_src)), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
+__device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
+__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
+// orders this thread's generic-proxy shared-memory writes before later async-proxy (bulk / TMA, tcgen05) accesses
+__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+
+// ---------------------------------------------------------------------------- cp.async (LDGSTS)
+// 8-byte copy through L1, 16-byte copy through L2 only; no register staging, so a thread can keep many in flight
+__device__ __forceinline__ void cp_async8(void* smem_dst, const void* gsrc) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_u32(smem_dst)), "l"(gsrc) : "memory");
+}
+__device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc) {
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(smem_dst)), "l"(gsrc) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N> __device__ __forceinline__ void cp_async_wait_group() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
+__device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
+
+// ---------------------------------------------------------------------------- tcgen05
+// TMEM allocation by one warp: the base address is written to shared memory at `slot`
+template <uint32_t NCOLS>
+__device__ __forceinline__ void tmem_alloc(uint32_t slot) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(slot), "n"(NCOLS) : "memory");
+}
+__device__ __forceinline__ void tmem_relinquish() { asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory"); }
+template <uint32_t NCOLS>
+__device__ __forceinline__ void tmem_dealloc(uint32_t taddr) {
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "n"(NCOLS) : "memory");
+}
+__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+
+// Shared-memory matrix descriptor, K-major, no swizzle: [k-chunk of 4 tf32][n][4]; LBO = bytes between the two
+// 16-byte K chunks of one MMA (= N * 16), SBO = bytes between 8-row groups (128); version 1 (sm_100).
+__device__ __forceinline__ uint64_t umma_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
+    return (uint64_t)((saddr >> 4) & 0x3FFFu) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16) |
+           ((uint64_t)((sbo_bytes >> 4) & 0x3FFFu) << 32) | (1ull << 46);
+}
+// Instruction descriptor of kind::tf32: D fp32, A/B tf32, both K-major, N >> 3 at bit 17, M >> 4 at bit 24.
+__host__ __device__ constexpr uint32_t umma_idesc_tf32(uint32_t m, uint32_t n) {
+    return (1u << 4) | (2u << 7) | (2u << 10) | ((n >> 3) << 17) | ((m >> 4) << 24);
+}
+// D[tmem] (+)= A[tmem: lane = row, one 32-bit column per k] * B[smem]
+__device__ __forceinline__ void umma_tf32_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n\t}"
+        ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
+}
+// arrives on the mbarrier once the MMAs issued so far have completed
+__device__ __forceinline__ void umma_commit(uint32_t bar) {
+    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
+}
+__device__ __forceinline__ void tmem_st4(uint32_t taddr, float a, float b, float c, float d) {
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};"
+                 ::"r"(taddr), "r"(__float_as_uint(a)), "r"(__float_as_uint(b)), "r"(__float_as_uint(c)), "r"(__float_as_uint(d)) : "memory");
+}
+// TMEM loads (32x32b: lane = row, one 32-bit column per register); the values are valid after tmem_wait_ld()
+__device__ __forceinline__ void tmem_ld1(uint32_t taddr, float& v) {
+    uint32_t r;
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x1.b32 {%0}, [%1];" : "=r"(r) : "r"(taddr));
+    v = __uint_as_float(r);
+}
+__device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&v)[8]) {
+    uint32_t r[8];
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]) : "r"(taddr));
+#pragma unroll
+    for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
+}
+__device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
+    uint32_t r[16];
+    asm volatile(
+        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
+        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
+          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+        : "r"(taddr));
+#pragma unroll
+    for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
+}
+__device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+__device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+
+// ---------------------------------------------------------------------------- warp groups
+template <int ID, int THREADS>
+__device__ __forceinline__ void group_sync() {               // named barrier of one warp group
+    asm volatile("bar.sync %0, %1;" ::"n"(ID), "n"(THREADS) : "memory");
+}
+__device__ __forceinline__ bool elect_one() {                // one lane of a converged warp (lets ptxas keep the
+    uint32_t p;                                              // descriptors of the MMA on the uniform datapath)
+    asm volatile("{\n\t.reg .pred P1;\n\telect.sync _|P1, 0xffffffff;\n\tselp.b32 %0, 1, 0, P1;\n\t}" : "=r"(p));
+    return p != 0u;
+}
