@@ -321,6 +321,22 @@ int fp_safety_load(FpHandle* h, const double* h_coef, const double* h_intercept,
 int fp_safety_project(FpHandle* h, const void* d_actions, int act_dtype, float* d_adjusted, int32_t type_major, double* d_slack,
                       uint8_t* d_intervened, void* stream);
 
+/* The same layer against the full fitted map as it was trained, V = A [P_1, Q_1, ..., P_nb, Q_nb] + c, instead of the
+ * reference's row-sum reading: every bus's prediction depends on every building's actions, so each env solves
+ *     min_y sum_k ||y_k - y0_k||^2 + w sum_n [max(0, v_min - V_n(y)) + max(0, V_n(y) - v_max)],  x, c, d >= 0
+ * (y0 = parse_actions of the proposal, the injections of safety_ref.solve_reference_qp) by an exact active-set method
+ * on the 2 na numbers V depends on (k_safety_project_affine).  The two forms keep separate models.
+ * fp_safety_load_affine: h_A [n_out][n_in] and h_c [n_out] (host, fp64: what fp_predictor_load takes) with
+ * n_in == 2 n_bus, n_out == n_bus, finite entries, v_min < v_max and slack_weight > 0, else FP_EINVAL.
+ * fp_safety_project_affine: inputs and d_adjusted as fp_safety_project; d_slack [N][n_bus] fp64 (remaining predicted
+ * violation per bus), d_intervened [N][na] (1 if any of the agent's four values moved) and d_status [N] int32
+ * (iterations, 0 if every bus was already inside -- then d_adjusted is the proposal cast to fp32 -- or -1 if the
+ * iteration cap was reached) may be NULL.  FP_ESTATE before fp_safety_load_affine or fp_load_profiles. */
+int fp_safety_load_affine(FpHandle* h, int32_t n_in, int32_t n_out, const double* h_A, const double* h_c, double v_min,
+                          double v_max, double slack_weight);
+int fp_safety_project_affine(FpHandle* h, const void* d_actions, int act_dtype, float* d_adjusted, int32_t type_major,
+                             double* d_slack, uint8_t* d_intervened, int32_t* d_status, void* stream);
+
 /* -- acting policy of the rollout loop, transitions, learner feed (SURVEY 8f ranks 1-2) ---- */
 
 /* The shared-parameter RNNAgent (madrl/agents/rnn_agent.py:8-32: fc1(144 obs + 5 agent-id -> 64) -> LayerNorm ->

@@ -44,6 +44,8 @@ struct FpHandle {
     double *d_pfl = nullptr, *d_qfl = nullptr, *d_isq = nullptr;
     double* d_stats_partial = nullptr;
     double safety_sP[8] = {0}, safety_sQ[8] = {0}, safety_b[8] = {0}, safety_vmin = 0, safety_vmax = 0, safety_w = 0; int safety_loaded = 0;
+    // the full affine map of fp_safety_load_affine: A transposed [2 nb][FP_MAX_BUS], c [nb]
+    double *d_saff_At = nullptr, *d_saff_c = nullptr, saff_vmin = 0, saff_vmax = 0, saff_w = 0; int saff_loaded = 0;
     uint8_t* d_retry_mask = nullptr; void* d_retry_count = nullptr;     // fp_reset_random_retry: device-built retry mask
     int stats_rows = 0, stats_cap = 0;     // rows of one launch's statistics block
     const uint8_t* d_inject = nullptr;
@@ -296,6 +298,7 @@ int fp_destroy(FpHandle* h) {
     cudaFree(h->d_rec); cudaFree(h->d_V); cudaFree(h->d_setp); cudaFree(h->d_hist); cudaFree(h->d_obsm); cudaFree(h->d_obsr);
     cudaFree(h->d_pfl); cudaFree(h->d_qfl); cudaFree(h->d_isq); cudaFree(h->d_stats_partial); cudaFree(h->d_retry_mask); cudaFree(h->d_retry_count);
     cudaFree(h->d_act_stage); cudaFree(h->d_act_xlat); cudaFree(h->d_reward_stage); cudaFree(h->d_done_stage); cudaFree(h->d_info_stage);
+    cudaFree(h->d_saff_At); cudaFree(h->d_saff_c);
     for (int i = 0; i < FP_HOST_STREAMS; ++i) {
         if (h->host_streams[i]) cudaStreamDestroy(h->host_streams[i]);
         if (h->host_ev_out[i]) cudaEventDestroy(h->host_ev_out[i]);
@@ -867,6 +870,55 @@ int fp_safety_project(FpHandle* h, const void* d_actions, int act_dtype, float* 
     p.actions = d_actions; p.act_f64 = (act_dtype == FP_F64);
     p.out = d_adjusted; p.type_major = type_major; p.slack = d_slack; p.intervened = d_intervened;
     CUDA_TRY(h, launch_safety_project(p, (cudaStream_t)stream));
+    h->launches++;
+    return FP_OK;
+}
+
+// The safety layer against the full affine map V = A [P_1, Q_1, ..., P_nb, Q_nb] + c: see k_safety_project_affine.
+int fp_safety_load_affine(FpHandle* h, int32_t n_in, int32_t n_out, const double* h_A, const double* h_c, double v_min,
+                          double v_max, double slack_weight) {
+    if (!h) return FP_EINVAL;
+    USE_DEVICE(h);
+    const int nb = h->dc.nb;
+    if (!h_A || !h_c) return fail(h, FP_EINVAL, "fp_safety_load_affine: null map");
+    if (n_in != 2 * nb || n_out != nb) return fail(h, FP_EINVAL, "fp_safety_load_affine: the map must be [n_bus][2 n_bus]");
+    if (!(slack_weight > 0.0) || !std::isfinite(slack_weight) || !(v_min < v_max) || !std::isfinite(v_min) || !std::isfinite(v_max))
+        return fail(h, FP_EINVAL, "fp_safety_load_affine: bad limits / weight");
+    std::vector<double> At((size_t)2 * nb * FP_MAX_BUS, 0.0);
+    for (int n = 0; n < nb; ++n) {
+        if (!std::isfinite(h_c[n])) return fail(h, FP_EINVAL, "fp_safety_load_affine: non-finite intercept");
+        for (int j = 0; j < 2 * nb; ++j) {
+            const double v = h_A[(size_t)n * 2 * nb + j];
+            if (!std::isfinite(v)) return fail(h, FP_EINVAL, "fp_safety_load_affine: non-finite map entry");
+            At[(size_t)j * FP_MAX_BUS + n] = v;
+        }
+    }
+    if (!h->d_saff_At) {
+        CUDA_TRY(h, cudaMalloc(&h->d_saff_At, (size_t)2 * FP_MAX_BUS * FP_MAX_BUS * sizeof(double)));
+        CUDA_TRY(h, cudaMalloc(&h->d_saff_c, FP_MAX_BUS * sizeof(double)));
+    }
+    CUDA_TRY(h, cudaMemcpy(h->d_saff_At, At.data(), At.size() * sizeof(double), cudaMemcpyHostToDevice));
+    CUDA_TRY(h, cudaMemcpy(h->d_saff_c, h_c, (size_t)nb * sizeof(double), cudaMemcpyHostToDevice));
+    h->saff_vmin = v_min; h->saff_vmax = v_max; h->saff_w = slack_weight; h->saff_loaded = 1;
+    return FP_OK;
+}
+
+int fp_safety_project_affine(FpHandle* h, const void* d_actions, int act_dtype, float* d_adjusted, int32_t type_major,
+                             double* d_slack, uint8_t* d_intervened, int32_t* d_status, void* stream) {
+    if (!h) return FP_EINVAL;
+    USE_DEVICE(h);
+    if (!h->saff_loaded) return fail(h, FP_ESTATE, "fp_safety_project_affine: call fp_safety_load_affine first");
+    if (!h->d_P) return fail(h, FP_ESTATE, "fp_safety_project_affine: call fp_load_profiles first");
+    if (!d_actions || !d_adjusted || (act_dtype != FP_F32 && act_dtype != FP_F64))
+        return fail(h, FP_EINVAL, "fp_safety_project_affine: bad arguments");
+    SafetyAffineParams p;
+    std::memset(&p, 0, sizeof(p));
+    fill_obs_params(h, p.o, nullptr, 0);
+    p.At = h->d_saff_At; p.cvec = h->d_saff_c;
+    p.v_min = h->saff_vmin; p.v_max = h->saff_vmax; p.w = h->saff_w;
+    p.actions = d_actions; p.act_f64 = (act_dtype == FP_F64);
+    p.out = d_adjusted; p.type_major = type_major; p.slack = d_slack; p.intervened = d_intervened; p.status = d_status;
+    CUDA_TRY(h, launch_safety_project_affine(p, (cudaStream_t)stream));
     h->launches++;
     return FP_OK;
 }

@@ -733,20 +733,12 @@ __global__ void k_safety_project(const SafetyParams prm) {
         const int i = (int)(t - e * na);
         // the env's current demands, PV and ESS energy (the row in force, quirk Q1)
         const uint64_t* rec = prm.o.rec + e * FP_REC_STRIDE;
-        const uint64_t tm = rec[FP_REC_TIME];
-        const int32_t start = (int32_t)(uint32_t)tm, steps = (int32_t)(tm >> 32);
-        const int64_t row = (int64_t)start + ((steps > 1) ? min(steps - 1, c.episode_limit + c.history) : 1);
+        const int64_t row = row_in_force(c, rec);
         const double* orow = prm.o.OBSROW + row * FP_OBS_STRIDE;
         const double Pd = __ldg(orow + FP_OBS_P + i), Qd = __ldg(orow + FP_OBS_Q + i), ppv = __ldg(orow + FP_OBS_PV + i);
         const double e_cur = __longlong_as_double((long long)rec[FP_REC_E_CUR + i]);
         double a0, a1, a2, a3;
-        if (prm.act_f64) {
-            const double* ap = reinterpret_cast<const double*>(prm.actions) + t * 4;
-            a0 = ap[0]; a1 = ap[1]; a2 = ap[2]; a3 = ap[3];
-        } else {
-            const float4 f = reinterpret_cast<const float4*>(prm.actions)[t];
-            a0 = f.x; a1 = f.y; a2 = f.z; a3 = f.w;
-        }
+        load_action4(prm.actions, prm.act_f64, t, a0, a1, a2, a3);
         // parse_actions (:143-174) = the env's own scaling / clipping / ESS logic
         const Setpoint sp = apply_actions_frac(c, true, a0, a1, a2, a3, ppv, e_cur);
         double y[4] = {sp.pred, sp.ch, sp.dis, sp.qpv};

@@ -102,6 +102,36 @@ struct SafetyParams {
     double* slack; uint8_t* intervened;            // per (env, agent): remaining slack, 1 if the layer moved the action (may be null)
 };
 cudaError_t launch_safety_project(const SafetyParams& prm, cudaStream_t st);
+// the same layer against the full affine voltage map V = A [P_1, Q_1, ..., P_nb, Q_nb] + c (fp_safety_project_affine)
+struct SafetyAffineParams {
+    ObsParams o;                                   // c, n, P, Q (full bus rows), OBSROW, rec
+    const double* At;                              // the map transposed: At[j * FP_MAX_BUS + n] = A[n][j], j < 2 nb
+    const double* cvec;                            // [nb]
+    double v_min, v_max, w;
+    const void* actions; int32_t act_f64;          // proposed raw policy actions [n][na][4]
+    float* out; int32_t type_major;                // adjusted setpoints, layouts as SafetyParams
+    double* slack; uint8_t* intervened; int32_t* status;   // [n][nb], [n][na], [n] (each may be null)
+};
+cudaError_t launch_safety_project_affine(const SafetyAffineParams& prm, cudaStream_t st);
+
+// the profile row in force for env `rec` (quirk Q1): what get_state / the safety layer read as the current demands
+__device__ __forceinline__ int64_t row_in_force(const DevCfg& c, const uint64_t* rec) {
+    const uint64_t tm = rec[FP_REC_TIME];
+    const int32_t start = (int32_t)(uint32_t)tm, steps = (int32_t)(tm >> 32);
+    return (int64_t)start + ((steps > 1) ? min(steps - 1, c.episode_limit + c.history) : 1);
+}
+
+// raw policy action t (= env * na + agent) of an [n][na][4] fp32 or fp64 array, widened to fp64
+__device__ __forceinline__ void load_action4(const void* actions, int32_t act_f64, int64_t t, double& a0, double& a1,
+                                             double& a2, double& a3) {
+    if (act_f64) {
+        const double* ap = reinterpret_cast<const double*>(actions) + t * 4;
+        a0 = ap[0]; a1 = ap[1]; a2 = ap[2]; a3 = ap[3];
+    } else {
+        const float4 f = reinterpret_cast<const float4*>(actions)[t];
+        a0 = f.x; a1 = f.y; a2 = f.z; a3 = f.w;
+    }
+}
 cudaError_t launch_reset_failed_mask(const uint64_t* rec, const uint8_t* mask, int64_t n, uint8_t* out, int32_t* count, cudaStream_t st);
 cudaError_t launch_stats_fold(const double* partial, int n_blocks, double* out, cudaStream_t st);
 cudaError_t launch_pack_obsrow(const double* P, const double* Q, const double* pvp, const int32_t* agent_col, int na, int nl,

@@ -491,6 +491,37 @@ class BatchedFlexProvisionEnv:
                                                 1 if tm else 0, _ptr(slack), _ptr(moved), _stream()), "fp_safety_project")
         return (out, slack, moved.bool()) if want_info else out
 
+    def load_safety_map(self, A, c, slack_weight=1000.0, v_min=None, v_max=None):
+        """The full affine voltage map V = A [P_1, Q_1, ..., P_nb, Q_nb] + c (A [n_bus, 2 n_bus], c [n_bus], fp64 --
+        e.g. pred.A, pred.c of a VoltagePredictor) for safety_project_affine.  The limits default to the env's."""
+        A = np.ascontiguousarray(A, dtype=np.float64); c = np.ascontiguousarray(c, dtype=np.float64)
+        if A.ndim != 2 or c.ndim != 1 or A.shape[0] != c.shape[0]:
+            raise ValueError("A must be [n_bus, 2 n_bus] and c [n_bus]")
+        v_min = float(self.args_dict["v_min"] if v_min is None else v_min)
+        v_max = float(self.args_dict["v_max"] if v_max is None else v_max)
+        self._check(self._lib.fp_safety_load_affine(self._h, A.shape[1], A.shape[0], A.ctypes.data_as(C.c_void_p),
+                                                    c.ctypes.data_as(C.c_void_p), v_min, v_max, float(slack_weight)),
+                    "fp_safety_load_affine")
+
+    def safety_project_affine(self, actions, layout="reference", want_info=False):
+        """The safety layer against the map of load_safety_map (every bus coupled to every building), for every env:
+        raw policy actions [N, na, 4] -> adjusted setpoints (fp32), layouts as safety_project.  want_info adds
+        (slack [N, n_bus] f64, intervened [N, na] bool, status [N] i32: iterations, 0 = already inside, -1 = cap hit)."""
+        a = actions.to(self.device).contiguous()
+        if a.dtype not in (torch.float32, torch.float64):
+            a = a.to(torch.float64)
+        if a.numel() != self.n_envs * self.n_agents * 4:
+            raise ValueError("actions must have n_envs * n_agents * 4 elements")
+        tm = layout == "reference"
+        out = torch.empty((self.n_envs, 4 * self.n_agents) if tm else (self.n_envs, self.n_agents, 4), dtype=torch.float32, device=self.device)
+        slack = torch.empty(self.n_envs, self.n_bus, dtype=torch.float64, device=self.device) if want_info else None
+        moved = torch.empty(self.n_envs, self.n_agents, dtype=torch.uint8, device=self.device) if want_info else None
+        status = torch.empty(self.n_envs, dtype=torch.int32, device=self.device) if want_info else None
+        self._check(self._lib.fp_safety_project_affine(self._h, _ptr(a), _lib.FP_F64 if a.dtype == torch.float64 else _lib.FP_F32,
+                                                       _ptr(out), 1 if tm else 0, _ptr(slack), _ptr(moved), _ptr(status), _stream()),
+                    "fp_safety_project_affine")
+        return (out, slack, moved.bool(), status) if want_info else out
+
     # ------------------------------------------------------------------ statistics
     def episode_stats(self, reduce=True, reset=False):
         """Sums accumulated by every step since the last reset of the statistics (the batched
