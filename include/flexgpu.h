@@ -22,6 +22,9 @@
  *   - all work is enqueued on the caller's CUDA stream (`stream` is a cudaStream_t cast
  *     to void*; NULL = legacy default stream).  No entry point synchronises the device
  *     unless it says so.  One handle per GPU per process; a handle is not thread-safe.
+ *   - a handle's work runs on the device it was created for, whatever the caller's current
+ *     device is: pointers and streams passed with it must belong to that device.  The
+ *     caller's current device is unchanged on return.
  *   - there is no CPU fallback: without a CUDA device fp_create fails.
  *
  * Layouts (all row-major, env-major: an env's row is the coalesced unit):

@@ -14,83 +14,8 @@
 #include <string>
 #include <vector>
 
-#include "flex_kernels.cuh"
-#include "predictor.cuh"
-
-#define FP_HOST_CHUNKS 4      // fp_step_host can pipeline the batch in up to this many chunks (copy engines || SMs)
-#define FP_HOST_STREAMS 3
-#define FP_HOST_CHUNKS_DEFAULT 4
-#define FP_HOST_GRAPHS 8
-
-struct FpHandle {
-    FpConfig cfg;
-    DevCfg dc;
-    DevTopo topo;
-    ThreadTopo tt;               // thread-per-env tables (by-value kernel parameter)
-    int variant = FP_VARIANT_THREAD, shape = SHAPE_RUNTIME;
-    int64_t n = 0;
-    int device = 0;
-    int64_t T = 0;
-    int32_t start_range = 0;
-    // device buffers
-    DevTopo* d_topo = nullptr;
-    double *d_P = nullptr, *d_Q = nullptr, *d_PVP = nullptr, *d_PQD = nullptr, *d_OBS = nullptr;
-    uint64_t* d_rec = nullptr;
-    double *d_V = nullptr, *d_setp = nullptr, *d_hist = nullptr;
-    // fp32 window ring of the observation history (fp_get_obs_view): [N][na][3H][6], last written slot, validity
-    float* d_obsm = nullptr; int obs_q = 0; bool obsm_valid = false;
-    // env-minor fp32 ring [H][na][6][n_pad] (fp_step_ring / fp_obs_ring): slot of the newest push, validity
-    float* d_obsr = nullptr; int ring_q = 0; bool obsr_valid = false; int64_t n_pad = 0;
-    double *d_pfl = nullptr, *d_qfl = nullptr, *d_isq = nullptr;
-    double* d_stats_partial = nullptr;
-    double safety_sP[8] = {0}, safety_sQ[8] = {0}, safety_b[8] = {0}, safety_vmin = 0, safety_vmax = 0, safety_w = 0; int safety_loaded = 0;
-    // the full affine map of fp_safety_load_affine: A transposed [2 nb][FP_MAX_BUS], c [nb]
-    double *d_saff_At = nullptr, *d_saff_c = nullptr, saff_vmin = 0, saff_vmax = 0, saff_w = 0; int saff_loaded = 0;
-    uint8_t* d_retry_mask = nullptr; void* d_retry_count = nullptr;     // fp_reset_random_retry: device-built retry mask
-    int stats_rows = 0, stats_cap = 0;     // rows of one launch's statistics block
-    const uint8_t* d_inject = nullptr;
-    int keep_flows = 0;
-    // staging for the host-buffer entry points
-    void* d_act_stage = nullptr; float* d_act_xlat = nullptr; double* d_reward_stage = nullptr; uint8_t* d_done_stage = nullptr;
-    double* d_info_stage = nullptr;
-    int grid_step = 0, grid_reset = 0, grid_pf = 0, grid_obs = 0;
-    cudaStream_t host_streams[FP_HOST_STREAMS] = {nullptr, nullptr, nullptr};
-    cudaEvent_t host_ev_in = nullptr, host_ev_out[FP_HOST_STREAMS] = {nullptr, nullptr, nullptr};
-    int fuse_obs = 0;            // set around the fp_step of fp_step_obs: the step kernel pushes the observation
-    int keep_hist = 1;           // fp_set_obs_history: 0 = the fused ring step does not maintain the fp64 history ring
-    bool hist_valid = true;      // false after a ring-only step: restored from the env-minor ring on demand (hist_ensure)
-    int host_chunks = 0;         // 0 = not decided yet (FLEXGPU_HOST_CHUNKS or the default)
-    // the chunk pipeline of fp_step_host as instantiated CUDA graphs, one per set of (pinned) host
-    // buffers: one launch per step instead of five API calls per chunk
-    cudaStream_t host_origin = nullptr;
-    struct HostGraph { cudaGraphExec_t exec = nullptr; std::vector<char> key; };
-    HostGraph host_graphs[FP_HOST_GRAPHS];
-    int host_graph_next = 0;
-    int64_t launches = 0;
-    std::string err;
-    PredictorState pred;
-};
-
-static thread_local std::string g_create_err;
-
-static int fail(FpHandle* h, int code, const std::string& msg) {
-    if (h) h->err = msg; else g_create_err = msg;
-    return code;
-}
-
-// Every entry point runs on the handle's device whatever the caller's current device is (two handles on two
-// GPUs in one process); cudaSetDevice on the current device is a no-op.
-#define USE_DEVICE(h)                                                                            \
-    do {                                                                                         \
-        cudaError_t e_ = cudaSetDevice((h)->device);                                             \
-        if (e_ != cudaSuccess) return fail((h), FP_ECUDA, std::string("cudaSetDevice: ") + cudaGetErrorString(e_)); \
-    } while (0)
-#define CUDA_TRY(h, expr)                                                              \
-    do {                                                                               \
-        cudaError_t e_ = (expr);                                                       \
-        if (e_ != cudaSuccess)                                                         \
-            return fail((h), FP_ECUDA, std::string(#expr) + ": " + cudaGetErrorString(e_)); \
-    } while (0)
+#include "api_handle.cuh"
+#include "flex_handle.cuh"
 
 // ------------------------------------------------------------------ topology preprocessing
 // Pre-order numbering (children visited in ascending bus position) + per-lane tables.
@@ -214,27 +139,27 @@ static int grid_for(int64_t n, int cap) {
 extern "C" {
 
 int fp_create(const FpConfig* cfg, int64_t n_envs, int device, FpHandle** out) {
-    if (!cfg || !out || n_envs < 1) return fail(nullptr, FP_EINVAL, "fp_create: bad arguments");
+    if (!cfg || !out || n_envs < 1) return fail<FpHandle>(nullptr, FP_EINVAL, "fp_create: bad arguments");
     if (cfg->history < 1 || cfg->episode_limit < 2 || cfg->pf_max_iter < 1 || !(cfg->pf_tol > 0.0) ||
         cfg->pf_f32_passes < 0 || cfg->pf_f32_passes >= cfg->pf_max_iter ||
         !(cfg->eta_ch > 0.0) || !(cfg->eta_dis > 0.0))
-        return fail(nullptr, FP_EINVAL, "fp_create: bad scalar configuration");
+        return fail<FpHandle>(nullptr, FP_EINVAL, "fp_create: bad scalar configuration");
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1)
-        return fail(nullptr, FP_ECUDA, "fp_create: no CUDA device (there is no CPU fallback)");
-    if (device < 0 || device >= ndev) return fail(nullptr, FP_EINVAL, "fp_create: bad device index");
+        return fail<FpHandle>(nullptr, FP_ECUDA, "fp_create: no CUDA device (there is no CPU fallback)");
+    if (device < 0 || device >= ndev) return fail<FpHandle>(nullptr, FP_EINVAL, "fp_create: bad device index");
     FpHandle* h = new (std::nothrow) FpHandle();
-    if (!h) return fail(nullptr, FP_ENOMEM, "fp_create: out of host memory");
+    if (!h) return fail<FpHandle>(nullptr, FP_ENOMEM, "fp_create: out of host memory");
     h->cfg = *cfg; h->n = n_envs; h->device = device;
     std::string err;
     int rc = build_topology(*cfg, h->topo, h->tt, h->shape, err);
-    if (rc != FP_OK) { delete h; return fail(nullptr, rc, "fp_create: " + err); }
+    if (rc != FP_OK) { delete h; return fail<FpHandle>(nullptr, rc, "fp_create: " + err); }
     if (cfg->variant != FP_VARIANT_THREAD && cfg->variant != FP_VARIANT_WARP) {
-        delete h; return fail(nullptr, FP_EINVAL, "fp_create: unknown kernel variant");
+        delete h; return fail<FpHandle>(nullptr, FP_EINVAL, "fp_create: unknown kernel variant");
     }
     h->variant = cfg->variant;
     if (h->variant == FP_VARIANT_THREAD && (h->tt.n_slots > FP_MAX_SLOTS || h->tt.n_chains > FP_MAX_CHAINS)) {
-        delete h; return fail(nullptr, FP_EINVAL, "fp_create: more than 8 branching buses or 16 laterals; use FP_VARIANT_WARP");
+        delete h; return fail<FpHandle>(nullptr, FP_EINVAL, "fp_create: more than 8 branching buses or 16 laterals; use FP_VARIANT_WARP");
     }
     fill_devcfg(*cfg, h->dc);
     const int nb = cfg->n_bus, na = cfg->n_agents, H = cfg->history;
@@ -244,10 +169,11 @@ int fp_create(const FpConfig* cfg, int64_t n_envs, int device, FpHandle** out) {
         if (e_ != cudaSuccess) {                                                           \
             std::string m = std::string("fp_create: " #expr ": ") + cudaGetErrorString(e_); \
             fp_destroy(h);                                                                 \
-            return fail(nullptr, e_ == cudaErrorMemoryAllocation ? FP_ENOMEM : FP_ECUDA, m); \
+            return fail<FpHandle>(nullptr, e_ == cudaErrorMemoryAllocation ? FP_ENOMEM : FP_ECUDA, m); \
         }                                                                                  \
     } while (0)
-    CREATE_TRY(cudaSetDevice(device));
+    const DeviceGuard on_device(device);
+    CREATE_TRY(on_device.error());
     CREATE_TRY(cudaMalloc(&h->d_topo, sizeof(DevTopo)));
     CREATE_TRY(cudaMemcpy(h->d_topo, &h->topo, sizeof(DevTopo), cudaMemcpyHostToDevice));
     CREATE_TRY(cudaMalloc(&h->d_rec, (size_t)n_envs * FP_REC_STRIDE * 8));
@@ -292,7 +218,7 @@ int fp_create(const FpConfig* cfg, int64_t n_envs, int device, FpHandle** out) {
 
 int fp_destroy(FpHandle* h) {
     if (!h) return FP_OK;
-    cudaSetDevice(h->device);
+    const DeviceGuard on_device(h->device);       // best effort: the handle is freed whatever happens
     predictor_free(&h->pred);
     cudaFree(h->d_topo); cudaFree(h->d_P); cudaFree(h->d_Q); cudaFree(h->d_PVP); cudaFree(h->d_PQD); cudaFree(h->d_OBS);
     cudaFree(h->d_rec); cudaFree(h->d_V); cudaFree(h->d_setp); cudaFree(h->d_hist); cudaFree(h->d_obsm); cudaFree(h->d_obsr);
@@ -310,7 +236,7 @@ int fp_destroy(FpHandle* h) {
     return FP_OK;
 }
 
-const char* fp_last_error(const FpHandle* h) { return h ? h->err.c_str() : g_create_err.c_str(); }
+const char* fp_last_error(const FpHandle* h) { return h ? h->err.c_str() : create_error<FpHandle>().c_str(); }
 int64_t fp_n_envs(const FpHandle* h) { return h ? h->n : 0; }
 int64_t fp_launch_count(const FpHandle* h) { return h ? h->launches : 0; }
 int32_t fp_sizeof_config(void) { return (int32_t)sizeof(FpConfig); }
@@ -323,7 +249,7 @@ int fp_load_profiles(FpHandle* h, const double* h_P, const double* h_Q, const do
     // the reference slices episode_limit + history + 1 rows per episode (:478)
     const int64_t need = (int64_t)h->cfg.episode_limit + h->cfg.history + 1;
     if (T < need) return fail(h, FP_EINVAL, "fp_load_profiles: fewer rows than one episode slice");
-    CUDA_TRY(h, cudaSetDevice(h->device));
+    USE_DEVICE(h);
     cudaFree(h->d_P); cudaFree(h->d_Q); cudaFree(h->d_PVP); cudaFree(h->d_PQD); cudaFree(h->d_OBS);
     h->d_P = h->d_Q = h->d_PVP = h->d_PQD = h->d_OBS = nullptr;
     double *d_pv = nullptr, *d_price = nullptr;
@@ -557,12 +483,9 @@ int fp_step_host(FpHandle* h, const void* h_actions, int act_dtype, double* h_re
     if (act_dtype != FP_F32 && act_dtype != FP_F64 && act_dtype != FP_F32_POLICY) return fail(h, FP_EINVAL, "fp_step_host: bad action dtype");
     cudaStream_t st = (cudaStream_t)stream;
     const size_t n = (size_t)h->n, na = (size_t)h->dc.na;
-    if (!h->d_act_stage) {
-        CUDA_TRY(h, cudaMalloc(&h->d_act_stage, n * na * 4 * 8));
-        CUDA_TRY(h, cudaMalloc(&h->d_reward_stage, n * 8));
-        CUDA_TRY(h, cudaMalloc(&h->d_done_stage, n));
-        CUDA_TRY(h, cudaMalloc(&h->d_info_stage, n * FP_INFO_STRIDE * 8));
-    }
+    if (!h->d_act_stage)
+        CUDA_TRY(h, alloc_group({{&h->d_act_stage, n * na * 4 * 8}, {&h->d_reward_stage, n * 8}, {&h->d_done_stage, n},
+                                 {&h->d_info_stage, n * FP_INFO_STRIDE * 8}}));
     const size_t abpe = na * 4 * (act_dtype == FP_F64 ? 8 : 4);          // action bytes per env
     const int64_t tiles = ((int64_t)n + 31) / 32;
     if (h->host_chunks == 0) {
@@ -583,7 +506,6 @@ int fp_step_host(FpHandle* h, const void* h_actions, int act_dtype, double* h_re
         return FP_OK;
     }
     if (!h->host_ev_in) {
-        CUDA_TRY(h, cudaSetDevice(h->device));
         for (int i = 0; i < FP_HOST_STREAMS; ++i) {
             CUDA_TRY(h, cudaStreamCreateWithFlags(&h->host_streams[i], cudaStreamNonBlocking));
             CUDA_TRY(h, cudaEventCreateWithFlags(&h->host_ev_out[i], cudaEventDisableTiming));
@@ -702,7 +624,6 @@ static int obs_ring_prepare(FpHandle* h, bool push, cudaStream_t st) {
     { const int rc = hist_ensure(h, st); if (rc != FP_OK) return rc; }   // the rebuild and the push below use the fp64 ring
     ObsParams p; fill_obs_params(h, p, nullptr, 1);
     if (!h->d_obsm) {
-        CUDA_TRY(h, cudaSetDevice(h->device));
         CUDA_TRY(h, cudaMalloc(&h->d_obsm, (size_t)h->n * per_env * 4));
         h->obsm_valid = false;
     }
@@ -756,7 +677,6 @@ int fp_step_obs(FpHandle* h, const void* d_actions, int act_dtype, double* d_rew
 static int obs_envminor_prepare(FpHandle* h, bool push, cudaStream_t st) {
     const int H = h->dc.history, na = h->dc.na;
     if (!h->d_obsr) {
-        CUDA_TRY(h, cudaSetDevice(h->device));
         h->n_pad = (h->n + 31) / 32 * 32;
         CUDA_TRY(h, cudaMalloc(&h->d_obsr, (size_t)H * na * 6 * h->n_pad * 4));
         h->obsr_valid = false;
@@ -893,10 +813,10 @@ int fp_safety_load_affine(FpHandle* h, int32_t n_in, int32_t n_out, const double
             At[(size_t)j * FP_MAX_BUS + n] = v;
         }
     }
-    if (!h->d_saff_At) {
-        CUDA_TRY(h, cudaMalloc(&h->d_saff_At, (size_t)2 * FP_MAX_BUS * FP_MAX_BUS * sizeof(double)));
-        CUDA_TRY(h, cudaMalloc(&h->d_saff_c, FP_MAX_BUS * sizeof(double)));
-    }
+    h->saff_loaded = 0;
+    if (!h->d_saff_At)
+        CUDA_TRY(h, alloc_group({{&h->d_saff_At, (size_t)2 * FP_MAX_BUS * FP_MAX_BUS * sizeof(double)},
+                                 {&h->d_saff_c, FP_MAX_BUS * sizeof(double)}}));
     CUDA_TRY(h, cudaMemcpy(h->d_saff_At, At.data(), At.size() * sizeof(double), cudaMemcpyHostToDevice));
     CUDA_TRY(h, cudaMemcpy(h->d_saff_c, h_c, (size_t)nb * sizeof(double), cudaMemcpyHostToDevice));
     h->saff_vmin = v_min; h->saff_vmax = v_max; h->saff_w = slack_weight; h->saff_loaded = 1;
@@ -950,8 +870,9 @@ int fp_state_ptrs(FpHandle* h, void** d_rec, void** d_voltage, void** d_setpoint
 // With write != 0 the caller is about to overwrite it (state restore): the derived fp32 rings are rebuilt on next use.
 int fp_history_ptr(FpHandle* h, void** d_hist, int64_t* doubles_per_env, int32_t write) {
     if (!h || !d_hist) return FP_EINVAL;
+    USE_DEVICE(h);
     if (write) h->hist_valid = true;               // about to be overwritten as a whole
-    else { const int rc = hist_ensure(h, nullptr); if (rc != FP_OK) return rc; cudaStreamSynchronize(nullptr); }
+    else { const int rc = hist_ensure(h, nullptr); if (rc != FP_OK) return rc; CUDA_TRY(h, cudaStreamSynchronize(nullptr)); }
     *d_hist = h->d_hist;
     if (doubles_per_env) *doubles_per_env = (int64_t)h->dc.history * FP_HIST_SLOT;
     if (write) { h->obsm_valid = false; h->obsr_valid = false; }
@@ -961,14 +882,9 @@ int fp_history_ptr(FpHandle* h, void** d_hist, int64_t* doubles_per_env, int32_t
 int fp_set_keep_flows(FpHandle* h, int keep) {
     if (!h) return FP_EINVAL;
     if (keep && !h->d_pfl) {
+        USE_DEVICE(h);
         const size_t bytes = (size_t)h->n * h->dc.nl * 8;
-        CUDA_TRY(h, cudaSetDevice(h->device));
-        CUDA_TRY(h, cudaMalloc(&h->d_pfl, bytes));
-        CUDA_TRY(h, cudaMalloc(&h->d_qfl, bytes));
-        CUDA_TRY(h, cudaMalloc(&h->d_isq, bytes));
-        CUDA_TRY(h, cudaMemset(h->d_pfl, 0, bytes));
-        CUDA_TRY(h, cudaMemset(h->d_qfl, 0, bytes));
-        CUDA_TRY(h, cudaMemset(h->d_isq, 0, bytes));
+        CUDA_TRY(h, alloc_group({{&h->d_pfl, bytes}, {&h->d_qfl, bytes}, {&h->d_isq, bytes}}, true));
     }
     h->keep_flows = keep ? 1 : 0;
     return FP_OK;
@@ -1016,9 +932,3 @@ int fp_inject_failure(FpHandle* h, const uint8_t* d_mask) {
 }
 
 }  // extern "C"
-
-// accessors used by the predictor / replay translation unit
-PredictorState* fp_internal_predictor(FpHandle* h) { return &h->pred; }
-int fp_internal_fail(FpHandle* h, int code, const char* msg) { return fail(h, code, msg); }
-void fp_internal_count_launch(FpHandle* h, int k) { h->launches += k; }
-int fp_internal_device(FpHandle* h) { return h->device; }

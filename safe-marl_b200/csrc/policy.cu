@@ -38,6 +38,7 @@
 #include <string>
 #include <vector>
 
+#include "api_handle.cuh"
 #include "flex_common.cuh"
 #include "sm100_ptx.cuh"
 
@@ -966,12 +967,6 @@ __global__ void k_reward_batchnorm(const float* __restrict__ reward, int64_t bat
     for (int64_t b = threadIdx.x; b < batch; b += blockDim.x) out[b * POL_NA + a] = (reward[b * POL_NA + a] - meanf) * rstd;
 }
 
-int grid_for(int64_t total) {
-    int64_t g = (total + 255) / 256;
-    if (g < 1) g = 1;
-    return (int)(g > 148 * 16 ? 148 * 16 : g);
-}
-
 int gt_grid(int64_t tiles, int per_sm) {       // persistent grid of the transposing gathers: per_sm CTAs per SM
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
@@ -1017,11 +1012,6 @@ EncodeTiledFn encode_tiled_fn() {                  // the driver entry point, wi
     }
     return fn;
 }
-thread_local std::string g_policy_err;
-int pfail(FpPolicy* p, int code, const std::string& msg) {
-    if (p) p->err = msg; else g_policy_err = msg;
-    return code;
-}
 }  // namespace
 
 // The ring as a 3-D tensor [24 slots][30 = agent x feature][n_pad envs] (innermost first); a tile is the box [24][6][128] at
@@ -1032,14 +1022,14 @@ static int ring_tensor_map(FpPolicy* p, const float* d_ring, int64_t n_pad, CUte
     *use_tma = 0;
     if (n_pad >= POL_M && ((uintptr_t)d_ring & 15) == 0) {
         EncodeTiledFn enc = encode_tiled_fn();
-        if (!enc) return pfail(p, FP_ECUDA, std::string(who) + ": cuTensorMapEncodeTiled is not available from this driver");
+        if (!enc) return fail(p, FP_ECUDA, std::string(who) + ": cuTensorMapEncodeTiled is not available from this driver");
         const cuuint64_t gdim[3] = {(cuuint64_t)n_pad, (cuuint64_t)(POL_NA * POL_F), (cuuint64_t)POL_H};
         const cuuint64_t gstride[2] = {(cuuint64_t)n_pad * 4, (cuuint64_t)n_pad * 4 * (POL_NA * POL_F)};
         const cuuint32_t box[3] = {POL_M, POL_F, (cuuint32_t)box_slots}, estr[3] = {1, 1, 1};
         const CUresult r = enc(tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(d_ring), gdim, gstride, box, estr,
                                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return pfail(p, FP_ECUDA, std::string(who) + ": cuTensorMapEncodeTiled failed (" + std::to_string((int)r) + ")");
+        if (r != CUDA_SUCCESS) return fail(p, FP_ECUDA, std::string(who) + ": cuTensorMapEncodeTiled failed (" + std::to_string((int)r) + ")");
         *use_tma = 1;
     }
     return FP_OK;
@@ -1050,8 +1040,8 @@ extern "C" {
 int fp_policy_create(int device, FpPolicy** out) {
     if (!out) return FP_EINVAL;
     int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) return pfail(nullptr, FP_ECUDA, "fp_policy_create: no CUDA device (there is no CPU fallback)");
-    if (device < 0 || device >= ndev) return pfail(nullptr, FP_EINVAL, "fp_policy_create: bad device index");
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) return fail<FpPolicy>(nullptr, FP_ECUDA, "fp_policy_create: no CUDA device (there is no CPU fallback)");
+    if (device < 0 || device >= ndev) return fail<FpPolicy>(nullptr, FP_EINVAL, "fp_policy_create: bad device index");
     FpPolicy* p = new FpPolicy();
     p->device = device;
     *out = p;
@@ -1060,14 +1050,14 @@ int fp_policy_create(int device, FpPolicy** out) {
 
 int fp_policy_destroy(FpPolicy* p) {
     if (!p) return FP_OK;
-    cudaSetDevice(p->device);
+    const DeviceGuard on_device(p->device);       // best effort: the handle is freed whatever happens
     cudaFree(p->d_W1rot); cudaFree(p->d_Wg); cudaFree(p->d_vec);
     cudaFree(p->d_Wc1rot); cudaFree(p->d_Wc2); cudaFree(p->d_Wca); cudaFree(p->d_cvec);
     delete p;
     return FP_OK;
 }
 
-const char* fp_policy_last_error(const FpPolicy* p) { return p ? p->err.c_str() : g_policy_err.c_str(); }
+const char* fp_policy_last_error(const FpPolicy* p) { return p ? p->err.c_str() : create_error<FpPolicy>().c_str(); }
 int64_t fp_policy_launch_count(const FpPolicy* p) { return p ? p->launches : 0; }
 
 // Host weights in torch's layouts (state_dict of RNNAgent, madrl/agents/rnn_agent.py:11-16):
@@ -1077,8 +1067,8 @@ int fp_policy_load(FpPolicy* p, const float* fc1_w, const float* fc1_b, const fl
                    const float* w_hh, const float* b_ih, const float* b_hh, const float* fc2_w, const float* fc2_b) {
     if (!p) return FP_EINVAL;
     if (!fc1_w || !fc1_b || !ln_g || !ln_b || !w_ih || !w_hh || !b_ih || !b_hh || !fc2_w || !fc2_b)
-        return pfail(p, FP_EINVAL, "fp_policy_load: null weight array");
-    cudaSetDevice(p->device);
+        return fail(p, FP_EINVAL, "fp_policy_load: null weight array");
+    USE_DEVICE(p);
     const int KIN = POL_OBS + POL_NA;
     // fc1: 24 column rotations, UMMA K-major layout [kc][n][4]; ring slot s holds history entry r = (s - q - 1) mod 24
     // when the newest slot is q, i.e. K index s * 6 + f must carry weight column r * 6 + f
@@ -1127,16 +1117,14 @@ int fp_policy_load(FpPolicy* p, const float* fc1_w, const float* fc1_b, const fl
     }
     for (int n = 0; n < 128; ++n) vec[V_BRZ + n] = (float)(-((double)b_ih[n] + (double)b_hh[n]) * (double)POL_L2E);
     for (int n = 0; n < POL_ACT; ++n) vec[V_B2 + n] = fc2_b[n];
+    p->loaded = 0;
     cudaFree(p->d_W1rot); cudaFree(p->d_Wg); cudaFree(p->d_vec);
     p->d_W1rot = p->d_Wg = p->d_vec = nullptr;
-    if (cudaMalloc(&p->d_W1rot, W1.size() * 4) != cudaSuccess || cudaMalloc(&p->d_Wg, Wg.size() * 4) != cudaSuccess ||
-        cudaMalloc(&p->d_vec, vec.size() * 4) != cudaSuccess)
-        return pfail(p, FP_ENOMEM, "fp_policy_load: cudaMalloc failed");
-    cudaMemcpy(p->d_W1rot, W1.data(), W1.size() * 4, cudaMemcpyHostToDevice);
-    cudaMemcpy(p->d_Wg, Wg.data(), Wg.size() * 4, cudaMemcpyHostToDevice);
-    cudaMemcpy(p->d_vec, vec.data(), vec.size() * 4, cudaMemcpyHostToDevice);
-    cudaError_t e = cudaFuncSetAttribute(k_policy, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)POL_SMEM);
-    if (e != cudaSuccess) return pfail(p, FP_ECUDA, cudaGetErrorString(e));
+    CUDA_TRY(p, alloc_group({{&p->d_W1rot, W1.size() * 4}, {&p->d_Wg, Wg.size() * 4}, {&p->d_vec, vec.size() * 4}}));
+    CUDA_TRY(p, cudaMemcpy(p->d_W1rot, W1.data(), W1.size() * 4, cudaMemcpyHostToDevice));
+    CUDA_TRY(p, cudaMemcpy(p->d_Wg, Wg.data(), Wg.size() * 4, cudaMemcpyHostToDevice));
+    CUDA_TRY(p, cudaMemcpy(p->d_vec, vec.data(), vec.size() * 4, cudaMemcpyHostToDevice));
+    CUDA_TRY(p, cudaFuncSetAttribute(k_policy, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)POL_SMEM));
     p->loaded = 1;
     return FP_OK;
 }
@@ -1150,11 +1138,11 @@ int fp_policy_act(FpPolicy* p, const float* d_ring, int32_t slot, int64_t n_pad,
                   const uint8_t* d_reset, float* d_hid_out, int32_t hid_env_minor, float* d_mean, float* d_action, float* d_logp,
                   const float* d_eps, uint64_t seed, uint64_t step, float std_, int32_t explore, void* stream) {
     if (!p) return FP_EINVAL;
-    if (!p->loaded) return pfail(p, FP_ESTATE, "fp_policy_act: call fp_policy_load first");
+    if (!p->loaded) return fail(p, FP_ESTATE, "fp_policy_act: call fp_policy_load first");
     if (!d_ring || !d_hid_out || !d_action || n_envs < 1 || slot < 0 || slot >= POL_H || n_pad < n_envs || (n_pad & 3))
-        return pfail(p, FP_EINVAL, "fp_policy_act: bad arguments");
-    if (!(std_ > 0.0f)) return pfail(p, FP_EINVAL, "fp_policy_act: std must be positive");
-    cudaSetDevice(p->device);
+        return fail(p, FP_EINVAL, "fp_policy_act: bad arguments");
+    if (!(std_ > 0.0f)) return fail(p, FP_EINVAL, "fp_policy_act: std must be positive");
+    USE_DEVICE(p);
     PolParams prm;
     std::memset(&prm, 0, sizeof(prm));
     prm.ring = d_ring; prm.n_pad = n_pad; prm.n = n_envs; prm.slot = slot;
@@ -1165,19 +1153,16 @@ int fp_policy_act(FpPolicy* p, const float* d_ring, int32_t slot, int64_t n_pad,
     alignas(64) CUtensorMap tmap;
     { const int rc = ring_tensor_map(p, d_ring, n_pad, &tmap, &prm.use_tma, "fp_policy_act"); if (rc != FP_OK) return rc; }
     if (p->sink_out) {                                  // one-shot `state` sink (fp_policy_state_sink); needs the TMA path
-        if (!prm.use_tma || p->sink_n > n_envs) { p->sink_out = nullptr; return pfail(p, FP_EINVAL, "fp_policy_act: the state sink needs n_pad >= 128 and at most n_envs rows"); }
+        if (!prm.use_tma || p->sink_n > n_envs) { p->sink_out = nullptr; return fail(p, FP_EINVAL, "fp_policy_act: the state sink needs n_pad >= 128 and at most n_envs rows"); }
         prm.st_out = p->sink_out; prm.st_pitch = p->sink_pitch; prm.st_row0 = p->sink_row0; prm.st_cap = p->sink_cap; prm.st_n = p->sink_n;
         p->sink_out = nullptr;
     }
     int sms = 0;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, p->device);
+    CUDA_TRY(p, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, p->device));
     const int64_t tiles = (n_envs + POL_M - 1) / POL_M * POL_NA;
     const int grid = (int)(tiles < sms ? tiles : sms);
     k_policy<<<grid, POL_THREADS, POL_SMEM, (cudaStream_t)stream>>>(prm, tmap);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return pfail(p, FP_ECUDA, cudaGetErrorString(e));
-    p->launches++;
-    return FP_OK;
+    return launched(p, "k_policy");
 }
 
 // select_action alone on stored fc2 outputs d_mean [n_envs][5][4] (fp_policy_act's d_mean): another exploration draw of the
@@ -1185,15 +1170,12 @@ int fp_policy_act(FpPolicy* p, const float* d_ring, int32_t slot, int64_t n_pad,
 int fp_policy_sample(FpPolicy* p, const float* d_mean, int64_t n_envs, float* d_action, float* d_logp, const float* d_eps,
                      uint64_t seed, uint64_t step, float std_, int32_t explore, void* stream) {
     if (!p) return FP_EINVAL;
-    if (!d_mean || !d_action || n_envs < 1) return pfail(p, FP_EINVAL, "fp_policy_sample: bad arguments");
-    if (!(std_ > 0.0f)) return pfail(p, FP_EINVAL, "fp_policy_sample: std must be positive");
-    cudaSetDevice(p->device);
+    if (!d_mean || !d_action || n_envs < 1) return fail(p, FP_EINVAL, "fp_policy_sample: bad arguments");
+    if (!(std_ > 0.0f)) return fail(p, FP_EINVAL, "fp_policy_sample: std must be positive");
+    USE_DEVICE(p);
     k_sample<<<grid_for(n_envs * POL_NA), 256, 0, (cudaStream_t)stream>>>(d_mean, n_envs * POL_NA, explore, d_eps, seed, step, std_, std::log(std_),
                                                                           d_action, d_logp);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return pfail(p, FP_ECUDA, cudaGetErrorString(e));
-    p->launches++;
-    return FP_OK;
+    return launched(p, "k_sample");
 }
 
 // One-shot sink for the NEXT fp_policy_act: while it evaluates the policy, its writer warps copy the dense get_obs windows
@@ -1203,7 +1185,7 @@ int fp_policy_sample(FpPolicy* p, const float* d_mean, int64_t n_envs, float* d_
 int fp_policy_state_sink(FpPolicy* p, float* d_field, int64_t pitch, int64_t row0, int64_t cap, int64_t n) {
     if (!p) return FP_EINVAL;
     if (!d_field || n < 1 || pitch < POL_NA * POL_OBS || (pitch & 3) || ((uintptr_t)d_field & 15) || row0 < 0 || cap < n || row0 >= cap)
-        return pfail(p, FP_EINVAL, "fp_policy_state_sink: bad arguments");
+        return fail(p, FP_EINVAL, "fp_policy_state_sink: bad arguments");
     p->sink_out = d_field; p->sink_pitch = pitch; p->sink_row0 = row0; p->sink_cap = cap; p->sink_n = n;
     return FP_OK;
 }
@@ -1215,15 +1197,12 @@ int fp_policy_gather_windows(FpPolicy* p, const float* d_ring, int32_t slot, int
                              int64_t row0, int64_t cap, void* stream) {
     if (!p) return FP_EINVAL;
     if (!d_ring || !d_out || n < 1 || pitch < POL_NA * POL_OBS || row0 < 0 || cap < n || row0 >= cap || slot < 0 || slot >= POL_H)
-        return pfail(p, FP_EINVAL, "fp_policy_gather_windows: bad arguments");
-    cudaSetDevice(p->device);
+        return fail(p, FP_EINVAL, "fp_policy_gather_windows: bad arguments");
+    USE_DEVICE(p);
     constexpr int smem_w = POL_OBS * GT_STRIDE * (int)sizeof(float);
-    if (!p->attr_window) { cudaFuncSetAttribute(k_window_gather, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_w); p->attr_window = 1; }
+    if (!p->attr_window) { CUDA_TRY(p, cudaFuncSetAttribute(k_window_gather, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_w)); p->attr_window = 1; }
     k_window_gather<<<gt_grid(((n + GT_ENVS - 1) / GT_ENVS) * POL_NA, 3), 256, smem_w, (cudaStream_t)stream>>>(d_ring, n_pad, slot, n, d_out, pitch, row0, cap);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return pfail(p, FP_ECUDA, cudaGetErrorString(e));
-    p->launches++;
-    return FP_OK;
+    return launched(p, "k_window_gather");
 }
 
 // Hidden states in the policy kernel's env-minor layout [5][64][n_pad] -> replay rows (last_hid / hid, 320 floats per env);
@@ -1231,38 +1210,29 @@ int fp_policy_gather_windows(FpPolicy* p, const float* d_ring, int32_t slot, int
 int fp_policy_hidden_to_ring(FpPolicy* p, const float* d_hid_em, int64_t n_pad, int64_t n, float* d_field, int64_t row0, int64_t cap,
                              const uint8_t* d_zero_mask, void* stream) {
     if (!p) return FP_EINVAL;
-    if (!d_hid_em || !d_field || n < 1 || n_pad < n || row0 < 0 || cap < n || row0 >= cap) return pfail(p, FP_EINVAL, "fp_policy_hidden_to_ring: bad arguments");
-    cudaSetDevice(p->device);
+    if (!d_hid_em || !d_field || n < 1 || n_pad < n || row0 < 0 || cap < n || row0 >= cap) return fail(p, FP_EINVAL, "fp_policy_hidden_to_ring: bad arguments");
+    USE_DEVICE(p);
     constexpr int smem_h = EM_KR * GT_STRIDE * (int)sizeof(float);
-    if (!p->attr_hidden) { cudaFuncSetAttribute(k_em_gather, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_h); p->attr_hidden = 1; }
+    if (!p->attr_hidden) { CUDA_TRY(p, cudaFuncSetAttribute(k_em_gather, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_h)); p->attr_hidden = 1; }
     k_em_gather<<<gt_grid(((n + GT_ENVS - 1) / GT_ENVS) * 2, 2), 256, smem_h, (cudaStream_t)stream>>>(d_hid_em, n_pad, n, d_field, row0, cap, d_zero_mask);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return pfail(p, FP_ECUDA, cudaGetErrorString(e));
-    p->launches++;
-    return FP_OK;
+    return launched(p, "k_em_gather");
 }
 
 int fp_policy_rows_to_ring(FpPolicy* p, const float* d_src, int64_t n, int32_t width, float* d_field, int64_t row0, int64_t cap, void* stream) {
     if (!p) return FP_EINVAL;
-    if (!d_src || !d_field || n < 1 || width < 1 || row0 < 0 || cap < n || row0 >= cap) return pfail(p, FP_EINVAL, "fp_policy_rows_to_ring: bad arguments");
-    cudaSetDevice(p->device);
+    if (!d_src || !d_field || n < 1 || width < 1 || row0 < 0 || cap < n || row0 >= cap) return fail(p, FP_EINVAL, "fp_policy_rows_to_ring: bad arguments");
+    USE_DEVICE(p);
     k_rows_to_ring<<<grid_for(n * width), 256, 0, (cudaStream_t)stream>>>(d_src, n, width, d_field, row0, cap);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return pfail(p, FP_ECUDA, cudaGetErrorString(e));
-    p->launches++;
-    return FP_OK;
+    return launched(p, "k_rows_to_ring");
 }
 
 int fp_policy_scalars_to_ring(FpPolicy* p, const double* d_reward, const uint8_t* d_done, int64_t n, int32_t last_step_all,
                               float* f_reward, float* f_done, float* f_last, float* f_avail, int64_t row0, int64_t cap, void* stream) {
     if (!p) return FP_EINVAL;
-    if (!d_reward || !d_done || n < 1 || row0 < 0 || cap < n || row0 >= cap) return pfail(p, FP_EINVAL, "fp_policy_scalars_to_ring: bad arguments");
-    cudaSetDevice(p->device);
+    if (!d_reward || !d_done || n < 1 || row0 < 0 || cap < n || row0 >= cap) return fail(p, FP_EINVAL, "fp_policy_scalars_to_ring: bad arguments");
+    USE_DEVICE(p);
     k_scalars_to_ring<<<grid_for(n), 256, 0, (cudaStream_t)stream>>>(d_reward, d_done, n, last_step_all, f_reward, f_done, f_last, f_avail, row0, cap);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return pfail(p, FP_ECUDA, cudaGetErrorString(e));
-    p->launches++;
-    return FP_OK;
+    return launched(p, "k_scalars_to_ring");
 }
 
 int fp_policy_transition_tail(FpPolicy* p, const float* d_action, const float* d_logp, const double* d_reward, const uint8_t* d_done,
@@ -1272,15 +1242,12 @@ int fp_policy_transition_tail(FpPolicy* p, const float* d_action, const float* d
     if (!p) return FP_EINVAL;
     if (!d_action || !d_reward || !d_done || !f_action || !f_reward || !f_done || !f_last || (f_logp && !d_logp) ||
         (zero_values && (!f_value || !f_next_value)) || n < 1 || row0 < 0 || cap < n || row0 >= cap)
-        return pfail(p, FP_EINVAL, "fp_policy_transition_tail: bad arguments");
-    cudaSetDevice(p->device);
+        return fail(p, FP_EINVAL, "fp_policy_transition_tail: bad arguments");
+    USE_DEVICE(p);
     k_transition_tail<<<grid_for(n * POL_NA * POL_ACT), 256, 0, (cudaStream_t)stream>>>(d_action, d_logp, d_reward, d_done, n, last_step_all,
                                                                                        zero_values, f_action, f_logp, f_value, f_next_value,
                                                                                        f_reward, f_done, f_last, f_avail, row0, cap);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return pfail(p, FP_ECUDA, cudaGetErrorString(e));
-    p->launches++;
-    return FP_OK;
+    return launched(p, "k_transition_tail");
 }
 
 // Critic weights, HOST fp32 arrays in torch's state_dict layouts (MLPCritic, madrl/critics/mlp_critic.py:5-20, as
@@ -1290,8 +1257,8 @@ int fp_policy_transition_tail(FpPolicy* p, const float* d_action, const float* d
 int fp_critic_load(FpPolicy* p, const float* fc1_w, const float* fc1_b, const float* ln_g, const float* ln_b, const float* fc2_w,
                    const float* fc2_b, const float* fc3_w, const float* fc3_b) {
     if (!p) return FP_EINVAL;
-    if (!fc1_w || !fc1_b || !ln_g || !ln_b || !fc2_w || !fc2_b || !fc3_w || !fc3_b) return pfail(p, FP_EINVAL, "fp_critic_load: null weight array");
-    cudaSetDevice(p->device);
+    if (!fc1_w || !fc1_b || !ln_g || !ln_b || !fc2_w || !fc2_b || !fc3_w || !fc3_b) return fail(p, FP_EINVAL, "fp_critic_load: null weight array");
+    USE_DEVICE(p);
     const int KIN = POL_NA * POL_OBS + POL_NA + POL_NA * POL_ACT;          // 745
     const size_t blk = CR_WB_BYTES / 4;
     // fc1, observation columns: per ring rotation q and agent block a, UMMA K-major layout [kc][n][4] (see fp_policy_load)
@@ -1315,17 +1282,16 @@ int fp_critic_load(FpPolicy* p, const float* fc1_w, const float* fc1_b, const fl
         vec[CV_LNG + n] = ln_g[n]; vec[CV_LNB + n] = ln_b[n]; vec[CV_B2 + n] = fc2_b[n]; vec[CV_W3 + n] = fc3_w[n];           // fc3 runs in fp32: unrounded
     }
     vec[CV_B3] = fc3_b[0];
+    p->critic_loaded = 0;
     cudaFree(p->d_Wc1rot); cudaFree(p->d_Wc2); cudaFree(p->d_Wca); cudaFree(p->d_cvec);
-    p->d_Wc1rot = p->d_Wc2 = p->d_Wca = p->d_cvec = nullptr; p->critic_loaded = 0;
-    if (cudaMalloc(&p->d_Wc1rot, W1.size() * 4) != cudaSuccess || cudaMalloc(&p->d_Wc2, W2.size() * 4) != cudaSuccess ||
-        cudaMalloc(&p->d_Wca, Wa.size() * 4) != cudaSuccess || cudaMalloc(&p->d_cvec, vec.size() * 4) != cudaSuccess)
-        return pfail(p, FP_ENOMEM, "fp_critic_load: cudaMalloc failed");
-    cudaMemcpy(p->d_Wc1rot, W1.data(), W1.size() * 4, cudaMemcpyHostToDevice);
-    cudaMemcpy(p->d_Wc2, W2.data(), W2.size() * 4, cudaMemcpyHostToDevice);
-    cudaMemcpy(p->d_Wca, Wa.data(), Wa.size() * 4, cudaMemcpyHostToDevice);
-    cudaMemcpy(p->d_cvec, vec.data(), vec.size() * 4, cudaMemcpyHostToDevice);
-    cudaError_t e = cudaFuncSetAttribute(k_critic, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CR_SMEM);
-    if (e != cudaSuccess) return pfail(p, FP_ECUDA, cudaGetErrorString(e));
+    p->d_Wc1rot = p->d_Wc2 = p->d_Wca = p->d_cvec = nullptr;
+    CUDA_TRY(p, alloc_group({{&p->d_Wc1rot, W1.size() * 4}, {&p->d_Wc2, W2.size() * 4}, {&p->d_Wca, Wa.size() * 4},
+                             {&p->d_cvec, vec.size() * 4}}));
+    CUDA_TRY(p, cudaMemcpy(p->d_Wc1rot, W1.data(), W1.size() * 4, cudaMemcpyHostToDevice));
+    CUDA_TRY(p, cudaMemcpy(p->d_Wc2, W2.data(), W2.size() * 4, cudaMemcpyHostToDevice));
+    CUDA_TRY(p, cudaMemcpy(p->d_Wca, Wa.data(), Wa.size() * 4, cudaMemcpyHostToDevice));
+    CUDA_TRY(p, cudaMemcpy(p->d_cvec, vec.data(), vec.size() * 4, cudaMemcpyHostToDevice));
+    CUDA_TRY(p, cudaFuncSetAttribute(k_critic, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CR_SMEM));
     p->critic_loaded = 1;
     return FP_OK;
 }
@@ -1336,10 +1302,10 @@ int fp_critic_load(FpPolicy* p, const float* fc1_w, const float* fc1_b, const fl
 int fp_critic_value(FpPolicy* p, const float* d_ring, int32_t slot, int64_t n_pad, int64_t n_envs, const float* d_actions,
                     float* d_value, void* stream) {
     if (!p) return FP_EINVAL;
-    if (!p->critic_loaded) return pfail(p, FP_ESTATE, "fp_critic_value: call fp_critic_load first");
+    if (!p->critic_loaded) return fail(p, FP_ESTATE, "fp_critic_value: call fp_critic_load first");
     if (!d_ring || !d_actions || !d_value || n_envs < 1 || slot < 0 || slot >= POL_H || n_pad < n_envs || (n_pad & 3))
-        return pfail(p, FP_EINVAL, "fp_critic_value: bad arguments");
-    cudaSetDevice(p->device);
+        return fail(p, FP_EINVAL, "fp_critic_value: bad arguments");
+    USE_DEVICE(p);
     CritParams prm;
     std::memset(&prm, 0, sizeof(prm));
     prm.ring = d_ring; prm.n_pad = n_pad; prm.n = n_envs; prm.slot = slot;
@@ -1348,14 +1314,11 @@ int fp_critic_value(FpPolicy* p, const float* d_ring, int32_t slot, int64_t n_pa
     alignas(64) CUtensorMap tmap;
     { const int rc = ring_tensor_map(p, d_ring, n_pad, &tmap, &prm.use_tma, "fp_critic_value", POL_H / 2); if (rc != FP_OK) return rc; }   // half-block boxes
     int sms = 0;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, p->device);
+    CUDA_TRY(p, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, p->device));
     const int64_t tiles = (n_envs + POL_M - 1) / POL_M;
     const int grid = (int)(tiles < sms ? tiles : sms);
     k_critic<<<grid, CRIT_THREADS, CR_SMEM, (cudaStream_t)stream>>>(prm, tmap);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return pfail(p, FP_ECUDA, cudaGetErrorString(e));
-    p->launches++;
-    return FP_OK;
+    return launched(p, "k_critic");
 }
 
 // Learner feed (unpack_data, madrl/models/model.py:308-323, on a sampled batch already on the device):
@@ -1364,19 +1327,12 @@ int fp_critic_value(FpPolicy* p, const float* d_ring, int32_t slot, int64_t n_pa
 int fp_learner_feed(FpPolicy* p, const float* d_state, const float* d_action, const float* d_reward, int64_t batch,
                     float* d_critic_in, float* d_reward_norm, void* stream) {
     if (!p) return FP_EINVAL;
-    if (batch < 1 || (d_critic_in && (!d_state || !d_action)) || (d_reward_norm && !d_reward)) return pfail(p, FP_EINVAL, "fp_learner_feed: bad arguments");
-    cudaSetDevice(p->device);
-    if (d_critic_in) {
+    if (batch < 1 || (d_critic_in && (!d_state || !d_action)) || (d_reward_norm && !d_reward)) return fail(p, FP_EINVAL, "fp_learner_feed: bad arguments");
+    USE_DEVICE(p);
+    if (d_critic_in)
         k_critic_input<<<grid_for(batch * POL_NA * 745), 256, 0, (cudaStream_t)stream>>>(d_state, d_action, batch, d_critic_in);
-        p->launches++;
-    }
-    if (d_reward_norm) {
-        k_reward_batchnorm<<<POL_NA, 256, 0, (cudaStream_t)stream>>>(d_reward, batch, d_reward_norm);
-        p->launches++;
-    }
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return pfail(p, FP_ECUDA, cudaGetErrorString(e));
-    return FP_OK;
+    if (d_reward_norm) k_reward_batchnorm<<<POL_NA, 256, 0, (cudaStream_t)stream>>>(d_reward, batch, d_reward_norm);
+    return launched(p, "fp_learner_feed", (d_critic_in != nullptr) + (d_reward_norm != nullptr));
 }
 
 }  // extern "C"

@@ -40,15 +40,9 @@
 #include <cmath>
 #include <cstring>
 
-#include "flex_kernels.cuh"
-#include "predictor.cuh"
+#include "api_handle.cuh"
+#include "flex_handle.cuh"
 #include "sm100_ptx.cuh"
-
-// implemented in flex_api.cu
-PredictorState* fp_internal_predictor(FpHandle* h);
-int fp_internal_fail(FpHandle* h, int code, const char* msg);
-void fp_internal_count_launch(FpHandle* h, int k);
-int fp_internal_device(FpHandle* h);
 
 namespace {
 
@@ -332,18 +326,6 @@ __global__ void k_replay_gather(const float* __restrict__ field, int64_t cap, in
     }
 }
 
-int grid_for_elems(int64_t total) {
-    int64_t g = (total + 255) / 256;
-    if (g < 1) g = 1;
-    return (int)(g > 148 * 16 ? 148 * 16 : g);
-}
-
-thread_local std::string g_replay_err;
-int rfail(FpReplay* r, int code, const std::string& msg) {
-    if (r) r->err = msg; else g_replay_err = msg;
-    return code;
-}
-
 }  // namespace
 
 void predictor_free(PredictorState* p) {
@@ -358,10 +340,10 @@ int fp_predictor_load(FpHandle* h, int32_t n_in, int32_t n_out, const double* h_
                       double v_max, double slack_weight) {
     if (!h) return FP_EINVAL;
     if (n_in != N_IN || n_out != N_OUT || !h_A || !h_c)
-        return fp_internal_fail(h, FP_EINVAL, "fp_predictor_load: expects a 66 -> 33 affine model (2*n_bus inputs, n_bus outputs)");
-    PredictorState* p = fp_internal_predictor(h);
-    cudaSetDevice(fp_internal_device(h));
-    predictor_free(p);
+        return fail(h, FP_EINVAL, "fp_predictor_load: expects a 66 -> 33 affine model (2*n_bus inputs, n_bus outputs)");
+    PredictorState* p = &h->pred;
+    USE_DEVICE(h);
+    predictor_free(p);                             // clears p->loaded: set again only after the last step below
     // weights: fp64 -> (hi, lo) TF32-representable pair, UMMA K-major layout [part][k-chunk][n][4], zero padded
     std::vector<float> B(2 * PRED_KC * PRED_N * 4, 0.0f), bias(PRED_N, 0.0f);
     for (int n = 0; n < N_OUT; ++n) {
@@ -375,12 +357,10 @@ int fp_predictor_load(FpHandle* h, int32_t n_in, int32_t n_out, const double* h_
         }
         bias[n] = (float)h_c[n];
     }
-    if (cudaMalloc(&p->d_B, B.size() * 4) != cudaSuccess || cudaMalloc(&p->d_bias, bias.size() * 4) != cudaSuccess)
-        return fp_internal_fail(h, FP_ENOMEM, "fp_predictor_load: cudaMalloc failed");
-    cudaMemcpy(p->d_B, B.data(), B.size() * 4, cudaMemcpyHostToDevice);
-    cudaMemcpy(p->d_bias, bias.data(), bias.size() * 4, cudaMemcpyHostToDevice);
-    cudaError_t e = cudaFuncSetAttribute(k_predict, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES);
-    if (e != cudaSuccess) return fp_internal_fail(h, FP_ECUDA, cudaGetErrorString(e));
+    CUDA_TRY(h, alloc_group({{&p->d_B, B.size() * 4}, {&p->d_bias, bias.size() * 4}}));
+    CUDA_TRY(h, cudaMemcpy(p->d_B, B.data(), B.size() * 4, cudaMemcpyHostToDevice));
+    CUDA_TRY(h, cudaMemcpy(p->d_bias, bias.data(), bias.size() * 4, cudaMemcpyHostToDevice));
+    CUDA_TRY(h, cudaFuncSetAttribute(k_predict, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
     p->n_in = n_in; p->n_out = n_out; p->v_min = v_min; p->v_max = v_max; p->slack_weight = slack_weight;
     p->loaded = 1;
     return FP_OK;
@@ -389,10 +369,10 @@ int fp_predictor_load(FpHandle* h, int32_t n_in, int32_t n_out, const double* h_
 int fp_predict(FpHandle* h, int64_t n, const float* d_X, float* d_vhat, double* d_penalty, FpReplay* sink,
                int32_t f_vhat, int32_t f_penalty, int64_t pos, void* stream) {
     if (!h) return FP_EINVAL;
-    PredictorState* p = fp_internal_predictor(h);
-    if (!p->loaded) return fp_internal_fail(h, FP_ESTATE, "fp_predict: call fp_predictor_load first");
-    if (n < 1 || !d_X) return fp_internal_fail(h, FP_EINVAL, "fp_predict: bad arguments");
-    if (((uintptr_t)d_X & 15) != 0) return fp_internal_fail(h, FP_EINVAL, "fp_predict: X must be 16-byte aligned (TMA)");
+    const PredictorState* p = &h->pred;
+    if (!p->loaded) return fail(h, FP_ESTATE, "fp_predict: call fp_predictor_load first");
+    if (n < 1 || !d_X) return fail(h, FP_EINVAL, "fp_predict: bad arguments");
+    if (((uintptr_t)d_X & 15) != 0) return fail(h, FP_EINVAL, "fp_predict: X must be 16-byte aligned (TMA)");
     PredParams prm;
     std::memset(&prm, 0, sizeof(prm));
     prm.X = d_X; prm.n = n; prm.B = p->d_B; prm.bias = p->d_bias; prm.vhat = d_vhat; prm.penalty = d_penalty;
@@ -403,44 +383,47 @@ int fp_predict(FpHandle* h, int64_t n, const float* d_X, float* d_vhat, double* 
     if (sink) {
         const int nf = (int)sink->widths.size();
         if (n > sink->capacity || pos < 0 || pos >= sink->capacity)
-            return fp_internal_fail(h, FP_EINVAL, "fp_predict: rows do not fit the replay ring");
+            return fail(h, FP_EINVAL, "fp_predict: rows do not fit the replay ring");
         if (f_vhat >= 0) {
-            if (f_vhat >= nf || sink->widths[f_vhat] != N_OUT) return fp_internal_fail(h, FP_EINVAL, "fp_predict: Vhat field must have width 33");
+            if (f_vhat >= nf || sink->widths[f_vhat] != N_OUT) return fail(h, FP_EINVAL, "fp_predict: Vhat field must have width 33");
             prm.ring_vhat = sink->d_fields[f_vhat];
         }
         if (f_penalty >= 0) {
-            if (f_penalty >= nf || sink->widths[f_penalty] != 1) return fp_internal_fail(h, FP_EINVAL, "fp_predict: penalty field must have width 1");
+            if (f_penalty >= nf || sink->widths[f_penalty] != 1) return fail(h, FP_EINVAL, "fp_predict: penalty field must have width 1");
             prm.ring_pen = sink->d_fields[f_penalty];
         }
         prm.ring_cap = sink->capacity; prm.ring_pos = pos;
     }
-    int dev = 0, sms = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    USE_DEVICE(h);
+    int sms = 0;
+    CUDA_TRY(h, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device));
     const int64_t tiles = (n + PRED_M - 1) / PRED_M;
     const int grid = (int)(tiles < sms ? tiles : sms);
     k_predict<<<grid, PRED_THREADS, SMEM_BYTES, (cudaStream_t)stream>>>(prm);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return fp_internal_fail(h, FP_ECUDA, cudaGetErrorString(e));
-    fp_internal_count_launch(h, 1);
-    return FP_OK;
+    return launched(h, "k_predict");
 }
 
 // ------------------------------------------------------------------ replay ring (TransReplayBuffer)
 int fp_replay_create(int64_t capacity, int32_t n_fields, const int32_t* widths, int device, FpReplay** out) {
-    if (!out || capacity < 1 || n_fields < 1 || n_fields > 64 || !widths) return rfail(nullptr, FP_EINVAL, "fp_replay_create: bad arguments");
+    if (!out || capacity < 1 || n_fields < 1 || n_fields > 64 || !widths) return fail<FpReplay>(nullptr, FP_EINVAL, "fp_replay_create: bad arguments");
     int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) return rfail(nullptr, FP_ECUDA, "fp_replay_create: no CUDA device (there is no CPU fallback)");
-    if (device < 0 || device >= ndev) return rfail(nullptr, FP_EINVAL, "fp_replay_create: bad device index");
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) return fail<FpReplay>(nullptr, FP_ECUDA, "fp_replay_create: no CUDA device (there is no CPU fallback)");
+    if (device < 0 || device >= ndev) return fail<FpReplay>(nullptr, FP_EINVAL, "fp_replay_create: bad device index");
+    for (int f = 0; f < n_fields; ++f)
+        if (widths[f] < 1) return fail<FpReplay>(nullptr, FP_EINVAL, "fp_replay_create: field width must be >= 1");
     FpReplay* r = new FpReplay();
     r->capacity = capacity; r->device = device;
-    cudaSetDevice(device);
-    for (int f = 0; f < n_fields; ++f) {
-        if (widths[f] < 1) { fp_replay_destroy(r); return rfail(nullptr, FP_EINVAL, "fp_replay_create: field width must be >= 1"); }
+    const DeviceGuard on_device(device);
+    cudaError_t e = on_device.error();
+    for (int f = 0; f < n_fields && e == cudaSuccess; ++f) {
         float* p = nullptr;
-        if (cudaMalloc(&p, (size_t)capacity * widths[f] * 4) != cudaSuccess) { fp_replay_destroy(r); return rfail(nullptr, FP_ENOMEM, "fp_replay_create: cudaMalloc failed"); }
-        cudaMemset(p, 0, (size_t)capacity * widths[f] * 4);
+        if ((e = cudaMalloc(&p, (size_t)capacity * widths[f] * 4)) != cudaSuccess) break;
         r->widths.push_back(widths[f]); r->d_fields.push_back(p);
+        e = cudaMemset(p, 0, (size_t)capacity * widths[f] * 4);
+    }
+    if (e != cudaSuccess) {
+        fp_replay_destroy(r);
+        return fail<FpReplay>(nullptr, e == cudaErrorMemoryAllocation ? FP_ENOMEM : FP_ECUDA, std::string("fp_replay_create: ") + cudaGetErrorString(e));
     }
     *out = r;
     return FP_OK;
@@ -448,13 +431,13 @@ int fp_replay_create(int64_t capacity, int32_t n_fields, const int32_t* widths, 
 
 int fp_replay_destroy(FpReplay* r) {
     if (!r) return FP_OK;
-    cudaSetDevice(r->device);
+    const DeviceGuard on_device(r->device);       // best effort: the ring is freed whatever happens
     for (float* p : r->d_fields) cudaFree(p);
     delete r;
     return FP_OK;
 }
 
-const char* fp_replay_last_error(const FpReplay* r) { return r ? r->err.c_str() : g_replay_err.c_str(); }
+const char* fp_replay_last_error(const FpReplay* r) { return r ? r->err.c_str() : create_error<FpReplay>().c_str(); }
 int64_t fp_replay_len(const FpReplay* r) { return r ? r->len : 0; }
 int64_t fp_replay_capacity(const FpReplay* r) { return r ? r->capacity : 0; }
 int fp_replay_clear(FpReplay* r) { if (!r) return FP_EINVAL; r->head = 0; r->len = 0; return FP_OK; }     // :29-30
@@ -462,7 +445,7 @@ int fp_replay_clear(FpReplay* r) { if (!r) return FP_EINVAL; r->head = 0; r->len
 // add_experience (:23-27) for n rows at once: the oldest rows are overwritten when the ring is full
 int fp_replay_reserve(FpReplay* r, int64_t n, int64_t* pos) {
     if (!r || !pos) return FP_EINVAL;
-    if (n < 1 || n > r->capacity) return rfail(r, FP_EINVAL, "fp_replay_reserve: 1 <= n <= capacity required");
+    if (n < 1 || n > r->capacity) return fail(r, FP_EINVAL, "fp_replay_reserve: 1 <= n <= capacity required");
     *pos = r->head;
     r->head = (r->head + n) % r->capacity;
     r->len = (r->len + n < r->capacity) ? r->len + n : r->capacity;
@@ -472,25 +455,27 @@ int fp_replay_reserve(FpReplay* r, int64_t n, int64_t* pos) {
 int fp_replay_write(FpReplay* r, int32_t field, int64_t pos, int64_t n, const float* d_src, void* stream) {
     if (!r) return FP_EINVAL;
     if (field < 0 || field >= (int)r->widths.size() || !d_src || n < 1 || n > r->capacity || pos < 0 || pos >= r->capacity)
-        return rfail(r, FP_EINVAL, "fp_replay_write: bad arguments");
+        return fail(r, FP_EINVAL, "fp_replay_write: bad arguments");
+    USE_DEVICE(r);
     const int w = r->widths[field];
-    k_replay_write<<<grid_for_elems(n * w), 256, 0, (cudaStream_t)stream>>>(r->d_fields[field], r->capacity, w, pos, n, d_src);
-    cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? FP_OK : rfail(r, FP_ECUDA, cudaGetErrorString(e));
+    k_replay_write<<<grid_for(n * w), 256, 0, (cudaStream_t)stream>>>(r->d_fields[field], r->capacity, w, pos, n, d_src);
+    CUDA_TRY(r, cudaGetLastError());
+    return FP_OK;
 }
 
 // get_batch (:14-21): `batch` consecutive rows from logical index `start` (0 = oldest)
 int fp_replay_sample(FpReplay* r, int64_t start, int64_t batch, float* const* d_out, void* stream) {
     if (!r || !d_out) return FP_EINVAL;
-    if (batch < 1 || start < 0 || start + batch > r->len) return rfail(r, FP_EINVAL, "fp_replay_sample: window outside the stored rows");
+    if (batch < 1 || start < 0 || start + batch > r->len) return fail(r, FP_EINVAL, "fp_replay_sample: window outside the stored rows");
+    USE_DEVICE(r);
     const int64_t first = ((r->head - r->len + start) % r->capacity + r->capacity) % r->capacity;
     for (size_t f = 0; f < r->widths.size(); ++f) {
         if (!d_out[f]) continue;
         const int w = r->widths[f];
-        k_replay_gather<<<grid_for_elems(batch * w), 256, 0, (cudaStream_t)stream>>>(r->d_fields[f], r->capacity, w, first, batch, d_out[f]);
+        k_replay_gather<<<grid_for(batch * w), 256, 0, (cudaStream_t)stream>>>(r->d_fields[f], r->capacity, w, first, batch, d_out[f]);
     }
-    cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? FP_OK : rfail(r, FP_ECUDA, cudaGetErrorString(e));
+    CUDA_TRY(r, cudaGetLastError());
+    return FP_OK;
 }
 
 int fp_replay_field_ptr(FpReplay* r, int32_t field, float** d_ptr) {

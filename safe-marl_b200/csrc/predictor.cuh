@@ -19,7 +19,6 @@ struct PredictorState {
     float* d_B = nullptr;      // [2 (hi, lo)][PRED_KC][PRED_N][4] tf32-splittable weights, UMMA K-major layout
     float* d_bias = nullptr;   // [PRED_N]
     double v_min = 0.0, v_max = 0.0, slack_weight = 0.0;
-    int64_t launches = 0;
 };
 
 void predictor_free(PredictorState* p);
@@ -29,6 +28,5 @@ struct FpReplay {
     int device = 0;
     std::vector<int32_t> widths;
     std::vector<float*> d_fields;      // [capacity][width] each
-    float** d_out_ptrs = nullptr;      // device copy of the output pointer table used by sample
     std::string err;
 };

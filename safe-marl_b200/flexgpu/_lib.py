@@ -7,6 +7,8 @@ module raises, and if no CUDA device is present `fp_create` fails.
 import ctypes as C
 import os
 
+import torch
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 # FLEXGPU_LIB: tuning builds of the same library (tools/); the product path is the in-tree default
 LIB_PATH = os.environ.get("FLEXGPU_LIB") or os.path.join(_HERE, "libflexgpu.so")
@@ -143,7 +145,14 @@ def lib():
     return _lib
 
 
-def check(rc, handle=None, what=""):
+def check(rc, handle=None, what="", last_error=None):
+    """Raise FlexGpuError for a failed entry point.  last_error: the *_last_error function of the handle's kind
+    (default fp_last_error, the env handle's); a NULL handle reads the last failed create of that kind."""
     if rc != 0:
-        msg = lib().fp_last_error(handle)
+        msg = (last_error or lib().fp_last_error)(handle)
         raise FlexGpuError(f"{what} failed (code {rc}): {msg.decode() if msg else ''}")
+
+
+def stream(device):
+    """torch's current stream on `device` (the handle's device, whatever torch's current device is) as a cudaStream_t."""
+    return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)

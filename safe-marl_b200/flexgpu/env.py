@@ -30,10 +30,6 @@ def _ptr(t):
     return C.c_void_p(t.data_ptr()) if t is not None else None
 
 
-def _stream():
-    return C.c_void_p(torch.cuda.current_stream().cuda_stream)
-
-
 class BatchedFlexProvisionEnv:
     def __init__(self, kwargs=None, n_envs=1, device="cuda:0", network=None, profiles=None,
                  seed=None, env_offset=0):
@@ -65,7 +61,7 @@ class BatchedFlexProvisionEnv:
         self._cfg = make_fp_config(self.args_dict, self.network)
         self._h = C.c_void_p()
         dev_index = self.device.index if self.device.index is not None else torch.cuda.current_device()
-        torch.cuda.set_device(dev_index)
+        self.device = torch.device("cuda", dev_index)    # the handle's device: torch's current device may change later
         _lib.check(self._lib.fp_create(C.byref(self._cfg), self.n_envs, dev_index, C.byref(self._h)),
                    None, "fp_create")
         self.profiles = None
@@ -249,10 +245,10 @@ class BatchedFlexProvisionEnv:
                 self._reset_failed = torch.zeros(1, dtype=torch.int32, device=self.device)
             n_retry = self.RESET_RETRIES if retries is None else int(retries)
             if n_retry == 0 and not check:         # per-step auto-reset: one launch, no failure count
-                self._check(self._lib.fp_reset_random(self._h, self.seed, self.env_offset, _ptr(m), _stream()), "fp_reset_random")
+                self._check(self._lib.fp_reset_random(self._h, self.seed, self.env_offset, _ptr(m), _lib.stream(self.device)), "fp_reset_random")
             else:
                 self._check(self._lib.fp_reset_random_retry(self._h, self.seed, self.env_offset, _ptr(m), n_retry,
-                                                            _ptr(self._reset_failed), _stream()), "fp_reset_random_retry")
+                                                            _ptr(self._reset_failed), _lib.stream(self.device)), "fp_reset_random_retry")
             if check and int(self._reset_failed.item()):
                 raise _lib.FlexGpuError(f"{int(self._reset_failed.item())} envs found no solvable initial state in "
                                         f"{self.RESET_RETRIES + 1} draws")
@@ -264,9 +260,9 @@ class BatchedFlexProvisionEnv:
             lo, hi = int(s.min()), int(s.max())
             if lo < 0 or hi >= self.max_start():
                 raise ValueError("start_index out of range for the loaded profiles")
-            self._check(self._lib.fp_reset(self._h, _ptr(s), _ptr(e), _ptr(a), _ptr(m), _stream()), "fp_reset")
+            self._check(self._lib.fp_reset(self._h, _ptr(s), _ptr(e), _ptr(a), _ptr(m), _lib.stream(self.device)), "fp_reset")
         if return_obs == "ring":                                        # reset()'s get_obs (:155) for the reset envs, ring form
-            self._check(self._lib.fp_obs_ring_reset_push(self._h, _ptr(m), _stream()), "fp_obs_ring_reset_push")
+            self._check(self._lib.fp_obs_ring_reset_push(self._h, _ptr(m), _lib.stream(self.device)), "fp_obs_ring_reset_push")
             return self.obs_ring()
         if return_obs:
             return self.get_obs(), self.get_state()                     # :155
@@ -299,17 +295,17 @@ class BatchedFlexProvisionEnv:
             p, sl, npad = C.c_void_p(), C.c_int32(), C.c_int64()
             self._check(self._lib.fp_step_ring(self._h, _ptr(actions), dt, _ptr(self._reward), _ptr(self._done),
                                                _ptr(self._info) if want_info else None, _ptr(m), C.byref(p), C.byref(sl),
-                                               C.byref(npad), _stream()), "fp_step_ring")
+                                               C.byref(npad), _lib.stream(self.device)), "fp_step_ring")
             obs = self._ring(p.value, sl.value, npad.value)
         elif return_obs:                             # step + pushing get_obs, dense strided view (fp_step_obs)
             p, ep, ap = C.c_void_p(), C.c_int64(), C.c_int64()
             self._check(self._lib.fp_step_obs(self._h, _ptr(actions), dt, _ptr(self._reward), _ptr(self._done),
                                               _ptr(self._info) if want_info else None, _ptr(m), C.byref(p), C.byref(ep),
-                                              C.byref(ap), _stream()), "fp_step_obs")
+                                              C.byref(ap), _lib.stream(self.device)), "fp_step_obs")
             obs = self._obs_view(p.value, ep.value, ap.value)
         else:
             self._check(self._lib.fp_step(self._h, _ptr(actions), dt, _ptr(self._reward), _ptr(self._done),
-                                          _ptr(self._info) if want_info else None, _ptr(m), _stream()), "fp_step")
+                                          _ptr(self._info) if want_info else None, _ptr(m), _lib.stream(self.device)), "fp_step")
         info = {k: self._info[:, i] for i, k in enumerate(_lib.INFO_KEYS)} if want_info else {}
         if return_obs:
             return self._reward, self._done, info, obs
@@ -336,7 +332,7 @@ class BatchedFlexProvisionEnv:
         self._check(self._lib.fp_step_host(
             self._h, a.ctypes.data_as(C.c_void_p), dt, C.c_void_p(hb["reward"].data_ptr()),
             C.c_void_p(hb["done"].data_ptr()), C.c_void_p(hb["info"].data_ptr()) if want_info else None,
-            _stream()), "fp_step_host")
+            _lib.stream(self.device)), "fp_step_host")
         info = {k: hb["info"].numpy()[:, i] for i, k in enumerate(_lib.INFO_KEYS)} if want_info else {}
         return hb["reward"].numpy(), hb["done"].numpy().astype(bool), info
 
@@ -353,7 +349,7 @@ class BatchedFlexProvisionEnv:
         contiguous=True go through their own buffers."""
         if push and dtype == torch.float32 and not contiguous:
             p, ep, ap = C.c_void_p(), C.c_int64(), C.c_int64()
-            self._check(self._lib.fp_get_obs_view(self._h, 1, C.byref(p), C.byref(ep), C.byref(ap), _stream()),
+            self._check(self._lib.fp_get_obs_view(self._h, 1, C.byref(p), C.byref(ep), C.byref(ap), _lib.stream(self.device)),
                         "fp_get_obs_view")
             return self._obs_view(p.value, ep.value, ap.value)
         buf = self._obs.get(dtype)
@@ -361,13 +357,13 @@ class BatchedFlexProvisionEnv:
             buf = torch.empty(self.n_envs, self.n_agents, self.obs_size, dtype=dtype, device=self.device)
             self._obs[dtype] = buf
         dt = _lib.FP_F64 if dtype == torch.float64 else _lib.FP_F32
-        self._check(self._lib.fp_get_obs(self._h, _ptr(buf), dt, 1 if push else 0, _stream()), "fp_get_obs")
+        self._check(self._lib.fp_get_obs(self._h, _ptr(buf), dt, 1 if push else 0, _lib.stream(self.device)), "fp_get_obs")
         return buf
 
     def obs_ring(self):
         """The observation history in its native device layout (fp_obs_ring): ObsRing, no push."""
         p, sl, npad = C.c_void_p(), C.c_int32(), C.c_int64()
-        self._check(self._lib.fp_obs_ring(self._h, C.byref(p), C.byref(sl), C.byref(npad), _stream()), "fp_obs_ring")
+        self._check(self._lib.fp_obs_ring(self._h, C.byref(p), C.byref(sl), C.byref(npad), _lib.stream(self.device)), "fp_obs_ring")
         return self._ring(p.value, sl.value, npad.value)
 
     def _ring(self, ptr, slot, n_pad):
@@ -395,7 +391,7 @@ class BatchedFlexProvisionEnv:
             buf = torch.empty(self.n_envs, self.state_size, dtype=dtype, device=self.device)
             self._state[dtype] = buf
         dt = _lib.FP_F64 if dtype == torch.float64 else _lib.FP_F32
-        self._check(self._lib.fp_get_state(self._h, _ptr(buf), dt, _stream()), "fp_get_state")
+        self._check(self._lib.fp_get_state(self._h, _ptr(buf), dt, _lib.stream(self.device)), "fp_get_state")
         return buf
 
     def get_avail_actions(self):                 # :721-726
@@ -433,7 +429,7 @@ class BatchedFlexProvisionEnv:
         iters = torch.empty(n, dtype=torch.int32, device=self.device)
         failed = torch.empty(n, dtype=torch.uint8, device=self.device)
         self._check(self._lib.fp_power_flow(self._h, n, _ptr(p), _ptr(q), _ptr(V), _ptr(Pl), _ptr(Ql),
-                                            _ptr(Isq), _ptr(iters), _ptr(failed), _stream()), "fp_power_flow")
+                                            _ptr(Isq), _ptr(iters), _ptr(failed), _lib.stream(self.device)), "fp_power_flow")
         return dict(V=V, P=Pl, Q=Ql, Isq=Isq, iters=iters, failed=failed.bool())
 
     def set_obs_history(self, keep=True):
@@ -488,7 +484,7 @@ class BatchedFlexProvisionEnv:
         slack = torch.empty(self.n_envs, self.n_agents, dtype=torch.float64, device=self.device) if want_info else None
         moved = torch.empty(self.n_envs, self.n_agents, dtype=torch.uint8, device=self.device) if want_info else None
         self._check(self._lib.fp_safety_project(self._h, _ptr(a), _lib.FP_F64 if a.dtype == torch.float64 else _lib.FP_F32, _ptr(out),
-                                                1 if tm else 0, _ptr(slack), _ptr(moved), _stream()), "fp_safety_project")
+                                                1 if tm else 0, _ptr(slack), _ptr(moved), _lib.stream(self.device)), "fp_safety_project")
         return (out, slack, moved.bool()) if want_info else out
 
     def load_safety_map(self, A, c, slack_weight=1000.0, v_min=None, v_max=None):
@@ -518,7 +514,7 @@ class BatchedFlexProvisionEnv:
         moved = torch.empty(self.n_envs, self.n_agents, dtype=torch.uint8, device=self.device) if want_info else None
         status = torch.empty(self.n_envs, dtype=torch.int32, device=self.device) if want_info else None
         self._check(self._lib.fp_safety_project_affine(self._h, _ptr(a), _lib.FP_F64 if a.dtype == torch.float64 else _lib.FP_F32,
-                                                       _ptr(out), 1 if tm else 0, _ptr(slack), _ptr(moved), _ptr(status), _stream()),
+                                                       _ptr(out), 1 if tm else 0, _ptr(slack), _ptr(moved), _ptr(status), _lib.stream(self.device)),
                     "fp_safety_project_affine")
         return (out, slack, moved.bool(), status) if want_info else out
 
@@ -527,12 +523,12 @@ class BatchedFlexProvisionEnv:
         """Sums accumulated by every step since the last reset of the statistics (the batched
         form of madrl/models/model.py:247-265).  With torch.distributed initialised and
         reduce=True the vector is all-reduced (NCCL) -- the only collective on this path."""
-        self._check(self._lib.fp_stats_read(self._h, _ptr(self._stats), _stream()), "fp_stats_read")
+        self._check(self._lib.fp_stats_read(self._h, _ptr(self._stats), _lib.stream(self.device)), "fp_stats_read")
         out = self._stats.clone()
         if reduce:
             sharding.reduce_stats(out)
         if reset:
-            self._check(self._lib.fp_stats_reset(self._h, _stream()), "fp_stats_reset")
+            self._check(self._lib.fp_stats_reset(self._h, _lib.stream(self.device)), "fp_stats_reset")
         return sharding.stats_dict(out)
 
     # ------------------------------------------------------------------ test hooks
@@ -558,7 +554,7 @@ class ObsRing:
         env = self.env
         if out is None:
             out = torch.empty(env.n_envs, env.n_agents, env.obs_size, dtype=torch.float32, device=env.device)
-        env._check(env._lib.fp_obs_ring_gather(env._h, _ptr(out), _stream()), "fp_obs_ring_gather")
+        env._check(env._lib.fp_obs_ring_gather(env._h, _ptr(out), _lib.stream(env.device)), "fp_obs_ring_gather")
         return out
 
 

@@ -34,10 +34,6 @@ def _ptr(t):
     return C.c_void_p(t.data_ptr())
 
 
-def _stream():
-    return C.c_void_p(torch.cuda.current_stream().cuda_stream)
-
-
 def round_tf32(w):
     """Round-to-nearest-even to TF32 (10-bit mantissa): how fp_policy_load holds the weights."""
     u = np.ascontiguousarray(w, dtype=np.float32).view(np.uint32).astype(np.uint64)
@@ -53,9 +49,8 @@ class DevicePolicy:
         self._lib = _lib.lib()
         self._p = C.c_void_p()
         idx = self.device.index if self.device.index is not None else torch.cuda.current_device()
-        rc = self._lib.fp_policy_create(idx, C.byref(self._p))
-        if rc != 0:
-            raise _lib.FlexGpuError(f"fp_policy_create failed ({rc}): {self._lib.fp_policy_last_error(None).decode()}")
+        self.device = torch.device("cuda", idx)
+        _lib.check(self._lib.fp_policy_create(idx, C.byref(self._p)), None, "fp_policy_create", self._lib.fp_policy_last_error)
         self.std = float(std)                       # fixed_policy_std (default.yaml: 1.0; gaussian_policy False)
         self.seed = int(seed)
         self._bufs = {}
@@ -64,8 +59,7 @@ class DevicePolicy:
             self.load_state_dict(state_dict)
 
     def _check(self, rc, what):
-        if rc != 0:
-            raise _lib.FlexGpuError(f"{what} failed ({rc}): {self._lib.fp_policy_last_error(self._p).decode()}")
+        _lib.check(rc, self._p, what, self._lib.fp_policy_last_error)
 
     def close(self):
         if getattr(self, "_p", None) is not None and self._p.value:
@@ -113,7 +107,7 @@ class DevicePolicy:
         if tuple(act.shape) != (N, N_AGENTS, ACT):
             raise ValueError("action must be [n_envs, 5, 4]")
         out = self._buf("value", (N, N_AGENTS, 1)) if out is None else out
-        self._check(self._lib.fp_critic_value(self._p, _ptr(ring), int(slot), int(ring.shape[-1]), N, _ptr(act), _ptr(out), _stream()),
+        self._check(self._lib.fp_critic_value(self._p, _ptr(ring), int(slot), int(ring.shape[-1]), N, _ptr(act), _ptr(out), _lib.stream(self.device)),
                     "fp_critic_value")
         return out
 
@@ -149,7 +143,7 @@ class DevicePolicy:
         e = None if eps is None else eps.to(device=self.device, dtype=torch.float32).contiguous()
         self._check(self._lib.fp_policy_act(self._p, _ptr(ring), int(slot), int(n_pad), N, _ptr(hid_in), _ptr(r), _ptr(hid_out),
                                             1 if em else 0, _ptr(mean), _ptr(action), _ptr(logp), _ptr(e), self.seed, int(step),
-                                            self.std, 1 if explore else 0, _stream()), "fp_policy_act")
+                                            self.std, 1 if explore else 0, _lib.stream(self.device)), "fp_policy_act")
         return action, logp, hid_out, mean
 
     def sample(self, mean, explore=True, eps=None, step=0, want_logp=True, out="action"):
@@ -160,13 +154,13 @@ class DevicePolicy:
         logp = self._buf("logp", (N, N_AGENTS, ACT)) if want_logp else None
         e = None if eps is None else eps.to(device=self.device, dtype=torch.float32).contiguous()
         self._check(self._lib.fp_policy_sample(self._p, _ptr(mean), N, _ptr(action), _ptr(logp), _ptr(e), self.seed, int(step),
-                                               self.std, 1 if explore else 0, _stream()), "fp_policy_sample")
+                                               self.std, 1 if explore else 0, _lib.stream(self.device)), "fp_policy_sample")
         return action, logp
 
     def gather_windows(self, ring, n, out, pitch, row0=0, cap=None):
         slot, ringt = ring.slot, ring.ring
         self._check(self._lib.fp_policy_gather_windows(self._p, _ptr(ringt), int(slot), int(ringt.shape[-1]), int(n), _ptr(out),
-                                                       int(pitch), int(row0), int(cap if cap is not None else n), _stream()),
+                                                       int(pitch), int(row0), int(cap if cap is not None else n), _lib.stream(self.device)),
                     "fp_policy_gather_windows")
 
 
@@ -242,12 +236,12 @@ class DeviceRollout:
         pol = self.policy
         w = TRANSITION_FIELDS[name]
         pol._check(pol._lib.fp_policy_rows_to_ring(pol._p, _ptr(src), self.R, w, self._fptr[name], pos, self.replay.size,
-                                                   _stream()), "fp_policy_rows_to_ring")
+                                                   _lib.stream(pol.device)), "fp_policy_rows_to_ring")
 
     def _hidden_rows(self, name, hid_em, pos, zero_mask=None):
         pol = self.policy
         pol._check(pol._lib.fp_policy_hidden_to_ring(pol._p, _ptr(hid_em), self._n_pad, self.R, self._fptr[name], pos, self.replay.size,
-                                                     _ptr(zero_mask), _stream()), "fp_policy_hidden_to_ring")
+                                                     _ptr(zero_mask), _lib.stream(pol.device)), "fp_policy_hidden_to_ring")
 
     def hidden(self):
         """The current hidden state in the reference's layout [N, 5, 64] (a copy)."""
@@ -308,7 +302,7 @@ class DeviceRollout:
             pol._check(pol._lib.fp_policy_transition_tail(
                 pol._p, _ptr(action), _ptr(logp), _ptr(reward), _ptr(done), self.R, 1 if self.t == self.max_steps else 0,
                 1 if self.value_fn is None else 0, f["action"], f["log_prob_a"], f["value"], f["next_value"], f["reward"], f["done"],
-                f["last_step"], f["action_avail"], pos, self.replay.size, _stream()), "fp_policy_transition_tail")
+                f["last_step"], f["action_avail"], pos, self.replay.size, _lib.stream(pol.device)), "fp_policy_transition_tail")
         self._cur = 1 - self._cur
         self._reset_mask = None
         if self.t >= env.episode_limit - 1 or self.t >= self.max_steps:        # every env of the batch has terminated (Q1)
@@ -342,7 +336,7 @@ def learner_batch(policy, replay, batch_size, start=None, reward_normalisation=T
     crit = torch.empty(B * N_AGENTS, N_AGENTS * OBS + N_AGENTS + N_AGENTS * ACT, device=replay.device) if critic_input else None
     rn = torch.empty(B, N_AGENTS, device=replay.device) if reward_normalisation else None
     policy._check(policy._lib.fp_learner_feed(policy._p, _ptr(b["state"]), _ptr(b["action"]), _ptr(b["reward"]), B, _ptr(crit),
-                                              _ptr(rn), _stream()), "fp_learner_feed")
+                                              _ptr(rn), _lib.stream(policy.device)), "fp_learner_feed")
     if reward_normalisation:
         out["reward"] = rn
     if critic_input:
@@ -395,5 +389,5 @@ def critic_input(policy, state, action):
     B = state.shape[0]
     st = state.reshape(B, N_AGENTS * OBS).contiguous(); ac = action.reshape(B, N_AGENTS * ACT).float().contiguous()
     out = torch.empty(B * N_AGENTS, N_AGENTS * OBS + N_AGENTS + N_AGENTS * ACT, device=st.device)
-    policy._check(policy._lib.fp_learner_feed(policy._p, _ptr(st), _ptr(ac), None, B, _ptr(out), None, _stream()), "fp_learner_feed")
+    policy._check(policy._lib.fp_learner_feed(policy._p, _ptr(st), _ptr(ac), None, B, _ptr(out), None, _lib.stream(policy.device)), "fp_learner_feed")
     return out

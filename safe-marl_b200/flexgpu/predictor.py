@@ -19,10 +19,6 @@ def _ptr(t):
     return C.c_void_p(t.data_ptr()) if t is not None else None
 
 
-def _stream():
-    return C.c_void_p(torch.cuda.current_stream().cuda_stream)
-
-
 class DeviceReplayBuffer:
     """FIFO of `size` transitions; every field is a [size, width] fp32 ring on the device."""
 
@@ -37,13 +33,12 @@ class DeviceReplayBuffer:
         self._r = C.c_void_p()
         widths = (C.c_int32 * len(self.names))(*[int(self.fields[k]) for k in self.names])
         idx = self.device.index if self.device.index is not None else torch.cuda.current_device()
-        rc = self._lib.fp_replay_create(self.size, len(self.names), widths, idx, C.byref(self._r))
-        if rc != 0:
-            raise _lib.FlexGpuError(f"fp_replay_create failed ({rc}): {self._lib.fp_replay_last_error(None).decode()}")
+        self.device = torch.device("cuda", idx)
+        _lib.check(self._lib.fp_replay_create(self.size, len(self.names), widths, idx, C.byref(self._r)), None, "fp_replay_create",
+                   self._lib.fp_replay_last_error)
 
     def _check(self, rc, what):
-        if rc != 0:
-            raise _lib.FlexGpuError(f"{what} failed ({rc}): {self._lib.fp_replay_last_error(self._r).decode()}")
+        _lib.check(rc, self._r, what, self._lib.fp_replay_last_error)
 
     def close(self):
         if getattr(self, "_r", None) is not None and self._r.value:
@@ -71,7 +66,7 @@ class DeviceReplayBuffer:
     def write(self, name, pos, rows):
         f = self.names.index(name)
         rows = rows.to(device=self.device, dtype=torch.float32).contiguous().view(-1, self.fields[name])
-        self._check(self._lib.fp_replay_write(self._r, f, int(pos), rows.shape[0], _ptr(rows), _stream()), "fp_replay_write")
+        self._check(self._lib.fp_replay_write(self._r, f, int(pos), rows.shape[0], _ptr(rows), _lib.stream(self.device)), "fp_replay_write")
 
     def add_experience(self, trans):                                       # :23-27, n rows at once
         n = next(iter(trans.values())).shape[0]
@@ -91,7 +86,7 @@ class DeviceReplayBuffer:
             start = int(np.random.choice(sample_range, 1, replace=False)[0])   # the reference's draw (:18)
         out = {k: torch.empty(batch_size, w, dtype=torch.float32, device=self.device) for k, w in self.fields.items()}
         ptrs = (C.c_void_p * len(self.names))(*[out[k].data_ptr() for k in self.names])
-        self._check(self._lib.fp_replay_sample(self._r, int(start), int(batch_size), ptrs, _stream()), "fp_replay_sample")
+        self._check(self._lib.fp_replay_sample(self._r, int(start), int(batch_size), ptrs, _lib.stream(self.device)), "fp_replay_sample")
         return out
 
 
@@ -171,7 +166,7 @@ class VoltagePredictor:
             fp_ = sink.names.index(penalty_field) if penalty_field in sink.names else -1
             if pos is None:
                 pos = sink.reserve(n)
-        env._check(env._lib.fp_predict(env._h, n, _ptr(X), _ptr(vhat), _ptr(pen), r, fv, fp_, int(pos or 0), _stream()),
+        env._check(env._lib.fp_predict(env._h, n, _ptr(X), _ptr(vhat), _ptr(pen), r, fv, fp_, int(pos or 0), _lib.stream(env.device)),
                    "fp_predict")
         return vhat, pen
 

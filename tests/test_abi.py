@@ -76,3 +76,14 @@ def test_null_handle_calls_are_rejected():
     assert l.fp_step(None, None, 0, None, None, None, None, None) == -1
     assert l.fp_n_envs(None) == 0 and l.fp_launch_count(None) == 0
     assert l.fp_destroy(None) == 0
+    assert l.fp_policy_act(None, None, 0, 0, 0, None, None, None, 0, None, None, None, None, 0, 0, 1.0, 0, None) == -1
+    assert l.fp_policy_load(None, *[None] * 10) == -1 and l.fp_critic_load(None, *[None] * 8) == -1
+    assert l.fp_critic_value(None, None, 0, 0, 0, None, None, None) == -1
+    assert l.fp_policy_rows_to_ring(None, None, 0, 0, None, 0, 0, None) == -1
+    assert l.fp_learner_feed(None, None, None, None, 0, None, None, None) == -1
+    assert l.fp_policy_launch_count(None) == 0 and l.fp_policy_destroy(None) == 0
+    assert l.fp_replay_write(None, 0, 0, 0, None, None) == -1
+    assert l.fp_replay_sample(None, 0, 0, None, None) == -1
+    assert l.fp_replay_reserve(None, 0, None) == -1 and l.fp_replay_clear(None) == -1
+    assert l.fp_replay_len(None) == 0 and l.fp_replay_destroy(None) == 0
+    assert l.fp_predict(None, 0, None, None, None, None, 0, 0, 0, None) == -1
