@@ -180,11 +180,11 @@ int fp_step(FpHandle* h, const void* d_actions, int act_dtype, double* d_reward,
 
 /* HOST-buffer variant of fp_step (the end-to-end path): reads h_actions, steps, delivers
  * reward/done/info into the host arrays and synchronises the stream.  h_info may be NULL.
- * With PINNED host buffers (thread variant, fp32 actions) the step kernel works on them directly
- * (zero-copy: its asynchronous input stage pulls the next tile's actions over PCIe while the
- * current tile is swept, its bulk stores write the results into host memory) -- one launch, no
- * staging.  Otherwise (pageable memory, fp64 actions, FLEXGPU_HOST_ZEROCOPY=0) the batch is cut
- * into FLEXGPU_HOST_CHUNKS chunks that flow through copy-in / kernel / copy-out streams. */
+ * With every buffer PINNED (thread variant, FP_F32 or FP_F32_POLICY actions) the step kernel works
+ * on them directly (zero-copy: its asynchronous input stage pulls the next tile's actions over PCIe
+ * while the current tile is swept, its bulk stores write the results into host memory) -- one
+ * launch, no staging.  Otherwise (pageable memory, fp64 actions, warp variant) the actions are
+ * copied into device staging buffers, the step runs there and the results are copied back. */
 int fp_step_host(FpHandle* h, const void* h_actions, int act_dtype, double* h_reward,
                  uint8_t* h_done, double* h_info, void* stream);
 

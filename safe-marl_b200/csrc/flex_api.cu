@@ -201,13 +201,12 @@ int fp_create(const FpConfig* cfg, int64_t n_envs, int device, FpHandle** out) {
         }
         h->grid_reset = (int)((tiles < cap_reset) ? tiles : cap_reset);
         h->grid_pf = thread_kernel_max_grid(MODE_PF, h->tt.n_slots, h->shape);
-        h->stats_cap = cap_step;
-        h->stats_rows = cap_step * (1 + FP_HOST_CHUNKS);     // + one block of rows per chunk of the pipelined host path
+        h->stats_rows = cap_step;
     } else {
         h->grid_step = grid_for(n_envs, max_resident_grid(MODE_STEP));
         h->grid_reset = grid_for(n_envs, max_resident_grid(MODE_RESET));
         h->grid_pf = max_resident_grid(MODE_PF);
-        h->stats_rows = max_resident_grid(MODE_STEP); h->stats_cap = h->stats_rows;
+        h->stats_rows = max_resident_grid(MODE_STEP);
     }
     CREATE_TRY(cudaMalloc(&h->d_stats_partial, (size_t)h->stats_rows * FP_NSTATS * 8));
     CREATE_TRY(cudaMemset(h->d_stats_partial, 0, (size_t)h->stats_rows * FP_NSTATS * 8));
@@ -225,13 +224,6 @@ int fp_destroy(FpHandle* h) {
     cudaFree(h->d_pfl); cudaFree(h->d_qfl); cudaFree(h->d_isq); cudaFree(h->d_stats_partial); cudaFree(h->d_retry_mask); cudaFree(h->d_retry_count);
     cudaFree(h->d_act_stage); cudaFree(h->d_act_xlat); cudaFree(h->d_reward_stage); cudaFree(h->d_done_stage); cudaFree(h->d_info_stage);
     cudaFree(h->d_saff_At); cudaFree(h->d_saff_c);
-    for (int i = 0; i < FP_HOST_STREAMS; ++i) {
-        if (h->host_streams[i]) cudaStreamDestroy(h->host_streams[i]);
-        if (h->host_ev_out[i]) cudaEventDestroy(h->host_ev_out[i]);
-    }
-    if (h->host_ev_in) cudaEventDestroy(h->host_ev_in);
-    for (auto& g : h->host_graphs) if (g.exec) cudaGraphExecDestroy(g.exec);
-    if (h->host_origin) cudaStreamDestroy(h->host_origin);
     delete h;
     return FP_OK;
 }
@@ -419,61 +411,12 @@ int fp_step(FpHandle* h, const void* d_actions, int act_dtype, double* d_reward,
     return FP_OK;
 }
 
-// The chunk pipeline of fp_step_host, enqueued behind everything already on `st` (no synchronisation).
-static int enqueue_host_chunks(FpHandle* h, const void* h_actions, int act_dtype, double* h_reward, uint8_t* h_done,
-                               double* h_info, int n_chunks, cudaStream_t st) {
-    const size_t n = (size_t)h->n, na = (size_t)h->dc.na;
-    const size_t abpe = na * 4 * (act_dtype == FP_F64 ? 8 : 4);          // action bytes per env
-    const int64_t tiles = ((int64_t)n + 31) / 32;
-    // everything already queued on the caller's stream happens before the chunks
-    cudaStream_t s_in = h->host_streams[0], s_k = h->host_streams[1], s_out = h->host_streams[2];
-    CUDA_TRY(h, cudaEventRecord(h->host_ev_in, st));
-    for (int i = 0; i < FP_HOST_STREAMS; ++i) CUDA_TRY(h, cudaStreamWaitEvent(h->host_streams[i], h->host_ev_in, 0));
-    const int cap = h->stats_cap;                                       // statistics rows of one launch
-    const int cap_grid = cap;
-    for (int c = 0; c < n_chunks; ++c) {
-        const int64_t t0 = tiles * c / n_chunks, t1 = tiles * (c + 1) / n_chunks;
-        const size_t e0 = (size_t)t0 * 32, e1 = ((size_t)t1 * 32 < n) ? (size_t)t1 * 32 : n, ne = e1 - e0;
-        // host -> device copies run back to back on their own stream (the link never idles) ...
-        CUDA_TRY(h, cudaMemcpyAsync((char*)h->d_act_stage + e0 * abpe, (const char*)h_actions + e0 * abpe, ne * abpe,
-                                    cudaMemcpyHostToDevice, s_in));
-        CUDA_TRY(h, cudaEventRecord(h->host_ev_out[0], s_in));
-        // ... the kernel of a chunk follows its copy ...
-        CUDA_TRY(h, cudaStreamWaitEvent(s_k, h->host_ev_out[0], 0));
-        EnvParams p; fill_env_params(h, p);
-        p.actions = h->d_act_stage; p.act_f64 = (act_dtype == FP_F64);
-        if (act_dtype == FP_F32_POLICY) set_translate(h, p);
-        p.reward = h->d_reward_stage; p.done = h->d_done_stage; p.info = h_info ? h->d_info_stage : nullptr;
-        p.stats_partial = h->d_stats_partial + (size_t)(1 + c) * cap * FP_NSTATS;
-        p.tile_begin = t0; p.tile_end = t1;
-        const int grid = (int)((t1 - t0 < cap_grid) ? (t1 - t0) : cap_grid);
-        {
-            EnvParamsT pt; pt.e = p; pt.t = h->tt;
-            pt.e.bulk_io = bulk_io_ok(p);
-            CUDA_TRY(h, launch_env_t(MODE_STEP, h->shape, pt, grid, s_k));
-        }
-        h->launches++;
-        CUDA_TRY(h, cudaEventRecord(h->host_ev_out[1], s_k));
-        // ... and its results leave on the other copy engine while the next chunk computes
-        CUDA_TRY(h, cudaStreamWaitEvent(s_out, h->host_ev_out[1], 0));
-        CUDA_TRY(h, cudaMemcpyAsync(h_reward + e0, h->d_reward_stage + e0, ne * 8, cudaMemcpyDeviceToHost, s_out));
-        CUDA_TRY(h, cudaMemcpyAsync(h_done + e0, h->d_done_stage + e0, ne, cudaMemcpyDeviceToHost, s_out));
-        if (h_info) CUDA_TRY(h, cudaMemcpyAsync(h_info + e0 * FP_INFO_STRIDE, h->d_info_stage + e0 * FP_INFO_STRIDE,
-                                                ne * FP_INFO_STRIDE * 8, cudaMemcpyDeviceToHost, s_out));
-    }
-    for (int i = 0; i < FP_HOST_STREAMS; ++i) {
-        CUDA_TRY(h, cudaEventRecord(h->host_ev_out[i], h->host_streams[i]));
-        CUDA_TRY(h, cudaStreamWaitEvent(st, h->host_ev_out[i], 0));
-    }
-    return FP_OK;
-}
-
-// Host-buffer step.  The batch is cut into chunks of 32-env tiles that flow through three internal
-// streams (copy in / kernels / copy out): the host->device copies run back to back, the kernel of
-// chunk c overlaps the copy of chunk c+1 and the device->host copies of chunk c-1 (both copy
-// engines and the SMs busy at once).  Chunks touch disjoint envs and disjoint statistics rows, so
-// results are identical to one full-batch launch.  With pinned host buffers the whole pipeline is
-// one instantiated CUDA graph per buffer set.
+// Host-buffer step, on one of two routes chosen from the call itself:
+//  * zero-copy (thread variant, every buffer pinned, fp32 actions): pinned host memory is part of the unified
+//    address space, so the step kernel reads the actions of tile i+1 straight over PCIe while it sweeps tile i (its
+//    input stage is asynchronous and one tile ahead) and stores reward / done / info straight into the host
+//    buffers -- one launch, no staging.  fp64 actions are read with plain loads, not LDGSTS, so they are staged.
+//  * staged, everything else: one copy in, the step on the device staging buffers, the copies out.
 int fp_step_host(FpHandle* h, const void* h_actions, int act_dtype, double* h_reward, uint8_t* h_done,
                  double* h_info, void* stream) {
     if (!h) return FP_EINVAL;
@@ -482,19 +425,21 @@ int fp_step_host(FpHandle* h, const void* h_actions, int act_dtype, double* h_re
     if (!h_actions || !h_reward || !h_done) return fail(h, FP_EINVAL, "fp_step_host: null buffer");
     if (act_dtype != FP_F32 && act_dtype != FP_F64 && act_dtype != FP_F32_POLICY) return fail(h, FP_EINVAL, "fp_step_host: bad action dtype");
     cudaStream_t st = (cudaStream_t)stream;
-    const size_t n = (size_t)h->n, na = (size_t)h->dc.na;
-    if (!h->d_act_stage)
-        CUDA_TRY(h, alloc_group({{&h->d_act_stage, n * na * 4 * 8}, {&h->d_reward_stage, n * 8}, {&h->d_done_stage, n},
-                                 {&h->d_info_stage, n * FP_INFO_STRIDE * 8}}));
-    const size_t abpe = na * 4 * (act_dtype == FP_F64 ? 8 : 4);          // action bytes per env
-    const int64_t tiles = ((int64_t)n + 31) / 32;
-    if (h->host_chunks == 0) {
-        const char* ev = std::getenv("FLEXGPU_HOST_CHUNKS");
-        int k = ev ? std::atoi(ev) : FP_HOST_CHUNKS_DEFAULT;
-        h->host_chunks = (k < 1) ? 1 : ((k > FP_HOST_CHUNKS) ? FP_HOST_CHUNKS : k);
-    }
-    const int n_chunks = h->host_chunks;
-    if (h->variant != FP_VARIANT_THREAD || n_chunks == 1 || tiles < 4 * n_chunks) {  // small batch / warp variant: one shot
+    auto pinned = [](const void* x) {
+        cudaPointerAttributes at;
+        if (cudaPointerGetAttributes(&at, x) != cudaSuccess) { cudaGetLastError(); return false; }
+        return at.type == cudaMemoryTypeHost;
+    };
+    if (h->variant == FP_VARIANT_THREAD && act_dtype != FP_F64 &&
+        pinned(h_actions) && pinned(h_reward) && pinned(h_done) && (!h_info || pinned(h_info))) {
+        int rc = fp_step(h, h_actions, act_dtype, h_reward, h_done, h_info, nullptr, stream);
+        if (rc != FP_OK) return rc;
+    } else {
+        const size_t n = (size_t)h->n, na = (size_t)h->dc.na;
+        if (!h->d_act_stage)
+            CUDA_TRY(h, alloc_group({{&h->d_act_stage, n * na * 4 * 8}, {&h->d_reward_stage, n * 8}, {&h->d_done_stage, n},
+                                     {&h->d_info_stage, n * FP_INFO_STRIDE * 8}}));
+        const size_t abpe = na * 4 * (act_dtype == FP_F64 ? 8 : 4);          // action bytes per env
         CUDA_TRY(h, cudaMemcpyAsync(h->d_act_stage, h_actions, n * abpe, cudaMemcpyHostToDevice, st));
         int rc = fp_step(h, h->d_act_stage, act_dtype, h->d_reward_stage, h->d_done_stage,
                          h_info ? h->d_info_stage : nullptr, nullptr, stream);
@@ -502,77 +447,7 @@ int fp_step_host(FpHandle* h, const void* h_actions, int act_dtype, double* h_re
         CUDA_TRY(h, cudaMemcpyAsync(h_reward, h->d_reward_stage, n * 8, cudaMemcpyDeviceToHost, st));
         CUDA_TRY(h, cudaMemcpyAsync(h_done, h->d_done_stage, n, cudaMemcpyDeviceToHost, st));
         if (h_info) CUDA_TRY(h, cudaMemcpyAsync(h_info, h->d_info_stage, n * FP_INFO_STRIDE * 8, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(h, cudaStreamSynchronize(st));
-        return FP_OK;
     }
-    if (!h->host_ev_in) {
-        for (int i = 0; i < FP_HOST_STREAMS; ++i) {
-            CUDA_TRY(h, cudaStreamCreateWithFlags(&h->host_streams[i], cudaStreamNonBlocking));
-            CUDA_TRY(h, cudaEventCreateWithFlags(&h->host_ev_out[i], cudaEventDisableTiming));
-        }
-        CUDA_TRY(h, cudaEventCreateWithFlags(&h->host_ev_in, cudaEventDisableTiming));
-    }
-    // Pinned buffers: the whole chunk pipeline is one instantiated graph per buffer set.
-    auto pinned = [](const void* x) {
-        cudaPointerAttributes at;
-        if (cudaPointerGetAttributes(&at, x) != cudaSuccess) { cudaGetLastError(); return false; }
-        return at.type == cudaMemoryTypeHost;
-    };
-    const bool all_pinned = pinned(h_actions) && pinned(h_reward) && pinned(h_done) && (!h_info || pinned(h_info));
-    // Zero-copy: pinned host memory is part of the unified address space, so the step kernel reads the
-    // actions of tile i+1 straight over PCIe while it sweeps tile i (its input stage is asynchronous and
-    // one tile ahead) and stores reward / done / info straight into the host buffers -- no staging copies,
-    // no chunking, one launch.  (thread variant, fp32 actions: their rows are staged by LDGSTS.)
-    // FLEXGPU_HOST_ZEROCOPY: 2 (default) = inputs and outputs, 1 = inputs only, 0 = staged chunk pipeline below
-    // (measured at 131 072 envs: 294 / 310 / 310 us per step; the 10.5 MB of actions alone take 240 us by DMA)
-    static const int zc_mode = std::getenv("FLEXGPU_HOST_ZEROCOPY") ? std::atoi(std::getenv("FLEXGPU_HOST_ZEROCOPY")) : 2;
-    if (all_pinned && zc_mode > 0 && act_dtype != FP_F64) {
-        double* out_r = h_reward; uint8_t* out_d = h_done; double* out_i = h_info;
-        if (zc_mode == 1) { out_r = h->d_reward_stage; out_d = h->d_done_stage; out_i = h_info ? h->d_info_stage : nullptr; }   // inputs only
-        int rc = fp_step(h, h_actions, act_dtype, out_r, out_d, out_i, nullptr, stream);
-        if (rc != FP_OK) return rc;
-        if (zc_mode == 1) {
-            CUDA_TRY(h, cudaMemcpyAsync(h_reward, h->d_reward_stage, n * 8, cudaMemcpyDeviceToHost, st));
-            CUDA_TRY(h, cudaMemcpyAsync(h_done, h->d_done_stage, n, cudaMemcpyDeviceToHost, st));
-            if (h_info) CUDA_TRY(h, cudaMemcpyAsync(h_info, h->d_info_stage, n * FP_INFO_STRIDE * 8, cudaMemcpyDeviceToHost, st));
-        }
-        CUDA_TRY(h, cudaStreamSynchronize(st));
-        return FP_OK;
-    }
-    const bool use_graph = all_pinned && !std::getenv("FLEXGPU_NO_HOST_GRAPH");
-    if (!use_graph) {
-        int rc = enqueue_host_chunks(h, h_actions, act_dtype, h_reward, h_done, h_info, n_chunks, st);
-        if (rc != FP_OK) return rc;
-        CUDA_TRY(h, cudaStreamSynchronize(st));
-        return FP_OK;
-    }
-    struct Key { EnvParams p; const void* a; void* r; void* d; void* i; int dtype, chunks; } key;
-    std::memset(&key, 0, sizeof(key));
-    fill_env_params(h, key.p);
-    key.a = h_actions; key.r = h_reward; key.d = h_done; key.i = h_info; key.dtype = act_dtype; key.chunks = n_chunks;
-    FpHandle::HostGraph* g = nullptr;
-    for (auto& c : h->host_graphs)
-        if (c.exec && c.key.size() == sizeof(key) && std::memcmp(c.key.data(), &key, sizeof(key)) == 0) { g = &c; break; }
-    if (!g) {
-        g = &h->host_graphs[h->host_graph_next];
-        h->host_graph_next = (h->host_graph_next + 1) % FP_HOST_GRAPHS;
-        if (g->exec) { cudaGraphExecDestroy(g->exec); g->exec = nullptr; }
-        if (!h->host_origin) CUDA_TRY(h, cudaStreamCreateWithFlags(&h->host_origin, cudaStreamNonBlocking));
-        cudaGraph_t graph = nullptr;
-        CUDA_TRY(h, cudaStreamBeginCapture(h->host_origin, cudaStreamCaptureModeThreadLocal));
-        const int64_t launches0 = h->launches;
-        int rc = enqueue_host_chunks(h, h_actions, act_dtype, h_reward, h_done, h_info, n_chunks, h->host_origin);
-        h->launches = launches0;                                         // counted per graph launch below
-        cudaError_t ce = cudaStreamEndCapture(h->host_origin, &graph);
-        if (rc != FP_OK) { if (graph) cudaGraphDestroy(graph); return rc; }
-        CUDA_TRY(h, ce);
-        ce = cudaGraphInstantiate(&g->exec, graph, 0);
-        cudaGraphDestroy(graph);
-        CUDA_TRY(h, ce);
-        g->key.assign(reinterpret_cast<const char*>(&key), reinterpret_cast<const char*>(&key) + sizeof(key));
-    }
-    CUDA_TRY(h, cudaGraphLaunch(g->exec, st));
-    h->launches += n_chunks;
     CUDA_TRY(h, cudaStreamSynchronize(st));
     return FP_OK;
 }

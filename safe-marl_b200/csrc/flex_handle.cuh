@@ -3,15 +3,9 @@
 #pragma once
 #include <cstdint>
 #include <string>
-#include <vector>
 
 #include "flex_kernels.cuh"
 #include "predictor.cuh"
-
-#define FP_HOST_CHUNKS 4      // fp_step_host can pipeline the batch in up to this many chunks (copy engines || SMs)
-#define FP_HOST_STREAMS 3
-#define FP_HOST_CHUNKS_DEFAULT 4
-#define FP_HOST_GRAPHS 8
 
 struct FpHandle {
     FpConfig cfg;
@@ -38,25 +32,16 @@ struct FpHandle {
     // the full affine map of fp_safety_load_affine: A transposed [2 nb][FP_MAX_BUS], c [nb]
     double *d_saff_At = nullptr, *d_saff_c = nullptr, saff_vmin = 0, saff_vmax = 0, saff_w = 0; int saff_loaded = 0;
     uint8_t* d_retry_mask = nullptr; void* d_retry_count = nullptr;     // fp_reset_random_retry: device-built retry mask
-    int stats_rows = 0, stats_cap = 0;     // rows of one launch's statistics block
+    int stats_rows = 0;          // rows of the statistics block: the step kernel's grid cap
     const uint8_t* d_inject = nullptr;
     int keep_flows = 0;
     // staging for the host-buffer entry points
     void* d_act_stage = nullptr; float* d_act_xlat = nullptr; double* d_reward_stage = nullptr; uint8_t* d_done_stage = nullptr;
     double* d_info_stage = nullptr;
     int grid_step = 0, grid_reset = 0, grid_pf = 0, grid_obs = 0;
-    cudaStream_t host_streams[FP_HOST_STREAMS] = {nullptr, nullptr, nullptr};
-    cudaEvent_t host_ev_in = nullptr, host_ev_out[FP_HOST_STREAMS] = {nullptr, nullptr, nullptr};
     int fuse_obs = 0;            // set around the fp_step of fp_step_obs: the step kernel pushes the observation
     int keep_hist = 1;           // fp_set_obs_history: 0 = the fused ring step does not maintain the fp64 history ring
     bool hist_valid = true;      // false after a ring-only step: restored from the env-minor ring on demand (hist_ensure)
-    int host_chunks = 0;         // 0 = not decided yet (FLEXGPU_HOST_CHUNKS or the default)
-    // the chunk pipeline of fp_step_host as instantiated CUDA graphs, one per set of (pinned) host
-    // buffers: one launch per step instead of five API calls per chunk
-    cudaStream_t host_origin = nullptr;
-    struct HostGraph { cudaGraphExec_t exec = nullptr; std::vector<char> key; };
-    HostGraph host_graphs[FP_HOST_GRAPHS];
-    int host_graph_next = 0;
     int64_t launches = 0;
     std::string err;
     PredictorState pred;

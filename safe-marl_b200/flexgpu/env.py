@@ -313,6 +313,9 @@ class BatchedFlexProvisionEnv:
 
     def step_host(self, actions, want_info=False, translate=False):
         """End-to-end variant: host (numpy, ideally pinned) in, host out, through fp_step_host.
+        Pinned fp32 actions (thread variant) are read by the step kernel straight from host memory, and the
+        results are written straight into the pinned output buffers (zero-copy).  Pageable or fp64 actions
+        are copied through device staging buffers.  The outputs are the same either way.
         translate: see step()."""
         a = np.ascontiguousarray(actions)
         if translate:
