@@ -309,6 +309,25 @@ int fp_predictor_load(FpHandle* h, int32_t n_in, int32_t n_out, const double* h_
 int fp_predict(FpHandle* h, int64_t n, const float* d_X, float* d_vhat, double* d_penalty, FpReplay* sink,
                int32_t f_vhat, int32_t f_penalty, int64_t pos, void* stream);
 
+/* The same predictor as a scikit-learn MLPRegressor: 1..3 hidden layers of width 1..128 sharing one activation,
+ * identity output layer.  n_layers = hidden layers + 1 (2..4); h_widths[n_layers + 1] = {66, hidden..., 33};
+ * h_W = the layers' [out][in] row-major fp64 matrices concatenated, h_b = their biases concatenated (host, copied;
+ * the caller folds the MinMax scalers into the first and last layer).  The model is held in its own slot of the
+ * handle: loading it does not evict the fp_predictor_load model.  The split-TF32 weights stay in shared memory, so a
+ * model is accepted only if they, the output staging and two 33 KB X staging buffers fit the 227 KB of one block, and
+ * its TMEM plan fits 512 columns; otherwise, and for bad widths, non-finite weights, an unknown activation,
+ * v_min >= v_max or slack_weight <= 0, FP_EINVAL with a message. */
+#define FP_ACT_IDENTITY 0
+#define FP_ACT_RELU 1
+#define FP_ACT_TANH 2
+#define FP_ACT_LOGISTIC 3
+int fp_predictor_load_mlp(FpHandle* h, int32_t n_layers, const int32_t* h_widths, const double* h_W, const double* h_b,
+                          int32_t activation, double v_min, double v_max, double slack_weight);
+/* fp_predict's contract (outputs, replay sink, field checks, 16-byte-aligned X) for the model of
+ * fp_predictor_load_mlp; FP_ESTATE before it. */
+int fp_predict_mlp(FpHandle* h, int64_t n, const float* d_X, float* d_vhat, double* d_penalty, FpReplay* sink,
+                   int32_t f_vhat, int32_t f_penalty, int64_t pos, void* stream);
+
 /* -- safety layer as a batched projection (SURVEY 8f rank 4) ------------------------------- */
 
 /* Replaces SAFEMADDPG.safety_layer_optimization (madrl/models/safemaddpg.py:176-299: a Pyomo QP solved by Gurobi per

@@ -219,6 +219,7 @@ int fp_destroy(FpHandle* h) {
     if (!h) return FP_OK;
     const DeviceGuard on_device(h->device);       // best effort: the handle is freed whatever happens
     predictor_free(&h->pred);
+    mlp_free(&h->mlp);
     cudaFree(h->d_topo); cudaFree(h->d_P); cudaFree(h->d_Q); cudaFree(h->d_PVP); cudaFree(h->d_PQD); cudaFree(h->d_OBS);
     cudaFree(h->d_rec); cudaFree(h->d_V); cudaFree(h->d_setp); cudaFree(h->d_hist); cudaFree(h->d_obsm); cudaFree(h->d_obsr);
     cudaFree(h->d_pfl); cudaFree(h->d_qfl); cudaFree(h->d_isq); cudaFree(h->d_stats_partial); cudaFree(h->d_retry_mask); cudaFree(h->d_retry_count);

@@ -45,4 +45,5 @@ struct FpHandle {
     int64_t launches = 0;
     std::string err;
     PredictorState pred;
+    MlpState mlp;                // fp_predictor_load_mlp: its own slot, next to the affine model
 };

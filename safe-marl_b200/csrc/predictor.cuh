@@ -23,6 +23,19 @@ struct PredictorState {
 
 void predictor_free(PredictorState* p);
 
+// The MLP of fp_predictor_load_mlp: split weights in the kernel's shared-memory image, padded biases, and the plan.
+struct MlpState {
+    int loaded = 0;
+    float* d_W = nullptr;      // per layer [2 (hi, lo)][k_pad / 4][n_pad][4], UMMA K-major layout
+    float* d_bias = nullptr;   // per layer [n_pad]
+    int n_layers = 0, act = 0, n_stages = 0, h_cols = 0, n_bias = 0;
+    int k_pad[4] = {0, 0, 0, 0}, n_pad[4] = {0, 0, 0, 0}, b_off[4] = {0, 0, 0, 0};
+    uint32_t w_off[4] = {0, 0, 0, 0}, w_bytes = 0, smem_bytes = 0;
+    double v_min = 0.0, v_max = 0.0, slack_weight = 0.0;
+};
+
+void mlp_free(MlpState* m);
+
 struct FpReplay {
     int64_t capacity = 0, head = 0, len = 0;
     int device = 0;

@@ -101,6 +101,12 @@ __device__ __forceinline__ void tmem_st4(uint32_t taddr, float a, float b, float
     asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};"
                  ::"r"(taddr), "r"(__float_as_uint(a)), "r"(__float_as_uint(b)), "r"(__float_as_uint(c)), "r"(__float_as_uint(d)) : "memory");
 }
+// x rounded to the nearest TF32 value (ties away from zero), in fp32 format with the low 13 mantissa bits zero
+__device__ __forceinline__ float tf32_rna(float x) {
+    uint32_t r;
+    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
+    return __uint_as_float(r);
+}
 // TMEM loads (32x32b: lane = row, one 32-bit column per register); the values are valid after tmem_wait_ld()
 __device__ __forceinline__ void tmem_ld1(uint32_t taddr, float& v) {
     uint32_t r;

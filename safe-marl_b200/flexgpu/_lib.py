@@ -21,6 +21,8 @@ FP_REC_STRIDE = 16
 FP_F32, FP_F64, FP_F32_POLICY = 0, 1, 2
 VARIANT_THREAD, VARIANT_WARP = 0, 1
 VARIANTS = {"thread": VARIANT_THREAD, "warp": VARIANT_WARP}
+# MLP activations (include/flexgpu.h FP_ACT_*), by scikit-learn's names
+ACTIVATIONS = {"identity": 0, "relu": 1, "tanh": 2, "logistic": 3}
 
 # record slots (include/flexgpu.h FP_REC_*)
 REC_E_INIT, REC_E_CUR, REC_CUM, REC_TIME, REC_HIST, REC_VMASK, REC_COUNTS, REC_LINES = 0, 5, 10, 11, 12, 13, 14, 15
@@ -97,6 +99,8 @@ _PROTOS = {
     "fp_replay_field_ptr": (C.c_int, [_P, C.c_int32, C.POINTER(_P)]),
     "fp_predictor_load": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, C.c_double, C.c_double, C.c_double]),
     "fp_predict": (C.c_int, [_P, C.c_int64, _P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int64, _P]),
+    "fp_predictor_load_mlp": (C.c_int, [_P, C.c_int32, _P, _P, _P, C.c_int32, C.c_double, C.c_double, C.c_double]),
+    "fp_predict_mlp": (C.c_int, [_P, C.c_int64, _P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int64, _P]),
     "fp_safety_load": (C.c_int, [_P, _P, _P, C.c_double, C.c_double, C.c_double]),
     "fp_safety_project": (C.c_int, [_P, _P, C.c_int, _P, C.c_int32, _P, _P, _P]),
     "fp_safety_load_affine": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, C.c_double, C.c_double, C.c_double]),

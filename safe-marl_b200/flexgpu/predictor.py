@@ -4,6 +4,9 @@ VoltagePredictor   batched `model.predict` of the reference's regressor
                    (safety_signal/train_safety_signal_model.py:33-46,73: MinMaxScaler on X and Y +
                    MultiOutputRegressor(LinearRegression), 66 -> 33) plus the safety layer's slack
                    penalty (madrl/models/safemaddpg.py:205-229), through fp_predict.
+MLPVoltagePredictor the same for a scikit-learn MLPRegressor swapped in for the regressor (1..3 hidden
+                   layers of width <= 128), through fp_predict_mlp; mlp_from_sklearn / fold_minmax turn the
+                   fitted model and its scalers into the raw-input layers it loads.
 DeviceReplayBuffer TransReplayBuffer (utils/replay_buffer.py:3-30) as a struct-of-arrays fp32 ring
                    on the device, through fp_replay_*.
 """
@@ -168,6 +171,102 @@ class VoltagePredictor:
                 pos = sink.reserve(n)
         env._check(env._lib.fp_predict(env._h, n, _ptr(X), _ptr(vhat), _ptr(pen), r, fv, fp_, int(pos or 0), _lib.stream(env.device)),
                    "fp_predict")
+        return vhat, pen
+
+
+def mlp_from_sklearn(model, scaler_x=None, scaler_y=None):
+    """A fitted MLPRegressor -> (weights [out, in] per layer, biases per layer, activation), fp64, with the MinMax
+    scalers (if given) folded into the first and last layer so that the layers act on raw inputs in p.u."""
+    if getattr(model, "out_activation_", "identity") != "identity":
+        raise ValueError(f"MLPRegressor output activation {model.out_activation_!r}: only 'identity' is supported")
+    if model.activation not in _lib.ACTIVATIONS:
+        raise ValueError(f"unknown activation {model.activation!r}")
+    W = [np.asarray(c, dtype=np.float64).T.copy() for c in model.coefs_]          # sklearn holds [in, out]
+    b = [np.asarray(c, dtype=np.float64).copy() for c in model.intercepts_]
+    if scaler_x is not None or scaler_y is not None:
+        W, b = fold_minmax(W, b, None if scaler_x is None else scaler_x.scale_, None if scaler_x is None else scaler_x.min_,
+                           None if scaler_y is None else scaler_y.scale_, None if scaler_y is None else scaler_y.min_)
+    return W, b, model.activation
+
+def fold_minmax(weights, biases, x_scale=None, x_min=None, y_scale=None, y_min=None):
+    """Folds x_s = x * x_scale + x_min into layer 1 and y = (y_s - y_min) / y_scale into the last layer (sklearn
+    MinMaxScaler.scale_ / min_, train_safety_signal_model.py:34-37), in fp64, as from_linear_model does for the
+    affine map.  Returns new lists; the inputs are not changed."""
+    W = [np.asarray(w, dtype=np.float64) for w in weights]
+    b = [np.asarray(c, dtype=np.float64) for c in biases]
+    if x_scale is not None:
+        sx = np.asarray(x_scale, dtype=np.float64)
+        mx = np.zeros_like(sx) if x_min is None else np.asarray(x_min, dtype=np.float64)
+        W[0], b[0] = W[0] * sx[None, :], W[0] @ mx + b[0]
+    if y_scale is not None:
+        sy = np.asarray(y_scale, dtype=np.float64)
+        my = np.zeros_like(sy) if y_min is None else np.asarray(y_min, dtype=np.float64)
+        W[-1], b[-1] = W[-1] / sy[:, None], (b[-1] - my) / sy
+    return W, b
+
+
+class MLPVoltagePredictor:
+    """Vhat = MLP(x) on raw interleaved inputs x = [P1, Q1, ..., P33, Q33]: hidden layers act(W h + b) with one
+    activation (identity, relu, tanh, logistic), identity output layer; weights [out, in] per layer.  predict() has
+    VoltagePredictor.predict's signature and returns, so either can serve a caller."""
+
+    def __init__(self, env, weights, biases, activation="relu", v_min=None, v_max=None, slack_weight=1000.0):
+        self.env = env
+        self.weights = [np.ascontiguousarray(w, dtype=np.float64) for w in weights]
+        self.biases = [np.ascontiguousarray(c, dtype=np.float64).reshape(-1) for c in biases]
+        if len(self.weights) != len(self.biases):
+            raise ValueError("one bias vector per weight matrix")
+        if activation not in _lib.ACTIVATIONS:
+            raise ValueError(f"unknown activation {activation!r} (one of {sorted(_lib.ACTIVATIONS)})")
+        self.activation = activation
+        self.widths = [self.weights[0].shape[1]] + [w.shape[0] for w in self.weights]
+        for l, w in enumerate(self.weights):
+            if w.shape != (self.widths[l + 1], self.widths[l]) or self.biases[l].shape != (self.widths[l + 1],):
+                raise ValueError(f"layer {l}: weights [out, in] and biases [out] do not chain")
+        self.n_in, self.n_out = self.widths[0], self.widths[-1]
+        self.v_min = float(env.args_dict["v_min"] if v_min is None else v_min)
+        self.v_max = float(env.args_dict["v_max"] if v_max is None else v_max)
+        self.slack_weight = float(slack_weight)
+        self._load()
+
+    def _load(self):
+        """The handle's MLP slot holds ONE model (fp_predictor_load_mlp), separate from the affine model of
+        VoltagePredictor; each MLPVoltagePredictor reloads its weights when it is not the resident one."""
+        env = self.env
+        widths = (C.c_int32 * len(self.widths))(*self.widths)
+        W = np.concatenate([w.reshape(-1) for w in self.weights])
+        b = np.concatenate(self.biases)
+        env._check(env._lib.fp_predictor_load_mlp(env._h, len(self.weights), widths, W.ctypes.data_as(C.c_void_p),
+                                                  b.ctypes.data_as(C.c_void_p), _lib.ACTIVATIONS[self.activation],
+                                                  self.v_min, self.v_max, self.slack_weight), "fp_predictor_load_mlp")
+        env._resident_mlp = self
+
+    @classmethod
+    def from_sklearn(cls, env, model, scaler_x=None, scaler_y=None, **kw):
+        W, b, act = mlp_from_sklearn(model, scaler_x, scaler_y)
+        return cls(env, W, b, activation=act, **kw)
+
+    def predict(self, X, want_vhat=True, want_penalty=True, sink=None, vhat_field="v_pred",
+                penalty_field="safety_penalty", pos=None):
+        """X [n, 66] fp32 on the device -> (Vhat [n, 33] fp32, penalty [n] fp64), as VoltagePredictor.predict."""
+        env = self.env
+        if getattr(env, "_resident_mlp", None) is not self:
+            self._load()
+        X = X.to(device=env.device, dtype=torch.float32).contiguous()
+        n = X.shape[0]
+        if X.dim() != 2 or X.shape[1] != self.n_in:
+            raise ValueError("X must be [n, 66]")
+        vhat = torch.empty(n, self.n_out, dtype=torch.float32, device=env.device) if want_vhat else None
+        pen = torch.empty(n, dtype=torch.float64, device=env.device) if want_penalty else None
+        r, fv, fp_ = None, -1, -1
+        if sink is not None:
+            r = sink._r
+            fv = sink.names.index(vhat_field) if vhat_field in sink.names else -1
+            fp_ = sink.names.index(penalty_field) if penalty_field in sink.names else -1
+            if pos is None:
+                pos = sink.reserve(n)
+        env._check(env._lib.fp_predict_mlp(env._h, n, _ptr(X), _ptr(vhat), _ptr(pen), r, fv, fp_, int(pos or 0),
+                                           _lib.stream(env.device)), "fp_predict_mlp")
         return vhat, pen
 
 
