@@ -178,6 +178,20 @@ int fp_reset_random_retry(FpHandle* h, uint64_t seed, int64_t env_offset, const 
 int fp_step(FpHandle* h, const void* d_actions, int act_dtype, double* d_reward,
             uint8_t* d_done, double* d_info, const uint8_t* d_mask, void* stream);
 
+/* "What would this action do?": what fp_step would compute for k candidate actions per env, bit for bit, WITHOUT
+ * committing it.  d_actions[k][N][na*4] of dtype act_dtype (as fp_step, FP_F32_POLICY included); outputs per
+ * (candidate, env): d_reward[k][N] fp64, d_done[k][N] uint8, d_info[k][N][FP_INFO_STRIDE] fp64, d_voltage[k][N][n_bus]
+ * fp64 (the voltages fp_step would leave behind: after a failed solve, the rolled-back ones), d_vmask[k][N] uint64
+ * (the violation mask it would leave in the record); d_info, d_voltage and d_vmask may be NULL.  Candidate c of env e
+ * sees env e's current state: the row in force, E_init / E_cur, the episode step and the failure-injection mask of
+ * fp_inject_failure.  A failed solve (NaN action included) is reported as fp_step reports it: -200, solver_failed, done.
+ * Nothing of the handle is written -- records, voltages, setpoints, line flows, observation history and rings, episode
+ * statistics -- so previews may be issued any number of times between two steps, and a step after them gives the
+ * same bits as a step without them.  FP_EINVAL for a null actions / reward / done, k < 1 or an unknown dtype;
+ * FP_ESTATE before fp_load_profiles. */
+int fp_step_preview(FpHandle* h, int32_t k, const void* d_actions, int act_dtype, double* d_reward, uint8_t* d_done,
+                    double* d_info, double* d_voltage, uint64_t* d_vmask, void* stream);
+
 /* HOST-buffer variant of fp_step (the end-to-end path): reads h_actions, steps, delivers
  * reward/done/info into the host arrays and synchronises the stream.  h_info may be NULL.
  * With every buffer PINNED (thread variant, FP_F32 or FP_F32_POLICY actions) the step kernel works

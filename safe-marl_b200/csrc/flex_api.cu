@@ -224,6 +224,7 @@ int fp_destroy(FpHandle* h) {
     cudaFree(h->d_rec); cudaFree(h->d_V); cudaFree(h->d_setp); cudaFree(h->d_hist); cudaFree(h->d_obsm); cudaFree(h->d_obsr);
     cudaFree(h->d_pfl); cudaFree(h->d_qfl); cudaFree(h->d_isq); cudaFree(h->d_stats_partial); cudaFree(h->d_retry_mask); cudaFree(h->d_retry_count);
     cudaFree(h->d_act_stage); cudaFree(h->d_act_xlat); cudaFree(h->d_reward_stage); cudaFree(h->d_done_stage); cudaFree(h->d_info_stage);
+    cudaFree(h->d_prev_xlat);
     cudaFree(h->d_saff_At); cudaFree(h->d_saff_c);
     delete h;
     return FP_OK;
@@ -408,6 +409,52 @@ int fp_step(FpHandle* h, const void* d_actions, int act_dtype, double* d_reward,
     p.stats_partial = h->d_stats_partial;
     if (h->fuse_obs) { p.obs_push = 1; p.obs_q = h->ring_q; p.hist = h->keep_hist ? h->d_hist : nullptr; p.obsr = h->d_obsr; p.n_pad = h->n_pad; }
     CUDA_TRY(h, launch_env_any(h, MODE_STEP, p, (cudaStream_t)stream));
+    h->launches++;
+    return FP_OK;
+}
+
+// The step's computation for k candidate actions per env, without committing it: one launch of the step kernel's
+// MODE_PREVIEW instantiation over k N virtual envs (see k_env_t).  It reads the handle's state and writes only the
+// caller's buffers, so any number of previews may run between two steps.
+int fp_step_preview(FpHandle* h, int32_t k, const void* d_actions, int act_dtype, double* d_reward, uint8_t* d_done,
+                    double* d_info, double* d_voltage, uint64_t* d_vmask, void* stream) {
+    if (!h) return FP_EINVAL;
+    USE_DEVICE(h);
+    if (!h->d_P) return fail(h, FP_ESTATE, "fp_step_preview: call fp_load_profiles first");
+    if (!d_actions || !d_reward || !d_done) return fail(h, FP_EINVAL, "fp_step_preview: null input/output");
+    if (k < 1) return fail(h, FP_EINVAL, "fp_step_preview: k must be >= 1");
+    if (act_dtype != FP_F32 && act_dtype != FP_F64 && act_dtype != FP_F32_POLICY) return fail(h, FP_EINVAL, "fp_step_preview: bad action dtype");
+    cudaStream_t st = (cudaStream_t)stream;
+    const int64_t n_virt = h->n * k;
+    EnvParams p; fill_env_params(h, p);
+    p.pv_V = d_voltage; p.pv_vmask = d_vmask; p.pv_k = k;            // (replaces the line-flow dump, which a preview never writes)
+    p.actions = d_actions; p.act_f64 = (act_dtype == FP_F64);
+    if (act_dtype == FP_F32_POLICY) {
+        if (h->variant == FP_VARIANT_THREAD) set_translate(h, p);      // fused, as in fp_step
+        else {                                                                     // the same elementwise pre-pass as fp_step
+            const int64_t cnt = n_virt * h->dc.na * 4;
+            if (cnt > h->prev_xlat_cap) {
+                cudaFree(h->d_prev_xlat); h->d_prev_xlat = nullptr; h->prev_xlat_cap = 0;
+                CUDA_TRY(h, cudaMalloc(&h->d_prev_xlat, (size_t)cnt * 4));
+                h->prev_xlat_cap = cnt;
+            }
+            EnvParams t; set_translate(h, t);
+            CUDA_TRY(h, launch_translate_actions((const float*)d_actions, h->d_prev_xlat, cnt, t.act_lo, t.act_hi, t.act_span, st));
+            h->launches++;
+            p.actions = h->d_prev_xlat;
+        }
+    }
+    p.reward = d_reward; p.done = d_done; p.info = d_info;
+    if (h->variant == FP_VARIANT_THREAD) {                            // the resident grid of the preview kernel, tiles of 32 envs
+        if (!h->cap_preview) h->cap_preview = thread_kernel_max_grid(MODE_PREVIEW, h->tt.n_slots, h->shape);
+        EnvParamsT pt;
+        pt.e = p; pt.t = h->tt;
+        const int64_t tiles = k * ((h->n + 31) / 32);
+        CUDA_TRY(h, launch_env_t(MODE_PREVIEW, h->shape, pt, (int)((tiles < h->cap_preview) ? tiles : h->cap_preview), st));
+    } else {                                                          // one warp per virtual env
+        if (!h->cap_preview) h->cap_preview = max_resident_grid(MODE_PREVIEW);
+        CUDA_TRY(h, launch_env(MODE_PREVIEW, p, grid_for(n_virt, h->cap_preview), st));
+    }
     h->launches++;
     return FP_OK;
 }

@@ -38,6 +38,8 @@ struct FpHandle {
     // staging for the host-buffer entry points
     void* d_act_stage = nullptr; float* d_act_xlat = nullptr; double* d_reward_stage = nullptr; uint8_t* d_done_stage = nullptr;
     double* d_info_stage = nullptr;
+    float* d_prev_xlat = nullptr; int64_t prev_xlat_cap = 0;          // fp_step_preview: translated candidates (warp variant)
+    int cap_preview = 0;         // fp_step_preview: resident grid of its kernel (0: not queried yet)
     int grid_step = 0, grid_reset = 0, grid_pf = 0, grid_obs = 0;
     int fuse_obs = 0;            // set around the fp_step of fp_step_obs: the step kernel pushes the observation
     int keep_hist = 1;           // fp_set_obs_history: 0 = the fused ring step does not maintain the fp64 history ring

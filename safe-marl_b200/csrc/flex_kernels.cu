@@ -2,6 +2,7 @@
 //
 //   k_env<STEP>   replaces FlexibilityProvisionEnv.step           (flexibility_provision_env.py:241-356)
 //   k_env<RESET>  replaces reset()/manual_reset()                  (:74-155, :157-239)
+//   k_env<PREVIEW> what k_env<STEP> computes for K candidate actions per env, without committing any of it
 //   k_power_flow  replaces power_flow_solver_simplified, batched   (utils/pf.py:115-192)
 //   k_obs         replaces get_obs() incl. its history side effect (:370-403)
 //   k_state       replaces get_state()                             (:358-368)
@@ -22,6 +23,8 @@ constexpr int SCRATCH_DOUBLES = 32;   // per-warp shared scratch
 
 template <int MODE>
 __global__ void __launch_bounds__(FP_CTA_THREADS) k_env(const EnvParams prm) {
+    // STEP and PREVIEW (MODE != MODE_RESET) share every stage up to the outputs; a preview walks K N virtual envs
+    // v = k N + e, reads the state of env e and the actions of v, and writes outputs of v only
     __shared__ DevTopo s_topo;
     __shared__ double s_scratch[WARPS_PER_CTA][SCRATCH_DOUBLES];
     __shared__ double s_stats[WARPS_PER_CTA][FP_NSTATS];
@@ -39,7 +42,9 @@ __global__ void __launch_bounds__(FP_CTA_THREADS) k_env(const EnvParams prm) {
     double stat_acc = 0.0;                                 // lane j < FP_NSTATS accumulates stat j
 
     const int64_t warps_total = (int64_t)gridDim.x * WARPS_PER_CTA;
-    for (int64_t e = (int64_t)blockIdx.x * WARPS_PER_CTA + warp; e < prm.n; e += warps_total) {
+    const int64_t n_virt = (MODE == MODE_PREVIEW) ? prm.n * prm.pv_k : prm.n;
+    for (int64_t v = (int64_t)blockIdx.x * WARPS_PER_CTA + warp; v < n_virt; v += warps_total) {
+        const int64_t e = (MODE == MODE_PREVIEW) ? v % prm.n : v;
         if (prm.mask != nullptr && prm.mask[e] == 0) continue;          // warp-uniform
 
         uint64_t* rec = prm.rec + e * FP_REC_STRIDE;
@@ -48,7 +53,7 @@ __global__ void __launch_bounds__(FP_CTA_THREADS) k_env(const EnvParams prm) {
         double e_init = 0.0, e_cur = 0.0, cum = 0.0;
         double a0, a1, a2, a3;
         a0 = a1 = a2 = a3 = 0.0;
-        if (MODE == MODE_STEP) {
+        if (MODE != MODE_RESET) {
             uint64_t tm = rec[FP_REC_TIME];                              // broadcast load
             start = (int32_t)(uint32_t)tm;
             steps = (int32_t)(tm >> 32);
@@ -56,11 +61,11 @@ __global__ void __launch_bounds__(FP_CTA_THREADS) k_env(const EnvParams prm) {
                 e_init = __longlong_as_double((long long)rec[FP_REC_E_INIT + lane]);
                 e_cur = __longlong_as_double((long long)rec[FP_REC_E_CUR + lane]);
                 if (prm.act_f64) {
-                    const double* a = reinterpret_cast<const double*>(prm.actions) + (e * na + lane) * 4;
+                    const double* a = reinterpret_cast<const double*>(prm.actions) + (v * na + lane) * 4;
                     a0 = a[0]; a1 = a[1]; a2 = a[2]; a3 = a[3];
                 } else {
                     // fp32 actions are widened exactly (SURVEY quirk Q6)
-                    float4 a = reinterpret_cast<const float4*>(prm.actions)[e * na + lane];
+                    float4 a = reinterpret_cast<const float4*>(prm.actions)[v * na + lane];
                     a0 = (double)a.x; a1 = (double)a.y; a2 = (double)a.z; a3 = (double)a.w;
                 }
             }
@@ -104,7 +109,7 @@ __global__ void __launch_bounds__(FP_CTA_THREADS) k_env(const EnvParams prm) {
 
         // ---------------------------------------------------------------- gather the profile row
         // Quirk Q1: the row in force is max(steps-1, 1); the row loaded after the solve is `steps`.
-        const int64_t row = (int64_t)start + ((MODE == MODE_STEP && steps > 1) ? min(steps - 1, c.episode_limit + c.history) : 1);
+        const int64_t row = (int64_t)start + ((MODE != MODE_RESET && steps > 1) ? min(steps - 1, c.episode_limit + c.history) : 1);
         double pl = 0.0, ql = 0.0;
         if (lane < nl) {
             pl = __ldg(prm.P + row * nl + my_col);
@@ -145,14 +150,14 @@ __global__ void __launch_bounds__(FP_CTA_THREADS) k_env(const EnvParams prm) {
             e_next = e_init + c.delta_t * (c.eta_ch * sp.ch - c.inv_eta_dis * sp.dis);
             e_bad = e_next < c.e_next_lb;                                // E_next in NonNegativeReals (pf.py:46)
             // a NaN action: np.clip keeps it, the reference's NLP gets a NaN injection and its solve raises (:314-337)
-            if (MODE == MODE_STEP) e_bad = e_bad || (a0 != a0) || (a1 != a1) || (a2 != a2) || (a3 != a3);
+            if (MODE != MODE_RESET) e_bad = e_bad || (a0 != a0) || (a1 != a1) || (a2 != a2) || (a3 != a3);
         }
         const bool ok = sw.ok && !__any_sync(FULL, e_bad);              // warp-uniform
 
         // ---------------------------------------------------------------- voltages, masks
         double V = sqrt(sw.v);                                           // pf.py:108
         double* Vrow = prm.V + e * c.nb;
-        if (ok) {
+        if (ok && MODE != MODE_PREVIEW) {
             if (lane < nl) Vrow[my_col + 1] = V;
             if (lane == 0) Vrow[0] = 1.0;                                // slack: sqrt(Vsqr = 1), pf.py:51-53
             if (prm.pfl != nullptr && lane < nl) {
@@ -160,7 +165,7 @@ __global__ void __launch_bounds__(FP_CTA_THREADS) k_env(const EnvParams prm) {
                 prm.qfl[e * nl + my_col] = sw.Q;
                 prm.isq[e * nl + my_col] = sw.ell;
             }
-        } else if (MODE == MODE_STEP) {
+        } else if (MODE == MODE_STEP || (MODE == MODE_PREVIEW && !ok)) {
             // roll back to the last valid state (:318-328): voltages and setpoints
             if (lane < nl) V = Vrow[my_col + 1];
             if (lane < na) {
@@ -168,6 +173,11 @@ __global__ void __launch_bounds__(FP_CTA_THREADS) k_env(const EnvParams prm) {
                 sp.pred = sprow[0 * na + lane]; sp.ch = sprow[1 * na + lane];
                 sp.dis = sprow[2 * na + lane]; sp.qpv = sprow[3 * na + lane];
             }
+        }
+        if (MODE == MODE_PREVIEW && prm.pv_V != nullptr) {             // what env.voltages would hold after the step
+            double* out = prm.pv_V + v * c.nb;
+            if (lane < nl) out[my_col + 1] = V;
+            if (lane == 0) out[0] = ok ? 1.0 : Vrow[0];
         }
         const double over = V - c.v_max, under = c.v_min - V;
         const bool viol = (lane < nl) && ((over > 0.0) || (under > 0.0));
@@ -179,7 +189,7 @@ __global__ void __launch_bounds__(FP_CTA_THREADS) k_env(const EnvParams prm) {
         const bool lviol = (lane < nl) && ok && (sw.ell > s_topo.imax2[lane]);       // utils/opf.py:124-126
         const uint32_t lm = __reduce_or_sync(FULL, lviol ? (1u << my_col) : 0u);
 
-        if (MODE == MODE_STEP) {
+        if (MODE != MODE_RESET) {
             // ------------------------------------------------------------ reward (:679-706)
             double vpen = warp_sum_xor(vterm) + c.slack_pen;
             if (lane < na) {
@@ -216,15 +226,20 @@ __global__ void __launch_bounds__(FP_CTA_THREADS) k_env(const EnvParams prm) {
             const bool done = (steps_new >= c.episode_limit) || !ok;              // :345-348
             if (lane < FP_INFO_STRIDE) {
                 double iv = scratch[24 + lane];
-                if (prm.info != nullptr) prm.info[e * FP_INFO_STRIDE + lane] = iv;
+                if (prm.info != nullptr) prm.info[v * FP_INFO_STRIDE + lane] = iv;
                 stat_acc += iv;                     // slots 0..6 info sums, 7 failures
             } else if (lane == 8) stat_acc += (double)vcount;
             else if (lane == 9) stat_acc += 1.0;
             else if (lane == 10) stat_acc += done ? 1.0 : 0.0;
             else if (lane == 11) stat_acc += (double)__popc(lm);
             if (lane == 0) {
-                prm.reward[e] = reward;
-                prm.done[e] = done ? 1 : 0;
+                prm.reward[v] = reward;
+                prm.done[v] = done ? 1 : 0;
+            }
+            if (MODE == MODE_PREVIEW) {
+                if (lane == 13 && prm.pv_vmask != nullptr) prm.pv_vmask[v] = vmask;
+                __syncwarp();                                                     // scratch is reused by the next env
+                continue;
             }
             // ------------------------------------------------------------ write back
             // success: E_cur <- E_next; failure: E_cur stays (rolled back). E_init <- E_cur (:354).
@@ -669,6 +684,7 @@ __global__ void k_pack_pvp(const double* __restrict__ pv, const double* __restri
 // ------------------------------------------------------------------------ launchers
 cudaError_t launch_env(int mode, const EnvParams& prm, int grid, cudaStream_t st) {
     if (mode == MODE_STEP) k_env<MODE_STEP><<<grid, FP_CTA_THREADS, 0, st>>>(prm);
+    else if (mode == MODE_PREVIEW) k_env<MODE_PREVIEW><<<grid, FP_CTA_THREADS, 0, st>>>(prm);
     else k_env<MODE_RESET><<<grid, FP_CTA_THREADS, 0, st>>>(prm);
     return cudaGetLastError();
 }
@@ -876,6 +892,7 @@ int max_resident_grid(int mode) {
     cudaError_t err;
     if (mode == MODE_STEP) err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_env<MODE_STEP>, FP_CTA_THREADS, 0);
     else if (mode == MODE_RESET) err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_env<MODE_RESET>, FP_CTA_THREADS, 0);
+    else if (mode == MODE_PREVIEW) err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_env<MODE_PREVIEW>, FP_CTA_THREADS, 0);
     else err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_power_flow, FP_CTA_THREADS, 0);
     if (err != cudaSuccess || per_sm < 1) per_sm = 1;
     return per_sm * sms;

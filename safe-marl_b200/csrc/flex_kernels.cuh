@@ -12,7 +12,9 @@
 #define FP_OBS_PV 10
 #define FP_OBS_PRICE 15
 
-enum { MODE_STEP = 0, MODE_RESET = 1, MODE_PF = 2 };
+// MODE_PREVIEW: the step's computation for K candidate actions per env, written to caller buffers; the env's state
+// (records, voltages, setpoints, flows, observation rings, statistics) is read and never written (fp_step_preview)
+enum { MODE_STEP = 0, MODE_RESET = 1, MODE_PF = 2, MODE_PREVIEW = 3 };
 
 // fp64 history ring: one slot = the agents' 6-vectors (<= 30 doubles) padded to 32 doubles = 256 bytes, so that a
 // push writes whole, aligned 32-byte sectors (a partial sector costs a DRAM read-modify-write under ECC)
@@ -34,7 +36,12 @@ struct EnvParams {
     double* hist; float* obsr; int64_t n_pad; int32_t obs_push; int32_t obs_q;   // hist: [N][H][FP_HIST_SLOT] doubles
     // per-env state
     uint64_t* rec; double* V; double* setp;
-    double* pfl; double* qfl; double* isq;       // optional line-flow dump (nullptr = off)
+    union {
+        struct { double* pfl; double* qfl; double* isq; };          // optional line-flow dump (nullptr = off)
+        // MODE_PREVIEW, which never dumps flows: candidates K; per (candidate, env) voltage rows [K][N][nb] and
+        // violation masks [K][N] (each may be null).  The actions and reward / done / info are [K][N][...] too.
+        struct { double* pv_V; uint64_t* pv_vmask; int64_t pv_k; };
+    };
     // step inputs/outputs
     const void* actions; int32_t act_f64;
     // fp32 policy outputs: translate_action (utils/util.py:121-129) in fp32 before widening

@@ -68,6 +68,7 @@ _PROTOS = {
     "fp_reset_random": (C.c_int, [_P, C.c_uint64, C.c_int64, _P, _P]),
     "fp_reset_random_retry": (C.c_int, [_P, C.c_uint64, C.c_int64, _P, C.c_int32, _P, _P]),
     "fp_step": (C.c_int, [_P, _P, C.c_int, _P, _P, _P, _P, _P]),
+    "fp_step_preview": (C.c_int, [_P, C.c_int32, _P, C.c_int, _P, _P, _P, _P, _P, _P]),
     "fp_step_host": (C.c_int, [_P, _P, C.c_int, _P, _P, _P, _P]),
     "fp_get_obs": (C.c_int, [_P, _P, C.c_int, C.c_int, _P]),
     "fp_get_obs_view": (C.c_int, [_P, C.c_int, C.POINTER(_P), C.POINTER(C.c_int64), C.POINTER(C.c_int64), _P]),

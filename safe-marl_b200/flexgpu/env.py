@@ -311,6 +311,45 @@ class BatchedFlexProvisionEnv:
             return self._reward, self._done, info, obs
         return self._reward, self._done, info
 
+    def preview_step(self, actions, translate=False, want_info=True, want_voltage=False, want_mask=False):
+        """What step(actions) would return and leave behind, without committing anything (fp_step_preview): no record,
+        voltage, setpoint, line-flow, observation-history or statistics write, so it may be called any number of times
+        between two steps.  actions: [N, na, 4] for one candidate per env, or [K, N, na, 4] for K candidates per env
+        (one launch); dtypes and translate as step().  Returns (reward, done, info) -- plus voltages [.., N, n_bus] f64
+        (what env.voltages would hold: after a failed solve the rolled-back ones) with want_voltage, plus the violation
+        mask [.., N] (what env.violation_mask would read) with want_mask -- with a leading K dimension for [K, N, na, 4]
+        actions.  info has step()'s keys.  Every returned tensor is freshly allocated."""
+        if not isinstance(actions, torch.Tensor):
+            actions = torch.as_tensor(np.ascontiguousarray(actions))
+        if translate:
+            actions = actions.to(torch.float32)
+        elif actions.dtype not in (torch.float32, torch.float64):
+            actions = actions.to(torch.float64)
+        actions = actions.to(self.device).contiguous()
+        N, na, nb = self.n_envs, self.n_agents, self.n_bus
+        tail = (N, na, self.n_actions)
+        if actions.dim() == 3 and tuple(actions.shape) == tail:
+            k, lead = 1, ()
+        elif actions.dim() == 4 and tuple(actions.shape[1:]) == tail and actions.shape[0] >= 1:
+            k = int(actions.shape[0]); lead = (k,)
+        else:
+            raise ValueError(f"actions must be [n_envs, n_agents, 4] or [K, n_envs, n_agents, 4], got {tuple(actions.shape)}")
+        dev = self.device
+        reward = torch.empty(*lead, N, dtype=torch.float64, device=dev)
+        done = torch.empty(*lead, N, dtype=torch.bool, device=dev)          # one byte per env, written as uint8
+        info = torch.empty(*lead, N, _lib.FP_INFO_STRIDE, dtype=torch.float64, device=dev) if want_info else None
+        volt = torch.empty(*lead, N, nb, dtype=torch.float64, device=dev) if want_voltage else None
+        vmask = torch.empty(*lead, N, dtype=torch.int64, device=dev) if want_mask else None
+        dt = _lib.FP_F32_POLICY if translate else (_lib.FP_F64 if actions.dtype == torch.float64 else _lib.FP_F32)
+        self._check(self._lib.fp_step_preview(self._h, k, _ptr(actions), dt, _ptr(reward), _ptr(done), _ptr(info), _ptr(volt),
+                                              _ptr(vmask), _lib.stream(dev)), "fp_step_preview")
+        out = (reward, done, {k_: info[..., i] for i, k_ in enumerate(_lib.INFO_KEYS)} if want_info else {})
+        if want_voltage:
+            out += (volt,)
+        if want_mask:
+            out += (vmask,)
+        return out
+
     def step_host(self, actions, want_info=False, translate=False):
         """End-to-end variant: host (numpy, ideally pinned) in, host out, through fp_step_host.
         Pinned fp32 actions (thread variant) are read by the step kernel straight from host memory, and the

@@ -1,0 +1,234 @@
+"""env.preview_step / fp_step_preview: the step's computation for K candidate actions per env without committing it.
+
+ * equals step bit for bit: reward, done, info, voltages and violation mask of preview_step(a) are those of a following
+   step(a) and of env.voltages / env.violation_mask after it, at every step of a whole episode;
+ * touches nothing: records, voltages, setpoints, line flows, both observation histories and the statistics partials
+   are byte-identical before and after previews, and a step after previews gives the bits of a step without them;
+ * K candidates in one launch equal K single-candidate calls;
+ * argument and call-sequence checks.
+"""
+import ctypes as C
+
+import numpy as np
+import pytest
+import torch
+
+from flexgpu import _lib
+
+
+def make(cuda, profiles, n, variant, **args):
+    from flexgpu import BatchedFlexProvisionEnv
+    a = dict(args)
+    a["kernel_variant"] = variant
+    return BatchedFlexProvisionEnv(a, n_envs=n, device=cuda, profiles=profiles)
+
+
+def reset(env, seed):
+    n = env.n_envs
+    rng = np.random.default_rng(seed)
+    start = rng.integers(0, env.max_start(), n).astype(np.int32)
+    e0 = rng.uniform(0.9 * 0.0125, 1.1 * 0.0125, (n, 5))
+    a0 = rng.uniform(0, 1, (n, 20))
+    env.reset(start, e0, a0, return_obs=False)
+
+
+def candidates(kind, rng, shape):
+    """Actions of one dtype kind: policy outputs for "policy", setpoints for the raw_actions ("raw") env."""
+    if kind == "raw":
+        a = rng.uniform(0, 1, shape) * np.array([0.5, 0.01, 0.01, 0.02])
+        return torch.from_numpy(a)
+    a = rng.normal(0.3, 0.6, shape)
+    return torch.from_numpy(a.astype(np.float64 if kind == "f64" else np.float32))
+
+
+def snapshot(env):
+    """Every byte of the handle's per-env state a step can write, and the statistics partials' sums."""
+    torch.cuda.synchronize()
+    ring = env.obs_ring()
+    pf, qf, isq = env.line_flows
+    out = {"rec": env.rec.clone(), "V": env.voltages.clone(), "setp": env.setpoints.clone(),
+           "hist": env._history(False).clone(), "ring": ring.ring.clone(), "slot": ring.slot}
+    if pf is not None:
+        out.update(pf=pf.clone(), qf=qf.clone(), isq=isq.clone())
+    out["stats"] = {k: v.clone() for k, v in env.episode_stats(reduce=False).items()}
+    torch.cuda.synchronize()
+    return out
+
+
+def assert_same_bytes(a, b):
+    assert a.keys() == b.keys()
+    for k in a:
+        if k == "stats":
+            for s in a[k]:
+                assert torch.equal(a[k][s].view(torch.int64), b[k][s].view(torch.int64)), s
+        elif isinstance(a[k], torch.Tensor):
+            x, y = a[k], b[k]
+            if x.dtype == torch.float64:
+                x, y = x.view(torch.int64), y.view(torch.int64)     # bits, NaN included
+            assert torch.equal(x, y), k
+        else:
+            assert a[k] == b[k], k
+
+
+def bits(t):
+    return t.view(torch.int64) if t.dtype == torch.float64 else t
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("n", [500, 3001])
+@pytest.mark.parametrize("kind", ["f32", "f64", "policy", "raw"])
+def test_preview_equals_the_following_step_over_an_episode(cuda, profiles, variant, kind, n):
+    """At every step of a 95-step episode (the first step, the episode limit, done and the row in force included),
+    preview_step(a) returns what step(a) then returns, and the voltages / mask that step leaves in the env."""
+    env = make(cuda, profiles, n, variant, **({"alg": "safemaddpg"} if kind == "raw" else {}))
+    reset(env, 1)
+    rng = np.random.default_rng(2)
+    translate = kind == "policy"
+    n_failed = 0
+    for t in range(env.episode_limit):
+        a = candidates(kind, rng, (n, 5, 4))
+        if t == 40:                                                 # NaN actions: the failure path
+            a[::97, 1, 2] = float("nan")
+        inj = None
+        if t == 60:                                                 # injected failures
+            inj = torch.zeros(n, dtype=torch.uint8); inj[5::31] = 1
+            env.inject_failure(inj)
+        r, d, info, V, vm = env.preview_step(a, translate=translate, want_voltage=True, want_mask=True)
+        r, d, V, vm = r.clone(), d.clone(), V.clone(), vm.clone()
+        info = {k: v.clone() for k, v in info.items()}
+        rs, ds, infos = env.step(a, translate=translate)
+        assert torch.equal(bits(r), bits(rs)), t
+        assert torch.equal(d, ds), t
+        assert info.keys() == infos.keys()
+        for k in info:
+            assert torch.equal(bits(info[k]), bits(infos[k])), (t, k)
+        assert torch.equal(bits(V), bits(env.voltages)), t
+        assert torch.equal(vm, env.violation_mask), t
+        n_failed += int(infos["solver_failed"].sum())
+        if inj is not None:
+            env.inject_failure(None)
+    assert bool(d.all()), "the last step reaches the episode limit"
+    assert n_failed > 0, "the episode must exercise the failure path"
+    env.close()
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("k", [1, 8])
+def test_preview_touches_nothing(cuda, profiles, variant, k):
+    """Heavy loading (thousands of violations), injected failures and NaN actions: the handle's state is
+    byte-identical before and after previews, and the next step gives the bits of a twin env that never previewed."""
+    from flexgpu import Profiles
+    heavy = Profiles(profiles.P * 2.4, profiles.Q * 2.4, profiles.PV, profiles.price)
+    n = 1000
+    envs = [make(cuda, heavy, n, variant) for _ in range(2)]
+    rng = np.random.default_rng(5)
+    for env in envs:
+        env.keep_line_flows(True)
+        reset(env, 3)
+    for t in range(3):                                              # some history in both observation rings
+        a = candidates("f32", np.random.default_rng(10 + t), (n, 5, 4))
+        for env in envs:
+            env.step(a, return_obs="ring")
+    inj = torch.zeros(n, dtype=torch.uint8); inj[::7] = 1
+    envs[0].inject_failure(inj)
+    before = snapshot(envs[0])
+    violations = 0
+    for rep in range(3):
+        cand = candidates("f32" if rep != 1 else "f64", rng, (k, n, 5, 4))
+        cand[:, ::13, 2, 1] = float("nan")
+        for translate in (False, True):
+            if translate and cand.dtype != torch.float32:
+                continue
+            r, d, info, V, vm = envs[0].preview_step(cand if k > 1 else cand[0], translate=translate, want_voltage=True,
+                                                     want_mask=True)
+            violations += int(((V > 1.1) | (V < 0.9)).sum())
+            assert bool(info["solver_failed"].bool().any())
+    assert violations > 1000, "the loading must produce violations"
+    assert_same_bytes(before, snapshot(envs[0]))
+    envs[0].inject_failure(None)
+    a = candidates("f32", rng, (n, 5, 4))
+    outs = []
+    for env in envs:
+        r, d, info = env.step(a)
+        outs.append((r.clone(), d.clone(), {k_: v.clone() for k_, v in info.items()}))
+    assert torch.equal(bits(outs[0][0]), bits(outs[1][0])) and torch.equal(outs[0][1], outs[1][1])
+    for k_ in outs[0][2]:
+        assert torch.equal(bits(outs[0][2][k_]), bits(outs[1][2][k_])), k_
+    assert_same_bytes(snapshot(envs[0]), snapshot(envs[1]))
+    for env in envs:
+        env.close()
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("k", [2, 5, 16])
+@pytest.mark.parametrize("kind", ["f32", "f64"])
+def test_k_candidates_equal_k_single_calls(cuda, profiles, variant, kind, k):
+    n = 777                                                         # not a multiple of 32
+    env = make(cuda, profiles, n, variant)
+    reset(env, 7)
+    rng = np.random.default_rng(8)
+    env.step(candidates(kind, rng, (n, 5, 4)))                      # past the first step: the row in force moves
+    cand = candidates(kind, rng, (k, n, 5, 4))
+    cand[k - 1, 3::50, 0, 0] = float("nan")
+    r, d, info, V, vm = env.preview_step(cand, want_voltage=True, want_mask=True)
+    assert r.shape == (k, n) and d.shape == (k, n) and V.shape == (k, n, 33) and vm.shape == (k, n)
+    assert info["reward"].shape == (k, n)
+    for j in range(k):
+        r1, d1, info1, V1, vm1 = env.preview_step(cand[j], want_voltage=True, want_mask=True)
+        assert torch.equal(bits(r[j]), bits(r1)) and torch.equal(d[j], d1), j
+        assert torch.equal(bits(V[j]), bits(V1)) and torch.equal(vm[j], vm1), j
+        for key in info:
+            assert torch.equal(bits(info[key][j]), bits(info1[key])), (j, key)
+    assert bool(info["solver_failed"][k - 1].bool().any())
+    # the outputs are fresh: a later call leaves earlier results alone
+    r_again = env.preview_step(cand[0] * 0.5)[0]
+    assert torch.equal(bits(r[0]), bits(env.preview_step(cand[0])[0])) and not torch.equal(r_again, r[0])
+    env.close()
+
+
+@pytest.mark.gpu
+def test_preview_argument_and_state_checks(cuda, profiles, variant):
+    from flexgpu import FlexGpuError
+    from flexgpu.config import make_fp_config, normalize_args
+    n = 40
+    env = make(cuda, profiles, n, variant)
+    reset(env, 1)
+    l, h = env._lib, env._h
+    a = torch.rand(n, 5, 4, device=cuda)
+    r = torch.empty(n, dtype=torch.float64, device=cuda)
+    d = torch.empty(n, dtype=torch.uint8, device=cuda)
+    p = lambda t: C.c_void_p(t.data_ptr())
+    s = _lib.stream(env.device)
+    assert l.fp_step_preview(h, 1, p(a), _lib.FP_F32, p(r), p(d), None, None, None, s) == 0
+    assert l.fp_step_preview(h, 1, None, _lib.FP_F32, p(r), p(d), None, None, None, s) == -1
+    assert l.fp_step_preview(h, 1, p(a), _lib.FP_F32, None, p(d), None, None, None, s) == -1
+    assert l.fp_step_preview(h, 1, p(a), _lib.FP_F32, p(r), None, None, None, None, s) == -1
+    assert l.fp_step_preview(h, 0, p(a), _lib.FP_F32, p(r), p(d), None, None, None, s) == -1
+    assert l.fp_step_preview(h, -3, p(a), _lib.FP_F32, p(r), p(d), None, None, None, s) == -1
+    assert l.fp_step_preview(h, 1, p(a), 7, p(r), p(d), None, None, None, s) == -1
+    assert b"fp_step_preview" in l.fp_last_error(h)
+    with pytest.raises(ValueError):
+        env.preview_step(torch.rand(n + 1, 5, 4))
+    with pytest.raises(ValueError):
+        env.preview_step(torch.rand(2, n, 5, 3))
+    env.close()
+    # before fp_load_profiles: FP_ESTATE, as fp_step
+    args = normalize_args({"kernel_variant": variant})
+    cfg = make_fp_config(args, env.network)
+    hh = C.c_void_p()
+    assert l.fp_create(C.byref(cfg), n, 0, C.byref(hh)) == 0
+    try:
+        assert l.fp_step_preview(hh, 1, p(a), _lib.FP_F32, p(r), p(d), None, None, None, s) == -3
+        assert l.fp_step(hh, p(a), _lib.FP_F32, p(r), p(d), None, None, s) == -3
+    finally:
+        l.fp_destroy(hh)
+    env = make(cuda, profiles, n, variant)
+    with pytest.raises(ValueError):
+        env.preview_step(torch.rand(0, n, 5, 4))
+    with pytest.raises(FlexGpuError):                                # failures of the entry point surface as FlexGpuError
+        env._check(l.fp_step_preview(env._h, 0, p(a), _lib.FP_F32, p(r), p(d), None, None, None, s), "fp_step_preview")
+    env.close()
+
+
+def test_null_handle_preview_is_rejected():
+    assert _lib.lib().fp_step_preview(None, 1, None, 0, None, None, None, None, None, None) == -1
