@@ -13,6 +13,7 @@ import numpy as np
 import pytest
 import torch
 
+from _feeders import assert_same_bytes, snapshot
 from flexgpu import _lib
 
 
@@ -39,35 +40,6 @@ def candidates(kind, rng, shape):
         return torch.from_numpy(a)
     a = rng.normal(0.3, 0.6, shape)
     return torch.from_numpy(a.astype(np.float64 if kind == "f64" else np.float32))
-
-
-def snapshot(env):
-    """Every byte of the handle's per-env state a step can write, and the statistics partials' sums."""
-    torch.cuda.synchronize()
-    ring = env.obs_ring()
-    pf, qf, isq = env.line_flows
-    out = {"rec": env.rec.clone(), "V": env.voltages.clone(), "setp": env.setpoints.clone(),
-           "hist": env._history(False).clone(), "ring": ring.ring.clone(), "slot": ring.slot}
-    if pf is not None:
-        out.update(pf=pf.clone(), qf=qf.clone(), isq=isq.clone())
-    out["stats"] = {k: v.clone() for k, v in env.episode_stats(reduce=False).items()}
-    torch.cuda.synchronize()
-    return out
-
-
-def assert_same_bytes(a, b):
-    assert a.keys() == b.keys()
-    for k in a:
-        if k == "stats":
-            for s in a[k]:
-                assert torch.equal(a[k][s].view(torch.int64), b[k][s].view(torch.int64)), s
-        elif isinstance(a[k], torch.Tensor):
-            x, y = a[k], b[k]
-            if x.dtype == torch.float64:
-                x, y = x.view(torch.int64), y.view(torch.int64)     # bits, NaN included
-            assert torch.equal(x, y), k
-        else:
-            assert a[k] == b[k], k
 
 
 def bits(t):

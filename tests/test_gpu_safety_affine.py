@@ -9,6 +9,7 @@ import numpy as np
 import pytest
 import torch
 
+from _feeders import lindistflow_map
 from oracle import env_ref, ieee33, safety_affine_ref, safety_ref
 
 pytestmark = pytest.mark.gpu
@@ -36,21 +37,7 @@ def _proposal(ref, a):
 
 def _lindistflow():
     """dV_n / dP_m = -sum R_l, dV_n / dQ_m = -sum X_l over the lines shared by the root paths of buses n and m."""
-    t = ieee33.tree_arrays(ieee33.create_network())
-    parent, R, X = np.asarray(t["parent"]), np.asarray(t["R"]), np.asarray(t["X"])
-    nb = len(parent)
-    path = []                                                       # lines (named by their far bus) from the root to n
-    for n in range(nb):
-        p, s = n, set()
-        while parent[p] >= 0:
-            s.add(p); p = parent[p]
-        path.append(s)
-    A = np.zeros((nb, 2 * nb))
-    for n in range(nb):
-        for m in range(nb):
-            shared = list(path[n] & path[m])
-            A[n, 2 * m] = -R[shared].sum(); A[n, 2 * m + 1] = -X[shared].sum()
-    return A, np.ones(nb)
+    return lindistflow_map(ieee33.tree_arrays(ieee33.create_network()))
 
 
 def _map(env, name):
