@@ -61,7 +61,7 @@ constexpr uint32_t WG_BYTES = 2 * WG_RZ_BYTES + 2 * WG_N_BYTES;            // 98
 constexpr int V_B1A = 0, V_LNG = 320, V_LNB = 384, V_BRZ = 448, V_BIN = 576, V_BHN = 640, V_W2 = 704, V_B2 = 960, V_FLOATS = 992;
 constexpr uint32_t OFF_W1 = 0, OFF_WG = OFF_W1 + W1_BYTES, OFF_VEC = OFF_WG + WG_BYTES;
 constexpr uint32_t OFF_STAGE = OFF_VEC + V_FLOATS * 4;                     // [144][128] fp32 = 73 728
-constexpr uint32_t OFF_LN = OFF_STAGE + POL_OBS * POL_M * 4;               // [TPR][128 rows] float2 (sum, sum of squares)
+constexpr uint32_t OFF_LN = OFF_STAGE + POL_OBS * POL_M * 4;               // [TPR][128 rows] float2 (quarter mean, sum of squared deviations)
 constexpr uint32_t OFF_FC = OFF_LN + TPR * POL_M * 8;                      // [TPR][128 rows] float4: fc2 partial sums
 constexpr uint32_t OFF_BAR = OFF_FC + TPR * POL_M * 16;                    // a_ready, mma_done, weights, x_full
 constexpr uint32_t OFF_TMEM = OFF_BAR + 56;                                // (+ mma_done of the two column halves of the GRU GEMMs, stage_copied)
@@ -147,6 +147,32 @@ __device__ __forceinline__ void tanh8_scaled(float (&v)[8]) {
     rcp4(a[4], a[5], a[6], a[7], a[4], a[5], a[6], a[7]);
 #pragma unroll
     for (int i = 0; i < 8; ++i) v[i] = copysignf(fmaf(-2.0f, a[i], 1.0f), v[i]);
+}
+
+// LayerNorm statistics of a row from its four column quarters, CENTRED: a thread reduces its 16 values to (mean_q, M2_q =
+// sum of squared deviations from mean_q), and the four pairs merge by Chan's formula, mean = sum mean_q / 4 and
+// var = (sum M2_q + 16 sum (mean_q - mean)^2) / 64 (biased, as torch.nn.LayerNorm).  The one-pass SS / 64 - mean^2 loses
+// ~(mean / std)^2 ulps of the variance to cancellation, i.e. its error grows with the square of a common offset of the
+// pre-activations; centred, only their fp32 representation (~ulp(mean) / std) remains.  A NaN input reaches mean and rstd.
+__device__ __forceinline__ float2 ln_quarter(const float (&v)[CPT]) {
+    float s = 0.0f;
+#pragma unroll
+    for (int i = 0; i < CPT; ++i) s = __fadd_rn(s, v[i]);
+    const float mq = __fmul_rn(s, 1.0f / CPT);
+    float m2 = 0.0f;
+#pragma unroll
+    for (int i = 0; i < CPT; ++i) { const float d = __fsub_rn(v[i], mq); m2 = fmaf(d, d, m2); }
+    return make_float2(mq, m2);
+}
+// q: the row's first quarter pair, the others POL_M pairs apart; every thread of the row merges them in the same order
+__device__ __forceinline__ void ln_merge(const float2* q, float& mean, float& rstd) {
+    const float2 t0 = q[0], t1 = q[POL_M], t2 = q[2 * POL_M], t3 = q[3 * POL_M];
+    mean = __fmul_rn(__fadd_rn(__fadd_rn(t0.x, t1.x), __fadd_rn(t2.x, t3.x)), 1.0f / TPR);
+    const float d0 = __fsub_rn(t0.x, mean), d1 = __fsub_rn(t1.x, mean), d2 = __fsub_rn(t2.x, mean), d3 = __fsub_rn(t3.x, mean);
+    const float between = fmaf(d3, d3, fmaf(d2, d2, fmaf(d1, d1, __fmul_rn(d0, d0))));
+    const float m2 = __fadd_rn(__fadd_rn(t0.y, t1.y), __fadd_rn(t2.y, t3.y));
+    const float var = __fmul_rn(fmaf((float)CPT, between, m2), 1.0f / POL_HID);
+    rstd = rsqrtf(__fadd_rn(var, 1e-5f));
 }
 
 // the row's four standard normals: the caller's array, or Philox4x32-10 keyed by the seed, counter = (row, step) + Box-Muller.
@@ -404,17 +430,12 @@ __global__ void __launch_bounds__(POL_THREADS, 1) k_policy(const PolParams prm, 
                 float v[CPT];
                 tmem_ld16(lane_base + C_ACC1 + c0, v);
                 tmem_wait_ld();
-                float s = 0.0f, ss = 0.0f;
 #pragma unroll
-                for (int i = 0; i < CPT; ++i) { v[i] = __fadd_rn(v[i], vec[V_B1A + a * POL_HID + c0 + i]); s = __fadd_rn(s, v[i]); ss = fmaf(v[i], v[i], ss); }
-                lnp[qt * POL_M + row] = make_float2(s, ss);
+                for (int i = 0; i < CPT; ++i) v[i] = __fadd_rn(v[i], vec[V_B1A + a * POL_HID + c0 + i]);
+                lnp[qt * POL_M + row] = ln_quarter(v);
                 group_sync<1, N_WORKERS>();
-                float S = 0.0f, SS = 0.0f;
-#pragma unroll
-                for (int j = 0; j < TPR; ++j) { const float2 t = lnp[j * POL_M + row]; S = __fadd_rn(S, t.x); SS = __fadd_rn(SS, t.y); }
-                const float mean = __fmul_rn(S, 1.0f / POL_HID);
-                const float var = max_nan(fmaf(-mean, mean, __fmul_rn(SS, 1.0f / POL_HID)), 0.0f);   // biased, as torch.nn.LayerNorm
-                const float rstd = rsqrtf(__fadd_rn(var, 1e-5f));
+                float mean, rstd;
+                ln_merge(lnp + row, mean, rstd);
 #pragma unroll
                 for (int i = 0; i < CPT; ++i) {
                     const float y = fmaf(__fmul_rn(__fsub_rn(v[i], mean), rstd), vec[V_LNG + c0 + i], vec[V_LNB + c0 + i]);
@@ -731,18 +752,13 @@ __global__ void __launch_bounds__(CRIT_THREADS, 1) k_critic(const CritParams prm
             tmem_wait_ld();
             auto e1 = [&](int i) {
                 float v[CPT];
-                float s = 0.0f, ss = 0.0f;
 #pragma unroll
-                for (int c = 0; c < CPT; ++c) { v[c] = __fadd_rn(y1[c], vec[CV_B1A + i * POL_HID + c0 + c]); s = __fadd_rn(s, v[c]); ss = fmaf(v[c], v[c], ss); }
+                for (int c = 0; c < CPT; ++c) v[c] = __fadd_rn(y1[c], vec[CV_B1A + i * POL_HID + c0 + c]);
                 float2* ln = lnp + (i & 1) * (TPR * POL_M);
-                ln[qt * POL_M + row] = make_float2(s, ss);
+                ln[qt * POL_M + row] = ln_quarter(v);
                 group_sync<1, N_WORKERS>();
-                float S = 0.0f, SS = 0.0f;
-#pragma unroll
-                for (int q4 = 0; q4 < TPR; ++q4) { const float2 t = ln[q4 * POL_M + row]; S = __fadd_rn(S, t.x); SS = __fadd_rn(SS, t.y); }
-                const float mean = __fmul_rn(S, 1.0f / POL_HID);
-                const float var = max_nan(fmaf(-mean, mean, __fmul_rn(SS, 1.0f / POL_HID)), 0.0f);   // biased, as torch.nn.LayerNorm
-                const float rstd = rsqrtf(__fadd_rn(var, 1e-5f));
+                float mean, rstd;
+                ln_merge(ln + row, mean, rstd);
 #pragma unroll
                 for (int c = 0; c < CPT; ++c) {
                     const float t = fmaf(__fmul_rn(__fsub_rn(v[c], mean), rstd), vec[CV_LNG + c0 + c], vec[CV_LNB + c0 + c]);
