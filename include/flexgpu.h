@@ -375,27 +375,30 @@ int fp_safety_project_affine(FpHandle* h, const void* d_actions, int act_dtype, 
 
 /* -- acting policy of the rollout loop, transitions, learner feed (SURVEY 8f ranks 1-2) ---- */
 
-/* The shared-parameter RNNAgent (madrl/agents/rnn_agent.py:8-32: fc1(144 obs + 5 agent-id -> 64) -> LayerNorm ->
- * ReLU -> GRUCell(64) -> fc2(64 -> 4)) evaluated for n_envs x 5 agents per call on tcgen05 tensor cores, reading the
+/* The shared-parameter RNNAgent (madrl/agents/rnn_agent.py:8-32: fc1(144 obs + na agent-id -> 64) -> LayerNorm ->
+ * ReLU -> GRUCell(64) -> fc2(64 -> 4)) evaluated for n_envs x na agents per call on tcgen05 tensor cores, reading the
  * observation ring of fp_step_ring / fp_obs_ring directly, followed by select_action (utils/util.py:50-64, continuous,
  * action_enforcebound) -- i.e. the device form of model.py:215-216 (prep_obs -> get_actions).  Weights are held as
- * TF32; activations keep fp32 accuracy (two-term split).  The handle is independent of FpHandle (one per GPU). */
+ * TF32; activations keep fp32 accuracy (two-term split).  The handle is independent of FpHandle (one per GPU).
+ * na = the handle's agent count, 1 .. 5, fixed for its lifetime (fp_policy_create_agents; fp_policy_create: na = 5).  It
+ * must equal the env's n_agents: every shape below is stated with it, and the ring is [24][na][6][n_pad]. */
 typedef struct FpPolicy FpPolicy;
-int fp_policy_create(int device, FpPolicy** out);
+int fp_policy_create_agents(int device, int32_t n_agents, FpPolicy** out);   /* FP_EINVAL unless 1 <= n_agents <= 5 */
+int fp_policy_create(int device, FpPolicy** out);                            /* = fp_policy_create_agents(device, 5, out) */
 int fp_policy_destroy(FpPolicy* p);
 const char* fp_policy_last_error(const FpPolicy* p);    /* p may be NULL: last fp_policy_create error */
 int64_t fp_policy_launch_count(const FpPolicy* p);
-/* HOST fp32 arrays in torch's state_dict layouts: fc1.weight [64][149], fc1.bias [64], layernorm.weight/.bias [64],
+/* HOST fp32 arrays in torch's state_dict layouts: fc1.weight [64][144 + na], fc1.bias [64], layernorm.weight/.bias [64],
  * rnn.weight_ih / weight_hh [192][64] (rows r | z | n), rnn.bias_ih / bias_hh [192], fc2.weight [4][64], fc2.bias [4]. */
 int fp_policy_load(FpPolicy* p, const float* fc1_w, const float* fc1_b, const float* ln_g, const float* ln_b,
                    const float* w_ih, const float* w_hh, const float* b_ih, const float* b_hh,
                    const float* fc2_w, const float* fc2_b);
 /* One acting step.  d_ring / slot / n_pad: the observation ring.  d_hid_in (NULL = zeros) / d_hid_out: hidden states
- * (last_hid / hid of the Transition), [n_envs][5][64] or -- hid_env_minor != 0, the kernel's native layout: every access a
- * coalesced 128-byte line -- [5][64][n_pad] (fp_policy_hidden_to_ring turns it into replay rows); d_reset (may be NULL): envs whose hidden state restarts at zero
- * (init_hidden, model.py:211).  Outputs [n_envs][5][4] fp32: d_mean (may be NULL), d_action = tanh(mean + std eps)
+ * (last_hid / hid of the Transition), [n_envs][na][64] or -- hid_env_minor != 0, the kernel's native layout: every access a
+ * coalesced 128-byte line -- [na][64][n_pad] (fp_policy_hidden_to_ring turns it into replay rows); d_reset (may be NULL): envs whose hidden state restarts at zero
+ * (init_hidden, model.py:211).  Outputs [n_envs][na][4] fp32: d_mean (may be NULL), d_action = tanh(mean + std eps)
  * (what translate_action receives: feed it to fp_step* with FP_F32_POLICY), d_logp (may be NULL).  explore = 1: status
- * 'train' with exploration, eps from d_eps (caller-supplied standard-normal draws, [n_envs][5][4]) or, if NULL, from
+ * 'train' with exploration, eps from d_eps (caller-supplied standard-normal draws, [n_envs][na][4]) or, if NULL, from
  * Philox4x32-10 keyed by (seed; row, step); explore = 0: status 'test' (action = tanh(mean)).  std = fixed_policy_std. */
 int fp_policy_act(FpPolicy* p, const float* d_ring, int32_t slot, int64_t n_pad, int64_t n_envs, const float* d_hid_in,
                   const uint8_t* d_reset, float* d_hid_out, int32_t hid_env_minor, float* d_mean, float* d_action, float* d_logp,
@@ -407,8 +410,9 @@ int fp_policy_act(FpPolicy* p, const float* d_ring, int32_t slot, int64_t n_pad,
 int fp_policy_sample(FpPolicy* p, const float* d_mean, int64_t n_envs, float* d_action, float* d_logp, const float* d_eps,
                      uint64_t seed, uint64_t step, float std_, int32_t explore, void* stream);
 /* Transition fields (madrl/models/model.py:19, :230-242) straight into a replay ring: field rows (row0 + e) mod cap.
- *   fp_policy_gather_windows   state / next_state: the dense get_obs windows [5][144] of envs [0, n) from the ring
- *                              (pitch = floats per destination row, >= 720; row0 = 0, cap >= n: a dense tensor)
+ *   fp_policy_gather_windows   state / next_state: the dense get_obs windows [na][144] of envs [0, n) from the ring
+ *                              (pitch = floats per destination row, >= na x 144; row0 = 0, cap >= n: a dense tensor)
+ *   fp_policy_hidden_to_ring   last_hid / hid: env-minor hidden states [na][64][n_pad] -> rows of na x 64 floats
  *   fp_policy_rows_to_ring     any dense [n][width] fp32 array (action, log_prob_a, last_hid, hid, value ...)
  *   fp_policy_scalars_to_ring  reward repeated per agent (model.py:221), done, last_step (= done, or every env when
  *                              last_step_all: t == max_steps - 1, model.py:229), all-ones action_avail; NULL fields skipped
@@ -416,7 +420,7 @@ int fp_policy_sample(FpPolicy* p, const float* d_mean, int64_t n_envs, float* d_
  *                              skipped), reward per agent, done, last_step, action_avail (NULL: skipped) and -- zero_values
  *                              != 0 -- value / next_value as zeros (MADDPG's losses recompute both, maddpg.py:104-107) */
 /* One-shot sink for the NEXT fp_policy_act: its writer warps copy the dense get_obs windows of envs [0, n) -- the blocks the
- * kernel stages anyway -- into rows (row0 + e) mod cap of pitch `pitch` floats (16-byte aligned field, pitch a multiple of 4):
+ * kernel stages anyway -- into rows (row0 + e) mod cap of pitch `pitch` floats (>= na x 144; 16-byte aligned field, pitch a multiple of 4):
  * the Transition's `state` without a separate pass over the ring.  Needs n_pad >= 128. */
 int fp_policy_state_sink(FpPolicy* p, float* d_field, int64_t pitch, int64_t row0, int64_t cap, int64_t n);
 int fp_policy_gather_windows(FpPolicy* p, const float* d_ring, int32_t slot, int64_t n_pad, int64_t n, float* d_out,
@@ -435,17 +439,18 @@ int fp_policy_transition_tail(FpPolicy* p, const float* d_action, const float* d
 /* The critic of the rollout loop: MADDPG.value (madrl/models/maddpg.py:29-76) with the shared-parameter MLPCritic
  * (madrl/critics/mlp_critic.py:5-36: fc1 -> LayerNorm -> ReLU -> fc2 -> ReLU -> fc3) as train_process evaluates it for the
  * Transition's value / next_value (madrl/models/model.py:217, :225-226), on tcgen05 (k_critic), reading the observation
- * ring directly.  fp_critic_load: HOST fp32 arrays in torch's state_dict layouts -- fc1.weight [64][745] (720 observation
- * columns | 5 agent-id columns | 20 action columns), fc1.bias [64], layernorm.weight / .bias [64], fc2.weight [64][64],
- * fc2.bias [64], fc3.weight [1][64], fc3.bias [1].  fp_critic_value: d_actions [n_envs][5][4] fp32 (what fp_policy_act
- * returned), d_value [n_envs][5] fp32. */
+ * ring directly.  fp_critic_load: HOST fp32 arrays in torch's state_dict layouts -- fc1.weight [64][na x 149] (na x 144
+ * observation columns | na agent-id columns | na x 4 action columns: 745 for five agents), fc1.bias [64], layernorm.weight
+ * / .bias [64], fc2.weight [64][64], fc2.bias [64], fc3.weight [1][64], fc3.bias [1].  fp_critic_value: d_actions
+ * [n_envs][na][4] fp32 (what fp_policy_act returned), d_value [n_envs][na] fp32. */
 int fp_critic_load(FpPolicy* p, const float* fc1_w, const float* fc1_b, const float* ln_g, const float* ln_b,
                    const float* fc2_w, const float* fc2_b, const float* fc3_w, const float* fc3_b);
 int fp_critic_value(FpPolicy* p, const float* d_ring, int32_t slot, int64_t n_pad, int64_t n_envs, const float* d_actions,
                     float* d_value, void* stream);
 /* Learner feed: the device part of unpack_data (model.py:308-323) on a batch sampled with fp_replay_sample.
- * d_critic_in [batch * 5][745] = the MADDPG critic's input rows (maddpg.py:29-66: all agents' observations, one-hot
- * agent id, all agents' actions); d_reward_norm [batch][5] = reward_normalisation (BatchNorm1d over the batch, training
+ * d_critic_in [batch * na][na x 149] = the MADDPG critic's input rows (maddpg.py:29-66: all agents' observations, one-hot
+ * agent id, all agents' actions; d_state [batch][na x 144], d_action [batch][na x 4]); d_reward [batch][na], d_reward_norm
+ * [batch][na] = reward_normalisation (BatchNorm1d over the batch, training
  * mode, initial affine parameters; model.py:321-322).  Either output may be NULL. */
 int fp_learner_feed(FpPolicy* p, const float* d_state, const float* d_action, const float* d_reward, int64_t batch,
                     float* d_critic_in, float* d_reward_norm, void* stream);

@@ -1,13 +1,13 @@
 // policy.cu -- the acting policy of the rollout loop on tcgen05 tensor cores (SURVEY 8f rank 1).
 //
-//   fp_policy_load / fp_policy_act   replace, for N envs x 5 agents at once, what train_process does per step
+//   fp_policy_load / fp_policy_act   replace, for N envs x NA agents (1 .. 5) at once, what train_process does per step
 //       (madrl/models/model.py:215-216): prep_obs -> Model.policy (model.py:102-140: agent-id one-hot appended,
 //       shared parameters) -> RNNAgent.forward (madrl/agents/rnn_agent.py:24-32: fc1 -> LayerNorm -> ReLU ->
 //       GRUCell -> fc2) -> select_action (utils/util.py:50-64, continuous / action_enforcebound: x = mean + std eps,
 //       action = tanh(x), log_prob = Normal(mean, std).log_prob(x) - log(1 - action^2 + 1e-6); status 'test':
 //       action = tanh(mean)).
 //
-// Input is the env-minor observation ring the step kernel pushes into (fp_step_ring: ring[24][5][6][n_pad] fp32):
+// Input is the env-minor observation ring the step kernel pushes into (fp_step_ring: ring[24][NA][6][n_pad] fp32):
 // a tile is (one agent, 128 consecutive envs), and its 144 x 128 input block -- row k = (ring slot, feature),
 // 128 contiguous envs -- arrives with coalesced 16-byte LDGSTS copies; nothing is re-materialised.  The rotation of
 // the ring (the newest slot moves every step) is absorbed by the WEIGHTS: fc1 is linear in the observation, so the
@@ -45,7 +45,11 @@
 namespace {
 
 constexpr int POL_M = 128;                 // rows per tile = envs of one agent
-constexpr int POL_OBS = 144, POL_HID = 64, POL_ACT = 4, POL_NA = 5, POL_H = 24, POL_F = 6;
+constexpr int POL_OBS = 144, POL_HID = 64, POL_ACT = 4, POL_H = 24, POL_F = 6;
+// Agents per env: NA = 1 .. 5, a template parameter of every kernel below, dispatched once on the handle's count (the
+// five-agent instantiations compile to the code of the single-count kernels they replace).  Shared memory, TMEM and the
+// small-array offsets stay sized for five agents: for NA < 5 they are upper bounds.
+constexpr int POL_NA_MAX = 5;
 constexpr int TPR = 4;                     // worker threads per row (column quarters)
 constexpr int N_WORKERS = TPR * POL_M;     // 512
 constexpr int N_WRITERS = 96;               // k_policy: three warps that copy the tile's observation block into the Transition's `state` rows
@@ -76,18 +80,18 @@ constexpr uint32_t C_A2HI = 0, C_A2LO = 64, C_A3HI = 128, C_A3LO = 192, C_RZ = 2
 struct PolParams {
     const float* ring; int64_t n_pad; int64_t n; int32_t slot;       // observation ring, newest slot
     const float* W1rot; const float* Wg; const float* vec;
-    const float* hid_in; const uint8_t* reset; float* hid_out;        // [n][5][64], or env-minor [5][64][n_pad] (hid_em); reset: h_in = 0 for these envs
+    const float* hid_in; const uint8_t* reset; float* hid_out;        // [n][NA][64], or env-minor [NA][64][n_pad] (hid_em); reset: h_in = 0 for these envs
     int32_t hid_em;
-    float* mean; float* action; float* logp;                          // [n][5][4]
-    const float* eps;                                                 // optional caller-supplied N(0,1) draws [n][5][4]
+    float* mean; float* action; float* logp;                          // [n][NA][4]
+    const float* eps;                                                 // optional caller-supplied N(0,1) draws [n][NA][4]
     uint64_t seed; uint64_t step; float std_; float log_std; int32_t explore;
     int32_t use_tma;                                                  // observation blocks by one 3-D TMA box copy per tile
-    // optional sink for the Transition's `state` (model.py:230-237): the dense get_obs windows [5][144] of envs [0, st_n) go to
+    // optional sink for the Transition's `state` (model.py:230-237): the dense get_obs windows [NA][144] of envs [0, st_n) go to
     // rows (st_row0 + e) mod st_cap of pitch st_pitch floats, written by the writer warps from the staged block (TMA path only)
     float* st_out; int64_t st_pitch, st_row0, st_cap, st_n;
 };
 
-// One box of the 3-D ring view [24 slots][30 = agent x feature][n_pad envs], starting at (c_env, c_row, c_slot): box_slots x 6
+// One box of the 3-D ring view [24 slots][NA x 6 = agent x feature][n_pad envs], starting at (c_env, c_row, c_slot): box_slots x 6
 // x 128 floats -> [6 box_slots][128] in shared memory (k_policy: all 24 slots, k_critic: 12)
 __device__ __forceinline__ void tma_load_box(uint32_t dst, const CUtensorMap* map, int32_t c_env, int32_t c_row, int32_t c_slot, uint32_t bar) {
     asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
@@ -233,6 +237,7 @@ __global__ void k_sample(const float* __restrict__ mean, int64_t rows, int explo
     }
 }
 
+template <int NA>
 __global__ void __launch_bounds__(POL_THREADS, 1) k_policy(const PolParams prm, const __grid_constant__ CUtensorMap tmap) {
     extern __shared__ __align__(128) uint8_t smem[];
     const float* vec = reinterpret_cast<const float*>(smem + OFF_VEC);
@@ -245,17 +250,17 @@ __global__ void __launch_bounds__(POL_THREADS, 1) k_policy(const PolParams prm, 
     const int tid = threadIdx.x, warp = __shfl_sync(0xFFFFFFFFu, tid >> 5, 0);
     const int row = tid & (POL_M - 1), qt = (tid >> 7) & (TPR - 1);        // row of the tile, column quarter
     const bool sink = prm.use_tma && prm.st_out != nullptr;               // the writer warps are at work
-    const int64_t n_blocks = (prm.n + POL_M - 1) / POL_M, n_tiles = n_blocks * POL_NA;
+    const int64_t n_blocks = (prm.n + POL_M - 1) / POL_M, n_tiles = n_blocks * NA;
 
     // this tile's observation block: 144 rows (ring slot s, feature f) x 128 envs, each row 512 contiguous bytes.
     // One TMA box copy by the MMA warp (tma_request); rings narrower than a tile take coalesced LDGSTS by the workers.
     auto tma_request = [&](int64_t tile) {                                   // one thread
         mbar_expect_tx(bar_x, POL_OBS * POL_M * 4);
-        tma_load_box(smem_u32(stage), &tmap, (int32_t)((tile / POL_NA) * POL_M), (int32_t)(tile % POL_NA) * POL_F, 0, bar_x);
+        tma_load_box(smem_u32(stage), &tmap, (int32_t)((tile / NA) * POL_M), (int32_t)(tile % NA) * POL_F, 0, bar_x);
     };
     auto request = [&](int64_t tile) {
-        const int a = (int)(tile % POL_NA);
-        const int64_t e0 = (tile / POL_NA) * POL_M;
+        const int a = (int)(tile % NA);
+        const int64_t e0 = (tile / NA) * POL_M;
         const int c4 = (tid & 31) * 4;
         const bool inside = e0 + c4 + 4 <= prm.n_pad;
 #pragma unroll
@@ -263,7 +268,7 @@ __global__ void __launch_bounds__(POL_THREADS, 1) k_policy(const PolParams prm, 
             const int k = (tid >> 5) + (N_WORKERS / 32) * i;
             const int s = k / POL_F, f = k - s * POL_F;
             float* dst = stage + k * POL_M + c4;
-            if (inside) cp_async16(dst, prm.ring + ((int64_t)(s * POL_NA + a) * POL_F + f) * prm.n_pad + e0 + c4);
+            if (inside) cp_async16(dst, prm.ring + ((int64_t)(s * NA + a) * POL_F + f) * prm.n_pad + e0 + c4);
             else *reinterpret_cast<float4*>(dst) = make_float4(0.f, 0.f, 0.f, 0.f);
         }
         cp_async_commit();
@@ -358,10 +363,10 @@ __global__ void __launch_bounds__(POL_THREADS, 1) k_policy(const PolParams prm, 
             const int rot = ((prm.slot + 1) % POL_H) * POL_F;
             uint32_t px = 0;
             for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-                const int a = (int)(tile % POL_NA);
+                const int a = (int)(tile % NA);
                 mbar_wait(bar_x, px); px ^= 1u;
                 for (int j = tid - (N_WORKERS + 32); j < POL_M; j += N_WRITERS) {      // env of the tile
-                    const int64_t e = (tile / POL_NA) * POL_M + j;
+                    const int64_t e = (tile / NA) * POL_M + j;
                     if (e >= prm.st_n) continue;
                     int64_t orow = prm.st_row0 + e; orow = orow >= prm.st_cap ? orow - prm.st_cap : orow;
                     float4* dst = reinterpret_cast<float4*>(prm.st_out + orow * prm.st_pitch + a * POL_OBS);
@@ -382,10 +387,10 @@ __global__ void __launch_bounds__(POL_THREADS, 1) k_policy(const PolParams prm, 
         uint32_t pm = 0, px = 0, pq = 0;
         bool first = true;
         for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-            const int a = (int)(tile % POL_NA);
-            const int64_t e = (tile / POL_NA) * POL_M + row;
+            const int a = (int)(tile % NA);
+            const int64_t e = (tile / NA) * POL_M + row;
             const bool live = e < prm.n;
-            const int64_t r_glob = e * POL_NA + a;                              // row of the reference's (b, n, .) tensors
+            const int64_t r_glob = e * NA + a;                                  // row of the reference's (b, n, .) tensors
 
             // ---- P0: observation block -> TMEM (this thread: 36 of the row's 144 inputs)
             if (prm.use_tma) { mbar_wait(bar_x, px); px ^= 1u; }
@@ -523,19 +528,19 @@ __global__ void __launch_bounds__(POL_THREADS, 1) k_policy(const PolParams prm, 
 }
 
 // ---------------------------------------------------------------------------- critic: MADDPG.value on tcgen05
-// k_critic replaces, for N envs x 5 agents at once, MADDPG.value (madrl/models/maddpg.py:29-76) with the shared-parameter
+// k_critic replaces, for N envs x NA agents at once, MADDPG.value (madrl/models/maddpg.py:29-76) with the shared-parameter
 // MLPCritic (madrl/critics/mlp_critic.py:5-36: fc1 -> LayerNorm -> ReLU -> fc2 -> ReLU -> fc3) as train_process calls it for
-// the Transition's value / next_value (madrl/models/model.py:217, :225-226).  The critic's 745-wide input row of (env, agent
-// i) is [all five agents' observations (720) | one-hot(i) (5) | all five agents' actions (20)]: only the one-hot differs
-// between the five rows of an env, so fc1 is evaluated ONCE per env on its 740 shared columns and the one-hot column is
+// the Transition's value / next_value (madrl/models/model.py:217, :225-226).  The critic's 149 NA-wide input row of (env,
+// agent i) is [all agents' observations (144 NA) | one-hot(i) (NA) | all agents' actions (4 NA)] (745 for five agents):
+// only the one-hot differs between the NA rows of an env, so fc1 is evaluated ONCE per env on its 148 NA shared columns and the one-hot column is
 // folded into a per-agent bias.  A tile is 128 envs, input = the env-minor observation ring, untouched:
-//   fc1: ten HALF-BLOCKS per tile (agent a, ring slots 12 hf .. 12 hf + 11: K = 72).  A half-block is one TMA box [12][6][128]
+//   fc1: 2 NA HALF-BLOCKS per tile (agent a, ring slots 12 hf .. 12 hf + 11: K = 72).  A half-block is one TMA box [12][6][128]
 //        into one of three staging buffers (requested three half-blocks ahead: the HBM stream never waits for the workers)
 //        plus the matching half of agent a's fc1 block -- ring rotation folded into the weights like k_policy's W1 -- into
 //        one of four weight buffers (two ahead); the workers split it into one of two TMEM operand buffers while the MMAs
 //        of the previous half-block run (acc1 += X Wc^T: 9 k-steps x (hi, lo)); the first half-block also adds the actions'
-//        20 columns (K padded to 24)
-//   per agent i = 0..4: E1: acc1 + bias(i) -> LayerNorm -> ReLU -> split -> A2[i & 1];  M2: acc2[i & 1] = A2 W2^T;  E2: ReLU,
+//        4 NA columns (K padded to 24)
+//   per agent i = 0 .. NA - 1: E1: acc1 + bias(i) -> LayerNorm -> ReLU -> split -> A2[i & 1];  M2: acc2[i & 1] = A2 W2^T;  E2: ReLU,
 //        dot with fc3 (fp32, CUDA cores), four-thread reduction, + bias -> value[env][i];  operand and accumulator are
 //        double-buffered: E1 of agent i + 1 runs under fc2 of agent i
 // Workers and the MMA warp meet through two mbarrier pairs (a_ready[b], mma_done[b], b = TMEM buffer); every commit is
@@ -549,7 +554,6 @@ constexpr uint32_t CR_WH_BYTES = CR_WB_BYTES / 2;                            // 
 constexpr uint32_t CR_W2_BYTES = POL_HID * POL_HID * 4;                      // fc2: [16 kc][64 n][4]
 constexpr int CR_KACT = 24;                                                  // 20 action columns + 4 zero columns
 constexpr uint32_t CR_WA_BYTES = CR_KACT * POL_HID * 4;                      // [6 kc][64 n][4]
-constexpr int CR_HB = 2 * POL_NA;                                            // half-blocks per tile
 // small arrays (floats): b1a[5][64] (fc1.bias + the one-hot column of agent i), ln_g[64], ln_b[64], b2[64], w3[64], b3 (+ pad)
 constexpr int CV_B1A = 0, CV_LNG = 320, CV_LNB = 384, CV_B2 = 448, CV_W3 = 512, CV_B3 = 576, CV_FLOATS = 592;
 constexpr uint32_t CO_ST = 0, CO_WB = CO_ST + CR_NST * CR_ST_BYTES, CO_W2 = CO_WB + CR_NWB * CR_WH_BYTES, CO_WA = CO_W2 + CR_W2_BYTES,
@@ -569,12 +573,14 @@ static_assert(2 * CC_XB == CC_ACC1 && CC_XB + 128 <= CC_ACC1 && CC_ACC2_1 + 64 <
 struct CritParams {
     const float* ring; int64_t n_pad; int64_t n; int32_t slot;
     const float* Wc1rot; const float* W2; const float* Wa; const float* vec;
-    const float* actions;                                             // [n][5][4]
-    float* value;                                                     // [n][5]
+    const float* actions;                                             // [n][NA][4]
+    float* value;                                                     // [n][NA]
     int32_t use_tma;
 };
 
+template <int NA>
 __global__ void __launch_bounds__(CRIT_THREADS, 1) k_critic(const CritParams prm, const __grid_constant__ CUtensorMap tmap) {
+    constexpr int CR_HB = 2 * NA;                                            // half-blocks per tile
     extern __shared__ __align__(128) uint8_t smem[];
     const float* vec = reinterpret_cast<const float*>(smem + CO_VEC);
     float2* lnp = reinterpret_cast<float2*>(smem + CO_LN);
@@ -585,7 +591,7 @@ __global__ void __launch_bounds__(CRIT_THREADS, 1) k_critic(const CritParams prm
     const int row = tid & (POL_M - 1), qt = (tid >> 7) & (TPR - 1);
     const int64_t n_tiles = (prm.n + POL_M - 1) / POL_M;
     const int64_t n_my = (n_tiles > (int64_t)blockIdx.x) ? (n_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
-    const int64_t n_hb = n_my * CR_HB;                                       // half-blocks of this CTA, in order: g = 10 tile + 2 a + hf
+    const int64_t n_hb = n_my * CR_HB;                                       // half-blocks of this CTA, in order: g = 2 NA tile + 2 a + hf
 
     auto tile_of = [&](int64_t g) -> int64_t { return (int64_t)blockIdx.x + (g / CR_HB) * gridDim.x; };
     auto tma_request = [&](int64_t g) {                                      // one thread: half-block g -> staging buffer g % 3
@@ -600,7 +606,7 @@ __global__ void __launch_bounds__(CRIT_THREADS, 1) k_critic(const CritParams prm
         const size_t a = (size_t)((g % CR_HB) >> 1), hf = (size_t)(g & 1);
         mbar_expect_tx(bar, CR_WH_BYTES);
         tma_load_1d(smem_u32(smem + CO_WB + (g % CR_NWB) * CR_WH_BYTES),
-                    prm.Wc1rot + (((size_t)prm.slot * POL_NA + a) * 2 + hf) * (CR_WH_BYTES / 4), CR_WH_BYTES, bar);
+                    prm.Wc1rot + (((size_t)prm.slot * NA + a) * 2 + hf) * (CR_WH_BYTES / 4), CR_WH_BYTES, bar);
     };
     auto request = [&](int64_t g) {                                          // workers, rings narrower than a tile: LDGSTS, not pipelined
         const int a = (int)((g % CR_HB) >> 1), hf = (int)(g & 1);
@@ -611,7 +617,7 @@ __global__ void __launch_bounds__(CRIT_THREADS, 1) k_critic(const CritParams prm
         for (int k = tid >> 5; k < CR_KH; k += N_WORKERS / 32) {              // 16-byte chunks: 32 per row, one row per warp and trip
             const int sl = hf * (POL_H / 2) + k / POL_F, f = k % POL_F;
             float* dst = stage + k * POL_M + c4;
-            if (inside) cp_async16(dst, prm.ring + ((int64_t)(sl * POL_NA + a) * POL_F + f) * prm.n_pad + e0 + c4);
+            if (inside) cp_async16(dst, prm.ring + ((int64_t)(sl * NA + a) * POL_F + f) * prm.n_pad + e0 + c4);
             else *reinterpret_cast<float4*>(dst) = make_float4(0.f, 0.f, 0.f, 0.f);
         }
         cp_async_commit();
@@ -681,7 +687,7 @@ __global__ void __launch_bounds__(CRIT_THREADS, 1) k_critic(const CritParams prm
             __syncwarp();
             if (hb != CR_HB - 1) continue;
             // ---- fc2, once per agent row, operand / accumulator buffer i & 1
-            for (int i = 0; i < POL_NA; ++i) {
+            for (int i = 0; i < NA; ++i) {
                 const int bi = i & 1;
                 if (bi) { mbar_wait(bar_a0 + 8, pa1); pa1 ^= 1u; } else { mbar_wait(bar_a0, pa0); pa0 ^= 1u; }
                 tc_fence_after();
@@ -726,12 +732,12 @@ __global__ void __launch_bounds__(CRIT_THREADS, 1) k_critic(const CritParams prm
                 split_st4(lane_base, xhi + k0, xlo + k0, stage[(k0 + 0) * POL_M + row], stage[(k0 + 1) * POL_M + row],
                           stage[(k0 + 2) * POL_M + row], stage[(k0 + 3) * POL_M + row]);
             }
-            if (hb == 0 && qt < 3) {                                            // the env's 20 action values (+ 4 zero columns): 8 per thread
+            if (hb == 0 && qt < 3) {                                            // the env's 4 NA action values (+ zero columns to 24): 8 per thread
                 float v[8];
 #pragma unroll
                 for (int i = 0; i < 8; ++i) {
                     const int k = 8 * qt + i;
-                    v[i] = (live && k < POL_NA * POL_ACT) ? __ldg(prm.actions + e * (POL_NA * POL_ACT) + k) : 0.0f;
+                    v[i] = (live && k < NA * POL_ACT) ? __ldg(prm.actions + e * (NA * POL_ACT) + k) : 0.0f;
                 }
                 split_st4(lane_base, CC_ACTHI + 8 * qt, CC_ACTLO + 8 * qt, v[0], v[1], v[2], v[3]);
                 split_st4(lane_base, CC_ACTHI + 8 * qt + 4, CC_ACTLO + 8 * qt + 4, v[4], v[5], v[6], v[7]);
@@ -773,9 +779,9 @@ __global__ void __launch_bounds__(CRIT_THREADS, 1) k_critic(const CritParams prm
                 mbar_arrive(bar_a0 + 8 * (i & 1));
             };
             e1(0);
-            for (int i = 0; i < POL_NA; ++i) {
+            for (int i = 0; i < NA; ++i) {
                 const int bi = i & 1;
-                if (i + 1 < POL_NA) e1(i + 1);                                  // (its operand buffer was released by E2 of agent i - 1)
+                if (i + 1 < NA) e1(i + 1);                                  // (its operand buffer was released by E2 of agent i - 1)
                 if (bi) { mbar_wait(bar_m0 + 8, pm1); pm1 ^= 1u; } else { mbar_wait(bar_m0, pm0); pm0 ^= 1u; }
                 tc_fence_after();
                 float u[CPT];
@@ -789,7 +795,7 @@ __global__ void __launch_bounds__(CRIT_THREADS, 1) k_critic(const CritParams prm
                 tc_fence_before();
                 group_sync<1, N_WORKERS>();
                 if (qt == 0 && live)
-                    prm.value[e * POL_NA + i] = __fadd_rn(__fadd_rn(__fadd_rn(__fadd_rn(fc[row], fc[POL_M + row]), fc[2 * POL_M + row]), fc[3 * POL_M + row]), vec[CV_B3]);
+                    prm.value[e * NA + i] = __fadd_rn(__fadd_rn(__fadd_rn(__fadd_rn(fc[row], fc[POL_M + row]), fc[2 * POL_M + row]), fc[3 * POL_M + row]), vec[CV_B3]);
             }
         }
     }
@@ -852,20 +858,21 @@ __device__ __forceinline__ void gt_drain(const float* t, float* __restrict__ out
     }
 }
 
-//   k_window_gather   dense observation windows [n][5][144] (oldest entry first: get_obs, :387-401) of envs [0, n) from
+//   k_window_gather   dense observation windows [n][NA][144] (oldest entry first: get_obs, :387-401) of envs [0, n) from
 //                     the env-minor ring into rows of pitch `pitch` floats (a replay field, or a dense tensor)
+template <int NA>
 __global__ void __launch_bounds__(256) k_window_gather(const float* __restrict__ ring, int64_t n_pad, int slot, int64_t n,
                                                        float* __restrict__ out, int64_t pitch, int64_t row0, int64_t cap) {
     extern __shared__ float gt_tile[];                            // [144][129]
     const int64_t n_blk = (n + GT_ENVS - 1) / GT_ENVS;
-    for (int64_t blk = blockIdx.x; blk < n_blk * POL_NA; blk += gridDim.x) {
-        const int a = (int)(blk % POL_NA);
-        const int64_t e0 = (blk / POL_NA) * GT_ENVS;
+    for (int64_t blk = blockIdx.x; blk < n_blk * NA; blk += gridDim.x) {
+        const int a = (int)(blk % NA);
+        const int64_t e0 = (blk / NA) * GT_ENVS;
         // k = r * 6 + f: the r-th oldest entry lives in ring slot (slot + 1 + r) mod 24
         gt_fill<POL_OBS>(gt_tile, ring, n_pad, e0, n, [&](int k) {
             const int r = k / POL_F, f = k - r * POL_F;
             int s = slot + 1 + r; s = s >= POL_H ? s - POL_H : s;
-            return (s * POL_NA + a) * POL_F + f;
+            return (s * NA + a) * POL_F + f;
         }, nullptr);
         __syncthreads();
         gt_drain<POL_OBS>(gt_tile, out, pitch, a * POL_OBS, e0, n, row0, cap);
@@ -873,14 +880,15 @@ __global__ void __launch_bounds__(256) k_window_gather(const float* __restrict__
     }
 }
 
-// env-minor [320 = 5 agents x 64 units][n_pad] -> ring rows (row0 + e) mod cap of 320 contiguous floats: the hidden
-// states of the Transition (last_hid / hid, (1, 5, 64) per env) from the policy kernel's native layout; a tile is
-// (128 envs, one half of the 320 rows)
-constexpr int EM_ROWS = POL_NA * POL_HID, EM_KR = EM_ROWS / 2;
+// env-minor [NA x 64 units][n_pad] -> ring rows (row0 + e) mod cap of NA x 64 contiguous floats: the hidden states of the
+// Transition (last_hid / hid, (1, NA, 64) per env) from the policy kernel's native layout; a tile is (128 envs, one half
+// of the NA x 64 rows)
+template <int NA>
 __global__ void __launch_bounds__(256) k_em_gather(const float* __restrict__ src, int64_t n_pad, int64_t n,
                                                    float* __restrict__ out, int64_t row0, int64_t cap,
                                                    const uint8_t* __restrict__ zero_mask) {
-    extern __shared__ float gt_tile[];                            // [160][129]
+    constexpr int EM_ROWS = NA * POL_HID, EM_KR = EM_ROWS / 2;
+    extern __shared__ float gt_tile[];                            // [EM_KR][129]
     const int64_t n_blk = (n + GT_ENVS - 1) / GT_ENVS;
     for (int64_t blk = blockIdx.x; blk < n_blk * 2; blk += gridDim.x) {
         const int h = (int)(blk & 1);
@@ -902,6 +910,7 @@ __global__ void k_rows_to_ring(const float* __restrict__ src, int64_t n, int wid
 }
 
 // reward (fp64, one per env) repeated for the agents (model.py:221), done / last_step flags, all-ones availability
+template <int NA>
 __global__ void k_scalars_to_ring(const double* __restrict__ reward, const uint8_t* __restrict__ done, int64_t n, int last_step_all,
                                   float* __restrict__ f_reward, float* __restrict__ f_done, float* __restrict__ f_last,
                                   float* __restrict__ f_avail, int64_t row0, int64_t cap) {
@@ -911,26 +920,27 @@ __global__ void k_scalars_to_ring(const double* __restrict__ reward, const uint8
         const float d = done[e] ? 1.0f : 0.0f;
         if (f_reward) {
 #pragma unroll
-            for (int a = 0; a < POL_NA; ++a) f_reward[o * POL_NA + a] = r;
+            for (int a = 0; a < NA; ++a) f_reward[o * NA + a] = r;
         }
         if (f_done) f_done[o] = d;
         if (f_last) f_last[o] = (done[e] || last_step_all) ? 1.0f : 0.0f;      // done_ = done or t == max_steps - 1 (model.py:229)
         if (f_avail) {
 #pragma unroll
-            for (int j = 0; j < POL_NA * POL_ACT; ++j) f_avail[o * (POL_NA * POL_ACT) + j] = 1.0f;
+            for (int j = 0; j < NA * POL_ACT; ++j) f_avail[o * (NA * POL_ACT) + j] = 1.0f;
         }
     }
 }
 
 // The small Transition fields of n envs in ONE launch (model.py:221, :229-242): action / log_prob_a rows, reward repeated per
 // agent, done, last_step (= done, or every env when last_step_all), all-ones action_avail, and -- zero_values -- value /
-// next_value as zeros (MADDPG's losses recompute both).  Thread = (env, column of the 20-wide rows): coalesced throughout.
+// next_value as zeros (MADDPG's losses recompute both).  Thread = (env, column of the NA x 4 wide rows): coalesced throughout.
+template <int NA>
 __global__ void k_transition_tail(const float* __restrict__ action, const float* __restrict__ logp, const double* __restrict__ reward,
                                   const uint8_t* __restrict__ done, int64_t n, int last_step_all, int zero_values,
                                   float* __restrict__ f_action, float* __restrict__ f_logp, float* __restrict__ f_value,
                                   float* __restrict__ f_next_value, float* __restrict__ f_reward, float* __restrict__ f_done,
                                   float* __restrict__ f_last, float* __restrict__ f_avail, int64_t row0, int64_t cap) {
-    constexpr int W = POL_NA * POL_ACT;
+    constexpr int W = NA * POL_ACT;
     const int64_t total = n * W;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
         const int64_t e = i / W;
@@ -939,48 +949,50 @@ __global__ void k_transition_tail(const float* __restrict__ action, const float*
         f_action[o * W + c] = action[i];
         if (f_logp) f_logp[o * W + c] = logp[i];
         if (f_avail) f_avail[o * W + c] = 1.0f;
-        if (c < POL_NA) {
-            f_reward[o * POL_NA + c] = (float)reward[e];
-            if (zero_values) { f_value[o * POL_NA + c] = 0.0f; f_next_value[o * POL_NA + c] = 0.0f; }
+        if (c < NA) {
+            f_reward[o * NA + c] = (float)reward[e];
+            if (zero_values) { f_value[o * NA + c] = 0.0f; f_next_value[o * NA + c] = 0.0f; }
         }
-        if (c == POL_NA) { const bool d = done[e] != 0; f_done[o] = d ? 1.0f : 0.0f; f_last[o] = (d || last_step_all) ? 1.0f : 0.0f; }
+        if (c == NA) { const bool d = done[e] != 0; f_done[o] = d ? 1.0f : 0.0f; f_last[o] = (d || last_step_all) ? 1.0f : 0.0f; }
     }
 }
 
 // MADDPG critic input (madrl/models/maddpg.py:29-66, shared parameters, agent_id): for batch row b and agent i
-//   [ obs of all agents (5 x 144) | one-hot(i) (5) | actions of all agents (5 x 4) ]   = 745 floats
+//   [ obs of all agents (NA x 144) | one-hot(i) (NA) | actions of all agents (NA x 4) ]   = 149 NA floats (745 for five agents)
+template <int NA>
 __global__ void k_critic_input(const float* __restrict__ state, const float* __restrict__ action, int64_t batch, float* __restrict__ out) {
-    constexpr int W = POL_NA * POL_OBS + POL_NA + POL_NA * POL_ACT;
-    const int64_t total = batch * POL_NA * W;
+    constexpr int W = NA * POL_OBS + NA + NA * POL_ACT;
+    const int64_t total = batch * NA * W;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
         const int c = (int)(i % W);
         const int64_t bi = i / W;
-        const int ag = (int)(bi % POL_NA);
-        const int64_t b = bi / POL_NA;
+        const int ag = (int)(bi % NA);
+        const int64_t b = bi / NA;
         float v;
-        if (c < POL_NA * POL_OBS) v = state[b * (POL_NA * POL_OBS) + c];
-        else if (c < POL_NA * POL_OBS + POL_NA) v = (c - POL_NA * POL_OBS == ag) ? 1.0f : 0.0f;
-        else v = action[b * (POL_NA * POL_ACT) + (c - POL_NA * POL_OBS - POL_NA)];
+        if (c < NA * POL_OBS) v = state[b * (NA * POL_OBS) + c];
+        else if (c < NA * POL_OBS + NA) v = (c - NA * POL_OBS == ag) ? 1.0f : 0.0f;
+        else v = action[b * (NA * POL_ACT) + (c - NA * POL_OBS - NA)];
         out[i] = v;
     }
 }
 
 // reward_normalisation (model.py:321-322): nn.BatchNorm1d(n_agents) in training mode with its initial affine
 // parameters (weight 1, bias 0: the module is in no optimiser): per agent column, (x - mean) / sqrt(var_biased + 1e-5)
+template <int NA>
 __global__ void k_reward_batchnorm(const float* __restrict__ reward, int64_t batch, float* __restrict__ out) {
     const int a = blockIdx.x;                                       // one block per agent column
     __shared__ double sh[2][256];
     double s = 0.0, ss = 0.0;
-    for (int64_t b = threadIdx.x; b < batch; b += blockDim.x) { const double x = reward[b * POL_NA + a]; s += x; }
+    for (int64_t b = threadIdx.x; b < batch; b += blockDim.x) { const double x = reward[b * NA + a]; s += x; }
     sh[0][threadIdx.x] = s; __syncthreads();
     for (int d = 128; d > 0; d >>= 1) { if ((int)threadIdx.x < d) sh[0][threadIdx.x] += sh[0][threadIdx.x + d]; __syncthreads(); }
     const double mean = sh[0][0] / (double)batch;
-    for (int64_t b = threadIdx.x; b < batch; b += blockDim.x) { const double x = reward[b * POL_NA + a] - mean; ss += x * x; }
+    for (int64_t b = threadIdx.x; b < batch; b += blockDim.x) { const double x = reward[b * NA + a] - mean; ss += x * x; }
     sh[1][threadIdx.x] = ss; __syncthreads();
     for (int d = 128; d > 0; d >>= 1) { if ((int)threadIdx.x < d) sh[1][threadIdx.x] += sh[1][threadIdx.x + d]; __syncthreads(); }
     const double var = sh[1][0] / (double)batch;
     const float rstd = (float)(1.0 / sqrt(var + 1e-5)), meanf = (float)mean;
-    for (int64_t b = threadIdx.x; b < batch; b += blockDim.x) out[b * POL_NA + a] = (reward[b * POL_NA + a] - meanf) * rstd;
+    for (int64_t b = threadIdx.x; b < batch; b += blockDim.x) out[b * NA + a] = (reward[b * NA + a] - meanf) * rstd;
 }
 
 int gt_grid(int64_t tiles, int per_sm) {       // persistent grid of the transposing gathers: per_sm CTAs per SM
@@ -990,6 +1002,18 @@ int gt_grid(int64_t tiles, int per_sm) {       // persistent grid of the transpo
     const int64_t g = (int64_t)sms * per_sm;
     return (int)(tiles < g ? (tiles < 1 ? 1 : tiles) : g);
 }
+
+// One instantiation per agent count, indexed by the handle's na (entry 0 unused)
+#define NA_TABLE(k) {nullptr, k<1>, k<2>, k<3>, k<4>, k<5>}
+decltype(&k_policy<5>) const K_POLICY[POL_NA_MAX + 1] = NA_TABLE(k_policy);
+decltype(&k_critic<5>) const K_CRITIC[POL_NA_MAX + 1] = NA_TABLE(k_critic);
+decltype(&k_window_gather<5>) const K_WINDOW_GATHER[POL_NA_MAX + 1] = NA_TABLE(k_window_gather);
+decltype(&k_em_gather<5>) const K_EM_GATHER[POL_NA_MAX + 1] = NA_TABLE(k_em_gather);
+decltype(&k_scalars_to_ring<5>) const K_SCALARS_TO_RING[POL_NA_MAX + 1] = NA_TABLE(k_scalars_to_ring);
+decltype(&k_transition_tail<5>) const K_TRANSITION_TAIL[POL_NA_MAX + 1] = NA_TABLE(k_transition_tail);
+decltype(&k_critic_input<5>) const K_CRITIC_INPUT[POL_NA_MAX + 1] = NA_TABLE(k_critic_input);
+decltype(&k_reward_batchnorm<5>) const K_REWARD_BATCHNORM[POL_NA_MAX + 1] = NA_TABLE(k_reward_batchnorm);
+#undef NA_TABLE
 
 float round_tf32(float x) {                    // round to nearest even on the 13 dropped mantissa bits
     uint32_t u; std::memcpy(&u, &x, 4);
@@ -1004,6 +1028,7 @@ float round_tf32(float x) {                    // round to nearest even on the 1
 
 struct FpPolicy {
     int device = 0;
+    int na = POL_NA_MAX;                           // agents per env, fixed at fp_policy_create_agents
     int loaded = 0;
     int attr_window = 0, attr_hidden = 0;          // opt-in shared-memory sizes of the gather kernels set on this handle's device
     float* d_W1rot = nullptr; float* d_Wg = nullptr; float* d_vec = nullptr;
@@ -1030,8 +1055,8 @@ EncodeTiledFn encode_tiled_fn() {                  // the driver entry point, wi
 }
 }  // namespace
 
-// The ring as a 3-D tensor [24 slots][30 = agent x feature][n_pad envs] (innermost first); a tile is the box [24][6][128] at
-// (env block, agent * 6, 0); envs past n_pad read as zeros.  Rings narrower than a tile: *use_tma = 0 (LDGSTS path).
+// The ring as a 3-D tensor [24 slots][na x 6 = agent x feature][n_pad envs] (innermost first); a tile is the box [24][6][128]
+// at (env block, agent * 6, 0); envs past n_pad read as zeros.  Rings narrower than a tile: *use_tma = 0 (LDGSTS path).
 static int ring_tensor_map(FpPolicy* p, const float* d_ring, int64_t n_pad, CUtensorMap* tmap, int32_t* use_tma, const char* who,
                            int box_slots = POL_H) {
     std::memset(tmap, 0, sizeof(*tmap));
@@ -1039,8 +1064,8 @@ static int ring_tensor_map(FpPolicy* p, const float* d_ring, int64_t n_pad, CUte
     if (n_pad >= POL_M && ((uintptr_t)d_ring & 15) == 0) {
         EncodeTiledFn enc = encode_tiled_fn();
         if (!enc) return fail(p, FP_ECUDA, std::string(who) + ": cuTensorMapEncodeTiled is not available from this driver");
-        const cuuint64_t gdim[3] = {(cuuint64_t)n_pad, (cuuint64_t)(POL_NA * POL_F), (cuuint64_t)POL_H};
-        const cuuint64_t gstride[2] = {(cuuint64_t)n_pad * 4, (cuuint64_t)n_pad * 4 * (POL_NA * POL_F)};
+        const cuuint64_t gdim[3] = {(cuuint64_t)n_pad, (cuuint64_t)(p->na * POL_F), (cuuint64_t)POL_H};
+        const cuuint64_t gstride[2] = {(cuuint64_t)n_pad * 4, (cuuint64_t)n_pad * 4 * (p->na * POL_F)};
         const cuuint32_t box[3] = {POL_M, POL_F, (cuuint32_t)box_slots}, estr[3] = {1, 1, 1};
         const CUresult r = enc(tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(d_ring), gdim, gstride, box, estr,
                                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
@@ -1053,16 +1078,21 @@ static int ring_tensor_map(FpPolicy* p, const float* d_ring, int64_t n_pad, CUte
 
 extern "C" {
 
-int fp_policy_create(int device, FpPolicy** out) {
+int fp_policy_create_agents(int device, int32_t n_agents, FpPolicy** out) {
     if (!out) return FP_EINVAL;
+    if (n_agents < 1 || n_agents > POL_NA_MAX)
+        return fail<FpPolicy>(nullptr, FP_EINVAL, "fp_policy_create_agents: n_agents must be in [1, 5], got " + std::to_string(n_agents));
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) return fail<FpPolicy>(nullptr, FP_ECUDA, "fp_policy_create: no CUDA device (there is no CPU fallback)");
     if (device < 0 || device >= ndev) return fail<FpPolicy>(nullptr, FP_EINVAL, "fp_policy_create: bad device index");
     FpPolicy* p = new FpPolicy();
     p->device = device;
+    p->na = n_agents;
     *out = p;
     return FP_OK;
 }
+
+int fp_policy_create(int device, FpPolicy** out) { return fp_policy_create_agents(device, POL_NA_MAX, out); }
 
 int fp_policy_destroy(FpPolicy* p) {
     if (!p) return FP_OK;
@@ -1077,7 +1107,7 @@ const char* fp_policy_last_error(const FpPolicy* p) { return p ? p->err.c_str() 
 int64_t fp_policy_launch_count(const FpPolicy* p) { return p ? p->launches : 0; }
 
 // Host weights in torch's layouts (state_dict of RNNAgent, madrl/agents/rnn_agent.py:11-16):
-//   fc1.weight [64][149] (144 observation columns + 5 agent-id columns), fc1.bias [64], layernorm.weight / .bias [64],
+//   fc1.weight [64][144 + na] (144 observation columns + na agent-id columns), fc1.bias [64], layernorm.weight / .bias [64],
 //   rnn.weight_ih / weight_hh [192][64] (rows r | z | n), rnn.bias_ih / bias_hh [192], fc2.weight [4][64], fc2.bias [4]
 int fp_policy_load(FpPolicy* p, const float* fc1_w, const float* fc1_b, const float* ln_g, const float* ln_b, const float* w_ih,
                    const float* w_hh, const float* b_ih, const float* b_hh, const float* fc2_w, const float* fc2_b) {
@@ -1085,7 +1115,7 @@ int fp_policy_load(FpPolicy* p, const float* fc1_w, const float* fc1_b, const fl
     if (!fc1_w || !fc1_b || !ln_g || !ln_b || !w_ih || !w_hh || !b_ih || !b_hh || !fc2_w || !fc2_b)
         return fail(p, FP_EINVAL, "fp_policy_load: null weight array");
     USE_DEVICE(p);
-    const int KIN = POL_OBS + POL_NA;
+    const int na = p->na, KIN = POL_OBS + na;
     // fc1: 24 column rotations, UMMA K-major layout [kc][n][4]; ring slot s holds history entry r = (s - q - 1) mod 24
     // when the newest slot is q, i.e. K index s * 6 + f must carry weight column r * 6 + f
     std::vector<float> W1((size_t)POL_H * POL_OBS * POL_HID, 0.0f);
@@ -1124,7 +1154,7 @@ int fp_policy_load(FpPolicy* p, const float* fc1_w, const float* fc1_b, const fl
     }
     for (int o = 0; o < POL_ACT; ++o)
         for (int k = 0; k < POL_HID; ++k) vec[V_W2 + 4 * k + o] = fc2_w[(size_t)o * POL_HID + k];      // fc2 runs in fp32: unrounded
-    for (int a = 0; a < POL_NA; ++a)
+    for (int a = 0; a < na; ++a)
         for (int n = 0; n < POL_HID; ++n) vec[V_B1A + a * POL_HID + n] = fc1_b[n] + fc1_w[(size_t)n * KIN + POL_OBS + a];   // one-hot column folded in
     for (int n = 0; n < POL_HID; ++n) { vec[V_LNG + n] = ln_g[n]; vec[V_LNB + n] = ln_b[n]; }
     // gate biases in the exponential's unit (see sigmoid8 / tanh8_scaled)
@@ -1140,15 +1170,15 @@ int fp_policy_load(FpPolicy* p, const float* fc1_w, const float* fc1_b, const fl
     CUDA_TRY(p, cudaMemcpy(p->d_W1rot, W1.data(), W1.size() * 4, cudaMemcpyHostToDevice));
     CUDA_TRY(p, cudaMemcpy(p->d_Wg, Wg.data(), Wg.size() * 4, cudaMemcpyHostToDevice));
     CUDA_TRY(p, cudaMemcpy(p->d_vec, vec.data(), vec.size() * 4, cudaMemcpyHostToDevice));
-    CUDA_TRY(p, cudaFuncSetAttribute(k_policy, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)POL_SMEM));
+    CUDA_TRY(p, cudaFuncSetAttribute(K_POLICY[na], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)POL_SMEM));
     p->loaded = 1;
     return FP_OK;
 }
 
-// One acting step for n_envs x 5 agents.  d_ring / slot / n_pad: the observation ring (fp_obs_ring, fp_step_ring).
-// d_hid_in (may be null = zeros) / d_hid_out: [n_envs][5][64]; d_reset (may be null): envs whose hidden state restarts
+// One acting step for n_envs x na agents (na = the handle's agent count).  d_ring / slot / n_pad: the observation ring (fp_obs_ring, fp_step_ring).
+// d_hid_in (may be null = zeros) / d_hid_out: [n_envs][na][64] (or env-minor [na][64][n_pad]); d_reset (may be null): envs whose hidden state restarts
 // at zero (init_hidden, model.py:211).  d_mean, d_logp may be null.  explore = 1: status 'train' with exploration
-// (d_eps = caller-supplied standard-normal draws [n_envs][5][4], or null: Philox keyed by (seed, row, step));
+// (d_eps = caller-supplied standard-normal draws [n_envs][na][4], or null: Philox keyed by (seed, row, step));
 // explore = 0: status 'test'.  std = fixed_policy_std (default.yaml: 1.0).
 int fp_policy_act(FpPolicy* p, const float* d_ring, int32_t slot, int64_t n_pad, int64_t n_envs, const float* d_hid_in,
                   const uint8_t* d_reset, float* d_hid_out, int32_t hid_env_minor, float* d_mean, float* d_action, float* d_logp,
@@ -1175,13 +1205,13 @@ int fp_policy_act(FpPolicy* p, const float* d_ring, int32_t slot, int64_t n_pad,
     }
     int sms = 0;
     CUDA_TRY(p, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, p->device));
-    const int64_t tiles = (n_envs + POL_M - 1) / POL_M * POL_NA;
+    const int64_t tiles = (n_envs + POL_M - 1) / POL_M * p->na;
     const int grid = (int)(tiles < sms ? tiles : sms);
-    k_policy<<<grid, POL_THREADS, POL_SMEM, (cudaStream_t)stream>>>(prm, tmap);
+    K_POLICY[p->na]<<<grid, POL_THREADS, POL_SMEM, (cudaStream_t)stream>>>(prm, tmap);
     return launched(p, "k_policy");
 }
 
-// select_action alone on stored fc2 outputs d_mean [n_envs][5][4] (fp_policy_act's d_mean): another exploration draw of the
+// select_action alone on stored fc2 outputs d_mean [n_envs][na][4] (fp_policy_act's d_mean): another exploration draw of the
 // same policy evaluation (same arguments as fp_policy_act's sampling part; bit-identical to re-running it with these draws).
 int fp_policy_sample(FpPolicy* p, const float* d_mean, int64_t n_envs, float* d_action, float* d_logp, const float* d_eps,
                      uint64_t seed, uint64_t step, float std_, int32_t explore, void* stream) {
@@ -1189,48 +1219,48 @@ int fp_policy_sample(FpPolicy* p, const float* d_mean, int64_t n_envs, float* d_
     if (!d_mean || !d_action || n_envs < 1) return fail(p, FP_EINVAL, "fp_policy_sample: bad arguments");
     if (!(std_ > 0.0f)) return fail(p, FP_EINVAL, "fp_policy_sample: std must be positive");
     USE_DEVICE(p);
-    k_sample<<<grid_for(n_envs * POL_NA), 256, 0, (cudaStream_t)stream>>>(d_mean, n_envs * POL_NA, explore, d_eps, seed, step, std_, std::log(std_),
+    k_sample<<<grid_for(n_envs * p->na), 256, 0, (cudaStream_t)stream>>>(d_mean, n_envs * p->na, explore, d_eps, seed, step, std_, std::log(std_),
                                                                           d_action, d_logp);
     return launched(p, "k_sample");
 }
 
 // One-shot sink for the NEXT fp_policy_act: while it evaluates the policy, its writer warps copy the dense get_obs windows
-// [5][144] of envs [0, n) -- the very blocks the kernel has staged -- into rows (row0 + e) mod cap of pitch `pitch` floats: the
+// [na][144] of envs [0, n) -- the very blocks the kernel has staged -- into rows (row0 + e) mod cap of pitch `pitch` floats: the
 // Transition's `state` (model.py:230-237) without a separate pass over the ring (fp_policy_gather_windows).  Needs a ring of
 // at least 128 envs (n_pad >= 128).
 int fp_policy_state_sink(FpPolicy* p, float* d_field, int64_t pitch, int64_t row0, int64_t cap, int64_t n) {
     if (!p) return FP_EINVAL;
-    if (!d_field || n < 1 || pitch < POL_NA * POL_OBS || (pitch & 3) || ((uintptr_t)d_field & 15) || row0 < 0 || cap < n || row0 >= cap)
+    if (!d_field || n < 1 || pitch < p->na * POL_OBS || (pitch & 3) || ((uintptr_t)d_field & 15) || row0 < 0 || cap < n || row0 >= cap)
         return fail(p, FP_EINVAL, "fp_policy_state_sink: bad arguments");
     p->sink_out = d_field; p->sink_pitch = pitch; p->sink_row0 = row0; p->sink_cap = cap; p->sink_n = n;
     return FP_OK;
 }
 
-// Dense observation windows of envs [0, n) (get_obs layout [n][5][144], oldest entry first) from the ring into rows
+// Dense observation windows of envs [0, n) (get_obs layout [n][na][144], oldest entry first) from the ring into rows
 // (row0 + e) mod cap of pitch `pitch` floats: a replay field (state / next_state of the Transition, model.py:230-237)
 // or, with row0 = 0 and cap >= n, a dense tensor.
 int fp_policy_gather_windows(FpPolicy* p, const float* d_ring, int32_t slot, int64_t n_pad, int64_t n, float* d_out, int64_t pitch,
                              int64_t row0, int64_t cap, void* stream) {
     if (!p) return FP_EINVAL;
-    if (!d_ring || !d_out || n < 1 || pitch < POL_NA * POL_OBS || row0 < 0 || cap < n || row0 >= cap || slot < 0 || slot >= POL_H)
+    if (!d_ring || !d_out || n < 1 || pitch < p->na * POL_OBS || row0 < 0 || cap < n || row0 >= cap || slot < 0 || slot >= POL_H)
         return fail(p, FP_EINVAL, "fp_policy_gather_windows: bad arguments");
     USE_DEVICE(p);
     constexpr int smem_w = POL_OBS * GT_STRIDE * (int)sizeof(float);
-    if (!p->attr_window) { CUDA_TRY(p, cudaFuncSetAttribute(k_window_gather, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_w)); p->attr_window = 1; }
-    k_window_gather<<<gt_grid(((n + GT_ENVS - 1) / GT_ENVS) * POL_NA, 3), 256, smem_w, (cudaStream_t)stream>>>(d_ring, n_pad, slot, n, d_out, pitch, row0, cap);
+    if (!p->attr_window) { CUDA_TRY(p, cudaFuncSetAttribute(K_WINDOW_GATHER[p->na], cudaFuncAttributeMaxDynamicSharedMemorySize, smem_w)); p->attr_window = 1; }
+    K_WINDOW_GATHER[p->na]<<<gt_grid(((n + GT_ENVS - 1) / GT_ENVS) * p->na, 3), 256, smem_w, (cudaStream_t)stream>>>(d_ring, n_pad, slot, n, d_out, pitch, row0, cap);
     return launched(p, "k_window_gather");
 }
 
-// Hidden states in the policy kernel's env-minor layout [5][64][n_pad] -> replay rows (last_hid / hid, 320 floats per env);
+// Hidden states in the policy kernel's env-minor layout [na][64][n_pad] -> replay rows (last_hid / hid, na x 64 floats per env);
 // d_zero_mask (may be null): envs whose row is written as zeros (a restarted env's last_hid is the zero state it acted from)
 int fp_policy_hidden_to_ring(FpPolicy* p, const float* d_hid_em, int64_t n_pad, int64_t n, float* d_field, int64_t row0, int64_t cap,
                              const uint8_t* d_zero_mask, void* stream) {
     if (!p) return FP_EINVAL;
     if (!d_hid_em || !d_field || n < 1 || n_pad < n || row0 < 0 || cap < n || row0 >= cap) return fail(p, FP_EINVAL, "fp_policy_hidden_to_ring: bad arguments");
     USE_DEVICE(p);
-    constexpr int smem_h = EM_KR * GT_STRIDE * (int)sizeof(float);
-    if (!p->attr_hidden) { CUDA_TRY(p, cudaFuncSetAttribute(k_em_gather, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_h)); p->attr_hidden = 1; }
-    k_em_gather<<<gt_grid(((n + GT_ENVS - 1) / GT_ENVS) * 2, 2), 256, smem_h, (cudaStream_t)stream>>>(d_hid_em, n_pad, n, d_field, row0, cap, d_zero_mask);
+    const int smem_h = p->na * POL_HID / 2 * GT_STRIDE * (int)sizeof(float);        // [na x 64 / 2][129]
+    if (!p->attr_hidden) { CUDA_TRY(p, cudaFuncSetAttribute(K_EM_GATHER[p->na], cudaFuncAttributeMaxDynamicSharedMemorySize, smem_h)); p->attr_hidden = 1; }
+    K_EM_GATHER[p->na]<<<gt_grid(((n + GT_ENVS - 1) / GT_ENVS) * 2, 2), 256, smem_h, (cudaStream_t)stream>>>(d_hid_em, n_pad, n, d_field, row0, cap, d_zero_mask);
     return launched(p, "k_em_gather");
 }
 
@@ -1247,7 +1277,7 @@ int fp_policy_scalars_to_ring(FpPolicy* p, const double* d_reward, const uint8_t
     if (!p) return FP_EINVAL;
     if (!d_reward || !d_done || n < 1 || row0 < 0 || cap < n || row0 >= cap) return fail(p, FP_EINVAL, "fp_policy_scalars_to_ring: bad arguments");
     USE_DEVICE(p);
-    k_scalars_to_ring<<<grid_for(n), 256, 0, (cudaStream_t)stream>>>(d_reward, d_done, n, last_step_all, f_reward, f_done, f_last, f_avail, row0, cap);
+    K_SCALARS_TO_RING[p->na]<<<grid_for(n), 256, 0, (cudaStream_t)stream>>>(d_reward, d_done, n, last_step_all, f_reward, f_done, f_last, f_avail, row0, cap);
     return launched(p, "k_scalars_to_ring");
 }
 
@@ -1260,41 +1290,41 @@ int fp_policy_transition_tail(FpPolicy* p, const float* d_action, const float* d
         (zero_values && (!f_value || !f_next_value)) || n < 1 || row0 < 0 || cap < n || row0 >= cap)
         return fail(p, FP_EINVAL, "fp_policy_transition_tail: bad arguments");
     USE_DEVICE(p);
-    k_transition_tail<<<grid_for(n * POL_NA * POL_ACT), 256, 0, (cudaStream_t)stream>>>(d_action, d_logp, d_reward, d_done, n, last_step_all,
+    K_TRANSITION_TAIL[p->na]<<<grid_for(n * p->na * POL_ACT), 256, 0, (cudaStream_t)stream>>>(d_action, d_logp, d_reward, d_done, n, last_step_all,
                                                                                        zero_values, f_action, f_logp, f_value, f_next_value,
                                                                                        f_reward, f_done, f_last, f_avail, row0, cap);
     return launched(p, "k_transition_tail");
 }
 
 // Critic weights, HOST fp32 arrays in torch's state_dict layouts (MLPCritic, madrl/critics/mlp_critic.py:5-20, as
-// MADDPG.construct_value_net builds it, maddpg.py:18-27): fc1.weight [64][745] (720 observation columns | 5 agent-id columns |
-// 20 action columns), fc1.bias [64], layernorm.weight / .bias [64], fc2.weight [64][64], fc2.bias [64], fc3.weight [1][64],
+// MADDPG.construct_value_net builds it, maddpg.py:18-27): fc1.weight [64][149 na] (144 na observation columns | na agent-id
+// columns | 4 na action columns), fc1.bias [64], layernorm.weight / .bias [64], fc2.weight [64][64], fc2.bias [64], fc3.weight [1][64],
 // fc3.bias [1].
 int fp_critic_load(FpPolicy* p, const float* fc1_w, const float* fc1_b, const float* ln_g, const float* ln_b, const float* fc2_w,
                    const float* fc2_b, const float* fc3_w, const float* fc3_b) {
     if (!p) return FP_EINVAL;
     if (!fc1_w || !fc1_b || !ln_g || !ln_b || !fc2_w || !fc2_b || !fc3_w || !fc3_b) return fail(p, FP_EINVAL, "fp_critic_load: null weight array");
     USE_DEVICE(p);
-    const int KIN = POL_NA * POL_OBS + POL_NA + POL_NA * POL_ACT;          // 745
+    const int na = p->na, KIN = na * POL_OBS + na + na * POL_ACT;          // 149 na: 745 for five agents
     const size_t blk = CR_WB_BYTES / 4;
     // fc1, observation columns: per ring rotation q and agent block a, UMMA K-major layout [kc][n][4] (see fp_policy_load)
-    std::vector<float> W1((size_t)POL_H * POL_NA * blk, 0.0f);
+    std::vector<float> W1((size_t)POL_H * na * blk, 0.0f);
     for (int q = 0; q < POL_H; ++q)
-        for (int a = 0; a < POL_NA; ++a)
+        for (int a = 0; a < na; ++a)
             for (int sl = 0; sl < POL_H; ++sl) {
                 const int r = ((sl - q - 1) % POL_H + POL_H) % POL_H;
                 for (int f = 0; f < POL_F; ++f) {
                     const int k = sl * POL_F + f, src = a * POL_OBS + r * POL_F + f;
                     for (int n = 0; n < POL_HID; ++n)
-                        W1[((size_t)q * POL_NA + a) * blk + ((size_t)(k >> 2) * POL_HID + n) * 4 + (k & 3)] = round_tf32(fc1_w[(size_t)n * KIN + src]);
+                        W1[((size_t)q * na + a) * blk + ((size_t)(k >> 2) * POL_HID + n) * 4 + (k & 3)] = round_tf32(fc1_w[(size_t)n * KIN + src]);
                 }
             }
     std::vector<float> W2(CR_W2_BYTES / 4, 0.0f), Wa(CR_WA_BYTES / 4, 0.0f), vec(CV_FLOATS, 0.0f);
     for (int n = 0; n < POL_HID; ++n) {
         for (int k = 0; k < POL_HID; ++k) W2[((size_t)(k >> 2) * POL_HID + n) * 4 + (k & 3)] = round_tf32(fc2_w[(size_t)n * POL_HID + k]);
-        for (int k = 0; k < POL_NA * POL_ACT; ++k)
-            Wa[((size_t)(k >> 2) * POL_HID + n) * 4 + (k & 3)] = round_tf32(fc1_w[(size_t)n * KIN + POL_NA * POL_OBS + POL_NA + k]);
-        for (int a = 0; a < POL_NA; ++a) vec[CV_B1A + a * POL_HID + n] = fc1_b[n] + fc1_w[(size_t)n * KIN + POL_NA * POL_OBS + a];   // one-hot column folded in
+        for (int k = 0; k < na * POL_ACT; ++k)
+            Wa[((size_t)(k >> 2) * POL_HID + n) * 4 + (k & 3)] = round_tf32(fc1_w[(size_t)n * KIN + na * POL_OBS + na + k]);
+        for (int a = 0; a < na; ++a) vec[CV_B1A + a * POL_HID + n] = fc1_b[n] + fc1_w[(size_t)n * KIN + na * POL_OBS + a];   // one-hot column folded in
         vec[CV_LNG + n] = ln_g[n]; vec[CV_LNB + n] = ln_b[n]; vec[CV_B2 + n] = fc2_b[n]; vec[CV_W3 + n] = fc3_w[n];           // fc3 runs in fp32: unrounded
     }
     vec[CV_B3] = fc3_b[0];
@@ -1307,13 +1337,13 @@ int fp_critic_load(FpPolicy* p, const float* fc1_w, const float* fc1_b, const fl
     CUDA_TRY(p, cudaMemcpy(p->d_Wc2, W2.data(), W2.size() * 4, cudaMemcpyHostToDevice));
     CUDA_TRY(p, cudaMemcpy(p->d_Wca, Wa.data(), Wa.size() * 4, cudaMemcpyHostToDevice));
     CUDA_TRY(p, cudaMemcpy(p->d_cvec, vec.data(), vec.size() * 4, cudaMemcpyHostToDevice));
-    CUDA_TRY(p, cudaFuncSetAttribute(k_critic, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CR_SMEM));
+    CUDA_TRY(p, cudaFuncSetAttribute(K_CRITIC[na], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CR_SMEM));
     p->critic_loaded = 1;
     return FP_OK;
 }
 
-// MADDPG.value (maddpg.py:29-76) for n_envs envs: d_value[n_envs][5] = the critic on (the observation ring's windows of all
-// agents, agent id, d_actions[n_envs][5][4]) -- the Transition's value (model.py:217) or, on the ring after the step and a
+// MADDPG.value (maddpg.py:29-76) for n_envs envs: d_value[n_envs][na] = the critic on (the observation ring's windows of all
+// agents, agent id, d_actions[n_envs][na][4]) -- the Transition's value (model.py:217) or, on the ring after the step and a
 // second sampled action, next_value (:225-226).
 int fp_critic_value(FpPolicy* p, const float* d_ring, int32_t slot, int64_t n_pad, int64_t n_envs, const float* d_actions,
                     float* d_value, void* stream) {
@@ -1333,12 +1363,12 @@ int fp_critic_value(FpPolicy* p, const float* d_ring, int32_t slot, int64_t n_pa
     CUDA_TRY(p, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, p->device));
     const int64_t tiles = (n_envs + POL_M - 1) / POL_M;
     const int grid = (int)(tiles < sms ? tiles : sms);
-    k_critic<<<grid, CRIT_THREADS, CR_SMEM, (cudaStream_t)stream>>>(prm, tmap);
+    K_CRITIC[p->na]<<<grid, CRIT_THREADS, CR_SMEM, (cudaStream_t)stream>>>(prm, tmap);
     return launched(p, "k_critic");
 }
 
 // Learner feed (unpack_data, madrl/models/model.py:308-323, on a sampled batch already on the device):
-//   d_critic_in [batch * 5][745]: the MADDPG critic's input rows (maddpg.py:29-66); d_reward_norm [batch][5]: the
+//   d_critic_in [batch * na][149 na]: the MADDPG critic's input rows (maddpg.py:29-66); d_reward_norm [batch][na]: the
 //   reward after reward_normalisation (BatchNorm1d over the batch, training mode).  Either may be null.
 int fp_learner_feed(FpPolicy* p, const float* d_state, const float* d_action, const float* d_reward, int64_t batch,
                     float* d_critic_in, float* d_reward_norm, void* stream) {
@@ -1346,8 +1376,8 @@ int fp_learner_feed(FpPolicy* p, const float* d_state, const float* d_action, co
     if (batch < 1 || (d_critic_in && (!d_state || !d_action)) || (d_reward_norm && !d_reward)) return fail(p, FP_EINVAL, "fp_learner_feed: bad arguments");
     USE_DEVICE(p);
     if (d_critic_in)
-        k_critic_input<<<grid_for(batch * POL_NA * 745), 256, 0, (cudaStream_t)stream>>>(d_state, d_action, batch, d_critic_in);
-    if (d_reward_norm) k_reward_batchnorm<<<POL_NA, 256, 0, (cudaStream_t)stream>>>(d_reward, batch, d_reward_norm);
+        K_CRITIC_INPUT[p->na]<<<grid_for(batch * p->na * (p->na * (POL_OBS + 1 + POL_ACT))), 256, 0, (cudaStream_t)stream>>>(d_state, d_action, batch, d_critic_in);
+    if (d_reward_norm) K_REWARD_BATCHNORM[p->na]<<<p->na, 256, 0, (cudaStream_t)stream>>>(d_reward, batch, d_reward_norm);
     return launched(p, "fp_learner_feed", (d_critic_in != nullptr) + (d_reward_norm != nullptr));
 }
 

@@ -107,6 +107,7 @@ _PROTOS = {
     "fp_safety_load_affine": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, C.c_double, C.c_double, C.c_double]),
     "fp_safety_project_affine": (C.c_int, [_P, _P, C.c_int, _P, C.c_int32, _P, _P, _P, _P]),
     "fp_policy_create": (C.c_int, [C.c_int, C.POINTER(_P)]),
+    "fp_policy_create_agents": (C.c_int, [C.c_int, C.c_int32, C.POINTER(_P)]),
     "fp_policy_destroy": (C.c_int, [_P]),
     "fp_policy_last_error": (C.c_char_p, [_P]),
     "fp_policy_launch_count": (C.c_int64, [_P]),

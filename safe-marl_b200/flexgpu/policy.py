@@ -1,8 +1,8 @@
 """The rollout loop on the device (SURVEY 8f ranks 1-2): acting policy, Transition writes, learner feed.
 
 DevicePolicy    the shared-parameter RNNAgent (madrl/agents/rnn_agent.py:8-32) + select_action
-                (utils/util.py:50-64) for N envs x 5 agents per call, through fp_policy_act (tcgen05), reading the
-                env's observation ring directly.
+                (utils/util.py:50-64) for N envs x n_agents (1 .. 5) per call, through fp_policy_act (tcgen05), reading
+                the env's observation ring directly.
 DeviceRollout   the body of train_process (madrl/models/model.py:213-254) with nothing crossing PCIe:
                 policy -> fused translate_action + step + get_obs -> Transition fields into a DeviceReplayBuffer.
 learner_batch   unpack_data (model.py:308-323) on a sampled window: the 12 batch tensors + the MADDPG critic input.
@@ -15,17 +15,34 @@ import torch
 from . import _lib
 from .predictor import DeviceReplayBuffer
 
-N_AGENTS, OBS, HID, ACT = 5, 144, 64, 4
-# Transition (model.py:19) as fp32 replay fields, widths per transition (one env-step)
-TRANSITION_FIELDS = {"state": N_AGENTS * OBS, "action": N_AGENTS * ACT, "log_prob_a": N_AGENTS * ACT, "value": N_AGENTS,
-                     "next_value": N_AGENTS, "reward": N_AGENTS, "next_state": N_AGENTS * OBS, "done": 1, "last_step": 1,
-                     "action_avail": N_AGENTS * ACT, "last_hid": N_AGENTS * HID, "hid": N_AGENTS * HID}
+N_AGENTS, OBS, HID, ACT = 5, 144, 64, 4          # N_AGENTS: the default agent count (IEEE-33 with five buildings)
+MAX_AGENTS = 5                                    # fp_policy_create_agents accepts 1 .. 5
+HISTORY, FEATURES = 24, 6                         # the observation ring [HISTORY, n_agents, FEATURES, n_pad] (OBS = 6 x 24)
+
+
+def transition_fields(n_agents):
+    """Transition (model.py:19) as fp32 replay fields, widths per transition (one env-step), for n_agents agents."""
+    na = int(n_agents)
+    return {"state": na * OBS, "action": na * ACT, "log_prob_a": na * ACT, "value": na, "next_value": na, "reward": na,
+            "next_state": na * OBS, "done": 1, "last_step": 1, "action_avail": na * ACT, "last_hid": na * HID, "hid": na * HID}
+
+
+def weight_shapes(n_agents):
+    """RNNAgent.state_dict() shapes, in _WEIGHT_KEYS order: fc1 takes 144 observations + n_agents agent-id columns."""
+    return ((HID, OBS + n_agents), (HID,), (HID,), (HID,), (3 * HID, HID), (3 * HID, HID), (3 * HID,), (3 * HID,), (ACT, HID), (ACT,))
+
+
+def critic_shapes(n_agents):
+    """MLPCritic.state_dict() shapes, in _CRITIC_KEYS order: fc1 takes n_agents x (144 + 4) + n_agents inputs."""
+    return ((HID, n_agents * (OBS + ACT) + n_agents), (HID,), (HID,), (HID,), (HID, HID), (HID,), (1, HID), (1,))
+
+
+TRANSITION_FIELDS = transition_fields(N_AGENTS)
 _WEIGHT_KEYS = ("fc1.weight", "fc1.bias", "layernorm.weight", "layernorm.bias", "rnn.weight_ih", "rnn.weight_hh",
                 "rnn.bias_ih", "rnn.bias_hh", "fc2.weight", "fc2.bias")
-_WEIGHT_SHAPES = ((HID, OBS + N_AGENTS), (HID,), (HID,), (HID,), (3 * HID, HID), (3 * HID, HID), (3 * HID,), (3 * HID,),
-                  (ACT, HID), (ACT,))
+_WEIGHT_SHAPES = weight_shapes(N_AGENTS)
 _CRITIC_KEYS = ("fc1.weight", "fc1.bias", "layernorm.weight", "layernorm.bias", "fc2.weight", "fc2.bias", "fc3.weight", "fc3.bias")
-_CRITIC_SHAPES = ((HID, N_AGENTS * (OBS + ACT) + N_AGENTS), (HID,), (HID,), (HID,), (HID, HID), (HID,), (1, HID), (1,))
+_CRITIC_SHAPES = critic_shapes(N_AGENTS)
 
 
 def _ptr(t):
@@ -42,7 +59,23 @@ def round_tf32(w):
 
 
 class DevicePolicy:
-    def __init__(self, state_dict=None, device="cuda:0", std=1.0, seed=0):
+    """n_agents: the agent count the handle serves (1 .. 5, fixed).  With a state dict it is read from fc1.weight's width
+    (144 + n_agents), and a different n_agents raises; without one it defaults to 5."""
+
+    def __init__(self, state_dict=None, device="cuda:0", std=1.0, seed=0, n_agents=None):
+        if state_dict is not None:
+            shape = tuple(np.shape(state_dict["fc1.weight"]))
+            inferred = shape[1] - OBS if len(shape) == 2 else None
+            if inferred is None or not 1 <= inferred <= MAX_AGENTS:
+                raise ValueError(f"fc1.weight: expected (64, 144 + n_agents) with n_agents in [1, 5], got {shape}")
+            if n_agents is not None and int(n_agents) != inferred:
+                raise ValueError(f"n_agents={n_agents} conflicts with fc1.weight {shape} (144 + {inferred} inputs: {inferred} agents)")
+            n_agents = inferred
+        n_agents = N_AGENTS if n_agents is None else int(n_agents)
+        if not 1 <= n_agents <= MAX_AGENTS:
+            raise ValueError(f"n_agents must be in [1, 5], got {n_agents}")
+        self.n_agents = n_agents
+        self._ring_dims = (HISTORY, n_agents, FEATURES)
         self.device = torch.device(device)
         if self.device.type != "cuda" or not torch.cuda.is_available():
             raise _lib.FlexGpuError("DevicePolicy needs a CUDA device; there is no CPU fallback")
@@ -50,7 +83,8 @@ class DevicePolicy:
         self._p = C.c_void_p()
         idx = self.device.index if self.device.index is not None else torch.cuda.current_device()
         self.device = torch.device("cuda", idx)
-        _lib.check(self._lib.fp_policy_create(idx, C.byref(self._p)), None, "fp_policy_create", self._lib.fp_policy_last_error)
+        _lib.check(self._lib.fp_policy_create_agents(idx, self.n_agents, C.byref(self._p)), None, "fp_policy_create_agents",
+                   self._lib.fp_policy_last_error)
         self.std = float(std)                       # fixed_policy_std (default.yaml: 1.0; gaussian_policy False)
         self.seed = int(seed)
         self._bufs = {}
@@ -74,12 +108,12 @@ class DevicePolicy:
 
     def load_state_dict(self, sd):
         """sd: RNNAgent.state_dict() (torch tensors) or a dict of arrays with the same keys."""
-        arrs = []
-        for k, shape in zip(_WEIGHT_KEYS, _WEIGHT_SHAPES):
+        arrs, na = [], self.n_agents
+        for k, shape in zip(_WEIGHT_KEYS, weight_shapes(na)):
             v = sd[k]
             a = np.ascontiguousarray(v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else v, dtype=np.float32)
             if a.shape != shape:
-                raise ValueError(f"{k}: expected {shape}, got {a.shape} (hid_size 64, obs 144 + 5 agent ids, 4 actions)")
+                raise ValueError(f"{k}: expected {shape}, got {a.shape} (hid_size 64, obs 144 + {na} agent ids, 4 actions)")
             arrs.append(a)
         self._check(self._lib.fp_policy_load(self._p, *[a.ctypes.data_as(C.c_void_p) for a in arrs]), "fp_policy_load")
 
@@ -87,26 +121,38 @@ class DevicePolicy:
         return int(self._lib.fp_policy_launch_count(self._p))
 
     def load_critic(self, sd):
-        """sd: MLPCritic.state_dict() (madrl/critics/mlp_critic.py, as MADDPG.construct_value_net builds it: input 745)."""
-        arrs = []
-        for k, shape in zip(_CRITIC_KEYS, _CRITIC_SHAPES):
+        """sd: MLPCritic.state_dict() (madrl/critics/mlp_critic.py, as MADDPG.construct_value_net builds it: input
+        n_agents x 149, 745 for five agents)."""
+        arrs, na = [], self.n_agents
+        for k, shape in zip(_CRITIC_KEYS, critic_shapes(na)):
             v = sd[k]
             a = np.ascontiguousarray(v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else v, dtype=np.float32)
             if a.shape != shape:
-                raise ValueError(f"critic {k}: expected {shape}, got {a.shape} (hid_size 64, 5 x (144 + 4) + 5 inputs)")
+                raise ValueError(f"critic {k}: expected {shape}, got {a.shape} (hid_size 64, {na} x (144 + 4) + {na} inputs)")
             arrs.append(a)
         self._check(self._lib.fp_critic_load(self._p, *[a.ctypes.data_as(C.c_void_p) for a in arrs]), "fp_critic_load")
         self.has_critic = True
 
-    def value(self, ring, action, slot=None, n_envs=None, out=None):
-        """MADDPG.value (maddpg.py:29-76) on the observation ring and `action` [N, 5, 4]: [N, 5, 1] (k_critic, tcgen05)."""
+    def _ring(self, ring, slot, n_envs):
+        """(ring tensor, slot, n_envs) of an ObsRing or a raw ring, whose shape must be [24, n_agents, 6, n_pad]."""
         if hasattr(ring, "ring"):
             slot, n_envs, ring = ring.slot, ring.env.n_envs, ring.ring
-        N = int(n_envs)
+        if tuple(ring.shape)[:-1] != self._ring_dims:
+            raise ValueError(f"the observation ring must be [24, {self.n_agents}, 6, n_pad] for this {self.n_agents}-agent policy, "
+                             f"got {tuple(ring.shape)}")
+        return ring, slot, n_envs
+
+    def value(self, ring, action, slot=None, n_envs=None, out=None):
+        """MADDPG.value (maddpg.py:29-76) on the observation ring and `action` [N, n_agents, 4]: [N, n_agents, 1]
+        (k_critic, tcgen05)."""
+        ring, slot, n_envs = self._ring(ring, slot, n_envs)
+        N, na = int(n_envs), self.n_agents
         act = action.to(device=self.device, dtype=torch.float32).contiguous()
-        if tuple(act.shape) != (N, N_AGENTS, ACT):
-            raise ValueError("action must be [n_envs, 5, 4]")
-        out = self._buf("value", (N, N_AGENTS, 1)) if out is None else out
+        if tuple(act.shape) != (N, na, ACT):
+            raise ValueError(f"action must be [n_envs, {na}, 4], got {tuple(act.shape)}")
+        if out is not None and tuple(out.shape) != (N, na, 1):
+            raise ValueError(f"out must be [n_envs, {na}, 1], got {tuple(out.shape)}")
+        out = self._buf("value", (N, na, 1)) if out is None else out
         self._check(self._lib.fp_critic_value(self._p, _ptr(ring), int(slot), int(ring.shape[-1]), N, _ptr(act), _ptr(out), _lib.stream(self.device)),
                     "fp_critic_value")
         return out
@@ -120,45 +166,58 @@ class DevicePolicy:
 
     def act(self, ring, slot=None, n_envs=None, hid_in=None, reset=None, explore=True, eps=None, step=0, hid_out=None,
             want_mean=False, want_logp=True, hid_layout="rows", out="action", mean_out=None):
-        """ring: an ObsRing (env.obs_ring() / step(..., return_obs='ring')) or a raw [24, 5, 6, n_pad] fp32 tensor with
-        `slot` / `n_envs`.  Returns (action [N,5,4], log_prob [N,5,4] or None, hid, mean or None); the output
-        tensors are reused by the next call unless hid_out is given (out: name of the reused action buffer).  hid_layout: "rows" = [N, 5, 64] (the reference's
-        (b, n, hid)), "env_minor" = [5, 64, n_pad] (the kernel's native layout: coalesced accesses; hid_out required)."""
-        if hasattr(ring, "ring"):
-            slot, n_envs, ring = ring.slot, ring.env.n_envs, ring.ring
+        """ring: an ObsRing (env.obs_ring() / step(..., return_obs='ring')) or a raw [24, n_agents, 6, n_pad] fp32 tensor
+        with `slot` / `n_envs`.  Returns (action [N, na, 4], log_prob [N, na, 4] or None, hid, mean or None), na =
+        n_agents; the output tensors are reused by the next call unless hid_out is given (out: name of the reused action
+        buffer).  hid_layout: "rows" = [N, na, 64] (the reference's (b, n, hid)), "env_minor" = [na, 64, n_pad] (the
+        kernel's native layout: coalesced accesses; hid_out required)."""
+        ring, slot, n_envs = self._ring(ring, slot, n_envs)
         n_pad = ring.shape[-1]
-        N = int(n_envs)
-        action = self._buf(out, (N, N_AGENTS, ACT))
-        logp = self._buf("logp", (N, N_AGENTS, ACT)) if want_logp else None
-        mean = mean_out if mean_out is not None else (self._buf("mean", (N, N_AGENTS, ACT)) if want_mean else None)
+        N, na = int(n_envs), self.n_agents
+        rows = (N, na, ACT)
+        if mean_out is not None and tuple(mean_out.shape) != rows:
+            raise ValueError(f"mean_out must be [n_envs, {na}, 4], got {tuple(mean_out.shape)}")
+        action = self._buf(out, rows)
+        logp = self._buf("logp", rows) if want_logp else None
+        mean = mean_out if mean_out is not None else (self._buf("mean", rows) if want_mean else None)
         em = hid_layout == "env_minor"
-        if em and (hid_out is None or tuple(hid_out.shape) != (N_AGENTS, HID, n_pad) or
-                   (hid_in is not None and tuple(hid_in.shape) != (N_AGENTS, HID, n_pad))):
-            raise ValueError("env-minor hidden states are [5, 64, n_pad] tensors (hid_out required)")
+        hshape = (na, HID, n_pad) if em else (N, na, HID)
+        if em and hid_out is None:
+            raise ValueError(f"env-minor hidden states are [{na}, 64, n_pad] tensors (hid_out required)")
+        if (hid_out is not None and tuple(hid_out.shape) != hshape) or (hid_in is not None and tuple(hid_in.shape) != hshape):
+            raise ValueError(f"hidden states of this {na}-agent policy ({hid_layout}) are {list(hshape)} tensors")
         if hid_out is None:
-            hid_out = self._buf("hid", (N, N_AGENTS, HID))
+            hid_out = self._buf("hid", hshape)
         if hid_in is not None and hid_in.data_ptr() == hid_out.data_ptr():
             raise ValueError("hid_in and hid_out must be different buffers")
         r = None if reset is None else reset.to(device=self.device, dtype=torch.uint8).contiguous()
         e = None if eps is None else eps.to(device=self.device, dtype=torch.float32).contiguous()
+        if e is not None and e.numel() != N * na * ACT:
+            raise ValueError(f"eps must hold n_envs x {na} x 4 draws, got {tuple(e.shape)}")
         self._check(self._lib.fp_policy_act(self._p, _ptr(ring), int(slot), int(n_pad), N, _ptr(hid_in), _ptr(r), _ptr(hid_out),
                                             1 if em else 0, _ptr(mean), _ptr(action), _ptr(logp), _ptr(e), self.seed, int(step),
                                             self.std, 1 if explore else 0, _lib.stream(self.device)), "fp_policy_act")
         return action, logp, hid_out, mean
 
     def sample(self, mean, explore=True, eps=None, step=0, want_logp=True, out="action"):
-        """select_action alone on stored fc2 outputs `mean` [N, 5, 4] (act(..., want_mean=True)): another exploration draw of
-        the same policy evaluation -- bit-identical to calling act() again on the same inputs with these draws."""
-        N = int(mean.shape[0])
-        action = self._buf(out, (N, N_AGENTS, ACT))
-        logp = self._buf("logp", (N, N_AGENTS, ACT)) if want_logp else None
+        """select_action alone on stored fc2 outputs `mean` [N, n_agents, 4] (act(..., want_mean=True)): another exploration
+        draw of the same policy evaluation -- bit-identical to calling act() again on the same inputs with these draws."""
+        N, na = int(mean.shape[0]), self.n_agents
+        if tuple(mean.shape) != (N, na, ACT) or not mean.is_contiguous():
+            raise ValueError(f"mean must be a contiguous [n_envs, {na}, 4] tensor, got {tuple(mean.shape)}")
+        action = self._buf(out, (N, na, ACT))
+        logp = self._buf("logp", (N, na, ACT)) if want_logp else None
         e = None if eps is None else eps.to(device=self.device, dtype=torch.float32).contiguous()
+        if e is not None and e.numel() != N * na * ACT:
+            raise ValueError(f"eps must hold n_envs x {na} x 4 draws, got {tuple(e.shape)}")
         self._check(self._lib.fp_policy_sample(self._p, _ptr(mean), N, _ptr(action), _ptr(logp), _ptr(e), self.seed, int(step),
                                                self.std, 1 if explore else 0, _lib.stream(self.device)), "fp_policy_sample")
         return action, logp
 
-    def gather_windows(self, ring, n, out, pitch, row0=0, cap=None):
-        slot, ringt = ring.slot, ring.ring
+    def gather_windows(self, ring, n, out, pitch, row0=0, cap=None, slot=None):
+        """Dense observation windows [n, n_agents, 144] of envs [0, n) into rows (row0 + e) mod cap of `pitch` floats of
+        `out` (a tensor or a device pointer)."""
+        ringt, slot, _ = self._ring(ring, slot, n)
         self._check(self._lib.fp_policy_gather_windows(self._p, _ptr(ringt), int(slot), int(ringt.shape[-1]), int(n), _ptr(out),
                                                        int(pitch), int(row0), int(cap if cap is not None else n), _lib.stream(self.device)),
                     "fp_policy_gather_windows")
@@ -167,7 +226,8 @@ class DevicePolicy:
 class DeviceRollout:
     """train_process (model.py:198-267) for N envs at once.  Per step: k_policy (act on the ring + last_hid) ->
     fp_step_ring with FP_F32_POLICY actions (translate_action + step + pushing get_obs, one launch) -> Transition
-    fields of the first `record_envs` envs into `replay` (a DeviceReplayBuffer with TRANSITION_FIELDS).  value /
+    fields of the first `record_envs` envs into `replay` (a DeviceReplayBuffer with transition_fields(n_agents)).
+    The env's n_agents must be the policy's, and its history 24 (the kernels' K = 6 x 24).  value /
     next_value are stored as zeros: MADDPG's losses recompute both from the critic (maddpg.py:104-107) and never read
     them.  Episodes end together (95 steps, quirk Q1): the finished envs are reset from their Philox streams and their
     hidden state restarts at zero (init_hidden, model.py:211).  An env can also terminate EARLY (solver failure,
@@ -178,28 +238,35 @@ class DeviceRollout:
 
     def __init__(self, env, policy, replay=None, record_envs=None, max_steps=240, reset_done_each_step=False, value_fn=None,
                  fp64_history=False):
+        if env.n_agents != policy.n_agents:
+            raise ValueError(f"the env has {env.n_agents} agents, the policy {policy.n_agents}: "
+                             f"build the policy with DevicePolicy(..., n_agents={env.n_agents})")
+        if env.history != HISTORY:
+            raise ValueError(f"the device rollout needs an observation history of {HISTORY} steps, the env has {env.history}")
+        na = self.na = policy.n_agents
+        self.fields = transition_fields(na)
         self.env, self.policy, self.replay = env, policy, replay
         # the loop consumes the fp32 ring only: by default the step stops pushing the fp64 history ring as well
         # (env.set_obs_history); a later env.get_obs() restores it from the ring at fp32 precision
         env.set_obs_history(bool(fp64_history))
         self.N = env.n_envs
         self.R = 0 if replay is None else int(self.N if record_envs is None else min(record_envs, self.N))
-        if replay is not None and (dict(replay.fields) != TRANSITION_FIELDS or self.R > replay.size):
-            raise ValueError("replay must be a DeviceReplayBuffer(TRANSITION_FIELDS) holding at least record_envs rows")
+        if replay is not None and (dict(replay.fields) != self.fields or self.R > replay.size):
+            raise ValueError(f"replay must be a DeviceReplayBuffer(transition_fields({na})) holding at least record_envs rows")
         self.max_steps = int(max_steps)
         self.reset_done_each_step = bool(reset_done_each_step)
         # value_fn: the critic behind the Transition's value / next_value, filled as train_process does (model.py:217, :225-226:
         # the critic on (state, action) and on (next_state, a SECOND sampled action from the policy with the new hidden state;
         # the second policy evaluation doubles k_policy's cost).  "native" = k_critic (tcgen05; policy.load_critic(...) holds the
-        # reference's MLPCritic), straight from the observation ring; or a callable (obs [R, 5, 144], action [R, 5, 4]) ->
-        # [R, 5, 1], e.g. behaviour_net.value (maddpg.py:29-76) as a torch module.
+        # reference's MLPCritic), straight from the observation ring; or a callable (obs [R, na, 144], action [R, na, 4]) ->
+        # [R, na, 1], e.g. behaviour_net.value (maddpg.py:29-76) as a torch module.
         self.value_fn = value_fn
         if value_fn == "native" and not policy.has_critic:
             raise ValueError('value_fn="native" needs the critic weights: policy.load_critic(MLPCritic.state_dict())')
         dev = env.device
         self._n_pad = (self.N + 31) // 32 * 32                      # the observation ring's padding (fp_obs_ring)
-        # hidden states in the policy kernel's env-minor layout [5, 64, n_pad]; hidden() gives the reference's [N, 5, 64]
-        self._hid = [torch.zeros(N_AGENTS, HID, self._n_pad, device=dev), torch.zeros(N_AGENTS, HID, self._n_pad, device=dev)]
+        # hidden states in the policy kernel's env-minor layout [na, 64, n_pad]; hidden() gives the reference's [N, na, 64]
+        self._hid = [torch.zeros(na, HID, self._n_pad, device=dev), torch.zeros(na, HID, self._n_pad, device=dev)]
         self._cur = 0
         self._reset_mask = None
         self._done_mask = None
@@ -207,7 +274,7 @@ class DeviceRollout:
         # evaluation the next step starts with (:215-216: same observations, same hidden state) -- only the exploration draw
         # differs.  Its fc2 outputs and new hidden state are kept, and the next step re-draws (fp_policy_sample) instead of
         # running k_policy again, unless a reset intervened.  Same bits as evaluating twice.
-        self._mean2 = torch.empty(self.N, N_AGENTS, ACT, device=dev) if value_fn is not None else None
+        self._mean2 = torch.empty(self.N, na, ACT, device=dev) if value_fn is not None else None
         self._cache_valid = False
         self.t = 0                                  # step within the episode
         self.total_steps = 0
@@ -218,11 +285,10 @@ class DeviceRollout:
                 p = C.c_void_p()
                 replay._check(replay._lib.fp_replay_field_ptr(replay._r, i, C.byref(p)), "fp_replay_field_ptr")
                 self._fptr[k] = p
-            self._zeros = torch.zeros(self.R, N_AGENTS, device=dev)
             if value_fn is not None:
                 if value_fn != "native":
-                    self._dense = torch.empty(self.R, N_AGENTS * OBS, device=dev)
-                self._hid_scratch = torch.empty(N_AGENTS, HID, self._n_pad, device=dev)
+                    self._dense = torch.empty(self.R, na * OBS, device=dev)
+                self._hid_scratch = torch.empty(na, HID, self._n_pad, device=dev)
 
     def reset(self):
         self.ring = self.env.reset(return_obs="ring")              # state, _ = env.reset() (model.py:208)
@@ -234,7 +300,7 @@ class DeviceRollout:
 
     def _rows(self, name, src, pos):
         pol = self.policy
-        w = TRANSITION_FIELDS[name]
+        w = self.fields[name]
         pol._check(pol._lib.fp_policy_rows_to_ring(pol._p, _ptr(src), self.R, w, self._fptr[name], pos, self.replay.size,
                                                    _lib.stream(pol.device)), "fp_policy_rows_to_ring")
 
@@ -244,20 +310,20 @@ class DeviceRollout:
                                                      _ptr(zero_mask), _lib.stream(pol.device)), "fp_policy_hidden_to_ring")
 
     def hidden(self):
-        """The current hidden state in the reference's layout [N, 5, 64] (a copy)."""
+        """The current hidden state in the reference's layout [N, n_agents, 64] (a copy)."""
         return self._hid[self._cur][:, :, :self.N].permute(2, 0, 1).contiguous()
 
     def _dense_obs(self):
-        self.policy.gather_windows(self.ring, self.R, self._dense, N_AGENTS * OBS, 0, self.R)
-        return self._dense.view(self.R, N_AGENTS, OBS)
+        self.policy.gather_windows(self.ring, self.R, self._dense, self.na * OBS, 0, self.R)
+        return self._dense.view(self.R, self.na, OBS)
 
     def _value(self, action, name):
-        """The critic on (the ring as it stands, action) for the recorded envs: [R, 5] fp32, contiguous."""
+        """The critic on (the ring as it stands, action) for the recorded envs: [R, na] fp32, contiguous."""
         if self.value_fn == "native":
-            out = self.policy._buf(name, (self.R, N_AGENTS, 1))              # the recorded envs only
-            return self.policy.value(self.ring.ring, action[:self.R], slot=self.ring.slot, n_envs=self.R, out=out).view(self.R, N_AGENTS)
+            out = self.policy._buf(name, (self.R, self.na, 1))              # the recorded envs only
+            return self.policy.value(self.ring.ring, action[:self.R], slot=self.ring.slot, n_envs=self.R, out=out).view(self.R, self.na)
         with torch.no_grad():
-            return self.value_fn(self._dense_obs(), action[:self.R]).reshape(self.R, N_AGENTS).float().contiguous()
+            return self.value_fn(self._dense_obs(), action[:self.R]).reshape(self.R, self.na).float().contiguous()
 
     def step(self, explore=True, eps=None, eps_next=None):
         if self.ring is None:
@@ -272,7 +338,7 @@ class DeviceRollout:
         else:
             pos, state_written = (self.replay.reserve(self.R) if self.R else None), False
             if self.R and self.ring.ring.shape[-1] >= 128:          # `state` rows written by k_policy's writer warps from the blocks it stages
-                pol._check(pol._lib.fp_policy_state_sink(pol._p, self._fptr["state"], TRANSITION_FIELDS["state"], pos, self.replay.size, self.R),
+                pol._check(pol._lib.fp_policy_state_sink(pol._p, self._fptr["state"], self.fields["state"], pos, self.replay.size, self.R),
                            "fp_policy_state_sink")
                 state_written = True
             action, logp, hid, _ = pol.act(self.ring, hid_in=last_hid, reset=self._reset_mask, explore=explore, eps=eps,
@@ -280,7 +346,7 @@ class DeviceRollout:
         self._cache_valid = False
         if self.R:
             if not state_written:
-                pol.gather_windows(self.ring, self.R, self._fptr["state"], TRANSITION_FIELDS["state"], pos, self.replay.size)
+                pol.gather_windows(self.ring, self.R, self._fptr["state"], self.fields["state"], pos, self.replay.size)
             self._hidden_rows("last_hid", last_hid, pos, self._reset_mask)     # a restarted env's last_hid is the zero state it acted from
             if self.value_fn is not None:                                      # value = critic(state, action) (model.py:217)
                 self._rows("value", self._value(action, "value"), pos)
@@ -289,7 +355,7 @@ class DeviceRollout:
         self.t += 1
         self.total_steps += 1
         if self.R:
-            pol.gather_windows(self.ring, self.R, self._fptr["next_state"], TRANSITION_FIELDS["next_state"], pos, self.replay.size)
+            pol.gather_windows(self.ring, self.R, self._fptr["next_state"], self.fields["next_state"], pos, self.replay.size)
             self._hidden_rows("hid", hid, pos)
             if self.value_fn is not None:   # next_value = critic(next_state, a second sampled action from the new hidden state) (model.py:225-226)
                 a2, _, _, _ = pol.act(self.ring, hid_in=hid, explore=explore, eps=eps_next, step=(1 << 40) + self.total_steps,
@@ -322,19 +388,23 @@ class DeviceRollout:
 def learner_batch(policy, replay, batch_size, start=None, reward_normalisation=True, critic_input=True):
     """unpack_data (model.py:308-323) on `batch_size` consecutive transitions (get_batch, replay_buffer.py:14-21):
     the reference's 12 tensors in its shapes -- including its quirk log_prob_a = action (:313) -- plus, for MADDPG,
-    `critic_in` [batch * 5, 745] (maddpg.py:29-66).  Everything stays on the device."""
+    `critic_in` [batch * na, na x 149] (maddpg.py:29-66; [batch * 5, 745] for five agents), na = policy.n_agents.
+    Everything stays on the device."""
+    na = policy.n_agents
+    if dict(replay.fields) != transition_fields(na):
+        raise ValueError(f"replay must be a DeviceReplayBuffer(transition_fields({na})) for this {na}-agent policy")
     b = replay.get_batch(batch_size, start=start)
     B = batch_size
     out = {
-        "state": b["state"].view(B, N_AGENTS, OBS), "action": b["action"].view(B, N_AGENTS, ACT),
-        "log_prob_a": b["action"].view(B, N_AGENTS, ACT),                     # sic: model.py:313 concatenates batch.action
-        "value": b["value"].view(B, N_AGENTS, 1), "next_value": b["next_value"].view(B, N_AGENTS, 1),
-        "reward": b["reward"], "next_state": b["next_state"].view(B, N_AGENTS, OBS), "done": b["done"].view(B, 1),
-        "last_step": b["last_step"].view(B, 1), "action_avail": b["action_avail"].view(B, N_AGENTS, ACT),
-        "last_hid": b["last_hid"].view(B, N_AGENTS, HID), "hid": b["hid"].view(B, N_AGENTS, HID),
+        "state": b["state"].view(B, na, OBS), "action": b["action"].view(B, na, ACT),
+        "log_prob_a": b["action"].view(B, na, ACT),                           # sic: model.py:313 concatenates batch.action
+        "value": b["value"].view(B, na, 1), "next_value": b["next_value"].view(B, na, 1),
+        "reward": b["reward"], "next_state": b["next_state"].view(B, na, OBS), "done": b["done"].view(B, 1),
+        "last_step": b["last_step"].view(B, 1), "action_avail": b["action_avail"].view(B, na, ACT),
+        "last_hid": b["last_hid"].view(B, na, HID), "hid": b["hid"].view(B, na, HID),
     }
-    crit = torch.empty(B * N_AGENTS, N_AGENTS * OBS + N_AGENTS + N_AGENTS * ACT, device=replay.device) if critic_input else None
-    rn = torch.empty(B, N_AGENTS, device=replay.device) if reward_normalisation else None
+    crit = torch.empty(B * na, na * (OBS + 1 + ACT), device=replay.device) if critic_input else None
+    rn = torch.empty(B, na, device=replay.device) if reward_normalisation else None
     policy._check(policy._lib.fp_learner_feed(policy._p, _ptr(b["state"]), _ptr(b["action"]), _ptr(b["reward"]), B, _ptr(crit),
                                               _ptr(rn), _lib.stream(policy.device)), "fp_learner_feed")
     if reward_normalisation:
@@ -346,15 +416,17 @@ def learner_batch(policy, replay, batch_size, start=None, reward_normalisation=T
 
 def smoke(env, device):
     """Tiny policy + rollout invocation for __graft_entry__.smoke(): k_policy on the env's own observation ring against
-    a plain torch fp32 evaluation of RNNAgent.forward (rnn_agent.py:24-32) with the same (TF32-rounded) matrices."""
+    a plain torch fp32 evaluation of RNNAgent.forward (rnn_agent.py:24-32) with the same (TF32-rounded) matrices, for the
+    env's own agent count."""
+    na = env.n_agents
     g = torch.Generator().manual_seed(0)
-    sd = {k: (torch.randn(s, generator=g) * 0.1) for k, s in zip(_WEIGHT_KEYS, _WEIGHT_SHAPES)}
+    sd = {k: (torch.randn(s, generator=g) * 0.1) for k, s in zip(_WEIGHT_KEYS, weight_shapes(na))}
     sd["layernorm.weight"] = 1.0 + sd["layernorm.weight"]
     pol = DevicePolicy(sd, device=device)
     ring = env.obs_ring()
     n = env.n_envs
-    h_in = (torch.rand(n, N_AGENTS, HID, generator=g) - 0.5).to(device)
-    act, _, hid, mean = pol.act(ring, hid_in=h_in, explore=False, want_mean=True, hid_out=torch.empty(n, N_AGENTS, HID, device=device))
+    h_in = (torch.rand(n, na, HID, generator=g) - 0.5).to(device)
+    act, _, hid, mean = pol.act(ring, hid_in=h_in, explore=False, want_mean=True, hid_out=torch.empty(n, na, HID, device=device))
     w = {k: v.to(device) for k, v in sd.items()}
     for k in ("rnn.weight_ih", "rnn.weight_hh"):
         w[k] = torch.from_numpy(round_tf32(sd[k].numpy())).to(device)
@@ -362,8 +434,8 @@ def smoke(env, device):
     prev = torch.backends.cuda.matmul.allow_tf32
     torch.backends.cuda.matmul.allow_tf32 = False
     try:
-        obs = ring.dense().view(n * N_AGENTS, OBS)
-        x = torch.cat([obs, torch.eye(N_AGENTS, device=device).repeat(n, 1)], dim=1) @ w["fc1.weight"].T + w["fc1.bias"]
+        obs = ring.dense().view(n * na, OBS)
+        x = torch.cat([obs, torch.eye(na, device=device).repeat(n, 1)], dim=1) @ w["fc1.weight"].T + w["fc1.bias"]
         x = torch.relu(torch.nn.functional.layer_norm(x, (HID,), w["layernorm.weight"], w["layernorm.bias"], 1e-5))
         h0 = h_in.view(-1, HID)
         gi = x @ w["rnn.weight_ih"].T + w["rnn.bias_ih"]; gh = h0 @ w["rnn.weight_hh"].T + w["rnn.bias_hh"]
@@ -384,10 +456,10 @@ def smoke(env, device):
 
 
 def critic_input(policy, state, action):
-    """The MADDPG critic's input rows (maddpg.py:29-66) for dense observations [B, 5, 144] and actions [B, 5, 4]:
-    [B * 5, 745] = all agents' observations | one-hot agent id | all agents' actions."""
-    B = state.shape[0]
-    st = state.reshape(B, N_AGENTS * OBS).contiguous(); ac = action.reshape(B, N_AGENTS * ACT).float().contiguous()
-    out = torch.empty(B * N_AGENTS, N_AGENTS * OBS + N_AGENTS + N_AGENTS * ACT, device=st.device)
+    """The MADDPG critic's input rows (maddpg.py:29-66) for dense observations [B, na, 144] and actions [B, na, 4], na =
+    policy.n_agents: [B * na, na x 149] = all agents' observations | one-hot agent id | all agents' actions."""
+    B, na = state.shape[0], policy.n_agents
+    st = state.reshape(B, na * OBS).contiguous(); ac = action.reshape(B, na * ACT).float().contiguous()
+    out = torch.empty(B * na, na * (OBS + 1 + ACT), device=st.device)
     policy._check(policy._lib.fp_learner_feed(policy._p, _ptr(st), _ptr(ac), None, B, _ptr(out), None, _lib.stream(policy.device)), "fp_learner_feed")
     return out
