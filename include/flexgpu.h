@@ -352,7 +352,9 @@ int fp_predict_mlp(FpHandle* h, int64_t n, const float* d_X, float* d_vhat, doub
  * slack price (1000, :205-206).  fp_safety_project: d_actions [N][na][4] raw policy outputs (FP_F32 / FP_F64) -> parse_actions
  * (:143-174, the env's own scaling / ESS logic on its current demands, PV and energy) -> projection -> d_adjusted fp32,
  * either in the reference's return layout [N][x(na) | c(na) | d(na) | g(na)] (type_major = 1, :290-296) or [N][na][4];
- * d_slack [N][na] (remaining predicted violation, p.u.) and d_intervened [N][na] may be NULL. */
+ * d_slack [N][na] (remaining predicted violation, p.u.) and d_intervened [N][na] may be NULL.
+ * NaN: parse_actions clips as numpy.clip does, so a NaN action component (or a3 = +-inf where PV = 0, or a1 = a2 = +inf,
+ * whose charge / discharge netting is inf - inf) leaves the agent's proposal NaN; it is returned as parsed, with NaN where numpy has it, and not projected: intervened 0, slack 0. */
 int fp_safety_load(FpHandle* h, const double* h_coef, const double* h_intercept, double v_min, double v_max, double slack_weight);
 int fp_safety_project(FpHandle* h, const void* d_actions, int act_dtype, float* d_adjusted, int32_t type_major, double* d_slack,
                       uint8_t* d_intervened, void* stream);
@@ -367,7 +369,10 @@ int fp_safety_project(FpHandle* h, const void* d_actions, int act_dtype, float* 
  * fp_safety_project_affine: inputs and d_adjusted as fp_safety_project; d_slack [N][n_bus] fp64 (remaining predicted
  * violation per bus), d_intervened [N][na] (1 if any of the agent's four values moved) and d_status [N] int32
  * (iterations, 0 if every bus was already inside -- then d_adjusted is the proposal cast to fp32 -- or -1 if the
- * iteration cap was reached) may be NULL.  FP_ESTATE before fp_safety_load_affine or fp_load_profiles. */
+ * iteration cap was reached) may be NULL.  FP_ESTATE before fp_safety_load_affine or fp_load_profiles.
+ * NaN: a proposal that is NaN after parse_actions (as for fp_safety_project) makes V(y0) non-finite, and the whole env
+ * is returned as parsed, unprojected: intervened 0 for every agent (the bits did not change), slack 0 on every bus,
+ * status 0.  The next fp_step treats the NaN as a solver failure for that env. */
 int fp_safety_load_affine(FpHandle* h, int32_t n_in, int32_t n_out, const double* h_A, const double* h_c, double v_min,
                           double v_max, double slack_weight);
 int fp_safety_project_affine(FpHandle* h, const void* d_actions, int act_dtype, float* d_adjusted, int32_t type_major,

@@ -146,12 +146,14 @@ def _piece_slope(a, t, lo, hi):
 def project_affine(y0, Pd, Qd, agent_bus, A, c, v_min, v_max, w=W_SLACK, max_iter=AFFINE_MAX_ITER):
     """One env: y0 [na, 4] proposed (x, c, d, g); Pd, Qd [nb] the current demands in bus order (0 at the slack bus);
     agent_bus [na] bus positions of the buildings; A [nb, 2 nb], c [nb].  Returns (y* [na, 4], slack [nb], status):
-    status = iterations (0: every bus already inside, y* = y0) or -1 if the cap was reached."""
+    status = iterations (0: every bus already inside, y* = y0) or -1 if the cap was reached.  A non-finite V(y0) (a NaN
+    in the proposal: parse_actions keeps a NaN action as numpy.clip does) leaves the env unprojected: y* = y0 with its
+    NaN, slack 0 on every bus, status 0."""
     y0 = np.asarray(y0, dtype=np.float64); agent_bus = np.asarray(agent_bus, dtype=np.int64)
     A = np.asarray(A, dtype=np.float64)
     na, nb = len(agent_bus), len(Pd)
     V0 = affine_prediction(y0, Pd, Qd, agent_bus, A, c)
-    if ((V0 >= v_min) & (V0 <= v_max)).all():
+    if not np.isfinite(V0).all() or ((V0 >= v_min) & (V0 <= v_max)).all():
         return y0.copy(), np.zeros(nb), 0
     B = np.concatenate([A[:, 2 * agent_bus], A[:, 2 * agent_bus + 1]], axis=1)          # [nb, 2 na]
     a = np.stack([-np.asarray(Pd, dtype=np.float64)[agent_bus], np.ones(na), -np.ones(na)], axis=1)

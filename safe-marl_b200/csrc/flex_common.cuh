@@ -163,10 +163,17 @@ __device__ __forceinline__ uint64_t pack2(int32_t lo, int32_t hi) {
     return (uint64_t)(uint32_t)lo | ((uint64_t)(uint32_t)hi << 32);
 }
 
+// numpy.clip for a non-NaN x (the same two selects, signed zeros included), but a NaN x returns lo where numpy keeps
+// the NaN.  The step kernels test their actions for NaN themselves (a NaN action is a solver failure and rolls the env
+// back), so what the clip makes of one never reaches their outputs; clip_np is the exact numpy.clip.
 __device__ __forceinline__ double clipd(double x, double lo, double hi) {
-    // numpy.clip == minimum(maximum(x, lo), hi)
     double t = (x > lo) ? x : lo;
     return (t < hi) ? t : hi;
+}
+
+// numpy.clip exactly (_NPY_CLIP: minimum(maximum(x, lo), hi), a NaN x propagates): the safety layer's parse_actions
+__device__ __forceinline__ double clip_np(double x, double lo, double hi) {
+    return (x != x) ? x : clipd(x, lo, hi);
 }
 
 // Inclusive Hillis-Steele scan over the warp (lane order).

@@ -756,7 +756,7 @@ __global__ void k_safety_project(const SafetyParams prm) {
         double a0, a1, a2, a3;
         load_action4(prm.actions, prm.act_f64, t, a0, a1, a2, a3);
         // parse_actions (:143-174) = the env's own scaling / clipping / ESS logic
-        const Setpoint sp = apply_actions_frac(c, true, a0, a1, a2, a3, ppv, e_cur);
+        const Setpoint sp = apply_actions_frac<true>(c, true, a0, a1, a2, a3, ppv, e_cur);
         double y[4] = {sp.pred, sp.ch, sp.dis, sp.qpv};
         const double sP = prm.sP[i], sQ = prm.sQ[i];
         const double V0 = fma(sQ, Qd + y[3], sP * ((Pd * (1.0 - y[0]) + y[1]) - y[2])) + prm.b[i];

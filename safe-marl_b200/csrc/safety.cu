@@ -104,7 +104,7 @@ __global__ void __launch_bounds__(SA_WARPS * 32) k_safety_project_affine(const S
             const double e_cur = __longlong_as_double((long long)rec[FP_REC_E_CUR + lane]);
             double a0, a1, a2, a3;
             load_action4(prm.actions, prm.act_f64, e * na + lane, a0, a1, a2, a3);
-            const Setpoint sp = apply_actions_frac(c, true, a0, a1, a2, a3, ppv, e_cur);
+            const Setpoint sp = apply_actions_frac<true>(c, true, a0, a1, a2, a3, ppv, e_cur);
             y0[0] = sp.pred; y0[1] = sp.ch; y0[2] = sp.dis; y0[3] = sp.qpv;
         }
         // full bus-order P/Q row (0 at the slack bus), with the proposal applied at the buildings' buses
@@ -136,7 +136,9 @@ __global__ void __launch_bounds__(SA_WARPS * 32) k_safety_project_affine(const S
         }
         const bool out0 = V0[0] < v_min || V0[0] > v_max;
         const bool out1 = own1 && (V0[1] < v_min || V0[1] > v_max);
-        const bool any_out = __any_sync(FULL, (lane < nb && out0) || out1);
+        // a NaN proposal (numpy.clip keeps a NaN action) makes V(y0) non-finite: the env is left as parsed, unprojected
+        const bool bad = (lane < nb && !isfinite(V0[0])) || (own1 && !isfinite(V0[1]));
+        const bool any_out = __any_sync(FULL, (lane < nb && out0) || out1) && !__any_sync(FULL, bad);
         double y[4] = {y0[0], y0[1], y0[2], y0[3]};
         int status = 0;
         int st[2] = {ST_IN, ST_IN};
@@ -366,8 +368,12 @@ __global__ void __launch_bounds__(SA_WARPS * 32) k_safety_project_affine(const S
             } else {
                 reinterpret_cast<float4*>(prm.out)[e * na + lane] = make_float4((float)y[0], (float)y[1], (float)y[2], (float)y[3]);
             }
-            if (prm.intervened != nullptr)
-                prm.intervened[e * na + lane] = (y[0] != y0[0] || y[1] != y0[1] || y[2] != y0[2] || y[3] != y0[3]) ? 1 : 0;
+            if (prm.intervened != nullptr) {                 // bits, not values: an untouched NaN has not moved
+                bool mv = false;
+#pragma unroll
+                for (int k = 0; k < 4; ++k) mv = mv || (__double_as_longlong(y[k]) != __double_as_longlong(y0[k]));
+                prm.intervened[e * na + lane] = mv ? 1 : 0;
+            }
         }
         if (prm.slack != nullptr) {
 #pragma unroll

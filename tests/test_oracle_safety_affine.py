@@ -112,3 +112,18 @@ def test_active_set_kkt_on_random_cases():
             z[:, :3] = np.maximum(z[:, :3], 0.0)
             assert cost(z) >= c0 - 1e-12 * max(1.0, c0), trial
     assert max(iters) < safety_affine_ref.AFFINE_MAX_ITER
+
+
+@pytest.mark.parametrize("kind", ["low", "high", "mixed", "hopeless"])
+def test_nan_proposal_is_left_unprojected(kind):
+    """A NaN in the proposal (parse_actions keeps a NaN action, as numpy.clip does) makes V(y0) non-finite: the env is
+    returned as proposed, NaN included, with no slack and status 0 -- what k_safety_project_affine writes."""
+    rng = np.random.default_rng({"low": 41, "high": 42, "mixed": 43, "hopeless": 44}[kind])
+    y0, Pd, Qd, A, c = _dense_case(rng, kind)
+    assert safety_affine_ref.project_affine(y0, Pd, Qd, BLDS, A, c, 0.9, 1.1)[2] > 0      # finite: it moves
+    for k in range(5):
+        for i in range(4):
+            bad = y0.copy(); bad[k, i] = np.nan
+            got, slack, status = safety_affine_ref.project_affine(bad, Pd, Qd, BLDS, A, c, 0.9, 1.1)
+            assert status == 0 and np.array_equal(slack, np.zeros(NB))
+            assert np.array_equal(got, bad, equal_nan=True) and np.isnan(got[k, i]) and np.isnan(got).sum() == 1
