@@ -1,8 +1,47 @@
-"""fp64 references of the device rollout's kernels for any agent count na in 1 .. 5, shared by the GPU tests.
+"""fp64 references of the device rollout's kernels (k_policy, k_sample, k_critic) for any agent count na in 1 .. 5, their
+per-element error model, and the drivers that run the kernels into sentinel-filled outputs and check every row.
 
-The error model is the one stated in tests/test_gpu_rollout_scale.py's docstring; only the shapes follow na: the policy's
-fc1 has 144 + na inputs (its kappa does not depend on na: K = 144 either way), the critic's fc1 na x 144 observation and
-na x 4 action columns, K padded to 24 for the actions: m = 2 (18 na + 3) MMA instructions, kappa = 1 + m / 4."""
+Reference.  torch float64 on the device, in chunks of 65 536 envs, from the raw observation ring by plain indexing
+(window entry r of env e, agent a, feature f = ring[(slot + 1 + r) % 24, a, f, e]), with exactly the matrices the loaders
+hold: fc1's observation (and, for the critic, action) columns, the GRU matrices and the critic's fc2 rounded to TF32
+(flexgpu.policy.round_tf32); biases, LayerNorm parameters, the policy's fc2 and the critic's fc3 unrounded fp32; the
+one-hot column folded into the bias by one fp32 addition.
+
+Error model, per element, propagated in float64 next to the reference (u = 2^-24, ulp = fp32 spacing of the value):
+  * tcgen05 GEMM, A = activations split x = hi + lo (hi TF32-exact), B = TF32 weights, fp32 accumulator, m MMA instructions
+    of K = 8 into one accumulator:  e <= kappa 2^-20 |W||x|,  kappa = 1 + m / 4.  The 1 is lo's own truncation to TF32
+    (|lo| < 2^-10 |x|, truncated to 11 bits: < 2^-20 |x|); hi x W is exact (11 x 11 bits).  Each instruction adds its
+    products to the accumulator with at most 2 ulp (truncating alignment) of a magnitude <= sum |W||x|: 2 m 2^-23 =
+    (m / 4) 2^-20.  fc1: m = 2 x 18 (policy, K = 144 whatever na: kappa = 19), 2 x (18 na + 3) (critic, na x 144
+    observation columns and na x 4 action columns padded to K = 24: kappa_critic_fc1(na), 47.5 at na = 5); GRU: m = 32
+    for r | z (x and h sides in one accumulator: kappa = 9), 16 for gi_n and gh_n (kappa = 5); critic fc2: m = 16
+    (kappa = 5).  A bias is added in fp32 after the MMA: + ulp(v).
+  * LayerNorm, centred (mean_q, M2_q per 16-column quarter, Chan merge): e_mu = mean(e1) + the rounding of the sums in
+    the kernel's order (u times every partial sum, from the reference values); e_var = 2 mean(|v - mu| e1) + mean(e1)^2
+    + e_mu^2 + 2^-19 var (the 16-term fma chains and the merge, 32 roundings); rstd: e_r = e_var / (2 (var + 1e-5 -
+    e_var)) + 2^-21 (rsqrtf 2 ulp, the + 1e-5);  e_y = |g| rstd (e1 + e_mu) + |g| |v - mu| rstd (e_r + 2^-23) + ulp(y).
+    ReLU: Lipschitz 1.  A common offset C of v enters only through ulp(v) and the sums' rounding: linear in C.
+  * GRU: gate arguments e = |W| e_x + kappa 2^-20 (|W_ih||x| + |W_hh||h|) + 2^-23 (|acc| + |b|) (the biases stored
+    pre-scaled by log2 e, one fma in the exponential's unit).  sigmoid8 / tanh8_scaled: ex2.approx (2 ulp), the + 1,
+    rcp4's four roundings (<= 2.4e-7 relative, policy.cu rcp4): c_sig = c_tanh = 6e-7 absolute.  r, z: 1/4 e + c_sig;
+    n: argument e_n = e_gin + r e_ghn + |gh_n + b_hn| e_r + 2^-22 (|gi_n| + |b_in| + r (|gh_n| + |b_hn|)), then
+    (1 - n^2 + e) e + c_tanh.  h' = n + z (h - n): |h - n| e_z + (1 - z + e_z) e_n + u |h - n| + ulp(h').
+  * fc2 (fp32 fma chains of 16, four partial sums, + bias): e_m = |W2| e_h + 2^-18 (|W2||h| + |b2|).
+  * action a = tanh_fast(x) (__expf, __fdividef: absolute error < 8 2^-23 on [0, 15]): e_a = min(1, 1 - a^2 + 2 e_x) e_x
+    + 8 2^-23, x = m (test mode) or fma(std, z, m) (e_x = e_m + std e_z + ulp(x)).
+  * log-probability: -(x - m)^2 / (2 std^2) - log std - log sqrt(2 pi) - log(1 - a^2 + 1e-6).  The Gaussian term from
+    d = x - m in fp32: (|z| / std)(ulp(x) + ulp(d) + std e_z) + 4 u z^2 / 2.  The tanh correction, conditioned on the row's
+    own a: w = 1 - a^2 + 1e-6 moves by dw = 2 |a| e_a + e_a^2 + 3 2^-25 (a^2, 1 - a^2, + 1e-6 in fp32), so the log by
+    dw / max(w - dw, 0.99e-6) (the kernel's a <= 1: w >= 1e-6), plus __logf (2^-21.41 absolute on [0.5, 2], else 3 ulp).
+    Near |a| = 1 one ulp of a moves logp by ~0.1: a flat tolerance cannot hold on millions of draws.  The formula alone is
+    checked separately: logp against the fp64 formula at the kernel's own fp32 a and x (caller eps, std = 1).
+  * Philox + Box-Muller: z_ref in fp64 from the exact uniforms of the numpy port.  ra = sqrt(-2 __logf(u0)): e_L =
+    2^-21.41 (u0 in [0.5, 1]) or 3 ulp(L) and e_ra = 2 e_L / (sqrt(2 |L| + 2 e_L) + sqrt(2 |L|)) + u ra; the angle
+    fp32(2 pi) u1 (up to 2 pi: __sincosf outside [-pi, pi], whose sin.approx / cos.approx absolute error is 2^-20.5 over
+    +-100 pi) + 2 u 2 pi; e_z = e_ra + ra e_trig + ulp(z).
+Worst.report prints max(err / bound) per quantity."""
+import contextlib
+
 import numpy as np
 import torch
 
@@ -14,7 +53,6 @@ C_TANH_FAST = 8 * 2.0 ** -23
 SENT = 7.25e6                                       # sentinel: no output of these kernels comes near it
 KEYS = ("fc1.weight", "fc1.bias", "layernorm.weight", "layernorm.bias", "rnn.weight_ih", "rnn.weight_hh", "rnn.bias_ih",
         "rnn.bias_hh", "fc2.weight", "fc2.bias")
-CKEYS = ("fc1.weight", "fc1.bias", "layernorm.weight", "layernorm.bias", "fc2.weight", "fc2.bias", "fc3.weight", "fc3.bias")
 
 
 def kappa_critic_fc1(na):
@@ -71,6 +109,19 @@ def windows(ring, slot, e0, e1):
     na = ring.shape[1]
     idx = torch.tensor([(slot + 1 + r) % 24 for r in range(24)], device=ring.device)
     return ring[:, :, :, e0:e1][idx].permute(3, 1, 0, 2).reshape(e1 - e0, na, 144)
+
+
+def ring_from_windows(obs, slot):
+    """The inverse of windows(): windows [n, na, 144] (oldest entry first; numpy or torch) -> the env-minor ring
+    [24, na, 6, n_pad] on obs's device with its newest entry in `slot`, zeros past env n."""
+    obs = torch.as_tensor(obs)
+    n, na = obs.shape[0], obs.shape[1]
+    n_pad = (n + 31) // 32 * 32
+    w = obs.reshape(n, na, 24, 6)
+    ring = torch.zeros(24, na, 6, n_pad, device=obs.device)
+    for r in range(24):
+        ring[(slot + 1 + r) % 24, :, :, :n] = w[:, :, r, :].permute(1, 2, 0)
+    return ring
 
 
 def policy_mats(sd, dev):
@@ -228,6 +279,7 @@ class Worst:
     def report(self):
         print(f"max(err/bound) {self.tag}: " + ", ".join(f"{k} {v:.3g}" for k, v in sorted(self.w.items())))
 
+
 def policy_reference(M, obs, h):
     """fp64 RNNAgent forward of obs [c, na, 144] (fp32 values) and h [c, na, 64]: mean, h', and their bounds."""
     x = obs.double()
@@ -319,3 +371,103 @@ def mlp_critic_torch(w, obs, act):
     finally:
         torch.backends.cuda.matmul.allow_tf32 = prev
     return v.view(N, na, 1)
+
+
+# ------------------------------------------------------------------------------------------------ drivers
+@contextlib.contextmanager
+def hbm_traffic():
+    """1 GB of HBM traffic on a side stream racing what the block launches; synchronises the device on exit."""
+    side = torch.cuda.Stream()
+    junk = torch.empty(1 << 28, device=torch.cuda.current_device())
+    side.wait_stream(torch.cuda.current_stream())
+    with torch.cuda.stream(side):
+        for _ in range(4):
+            junk.mul_(0.5)
+    yield
+    torch.cuda.current_stream().wait_stream(side)
+    torch.cuda.synchronize()
+
+
+def hidden_input(n, na, n_pad, kind, layout, cuda, seed):
+    """act()'s hidden-state input of `kind` none / given / reset (every third env) in `layout` rows / env_minor:
+    (hid_in, reset, h_ref), h_ref [n, na, 64] the rows the kernel must start from."""
+    g = torch.Generator(device=cuda).manual_seed(seed)
+    h = 0.9 * (2 * torch.rand(n, na, 64, device=cuda, generator=g) - 1)
+    reset = None
+    if kind == "reset":
+        reset = torch.zeros(n, dtype=torch.uint8, device=cuda); reset[::3] = 1
+    h_ref = torch.zeros_like(h) if kind == "none" else h.clone()
+    if reset is not None:
+        h_ref[reset.bool()] = 0
+    if kind == "none":
+        return None, None, h_ref
+    if layout == "rows":
+        return h, reset, h_ref
+    em = torch.zeros(na, 64, n_pad, device=cuda); em[:, :, :n] = h.permute(1, 2, 0)
+    return em, reset, h_ref
+
+
+def run_policy(pol, ring, slot, n, hid_in, reset, layout, mode, eps, step):
+    """act() in `mode` eps / philox / test, under side-stream HBM traffic, into sentinel-filled outputs with a guard band
+    past row n (and, env-minor, past column n and agent na): (action, logp, hid rows, mean)."""
+    na, n_pad, dev = pol.n_agents, ring.shape[-1], ring.device
+    full = {k: torch.full((n + 64, na, 4), SENT, device=dev) for k in ("action", "logp", "mean")}
+    for k in ("action", "logp"):
+        pol._bufs[k] = full[k][:n]
+    if layout == "rows":
+        hfull = torch.full((n + 8, na, 64), SENT, device=dev); hid_out = hfull[:n]
+    else:
+        hfull = torch.full((na + 1, 64, n_pad), SENT, device=dev); hid_out = hfull[:na]
+    with hbm_traffic():
+        pol.act(ring, slot=slot, n_envs=n, hid_in=hid_in, reset=reset, explore=mode != "test",
+                eps=eps if mode == "eps" else None, step=step, hid_out=hid_out, hid_layout=layout, want_mean=True,
+                mean_out=full["mean"][:n])
+    for k in ("action", "logp", "mean"):
+        assert bool((full[k][n:] == SENT).all()), ("written past row n", k)
+    if layout == "rows":
+        assert bool((hfull[n:] == SENT).all()), "hidden rows written past n"
+        h_rows = hid_out
+    else:
+        assert bool((hfull[na:] == SENT).all()) and bool((hfull[:na, :, n:] == SENT).all()), "env-minor hidden written past n / na"
+        h_rows = hfull[:na, :, :n].permute(2, 0, 1)
+    return full["action"][:n].clone(), full["logp"][:n].clone(), h_rows.clone(), full["mean"][:n].clone()
+
+
+def check_policy(wst, pol, M, ring, slot, n, h_ref, eps, step, outs, *, rms):
+    """run_policy's outputs `outs` by mode, every row in chunks against policy_reference: mean and hid (the same in every
+    mode), then action and log-probability with the caller's eps, with the Philox port's draws and in test mode."""
+    na, dev = pol.n_agents, ring.device
+    for mode in ("philox", "test"):                                          # the network's outputs do not depend on the draw
+        assert torch.equal(outs[mode][3], outs["eps"][3]) and torch.equal(outs[mode][2], outs["eps"][2])
+    for e0 in range(0, n, CHUNK):
+        e1 = min(n, e0 + CHUNK)
+        m, e_m, h1, e_h = policy_reference(M, windows(ring, slot, e0, e1), h_ref[e0:e1].double())
+        wst.check("mean", outs["eps"][3][e0:e1], m, e_m, rms=rms)
+        wst.check("hid", outs["eps"][2][e0:e1], h1, e_h, rms=rms)
+        rows = (np.arange(e0, e1, dtype=np.uint64)[:, None] * np.uint64(na) + np.arange(na, dtype=np.uint64)[None]).reshape(-1)
+        zp, ezp = philox_normals(rows, pol.seed, step)
+        z_ph = torch.from_numpy(zp).to(dev).view(e1 - e0, na, 4); e_ph = torch.from_numpy(ezp).to(dev).view(e1 - e0, na, 4)
+        z_eps = eps[e0:e1].double()
+        for mode, z, ez in (("eps", z_eps, torch.zeros_like(z_eps)), ("philox", z_ph, e_ph), ("test", None, None)):
+            act, logp = outs[mode][0][e0:e1], outs[mode][1][e0:e1]
+            a, e_a, x, e_x = action_bound(m, e_m, z, ez, pol.std, mode != "test")
+            wst.check("action", act, a, e_a, f"[{mode}]")
+            if mode == "test":
+                assert bool((logp == 0).all())
+                continue
+            lp, e_lp = logp_bound(a, e_a, z, ez, x, pol.std)
+            wst.check("logp", logp, lp, e_lp, f"[{mode}]")
+
+
+def critic_rows(wst, pol, M, ring, slot, n, act, key="", *, rms):
+    """value() of the first n envs under side-stream HBM traffic into a sentinel-filled output (the rows past n_envs keep
+    their sentinels), every row in chunks against critic_reference."""
+    na = ring.shape[1]
+    out_full = torch.full((ring.shape[-1] + 16, na, 1), SENT, device=ring.device)
+    with hbm_traffic():
+        pol.value(ring, act[:n], slot=slot, n_envs=n, out=out_full[:n])
+    assert bool((out_full[n:] == SENT).all()), "value written past n_envs"
+    for e0 in range(0, n, CHUNK):
+        e1 = min(n, e0 + CHUNK)
+        val, e_val = critic_reference(M, windows(ring, slot, e0, e1).reshape(e1 - e0, na * 144), act[e0:e1].reshape(e1 - e0, na * 4))
+        wst.check("value", out_full[e0:e1, :, 0], val, e_val, key, rms=rms)

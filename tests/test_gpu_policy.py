@@ -16,11 +16,10 @@ import numpy as np
 import pytest
 import torch
 from _golden import load_ref_policy
+from _rollout_ref import KEYS, mlp_critic_torch, ring_from_windows, torch_mats
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "ref_policy.npz")
-KEYS = ("fc1.weight", "fc1.bias", "layernorm.weight", "layernorm.bias", "rnn.weight_ih", "rnn.weight_hh", "rnn.bias_ih",
-        "rnn.bias_hh", "fc2.weight", "fc2.bias")
 
 
 @pytest.fixture(scope="module")
@@ -33,17 +32,6 @@ def hidden_rows(gold, n):
     return np.resize(gold["t_hid0"], (n, 5, 64))
 
 
-def make_ring(obs, slot, cuda, n_pad=None):
-    """[n, 5, 144] windows (oldest entry first) -> the env-minor ring [24, 5, 6, n_pad] with its newest entry in `slot`."""
-    n = obs.shape[0]
-    n_pad = n_pad or (n + 31) // 32 * 32
-    w = torch.from_numpy(obs).view(n, 5, 24, 6)
-    ring = torch.zeros(24, 5, 6, n_pad)
-    for r in range(24):
-        ring[(slot + 1 + r) % 24, :, :, :n] = w[:, :, r, :].permute(1, 2, 0)
-    return ring.to(cuda).contiguous()
-
-
 @pytest.mark.parametrize("tag,tol,tol_lp", [("t_", 2e-5, 2e-4), ("", 5e-4, 5e-3)])
 def test_policy_matches_reference_rnn_agent(gold, cuda, tag, tol, tol_lp):
     from flexgpu.policy import DevicePolicy
@@ -54,7 +42,7 @@ def test_policy_matches_reference_rnn_agent(gold, cuda, tag, tol, tol_lp):
     worst = {}
     rows = torch.from_numpy(gold["hid_rows"]).to(cuda)           # the envs whose hidden states the fixture keeps
     for t, slot in enumerate((7, 23, 0)):                       # three recurrent steps, three rotations of the ring
-        ring = make_ring(gold[f"obs{t}"], slot, cuda)
+        ring = ring_from_windows(gold[f"obs{t}"], slot).to(cuda)
         hid_out = torch.empty(n, 5, 64, device=cuda)
         act, logp, hid_new, mean = pol.act(ring, slot=slot, n_envs=n, hid_in=hid, explore=True, eps=torch.from_numpy(gold[f"eps{t}"]),
                                            hid_out=hid_out, want_mean=True)
@@ -77,7 +65,7 @@ def test_policy_rows_are_independent_and_ragged_sizes(gold, cuda):
     h0 = hidden_rows(gold, 160)
     full = None
     for n in (160, 129, 128, 33, 1):
-        ring = make_ring(obs[:n], 5, cuda)
+        ring = ring_from_windows(obs[:n], 5).to(cuda)
         h_in = torch.from_numpy(h0[:n]).to(cuda).contiguous()
         act, _, hid, mean = pol.act(ring, slot=5, n_envs=n, hid_in=h_in, explore=False, want_mean=True, hid_out=torch.empty(n, 5, 64, device=cuda))
         got = (mean.cpu().numpy().copy(), hid.cpu().numpy().copy())
@@ -87,7 +75,7 @@ def test_policy_rows_are_independent_and_ragged_sizes(gold, cuda):
             assert np.array_equal(got[0], full[0][:n]) and np.array_equal(got[1], full[1][:n])
     # the env-minor hidden-state layout [5, 64, n_pad] (the kernel's native one) gives the same bits
     n = 160
-    ring = make_ring(obs, 5, cuda)
+    ring = ring_from_windows(obs, 5).to(cuda)
     h_rows = torch.from_numpy(h0).to(cuda).contiguous()
     h_em = torch.zeros(5, 64, 160, device=cuda); h_em[:, :, :n] = h_rows.permute(1, 2, 0)
     out_em = torch.empty(5, 64, 160, device=cuda)
@@ -96,7 +84,7 @@ def test_policy_rows_are_independent_and_ragged_sizes(gold, cuda):
     assert np.array_equal(mean_em.cpu().numpy(), full[0]) and np.array_equal(hid_em[:, :, :n].permute(2, 0, 1).cpu().numpy(), full[1])
     # reset mask: the masked envs act from a zero hidden state
     n = 160
-    ring = make_ring(obs, 5, cuda)
+    ring = ring_from_windows(obs, 5).to(cuda)
     h_in = torch.from_numpy(h0).to(cuda).contiguous()
     mask = torch.zeros(n, dtype=torch.uint8, device=cuda); mask[::3] = 1
     _, _, hid_m, mean_m = pol.act(ring, slot=5, n_envs=n, hid_in=h_in, reset=mask, explore=False, want_mean=True, hid_out=torch.empty(n, 5, 64, device=cuda))
@@ -119,7 +107,7 @@ def test_policy_saturated_gates_stay_finite(gold, cuda):
     obs = gold["obs1"]
     n = obs.shape[0]
     h0 = (np.random.default_rng(3).uniform(-1, 1, (n, 5, 64))).astype(np.float32)
-    ring = make_ring(obs, 11, cuda)
+    ring = ring_from_windows(obs, 11).to(cuda)
     _, _, hid, mean = pol.act(ring, slot=11, n_envs=n, hid_in=torch.from_numpy(h0).to(cuda), explore=False, want_mean=True,
                               hid_out=torch.empty(n, 5, 64, device=cuda))
     t = {k: torch.from_numpy(v).double() for k, v in w.items()}
@@ -150,7 +138,7 @@ def test_policy_nan_observation_poisons_its_row_only(gold, cuda):
         o = obs.copy()
         if poison:
             o[37, 2, 100] = np.nan
-        ring = make_ring(o, 5, cuda)
+        ring = ring_from_windows(o, 5).to(cuda)
         _, _, hid, mean = pol.act(ring, slot=5, n_envs=n, hid_in=None, explore=False, want_mean=True, hid_out=torch.empty(n, 5, 64, device=cuda))
         outs.append((hid.cpu().numpy().copy(), mean.cpu().numpy().copy()))
     (h0, m0), (h1, m1) = outs
@@ -166,7 +154,7 @@ def test_policy_philox_sampling(gold, cuda):
     pol = DevicePolicy({k: gold["wt_" + k] for k in KEYS}, device=cuda, std=1.0, seed=1234)
     n = 4096
     obs = np.tile(gold["obs0"], (26, 1, 1))[:n]
-    ring = make_ring(obs, 3, cuda)
+    ring = ring_from_windows(obs, 3).to(cuda)
     a1, lp1, _, m1 = pol.act(ring, slot=3, n_envs=n, explore=True, step=7, want_mean=True)
     a1, lp1, m1 = a1.double().cpu().numpy().copy(), lp1.cpu().numpy().copy(), m1.double().cpu().numpy().copy()
     a2, _, _, _ = pol.act(ring, slot=3, n_envs=n, explore=True, step=7)
@@ -369,26 +357,13 @@ def test_rollout_resets_early_terminations_each_step(gold, cuda, profiles):
     pol.close(); buf.close(); env.close()
 
 
-def _critic_torch(w, obs_all, act_all, cuda):
-    """MADDPG.value (maddpg.py:29-76) + MLPCritic.forward (mlp_critic.py:27-36) in plain torch fp32 on [n, 720] observations
-    and [n, 20] actions: rows (env, agent i) = [obs of all agents | one-hot(i) | actions of all agents]."""
-    F = torch.nn.functional
-    n = obs_all.shape[0]
-    eye = torch.eye(5, device=cuda)
-    x = torch.cat([obs_all[:, None, :].expand(n, 5, 720), eye[None].expand(n, 5, 5), act_all[:, None, :].expand(n, 5, 20)], dim=-1).reshape(n * 5, 745)
-    y = F.linear(x, w["fc1.weight"], w["fc1.bias"])
-    y = torch.relu(F.layer_norm(y, (64,), w["layernorm.weight"], w["layernorm.bias"], 1e-5))
-    h = torch.relu(F.linear(y, w["fc2.weight"], w["fc2.bias"]))
-    return F.linear(h, w["fc3.weight"], w["fc3.bias"]).view(n, 5, 1)
-
-
 @pytest.mark.parametrize("n", [300, 40, 1, 2 * 148 * 128 + 77])
 def test_native_critic_matches_torch(cuda, n):
     """fp_critic_value (k_critic, tcgen05) against plain torch fp32 with the same TF32-rounded fc1 / fc2 matrices (the
     device holds them as TF32, activations keep fp32 accuracy; bound 2e-5, observed ~1e-6): the TMA path with a ragged last
     tile, the LDGSTS path of rings narrower than a tile, a single env, and several tiles per CTA (weight blocks cycling
     through their three buffers); three ring rotations."""
-    from flexgpu.policy import DevicePolicy, round_tf32
+    from flexgpu.policy import DevicePolicy
     rng = np.random.default_rng(11)
     sd = {"fc1.weight": rng.normal(0, 0.05, (64, 745)), "fc1.bias": rng.uniform(-0.04, 0.04, 64), "layernorm.weight": 1 + rng.normal(0, 0.1, 64),
           "layernorm.bias": rng.normal(0, 0.1, 64), "fc2.weight": rng.uniform(-0.125, 0.125, (64, 64)), "fc2.bias": rng.uniform(-0.125, 0.125, 64),
@@ -396,25 +371,13 @@ def test_native_critic_matches_torch(cuda, n):
     sd = {k: v.astype(np.float32) for k, v in sd.items()}
     pol = DevicePolicy(None, device=cuda)
     pol.load_critic(sd)
-    w = {k: torch.from_numpy(v).to(cuda) for k, v in sd.items()}
-    w1 = sd["fc1.weight"].copy(); w1[:, :720] = round_tf32(w1[:, :720]); w1[:, 725:] = round_tf32(w1[:, 725:])
-    w["fc1.weight"] = torch.from_numpy(w1).to(cuda); w["fc2.weight"] = torch.from_numpy(round_tf32(sd["fc2.weight"])).to(cuda)
+    w = torch_mats(sd, cuda, critic=True)
     g = torch.Generator(device=cuda).manual_seed(3)
-    prev = torch.backends.cuda.matmul.allow_tf32
-    torch.backends.cuda.matmul.allow_tf32 = False
-    try:
-        for slot in (0, 9, 23):
-            obs = torch.rand(n, 5, 144, device=cuda, generator=g) * 2 - 0.5
-            act = torch.tanh(torch.randn(n, 5, 4, device=cuda, generator=g))
-            n_pad = (n + 31) // 32 * 32
-            ring = torch.zeros(24, 5, 6, n_pad, device=cuda)
-            wv = obs.view(n, 5, 24, 6)
-            for r in range(24):
-                ring[(slot + 1 + r) % 24, :, :, :n] = wv[:, :, r, :].permute(1, 2, 0)
-            got = pol.value(ring.contiguous(), act, slot=slot, n_envs=n).clone()
-            want = _critic_torch(w, obs.reshape(n, 720), act.reshape(n, 20), cuda)
-            err = float((got - want).abs().max())
-            assert got.shape == (n, 5, 1) and err < 2e-5, (slot, err)
-    finally:
-        torch.backends.cuda.matmul.allow_tf32 = prev
+    for slot in (0, 9, 23):
+        obs = torch.rand(n, 5, 144, device=cuda, generator=g) * 2 - 0.5
+        act = torch.tanh(torch.randn(n, 5, 4, device=cuda, generator=g))
+        got = pol.value(ring_from_windows(obs, slot), act, slot=slot, n_envs=n).clone()
+        want = mlp_critic_torch(w, obs, act)
+        err = float((got - want).abs().max())
+        assert got.shape == (n, 5, 1) and err < 2e-5, (slot, err)
     pol.close()

@@ -1,10 +1,9 @@
 """The device rollout at one to four agents: k_policy, k_sample, k_critic, the Transition writers and the learner feed of
-a DevicePolicy built for n_agents = na, every row against the fp64 references of tests/_rollout_ref.py (the error model of
-tests/test_gpu_rollout_scale.py), DeviceRollout on the catalogue feeders of each agent count, and the rejection of every
-agent-count or history mismatch."""
+a DevicePolicy built for n_agents = na, every row against the fp64 references and within the error model of
+tests/_rollout_ref.py, DeviceRollout on the catalogue feeders of each agent count, and the rejection of every agent-count
+or history mismatch."""
 import ctypes as C
 
-import numpy as np
 import pytest
 import torch
 
@@ -19,47 +18,6 @@ def _policy(na, seed=21, **kw):
     from flexgpu.policy import DevicePolicy
     sd = R.realistic_policy(seed + na, na)
     return DevicePolicy(sd, device="cuda:0", std=1.0, seed=(5 << 32) + 77, **kw), sd
-
-
-def _hidden(n, na, n_pad, kind, layout, cuda, seed):
-    g = torch.Generator(device=cuda).manual_seed(seed)
-    h = 0.9 * (2 * torch.rand(n, na, 64, device=cuda, generator=g) - 1)
-    reset = None
-    if kind == "reset":
-        reset = torch.zeros(n, dtype=torch.uint8, device=cuda); reset[::3] = 1
-    h_ref = torch.zeros_like(h) if kind == "none" else h.clone()
-    if reset is not None:
-        h_ref[reset.bool()] = 0
-    if kind == "none":
-        return None, None, h_ref
-    if layout == "rows":
-        return h, reset, h_ref
-    em = torch.zeros(na, 64, n_pad, device=cuda); em[:, :, :n] = h.permute(1, 2, 0)
-    return em, reset, h_ref
-
-
-def _run_policy(pol, ring, slot, n, hid_in, reset, layout, mode, eps, step):
-    """act() into sentinel-filled outputs with a guard band after each; returns (action, logp, hid rows, mean)."""
-    na, n_pad, dev = pol.n_agents, ring.shape[-1], ring.device
-    full = {k: torch.full((n + 64, na, 4), R.SENT, device=dev) for k in ("action", "logp", "mean")}
-    for k in ("action", "logp"):
-        pol._bufs[k] = full[k][:n]
-    if layout == "rows":
-        hfull = torch.full((n + 8, na, 64), R.SENT, device=dev); hid_out = hfull[:n]
-    else:
-        hfull = torch.full((na + 1, 64, n_pad), R.SENT, device=dev); hid_out = hfull[:na]
-    pol.act(ring, slot=slot, n_envs=n, hid_in=hid_in, reset=reset, explore=mode != "test", eps=eps if mode == "eps" else None,
-            step=step, hid_out=hid_out, hid_layout=layout, want_mean=True, mean_out=full["mean"][:n])
-    torch.cuda.synchronize()
-    for k in ("action", "logp", "mean"):
-        assert bool((full[k][n:] == R.SENT).all()), ("written past row n", k)
-    if layout == "rows":
-        assert bool((hfull[n:] == R.SENT).all()), "hidden rows written past n"
-        h_rows = hid_out
-    else:
-        assert bool((hfull[na:] == R.SENT).all()) and bool((hfull[:na, :, n:] == R.SENT).all()), "env-minor hidden written past n / na"
-        h_rows = hfull[:na, :, :n].permute(2, 0, 1)
-    return full["action"][:n].clone(), full["logp"][:n].clone(), h_rows.clone(), full["mean"][:n].clone()
 
 
 CONFIGS = [("rows", "none", 0), ("env_minor", "given", 11), ("rows", "reset", 23), ("env_minor", "reset", 5)]
@@ -77,29 +35,10 @@ def test_policy_every_row_against_fp64(cuda, na, n):
     wst = R.Worst(f"k_policy na={na} n={n}")
     for ci, (layout, hkind, slot) in enumerate(CONFIGS):
         ring, whole = R.random_ring(n, na, 100 * na + ci, cuda)
-        hid_in, reset, h_ref = _hidden(n, na, n_pad, hkind, layout, cuda, ci + n)
+        hid_in, reset, h_ref = R.hidden_input(n, na, n_pad, hkind, layout, cuda, ci + n)
         eps = torch.randn(n, na, 4, device=cuda, generator=torch.Generator(device=cuda).manual_seed(ci))
-        outs = {mode: _run_policy(pol, ring, slot, n, hid_in, reset, layout, mode, eps, step) for mode in ("eps", "philox", "test")}
-        for mode in ("philox", "test"):
-            assert torch.equal(outs[mode][3], outs["eps"][3]) and torch.equal(outs[mode][2], outs["eps"][2])
-        for e0 in range(0, n, R.CHUNK):
-            e1 = min(n, e0 + R.CHUNK)
-            m, e_m, h1, e_h = R.policy_reference(M, R.windows(ring, slot, e0, e1), h_ref[e0:e1].double())
-            wst.check("mean", outs["eps"][3][e0:e1], m, e_m, rms=n >= 3917)
-            wst.check("hid", outs["eps"][2][e0:e1], h1, e_h, rms=n >= 3917)
-            rows = (np.arange(e0, e1, dtype=np.uint64)[:, None] * np.uint64(na) + np.arange(na, dtype=np.uint64)[None]).reshape(-1)
-            zp, ezp = R.philox_normals(rows, pol.seed, step)
-            z_ph = torch.from_numpy(zp).to(cuda).view(e1 - e0, na, 4); e_ph = torch.from_numpy(ezp).to(cuda).view(e1 - e0, na, 4)
-            z_eps = eps[e0:e1].double()
-            for mode, z, ez in (("eps", z_eps, torch.zeros_like(z_eps)), ("philox", z_ph, e_ph), ("test", None, None)):
-                act, logp = outs[mode][0][e0:e1], outs[mode][1][e0:e1]
-                a, e_a, x, e_x = R.action_bound(m, e_m, z, ez, pol.std, mode != "test")
-                wst.check("action", act, a, e_a, f"[{mode}]")
-                if mode == "test":
-                    assert bool((logp == 0).all())
-                    continue
-                lp, e_lp = R.logp_bound(a, e_a, z, ez, x, pol.std)
-                wst.check("logp", logp, lp, e_lp, f"[{mode}]")
+        outs = {mode: R.run_policy(pol, ring, slot, n, hid_in, reset, layout, mode, eps, step) for mode in ("eps", "philox", "test")}
+        R.check_policy(wst, pol, M, ring, slot, n, h_ref, eps, step, outs, rms=n >= 3917)
         del whole
     wst.report()
     pol.close()
@@ -136,14 +75,7 @@ def test_critic_every_row_against_fp64(cuda, na, n):
     wst = R.Worst(f"k_critic na={na} n={n}")
     for slot in (0, 11, 23):
         ring, whole = R.random_ring(n, na, 7 + slot, cuda)
-        out_full = torch.full((n + 16, na, 1), R.SENT, device=cuda)
-        pol.value(ring, act, slot=slot, n_envs=n, out=out_full[:n])
-        torch.cuda.synchronize()
-        assert bool((out_full[n:] == R.SENT).all()), "value written past n_envs"
-        for e0 in range(0, n, R.CHUNK):
-            e1 = min(n, e0 + R.CHUNK)
-            val, e_val = R.critic_reference(M, R.windows(ring, slot, e0, e1).reshape(e1 - e0, na * 144), act[e0:e1].reshape(e1 - e0, na * 4))
-            wst.check("value", out_full[e0:e1, :, 0], val, e_val, f"[slot {slot}]", rms=n > 77)
+        R.critic_rows(wst, pol, M, ring, slot, n, act, f"[slot {slot}]", rms=n > 77)
         del whole
     wst.report()
     pol.close()
