@@ -450,7 +450,10 @@ static void env_core(const FoNet* c, const double* P, const double* Q, const dou
                      double* reward, uint8_t* done, double* info) {
     const int nl = c->nl, nb = c->nb, na = c->na;
     int32_t steps = is_reset ? 1 : s->steps[e];
-    const int64_t row = (int64_t)s->start[e] + ((!is_reset && steps > 1) ? steps - 1 : 1);   /* quirk Q1 */
+    /* quirk Q1; an env stepped on past `done` without a reset stays on the last row of its slice (episode_limit +
+       history + 1 rows), as the kernels do (row_in_force) */
+    const int max_off = c->episode_limit + c->history;
+    const int64_t row = (int64_t)s->start[e] + ((!is_reset && steps > 1) ? (steps - 1 < max_off ? steps - 1 : max_off) : 1);
     double pl[NL] = {0}, ql[NL] = {0};
     Setp sp[8];
     for (int k = 0; k < nl; ++k) { pl[k] = P[row * nl + c->col[k]]; ql[k] = Q[row * nl + c->col[k]]; }

@@ -212,7 +212,9 @@ class MirrorBatch:
 
     # numpy restatement of get_state / get_obs for the batch (flexibility_provision_env.py:358-403)
     def row(self):
-        return self.start.astype(np.int64) + np.where(self.steps > 1, self.steps - 1, 1)
+        """The profile row in force, clamped to the last row of the episode slice as the kernels clamp it."""
+        max_off = self.net.episode_limit + self.net.history
+        return self.start.astype(np.int64) + np.where(self.steps > 1, np.minimum(self.steps - 1, max_off), 1)
 
     def get_state(self):
         r = self.row()

@@ -220,6 +220,33 @@ def test_mirror_vs_env_ref_random_batch(fonet, profiles):
             assert int(viol.sum()) == mb.vcount[i]
 
 
+@pytest.mark.parametrize("variant", ["thread", "warp"])
+def test_mirror_clamps_the_row_past_the_episode_slice(fonets, profiles, variant):
+    """An env stepped on past `done` without a reset stays on the last row of its episode slice (start + episode_limit +
+    history), as the kernels' row_in_force does.  Every row after the slice of the latest start is NaN but inside the
+    table: 130 steps without a reset (past the end of the episode, steps 119-123 around the clamp) stay finite and
+    bit-identical to a run on the finite table."""
+    from _obs_ref import clamp_tables
+    s0, n = 1000, 41
+    finite, poisoned = clamp_tables(profiles, s0)
+    start = (s0 - np.arange(n)).astype(np.int32)                       # starts s0 - 40 .. s0
+    rng = np.random.default_rng(3)
+    e0 = rng.uniform(0.9 * 0.0125, 1.1 * 0.0125, (n, 5)); a0 = rng.uniform(0, 1, (n, 20))
+    runs = []
+    for prof in (poisoned, finite):
+        mb = c_mirror.MirrorBatch(fonets[variant], prof.as_dict(), n)
+        mb.reset(start, e0, a0)
+        out = []
+        act = np.random.default_rng(4)
+        for t in range(130):
+            r, d, info = mb.step(act.uniform(0, 1, (n, 20)))
+            out += [r.copy(), info.copy(), mb.V.copy(), mb.E_cur.copy(), mb.setp.copy(), mb.current_obs(), mb.get_state()]
+        assert d.all() and int(mb.steps.min()) == 131
+        runs.append(out)
+    for k, (x, y) in enumerate(zip(*runs)):
+        assert np.isfinite(x).all() and np.array_equal(x, y), (k // 7, k % 7)
+
+
 def test_mirror_failure_injection_matches_env_ref(fonet, profiles):
     flag = {'on': False}
     env = make_env(profiles, seed=9, force_fail=lambda e: flag['on'])
