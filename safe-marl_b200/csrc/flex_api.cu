@@ -130,11 +130,8 @@ static void fill_devcfg(const FpConfig& c, DevCfg& d) {
     d.pf_f32 = c.pf_f32_passes;
 }
 
-static int grid_for(int64_t n, int cap) {
-    int64_t ctas = (n + (FP_CTA_THREADS / 32) - 1) / (FP_CTA_THREADS / 32);
-    if (ctas < 1) ctas = 1;
-    return (int)((ctas < cap) ? ctas : cap);
-}
+// envs per CTA of the warp variant's kernels and of the observation kernels: one env per warp
+constexpr int64_t ENVS_PER_CTA = FP_CTA_THREADS / 32;
 
 extern "C" {
 
@@ -187,26 +184,17 @@ int fp_create(const FpConfig* cfg, int64_t n_envs, int device, FpHandle** out) {
     {   // observation / state kernels are streaming kernels: a full SM worth of warps (8 CTAs of 256 threads)
         int sms = 0;
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-        h->grid_obs = grid_for(n_envs, 8 * (sms > 0 ? sms : 1));
+        const int64_t ctas = (n_envs + ENVS_PER_CTA - 1) / ENVS_PER_CTA, cap = 8 * (sms > 0 ? sms : 1);
+        h->grid_obs = (int)((ctas < cap) ? ctas : cap);
     }
-    if (h->variant == FP_VARIANT_THREAD) {
-        CREATE_TRY(thread_kernels_configure(FP_MAX_SLOTS));
-        const int64_t tiles = (n_envs + 31) / 32;
-        const int cap_step = thread_kernel_max_grid(MODE_STEP, h->tt.n_slots, h->shape);
-        const int cap_reset = thread_kernel_max_grid(MODE_RESET, h->tt.n_slots, h->shape);
-        h->grid_step = (int)((tiles < cap_step) ? tiles : cap_step);
-        if (const char* gs = std::getenv("FLEXGPU_GRID_STEP")) {      // tuning knob: persistent CTAs of the step kernel
-            const int g = std::atoi(gs);
-            if (g > 0 && g <= cap_step) h->grid_step = (int)((tiles < g) ? tiles : g);
-        }
-        h->grid_reset = (int)((tiles < cap_reset) ? tiles : cap_reset);
-        h->grid_pf = thread_kernel_max_grid(MODE_PF, h->tt.n_slots, h->shape);
-        h->stats_rows = cap_step;
-    } else {
-        h->grid_step = grid_for(n_envs, max_resident_grid(MODE_STEP));
-        h->grid_reset = grid_for(n_envs, max_resident_grid(MODE_RESET));
-        h->grid_pf = max_resident_grid(MODE_PF);
-        h->stats_rows = max_resident_grid(MODE_STEP);
+    const bool thread = h->variant == FP_VARIANT_THREAD;
+    if (thread) CREATE_TRY(thread_kernels_configure(FP_MAX_SLOTS));
+    for (int mode : {MODE_STEP, MODE_RESET, MODE_PF, MODE_PREVIEW})
+        h->cap[mode] = thread ? thread_kernel_max_grid(mode, h->tt.n_slots, h->shape) : max_resident_grid(mode);
+    h->stats_rows = h->cap[MODE_STEP];
+    if (const char* gs = std::getenv("FLEXGPU_GRID_STEP")) {          // tuning knob: persistent CTAs of the thread step kernel
+        const int g = std::atoi(gs);
+        if (thread && g > 0 && g <= h->cap[MODE_STEP]) h->cap[MODE_STEP] = g;
     }
     CREATE_TRY(cudaMalloc(&h->d_stats_partial, (size_t)h->stats_rows * FP_NSTATS * 8));
     CREATE_TRY(cudaMemset(h->d_stats_partial, 0, (size_t)h->stats_rows * FP_NSTATS * 8));
@@ -224,7 +212,6 @@ int fp_destroy(FpHandle* h) {
     cudaFree(h->d_rec); cudaFree(h->d_V); cudaFree(h->d_setp); cudaFree(h->d_hist); cudaFree(h->d_obsm); cudaFree(h->d_obsr);
     cudaFree(h->d_pfl); cudaFree(h->d_qfl); cudaFree(h->d_isq); cudaFree(h->d_stats_partial); cudaFree(h->d_retry_mask); cudaFree(h->d_retry_count);
     cudaFree(h->d_act_stage); cudaFree(h->d_act_xlat); cudaFree(h->d_reward_stage); cudaFree(h->d_done_stage); cudaFree(h->d_info_stage);
-    cudaFree(h->d_prev_xlat);
     cudaFree(h->d_saff_At); cudaFree(h->d_saff_c);
     delete h;
     return FP_OK;
@@ -289,45 +276,74 @@ static int bulk_io_ok(const EnvParams& p) {
     return (al16(p.rec) && al16(p.setp) && al16(p.V) && al16(p.reward) && al16(p.done) && (p.info == nullptr || al16(p.info))) ? 1 : 0;
 }
 
-// translate_action's constants exactly as torch forms them (utils/util.py:124-128): the clamp bounds
-// and `low` become fp32 scalars, `high - low` is a Python (double) difference turned into an fp32 scalar
-static void set_translate(const FpHandle* h, EnvParams& p) {
-    p.act_translate = 1;
-    p.act_lo = (float)h->cfg.action_low; p.act_hi = (float)h->cfg.action_high;
-    p.act_span = (float)(h->cfg.action_high - h->cfg.action_low);
-}
-
-static cudaError_t launch_env_any(FpHandle* h, int mode, const EnvParams& p, cudaStream_t st) {
-    const int grid = (mode == MODE_STEP) ? h->grid_step : h->grid_reset;
+// The env kernel of `mode` on the handle's variant, over k candidates per env for MODE_PREVIEW (k = 1 otherwise), on
+// at most its resident grid.  translate: p.actions are raw fp32 policy outputs (FP_F32_POLICY), translated into the
+// step kernel (thread variant) or by an elementwise pre-pass into the handle's scratch (warp variant).
+static int launch_env_any(FpHandle* h, int mode, EnvParams p, bool translate, int64_t k, cudaStream_t st) {
+    // translate_action's constants exactly as torch forms them (utils/util.py:124-128): the clamp bounds
+    // and `low` become fp32 scalars, `high - low` is a Python (double) difference turned into an fp32 scalar
+    const float lo = (float)h->cfg.action_low, hi = (float)h->cfg.action_high;
+    const float span = (float)(h->cfg.action_high - h->cfg.action_low);
+    const int cap = h->cap[mode];
     if (h->variant == FP_VARIANT_THREAD) {
         EnvParamsT pt;
         pt.e = p; pt.t = h->tt;
+        if (translate) { pt.e.act_translate = 1; pt.e.act_lo = lo; pt.e.act_hi = hi; pt.e.act_span = span; }
         if (mode == MODE_STEP) pt.e.bulk_io = bulk_io_ok(p);
-        return launch_env_t(mode, h->shape, pt, grid, st);
+        const int64_t tiles = k * ((h->n + 31) / 32);           // 32-env tiles; every candidate's envs start a tile
+        CUDA_TRY(h, launch_env_t(mode, h->shape, pt, (int)((tiles < cap) ? tiles : cap), st));
+    } else {
+        if (translate) {
+            const int64_t cnt = k * h->n * h->dc.na * 4;
+            if (cnt > h->act_xlat_cap) {
+                cudaFree(h->d_act_xlat); h->d_act_xlat = nullptr; h->act_xlat_cap = 0;
+                CUDA_TRY(h, cudaMalloc(&h->d_act_xlat, (size_t)cnt * 4));
+                h->act_xlat_cap = cnt;
+            }
+            CUDA_TRY(h, launch_translate_actions((const float*)p.actions, h->d_act_xlat, cnt, lo, hi, span, st));
+            h->launches++;
+            p.actions = h->d_act_xlat;
+        }
+        const int64_t ctas = (k * h->n + ENVS_PER_CTA - 1) / ENVS_PER_CTA;
+        CUDA_TRY(h, launch_env(mode, p, (int)((ctas < cap) ? ctas : cap), st));
     }
-    return launch_env(mode, p, grid, st);
+    h->launches++;
+    return FP_OK;
 }
+
+// Restarts the observation rings of the envs of d_mask (all envs: null) after their reset: the zero padding of their
+// windows in the window ring, their history in the env-minor ring.  A ring that is not valid is rebuilt on its next use.
+static int restart_obs_rings(FpHandle* h, const uint8_t* d_mask, cudaStream_t st) {
+    if (h->d_obsm && h->obsm_valid) {
+        CUDA_TRY(h, launch_obsm_clear(h->d_obsm, d_mask, h->n, h->dc.na * 3 * h->dc.history * 6, st));
+        h->launches++;
+    }
+    if (h->d_obsr && h->obsr_valid) {
+        CUDA_TRY(h, launch_obsr_clear(h->d_obsr, d_mask, h->n, h->n_pad, h->dc.history * h->dc.na * 6, st));
+        h->launches++;
+    }
+    return FP_OK;
+}
+
+// The preamble of the entry points that need the profile dataset: a handle, its device current for the rest of the
+// call, profiles loaded.  `what` is the entry point's name, a string literal.
+#define ENV_ENTRY(h, what)                                                                                \
+    if (!(h)) return FP_EINVAL;                                                                           \
+    USE_DEVICE(h);                                                                                        \
+    if (!(h)->d_P) return fail((h), FP_ESTATE, what ": call fp_load_profiles first")
+
+// The action dtypes of the stepping entry points
+static bool step_dtype_ok(int act_dtype) { return act_dtype == FP_F32 || act_dtype == FP_F64 || act_dtype == FP_F32_POLICY; }
 
 int fp_reset(FpHandle* h, const int32_t* d_start, const double* d_e0, const double* d_a0,
              const uint8_t* d_mask, void* stream) {
-    if (!h) return FP_EINVAL;
-    USE_DEVICE(h);
-    if (!h->d_P) return fail(h, FP_ESTATE, "fp_reset: call fp_load_profiles first");
+    ENV_ENTRY(h, "fp_reset");
     if (!d_start || !d_e0 || !d_a0) return fail(h, FP_EINVAL, "fp_reset: null input");
     EnvParams p; fill_env_params(h, p);
     p.start = d_start; p.e0 = d_e0; p.a0 = d_a0; p.mask = d_mask; p.random = 0;
     p.inject = nullptr;
-    CUDA_TRY(h, launch_env_any(h, MODE_RESET, p, (cudaStream_t)stream));
-    h->launches++;
-    if (h->d_obsm && h->obsm_valid) {              // restart the zero padding of the reset envs' observation windows
-        CUDA_TRY(h, launch_obsm_clear(h->d_obsm, d_mask, h->n, h->dc.na * 3 * h->dc.history * 6, (cudaStream_t)stream));
-        h->launches++;
-    }
-    if (h->d_obsr && h->obsr_valid) {
-        CUDA_TRY(h, launch_obsr_clear(h->d_obsr, d_mask, h->n, h->n_pad, h->dc.history * h->dc.na * 6, (cudaStream_t)stream));
-        h->launches++;
-    }
-    return FP_OK;
+    const int rc = launch_env_any(h, MODE_RESET, p, false, 1, (cudaStream_t)stream);
+    return (rc != FP_OK) ? rc : restart_obs_rings(h, d_mask, (cudaStream_t)stream);
 }
 
 // One launch of the random reset for the envs of d_mask (+ the observation rings' restart).
@@ -335,23 +351,12 @@ static int reset_random_once(FpHandle* h, uint64_t seed, int64_t env_offset, con
     EnvParams p; fill_env_params(h, p);
     p.mask = d_mask; p.random = 1; p.seed = seed; p.env_offset = env_offset;
     p.inject = nullptr;
-    CUDA_TRY(h, launch_env_any(h, MODE_RESET, p, (cudaStream_t)stream));
-    h->launches++;
-    if (h->d_obsm && h->obsm_valid) {
-        CUDA_TRY(h, launch_obsm_clear(h->d_obsm, d_mask, h->n, h->dc.na * 3 * h->dc.history * 6, (cudaStream_t)stream));
-        h->launches++;
-    }
-    if (h->d_obsr && h->obsr_valid) {
-        CUDA_TRY(h, launch_obsr_clear(h->d_obsr, d_mask, h->n, h->n_pad, h->dc.history * h->dc.na * 6, (cudaStream_t)stream));
-        h->launches++;
-    }
-    return FP_OK;
+    const int rc = launch_env_any(h, MODE_RESET, p, false, 1, (cudaStream_t)stream);
+    return (rc != FP_OK) ? rc : restart_obs_rings(h, d_mask, (cudaStream_t)stream);
 }
 
 int fp_reset_random(FpHandle* h, uint64_t seed, int64_t env_offset, const uint8_t* d_mask, void* stream) {
-    if (!h) return FP_EINVAL;
-    USE_DEVICE(h);
-    if (!h->d_P) return fail(h, FP_ESTATE, "fp_reset_random: call fp_load_profiles first");
+    ENV_ENTRY(h, "fp_reset_random");
     return reset_random_once(h, seed, env_offset, d_mask, stream);
 }
 
@@ -362,9 +367,7 @@ int fp_reset_random(FpHandle* h, uint64_t seed, int64_t env_offset, const uint8_
 // still flagged after the last attempt (int32 on the device).
 int fp_reset_random_retry(FpHandle* h, uint64_t seed, int64_t env_offset, const uint8_t* d_mask, int32_t retries,
                           int32_t* d_failed, void* stream) {
-    if (!h) return FP_EINVAL;
-    USE_DEVICE(h);
-    if (!h->d_P) return fail(h, FP_ESTATE, "fp_reset_random_retry: call fp_load_profiles first");
+    ENV_ENTRY(h, "fp_reset_random_retry");
     if (retries < 0 || retries > 64) return fail(h, FP_EINVAL, "fp_reset_random_retry: 0 <= retries <= 64");
     int rc = reset_random_once(h, seed, env_offset, d_mask, stream);
     if (rc != FP_OK) return rc;
@@ -386,31 +389,15 @@ int fp_reset_random_retry(FpHandle* h, uint64_t seed, int64_t env_offset, const 
 
 int fp_step(FpHandle* h, const void* d_actions, int act_dtype, double* d_reward, uint8_t* d_done,
             double* d_info, const uint8_t* d_mask, void* stream) {
-    if (!h) return FP_EINVAL;
-    USE_DEVICE(h);
-    if (!h->d_P) return fail(h, FP_ESTATE, "fp_step: call fp_load_profiles first");
+    ENV_ENTRY(h, "fp_step");
     if (!d_actions || !d_reward || !d_done) return fail(h, FP_EINVAL, "fp_step: null input/output");
-    if (act_dtype != FP_F32 && act_dtype != FP_F64 && act_dtype != FP_F32_POLICY) return fail(h, FP_EINVAL, "fp_step: bad action dtype");
+    if (!step_dtype_ok(act_dtype)) return fail(h, FP_EINVAL, "fp_step: bad action dtype");
     EnvParams p; fill_env_params(h, p);
     p.actions = d_actions; p.act_f64 = (act_dtype == FP_F64);
-    if (act_dtype == FP_F32_POLICY) {
-        if (h->variant == FP_VARIANT_THREAD) set_translate(h, p);      // fused into the step kernel
-        else {                                                                     // other variants: elementwise pre-pass
-            const size_t cnt = (size_t)h->n * h->dc.na * 4;
-            if (!h->d_act_xlat) CUDA_TRY(h, cudaMalloc(&h->d_act_xlat, cnt * 4));
-            EnvParams t; set_translate(h, t);
-            CUDA_TRY(h, launch_translate_actions((const float*)d_actions, h->d_act_xlat, (int64_t)cnt, t.act_lo, t.act_hi, t.act_span,
-                                                 (cudaStream_t)stream));
-            h->launches++;
-            p.actions = h->d_act_xlat;
-        }
-    }
     p.reward = d_reward; p.done = d_done; p.info = d_info; p.mask = d_mask;
     p.stats_partial = h->d_stats_partial;
     if (h->fuse_obs) { p.obs_push = 1; p.obs_q = h->ring_q; p.hist = h->keep_hist ? h->d_hist : nullptr; p.obsr = h->d_obsr; p.n_pad = h->n_pad; }
-    CUDA_TRY(h, launch_env_any(h, MODE_STEP, p, (cudaStream_t)stream));
-    h->launches++;
-    return FP_OK;
+    return launch_env_any(h, MODE_STEP, p, act_dtype == FP_F32_POLICY, 1, (cudaStream_t)stream);
 }
 
 // The step's computation for k candidate actions per env, without committing it: one launch of the step kernel's
@@ -418,45 +405,15 @@ int fp_step(FpHandle* h, const void* d_actions, int act_dtype, double* d_reward,
 // caller's buffers, so any number of previews may run between two steps.
 int fp_step_preview(FpHandle* h, int32_t k, const void* d_actions, int act_dtype, double* d_reward, uint8_t* d_done,
                     double* d_info, double* d_voltage, uint64_t* d_vmask, void* stream) {
-    if (!h) return FP_EINVAL;
-    USE_DEVICE(h);
-    if (!h->d_P) return fail(h, FP_ESTATE, "fp_step_preview: call fp_load_profiles first");
+    ENV_ENTRY(h, "fp_step_preview");
     if (!d_actions || !d_reward || !d_done) return fail(h, FP_EINVAL, "fp_step_preview: null input/output");
     if (k < 1) return fail(h, FP_EINVAL, "fp_step_preview: k must be >= 1");
-    if (act_dtype != FP_F32 && act_dtype != FP_F64 && act_dtype != FP_F32_POLICY) return fail(h, FP_EINVAL, "fp_step_preview: bad action dtype");
-    cudaStream_t st = (cudaStream_t)stream;
-    const int64_t n_virt = h->n * k;
+    if (!step_dtype_ok(act_dtype)) return fail(h, FP_EINVAL, "fp_step_preview: bad action dtype");
     EnvParams p; fill_env_params(h, p);
     p.pv_V = d_voltage; p.pv_vmask = d_vmask; p.pv_k = k;            // (replaces the line-flow dump, which a preview never writes)
     p.actions = d_actions; p.act_f64 = (act_dtype == FP_F64);
-    if (act_dtype == FP_F32_POLICY) {
-        if (h->variant == FP_VARIANT_THREAD) set_translate(h, p);      // fused, as in fp_step
-        else {                                                                     // the same elementwise pre-pass as fp_step
-            const int64_t cnt = n_virt * h->dc.na * 4;
-            if (cnt > h->prev_xlat_cap) {
-                cudaFree(h->d_prev_xlat); h->d_prev_xlat = nullptr; h->prev_xlat_cap = 0;
-                CUDA_TRY(h, cudaMalloc(&h->d_prev_xlat, (size_t)cnt * 4));
-                h->prev_xlat_cap = cnt;
-            }
-            EnvParams t; set_translate(h, t);
-            CUDA_TRY(h, launch_translate_actions((const float*)d_actions, h->d_prev_xlat, cnt, t.act_lo, t.act_hi, t.act_span, st));
-            h->launches++;
-            p.actions = h->d_prev_xlat;
-        }
-    }
     p.reward = d_reward; p.done = d_done; p.info = d_info;
-    if (h->variant == FP_VARIANT_THREAD) {                            // the resident grid of the preview kernel, tiles of 32 envs
-        if (!h->cap_preview) h->cap_preview = thread_kernel_max_grid(MODE_PREVIEW, h->tt.n_slots, h->shape);
-        EnvParamsT pt;
-        pt.e = p; pt.t = h->tt;
-        const int64_t tiles = k * ((h->n + 31) / 32);
-        CUDA_TRY(h, launch_env_t(MODE_PREVIEW, h->shape, pt, (int)((tiles < h->cap_preview) ? tiles : h->cap_preview), st));
-    } else {                                                          // one warp per virtual env
-        if (!h->cap_preview) h->cap_preview = max_resident_grid(MODE_PREVIEW);
-        CUDA_TRY(h, launch_env(MODE_PREVIEW, p, grid_for(n_virt, h->cap_preview), st));
-    }
-    h->launches++;
-    return FP_OK;
+    return launch_env_any(h, MODE_PREVIEW, p, act_dtype == FP_F32_POLICY, k, (cudaStream_t)stream);
 }
 
 // Host-buffer step, on one of two routes chosen from the call itself:
@@ -467,11 +424,9 @@ int fp_step_preview(FpHandle* h, int32_t k, const void* d_actions, int act_dtype
 //  * staged, everything else: one copy in, the step on the device staging buffers, the copies out.
 int fp_step_host(FpHandle* h, const void* h_actions, int act_dtype, double* h_reward, uint8_t* h_done,
                  double* h_info, void* stream) {
-    if (!h) return FP_EINVAL;
-    USE_DEVICE(h);
-    if (!h->d_P) return fail(h, FP_ESTATE, "fp_step_host: call fp_load_profiles first");
+    ENV_ENTRY(h, "fp_step_host");
     if (!h_actions || !h_reward || !h_done) return fail(h, FP_EINVAL, "fp_step_host: null buffer");
-    if (act_dtype != FP_F32 && act_dtype != FP_F64 && act_dtype != FP_F32_POLICY) return fail(h, FP_EINVAL, "fp_step_host: bad action dtype");
+    if (!step_dtype_ok(act_dtype)) return fail(h, FP_EINVAL, "fp_step_host: bad action dtype");
     cudaStream_t st = (cudaStream_t)stream;
     auto pinned = [](const void* x) {
         cudaPointerAttributes at;
@@ -527,9 +482,7 @@ int fp_set_obs_history(FpHandle* h, int keep) {
 }
 
 int fp_get_obs(FpHandle* h, void* d_out, int dtype, int push, void* stream) {
-    if (!h) return FP_EINVAL;
-    USE_DEVICE(h);
-    if (!h->d_P) return fail(h, FP_ESTATE, "fp_get_obs: call fp_load_profiles first");
+    ENV_ENTRY(h, "fp_get_obs");
     if (!d_out || (dtype != FP_F32 && dtype != FP_F64)) return fail(h, FP_EINVAL, "fp_get_obs: bad arguments");
     { const int rc = hist_ensure(h, (cudaStream_t)stream); if (rc != FP_OK) return rc; }
     ObsParams p; fill_obs_params(h, p, d_out, push ? 1 : 0);
@@ -567,9 +520,8 @@ static int obs_ring_prepare(FpHandle* h, bool push, cudaStream_t st) {
 }
 
 int fp_get_obs_view(FpHandle* h, int push, float** d_view, int64_t* env_pitch, int64_t* agent_pitch, void* stream) {
-    if (!h || !d_view) return FP_EINVAL;
-    USE_DEVICE(h);
-    if (!h->d_P) return fail(h, FP_ESTATE, "fp_get_obs_view: call fp_load_profiles first");
+    if (!d_view) return FP_EINVAL;
+    ENV_ENTRY(h, "fp_get_obs_view");
     const int H = h->dc.history, na = h->dc.na;
     cudaStream_t st = (cudaStream_t)stream;
     int rc = obs_ring_prepare(h, push != 0, st);
@@ -616,9 +568,8 @@ static int obs_envminor_prepare(FpHandle* h, bool push, cudaStream_t st) {
 }
 
 int fp_obs_ring(FpHandle* h, float** d_ring, int32_t* slot, int64_t* n_pad, void* stream) {
-    if (!h || !d_ring) return FP_EINVAL;
-    USE_DEVICE(h);
-    if (!h->d_P) return fail(h, FP_ESTATE, "fp_obs_ring: call fp_load_profiles first");
+    if (!d_ring) return FP_EINVAL;
+    ENV_ENTRY(h, "fp_obs_ring");
     int rc = obs_envminor_prepare(h, false, (cudaStream_t)stream);
     if (rc != FP_OK) return rc;
     *d_ring = h->d_obsr;
@@ -629,9 +580,8 @@ int fp_obs_ring(FpHandle* h, float** d_ring, int32_t* slot, int64_t* n_pad, void
 
 int fp_step_ring(FpHandle* h, const void* d_actions, int act_dtype, double* d_reward, uint8_t* d_done, double* d_info,
                  const uint8_t* d_mask, float** d_ring, int32_t* slot, int64_t* n_pad, void* stream) {
-    if (!h || !d_ring) return FP_EINVAL;
-    USE_DEVICE(h);
-    if (!h->d_P) return fail(h, FP_ESTATE, "fp_step_ring: call fp_load_profiles first");
+    if (!d_ring) return FP_EINVAL;
+    ENV_ENTRY(h, "fp_step_ring");
     // one launch for the built-in feeder shape; the run-time-table kernels, the warp variant and masked steps push
     // through the generic path (fp64 history ring) and rebuild the ring from it: same contents
     const bool fuse = (h->variant == FP_VARIANT_THREAD) && d_mask == nullptr && h->shape == SHAPE_IEEE33;
@@ -658,9 +608,7 @@ int fp_step_ring(FpHandle* h, const void* d_actions, int act_dtype, double* d_re
 }
 
 int fp_obs_ring_reset_push(FpHandle* h, const uint8_t* d_mask, void* stream) {
-    if (!h) return FP_EINVAL;
-    USE_DEVICE(h);
-    if (!h->d_P) return fail(h, FP_ESTATE, "fp_obs_ring_reset_push: call fp_load_profiles first");
+    ENV_ENTRY(h, "fp_obs_ring_reset_push");
     int rc = obs_envminor_prepare(h, false, (cudaStream_t)stream);
     if (rc != FP_OK) return rc;
     ObsParams p; fill_obs_params(h, p, nullptr, 1);
@@ -671,9 +619,8 @@ int fp_obs_ring_reset_push(FpHandle* h, const uint8_t* d_mask, void* stream) {
 }
 
 int fp_obs_ring_gather(FpHandle* h, float* d_out, void* stream) {
-    if (!h || !d_out) return FP_EINVAL;
-    USE_DEVICE(h);
-    if (!h->d_P) return fail(h, FP_ESTATE, "fp_obs_ring_gather: call fp_load_profiles first");
+    if (!d_out) return FP_EINVAL;
+    ENV_ENTRY(h, "fp_obs_ring_gather");
     int rc = obs_envminor_prepare(h, false, (cudaStream_t)stream);
     if (rc != FP_OK) return rc;
     CUDA_TRY(h, launch_obsr_gather(h->d_obsr, d_out, h->n, h->n_pad, h->dc.na, h->dc.history, h->ring_q, (cudaStream_t)stream));
@@ -700,10 +647,8 @@ int fp_safety_load(FpHandle* h, const double* h_coef, const double* h_intercept,
 
 int fp_safety_project(FpHandle* h, const void* d_actions, int act_dtype, float* d_adjusted, int32_t type_major, double* d_slack,
                       uint8_t* d_intervened, void* stream) {
-    if (!h) return FP_EINVAL;
-    USE_DEVICE(h);
-    if (!h->safety_loaded) return fail(h, FP_ESTATE, "fp_safety_project: call fp_safety_load first");
-    if (!h->d_P) return fail(h, FP_ESTATE, "fp_safety_project: call fp_load_profiles first");
+    if (h && !h->safety_loaded) return fail(h, FP_ESTATE, "fp_safety_project: call fp_safety_load first");
+    ENV_ENTRY(h, "fp_safety_project");
     if (!d_actions || !d_adjusted || (act_dtype != FP_F32 && act_dtype != FP_F64)) return fail(h, FP_EINVAL, "fp_safety_project: bad arguments");
     SafetyParams p;
     std::memset(&p, 0, sizeof(p));
@@ -748,10 +693,8 @@ int fp_safety_load_affine(FpHandle* h, int32_t n_in, int32_t n_out, const double
 
 int fp_safety_project_affine(FpHandle* h, const void* d_actions, int act_dtype, float* d_adjusted, int32_t type_major,
                              double* d_slack, uint8_t* d_intervened, int32_t* d_status, void* stream) {
-    if (!h) return FP_EINVAL;
-    USE_DEVICE(h);
-    if (!h->saff_loaded) return fail(h, FP_ESTATE, "fp_safety_project_affine: call fp_safety_load_affine first");
-    if (!h->d_P) return fail(h, FP_ESTATE, "fp_safety_project_affine: call fp_load_profiles first");
+    if (h && !h->saff_loaded) return fail(h, FP_ESTATE, "fp_safety_project_affine: call fp_safety_load_affine first");
+    ENV_ENTRY(h, "fp_safety_project_affine");
     if (!d_actions || !d_adjusted || (act_dtype != FP_F32 && act_dtype != FP_F64))
         return fail(h, FP_EINVAL, "fp_safety_project_affine: bad arguments");
     SafetyAffineParams p;
@@ -767,9 +710,7 @@ int fp_safety_project_affine(FpHandle* h, const void* d_actions, int act_dtype, 
 }
 
 int fp_get_state(FpHandle* h, void* d_out, int dtype, void* stream) {
-    if (!h) return FP_EINVAL;
-    USE_DEVICE(h);
-    if (!h->d_P) return fail(h, FP_ESTATE, "fp_get_state: call fp_load_profiles first");
+    ENV_ENTRY(h, "fp_get_state");
     if (!d_out || (dtype != FP_F32 && dtype != FP_F64)) return fail(h, FP_EINVAL, "fp_get_state: bad arguments");
     ObsParams p; fill_obs_params(h, p, d_out, 0);
     CUDA_TRY(h, launch_state(p, dtype == FP_F64, h->grid_obs, (cudaStream_t)stream));
@@ -821,13 +762,15 @@ int fp_power_flow(FpHandle* h, int64_t n, const double* d_p, const double* d_q, 
     PfParams p;
     p.topo = h->d_topo; p.n = n; p.nl = h->dc.nl; p.max_iter = h->dc.pf_max_iter; p.tol = h->dc.pf_tol; p.n32 = h->dc.pf_f32; p.pad_ = 0;
     p.p = d_p; p.q = d_q; p.V = d_V; p.Pl = d_Pl; p.Ql = d_Ql; p.Isq = d_Isq; p.iters = d_iters; p.fail = d_fail;
-    if (h->variant == FP_VARIANT_THREAD) {
+    const int cap = h->cap[MODE_PF];
+    if (h->variant == FP_VARIANT_THREAD) {                           // grids as launch_env_any's
         PfParamsT pt;
         pt.p = p; pt.t = h->tt;
         const int64_t tiles = (n + 31) / 32;
-        CUDA_TRY(h, launch_power_flow_t(h->shape, pt, (int)((tiles < h->grid_pf) ? tiles : h->grid_pf), (cudaStream_t)stream));
+        CUDA_TRY(h, launch_power_flow_t(h->shape, pt, (int)((tiles < cap) ? tiles : cap), (cudaStream_t)stream));
     } else {
-        CUDA_TRY(h, launch_power_flow(p, grid_for(n, h->grid_pf), (cudaStream_t)stream));
+        const int64_t ctas = (n + ENVS_PER_CTA - 1) / ENVS_PER_CTA;
+        CUDA_TRY(h, launch_power_flow(p, (int)((ctas < cap) ? ctas : cap), (cudaStream_t)stream));
     }
     h->launches++;
     return FP_OK;

@@ -36,11 +36,11 @@ struct FpHandle {
     const uint8_t* d_inject = nullptr;
     int keep_flows = 0;
     // staging for the host-buffer entry points
-    void* d_act_stage = nullptr; float* d_act_xlat = nullptr; double* d_reward_stage = nullptr; uint8_t* d_done_stage = nullptr;
+    void* d_act_stage = nullptr; double* d_reward_stage = nullptr; uint8_t* d_done_stage = nullptr;
     double* d_info_stage = nullptr;
-    float* d_prev_xlat = nullptr; int64_t prev_xlat_cap = 0;          // fp_step_preview: translated candidates (warp variant)
-    int cap_preview = 0;         // fp_step_preview: resident grid of its kernel (0: not queried yet)
-    int grid_step = 0, grid_reset = 0, grid_pf = 0, grid_obs = 0;
+    float* d_act_xlat = nullptr; int64_t act_xlat_cap = 0;            // FP_F32_POLICY actions translated for the warp kernels
+    int cap[4] = {0, 0, 0, 0};   // grid caps of the env kernels by MODE_*: the resident grid, or FLEXGPU_GRID_STEP's below it
+    int grid_obs = 0;
     int fuse_obs = 0;            // set around the fp_step of fp_step_obs: the step kernel pushes the observation
     int keep_hist = 1;           // fp_set_obs_history: 0 = the fused ring step does not maintain the fp64 history ring
     bool hist_valid = true;      // false after a ring-only step: restored from the env-minor ring on demand (hist_ensure)
