@@ -8,6 +8,7 @@ import pytest
 import torch
 
 import _feeders as F
+from _preview_ref import mirror_copy, mirror_restore
 from oracle import c_mirror, env_ref, ieee33, pf_ref, safety_affine_ref, safety_ref
 
 pytestmark = pytest.mark.gpu
@@ -239,15 +240,6 @@ def test_episode_bit_exact_vs_mirror(cuda, monkeypatch, case, kind):
     env.close()
 
 
-def _mirror_copy(mb):
-    return {k: v.copy() for k, v in vars(mb).items() if isinstance(v, np.ndarray)}
-
-
-def _mirror_restore(mb, saved):
-    for k, v in saved.items():
-        getattr(mb, k)[...] = v
-
-
 @pytest.mark.parametrize("case", CASES, ids=IDS)
 def test_preview_equals_step_and_mirror(cuda, case):
     """preview_step with K = 1 and K = 3 (fp32, fp64 and translated candidates) returns the following step's reward,
@@ -274,13 +266,13 @@ def test_preview_equals_step_and_mirror(cuda, case):
         F.assert_same_bytes(before, F.snapshot(env))
         r, d, V, vm = (x.reshape(k, n, *x.shape[(2 if k > 1 else 1):]) for x in (r, d, V, vm))
         info = {key: v.reshape(k, n) for key, v in info.items()}
-        saved = _mirror_copy(mb)
+        saved = mirror_copy(mb)
         for j in range(k):                                          # the mirror's step for each candidate, then undone
             rr, dd, ii = mb.step(_mirror_actions(kind, cand[j]))
             assert np.array_equal(r[j].cpu().numpy(), rr) and np.array_equal(d[j].cpu().numpy(), dd), (t, j)
             assert np.array_equal(np.stack([info[key][j].cpu().numpy() for key in INFO7 + ("solver_failed",)], 1), ii)
             assert np.array_equal(V[j].cpu().numpy(), mb.V) and np.array_equal(vm[j].cpu().numpy().view(np.uint64), mb.vmask)
-            _mirror_restore(mb, saved)
+            mirror_restore(mb, saved)
         j = k - 1                                                   # commit the last candidate
         rs, ds, infos = env.step(torch.from_numpy(cand[j]), translate=kind == "policy")
         mb.step(_mirror_actions(kind, cand[j]))
