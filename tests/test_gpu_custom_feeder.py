@@ -8,67 +8,26 @@ import pytest
 import torch
 
 import _feeders as F
+from _env_check import (actions, bits, check_state, draws, feeder_profiles, make_env, mirror_actions, reset_both,
+                        scaled_profiles)
 from _preview_ref import mirror_copy, mirror_restore
+from flexgpu._lib import INFO_KEYS
 from oracle import c_mirror, env_ref, ieee33, pf_ref, safety_affine_ref, safety_ref
 
 pytestmark = pytest.mark.gpu
 
 CASES = F.cases()
 IDS = [f"{f}-{v}" for f, v in CASES]
-INFO7 = ("reward", "revenue", "der_cost", "ess_cost", "discomfort_penalty", "voltage_penalty", "cumulative_reward")
 
 
 def _variant(v):
     return c_mirror.VARIANT_WARP if v == "warp" else c_mirror.VARIANT_THREAD
 
 
-def _profiles(net, heavy=False, T=1500, seed=3):
-    """Synthetic profiles of the feeder; heavy: every other day's demand scaled by 2.4, so that an episode (121 rows)
-    runs through both a normal and a heavily loaded day, with voltage violations on the latter."""
-    from flexgpu.network import Network
-    from flexgpu.profiles import Profiles, synthetic_profiles
-    p = synthetic_profiles(Network(net), len(net['buildings']), T=T, seed=seed)
-    if not heavy:
-        return p
-    f = np.where((np.arange(T) // 96) % 2 == 1, 2.4, 1.0)[:, None]
-    return Profiles(p.P * f, p.Q * f, p.PV, p.price)
-
-
-def _make(cuda, net, variant, n, profiles, **extra):
-    from flexgpu import BatchedFlexProvisionEnv
-    return BatchedFlexProvisionEnv(F.env_args(net, variant, **extra), n_envs=n, device=cuda, network=net, profiles=profiles)
-
-
-def _draws(env, n, na, seed):
-    rng = np.random.default_rng(seed)
-    start = rng.integers(0, env.max_start(), n).astype(np.int32)
-    e0 = rng.uniform(0.9 * 0.0125, 1.1 * 0.0125, (n, na)); a0 = rng.uniform(0, 1, (n, 4 * na))
-    return start, e0, a0
-
-
-def _actions(kind, rng, shape):
-    """Actions of one kind: fp32 / fp64 policy outputs, raw fp32 outputs to translate ("policy"), setpoints ("raw")."""
-    if kind == "raw":
-        return rng.uniform(0, 1, shape) * np.array([0.5, 0.01, 0.01, 0.02])
-    a = rng.normal(0.4, 0.6, shape)
-    return a.astype(np.float64 if kind == "f64" else np.float32)
-
-
-def _mirror_actions(kind, a):
-    return c_mirror.translate_action_f32(a) if kind == "policy" else a
-
-
-def _bits(t):
-    return t.view(torch.int64) if t.dtype == torch.float64 else t
-
-
-def _assert_state(env, mb, sel=slice(None)):
-    assert np.array_equal(env.voltages.cpu().numpy()[sel], mb.V[sel])
-    assert np.array_equal(env.ess_energy.cpu().numpy()[sel], mb.E_cur[sel])
-    assert np.array_equal(env.setpoints.cpu().numpy()[sel], mb.setp[sel])
-    assert np.array_equal(env.violation_mask.cpu().numpy().view(np.uint64)[sel], mb.vmask[sel])
-    assert np.array_equal(env.violation_count.cpu().numpy()[sel], mb.vcount[sel])
-    assert np.array_equal(env.pf_iterations.cpu().numpy()[sel], mb.iters[sel])
+def _heavy(net):
+    """Every other day's demand x 2.4: an episode (121 rows) runs through both a normal and a heavily loaded day, with
+    voltage violations on the latter."""
+    return scaled_profiles(feeder_profiles(net), every_other_day=True)
 
 
 @pytest.fixture(scope="module", params=CASES, ids=IDS)
@@ -76,11 +35,11 @@ def setup(request, cuda):
     from flexgpu.network import Network
     name, variant = request.param
     net = F.feeder(name)
-    prof = _profiles(net)
+    prof = feeder_profiles(net)
     tree = ieee33.tree_arrays(net)
     fonet = c_mirror.make_net(tree, F.env_args(net, variant), net['buildings'], variant=_variant(variant))
     n = 200
-    env = _make(cuda, net, variant, n, prof)
+    env = make_env(cuda, prof, n, variant, net=net)
     yield env, fonet, prof, tree, Network(net), n
     env.close()
 
@@ -105,16 +64,15 @@ def test_env_steps_bit_exact_vs_mirror(setup):
     env, fonet, prof, tree, network, n = setup
     mb = c_mirror.MirrorBatch(fonet, prof.as_dict(), n)
     na, nb = env.n_agents, env.n_bus
-    start, e0, a0 = _draws(env, n, na, 2)
+    reset_both(env, mb, np.random.default_rng(2))
     rng = np.random.default_rng(2)
-    env.reset(start, e0, a0, return_obs=False); mb.reset(start, e0, a0)
     for t in range(6):
         a = rng.normal(0.4, 0.5, (n, 4 * na))
         r, d, info = env.step(torch.from_numpy(a), want_info=True)
         rr, dd, ii = mb.step(a)
         assert np.array_equal(r.cpu().numpy(), rr) and np.array_equal(d.cpu().numpy(), dd)
         assert np.array_equal(info["voltage_penalty"].cpu().numpy(), ii[:, 5])
-    _assert_state(env, mb)
+    check_state(env, mb, "6 steps")
     obs = env.get_obs(); state = env.get_state()
     assert obs.shape == (n, na, 6 * env.history) and state.shape == (n, 3 * nb + 2 * na + 1)
     # step(return_obs=True) on a run-time-table feeder (fewer agents: packed observation row, two-launch
@@ -139,7 +97,7 @@ def test_power_flow_across_loading_to_collapse(cuda, case):
     net = F.feeder(name)
     tree = ieee33.tree_arrays(net)
     network = Network(net)
-    env = _make(cuda, net, variant, 64, _profiles(net))
+    env = make_env(cuda, feeder_profiles(net), 64, variant, net=net)
     fonet = c_mirror.make_net(tree, F.env_args(net, variant), net['buildings'], variant=_variant(variant))
     rng = np.random.default_rng(21)
     m = 2000
@@ -187,16 +145,15 @@ def test_episode_bit_exact_vs_mirror(cuda, monkeypatch, case, kind):
     monkeypatch.setenv("FLEXGPU_GRID_STEP", "2")                    # 2 persistent CTAs: 4 trips over 8 tiles
     net = F.feeder(name)
     raw = kind == "raw"
-    prof = _profiles(net, heavy=True)
+    prof = _heavy(net)
     n = 32 * 7 + 7
-    env = _make(cuda, net, variant, n, prof, **({"alg": "safemaddpg"} if raw else {}))
+    env = make_env(cuda, prof, n, variant, net=net, **({"alg": "safemaddpg"} if raw else {}))
     na = env.n_agents
     fonet = c_mirror.make_net(ieee33.tree_arrays(net), F.env_args(net, variant), net['buildings'], raw_actions=raw,
                               variant=_variant(variant))
     mb = c_mirror.MirrorBatch(fonet, prof.as_dict(), n)
-    start, e0, a0 = _draws(env, n, na, 11)
-    env.reset(start, e0, a0, return_obs=False); mb.reset(start, e0, a0)
-    _assert_state(env, mb)
+    start, e0, a0 = reset_both(env, mb, np.random.default_rng(11))
+    check_state(env, mb, "reset")
     idx = [0, 3, n // 2, n - 1]                                     # NaN actions, injected failure, plain, masked out
     injected = [None]
     refs = _ref_envs(net, prof, idx, start, e0, a0, raw, injected) if kind == "f64" else []
@@ -205,7 +162,7 @@ def test_episode_bit_exact_vs_mirror(cuda, monkeypatch, case, kind):
     rng = np.random.default_rng(12)
     violations = failures = 0
     for t in range(env.episode_limit - 1):
-        a = _actions(kind, rng, (n, na, 4))
+        a = actions(kind, rng, (n, na, 4), 0.4)
         inj = mask = None
         if t == 30:
             a[::13, 0, 1] = np.nan
@@ -215,18 +172,18 @@ def test_episode_bit_exact_vs_mirror(cuda, monkeypatch, case, kind):
         if t == 70:
             mask = (rng.uniform(size=n) < 0.6).astype(np.uint8); mask[0] = 1; mask[n - 1] = 0
         r, d, info = env.step(torch.from_numpy(a), mask=mask, translate=kind == "policy")
-        rr, dd, ii = mb.step(_mirror_actions(kind, a), inject=inj, mask=mask)
+        rr, dd, ii = mb.step(mirror_actions(kind, a), inject=inj, mask=mask)
         sel = slice(None) if mask is None else mask.astype(bool)
         assert np.array_equal(r.cpu().numpy()[sel], rr[sel]), t
         assert np.array_equal(d.cpu().numpy()[sel], dd[sel]), t
-        got = np.stack([info[k].cpu().numpy() for k in INFO7 + ("solver_failed",)], 1)
+        got = np.stack([info[k].cpu().numpy() for k in INFO_KEYS], 1)
         assert np.array_equal(got[sel], ii[sel]), t
-        _assert_state(env, mb)
+        check_state(env, mb, f"step {t}")
         violations += int(mb.vcount.sum()); failures += int(ii[:, 7].sum())
         for e, ref in zip(idx, refs):
             if mask is not None and not mask[e]:
                 continue
-            rw, dn, inf = ref.step(_mirror_actions(kind, a[e]).reshape(-1))
+            rw, dn, inf = ref.step(mirror_actions(kind, a[e]).reshape(-1))
             assert abs(rr[e] - rw) <= 1e-6 * abs(rw) + 1e-12, (t, e, rr[e], rw)
             assert bool(dd[e]) == dn, (t, e)
             assert (ii[e, 7] == 1.0) == bool(inf.get("solver_failed", False)), (t, e)
@@ -246,19 +203,18 @@ def test_preview_equals_step_and_mirror(cuda, case):
     done, info, voltages and mask, and the mirror's; the handle's bytes are unchanged by the previews."""
     name, variant = case
     net = F.feeder(name)
-    prof = _profiles(net, heavy=True)
+    prof = _heavy(net)
     n = 32 * 3 + 5
-    env = _make(cuda, net, variant, n, prof)
+    env = make_env(cuda, prof, n, variant, net=net)
     na = env.n_agents
     fonet = c_mirror.make_net(ieee33.tree_arrays(net), F.env_args(net, variant), net['buildings'], variant=_variant(variant))
     mb = c_mirror.MirrorBatch(fonet, prof.as_dict(), n)
-    start, e0, a0 = _draws(env, n, na, 31)
-    env.reset(start, e0, a0, return_obs=False); mb.reset(start, e0, a0)
+    reset_both(env, mb, np.random.default_rng(31))
     env.keep_line_flows(True)
     rng = np.random.default_rng(32)
     for t, kind in enumerate(["f32", "f64", "policy", "f32", "f64"]):
         k = 1 if t % 2 == 0 else 3
-        cand = _actions(kind, rng, (k, n, na, 4))
+        cand = actions(kind, rng, (k, n, na, 4), 0.4)
         cand[k - 1, ::11, 0, 2] = np.nan
         before = F.snapshot(env)
         c = torch.from_numpy(cand if k > 1 else cand[0])
@@ -268,19 +224,19 @@ def test_preview_equals_step_and_mirror(cuda, case):
         info = {key: v.reshape(k, n) for key, v in info.items()}
         saved = mirror_copy(mb)
         for j in range(k):                                          # the mirror's step for each candidate, then undone
-            rr, dd, ii = mb.step(_mirror_actions(kind, cand[j]))
+            rr, dd, ii = mb.step(mirror_actions(kind, cand[j]))
             assert np.array_equal(r[j].cpu().numpy(), rr) and np.array_equal(d[j].cpu().numpy(), dd), (t, j)
-            assert np.array_equal(np.stack([info[key][j].cpu().numpy() for key in INFO7 + ("solver_failed",)], 1), ii)
+            assert np.array_equal(np.stack([info[key][j].cpu().numpy() for key in INFO_KEYS], 1), ii)
             assert np.array_equal(V[j].cpu().numpy(), mb.V) and np.array_equal(vm[j].cpu().numpy().view(np.uint64), mb.vmask)
             mirror_restore(mb, saved)
         j = k - 1                                                   # commit the last candidate
         rs, ds, infos = env.step(torch.from_numpy(cand[j]), translate=kind == "policy")
-        mb.step(_mirror_actions(kind, cand[j]))
-        assert torch.equal(_bits(r[j]), _bits(rs)) and torch.equal(d[j], ds), t
+        mb.step(mirror_actions(kind, cand[j]))
+        assert torch.equal(bits(r[j]), bits(rs)) and torch.equal(d[j], ds), t
         for key in infos:
-            assert torch.equal(_bits(info[key][j]), _bits(infos[key])), (t, key)
-        assert torch.equal(_bits(V[j]), _bits(env.voltages)) and torch.equal(vm[j], env.violation_mask), t
-        _assert_state(env, mb)
+            assert torch.equal(bits(info[key][j]), bits(infos[key])), (t, key)
+        assert torch.equal(bits(V[j]), bits(env.voltages)) and torch.equal(vm[j], env.violation_mask), t
+        check_state(env, mb, f"step {t}")
     env.close()
 
 
@@ -290,16 +246,16 @@ def test_observations_and_host_step(cuda, name, variant):
     """step(return_obs=True) and step(return_obs="ring") equal step + get_obs / obs_ring().dense(); step_host through
     the zero-copy route (pinned fp32) and the staged route (pageable, fp64) equals step bit for bit."""
     net = F.feeder(name)
-    prof = _profiles(net, heavy=True)
+    prof = _heavy(net)
     n = 32 * 4 + 9
-    envs = [_make(cuda, net, variant, n, prof) for _ in range(3)]
+    envs = [make_env(cuda, prof, n, variant, net=net) for _ in range(3)]
     na = envs[0].n_agents
-    start, e0, a0 = _draws(envs[0], n, na, 41)
+    start, e0, a0 = draws(41, envs[0])
     for env in envs:
         env.reset(start, e0, a0, return_obs=False)
     rng = np.random.default_rng(42)
     for t in range(30):
-        a = _actions("f32" if t % 3 else "f64", rng, (n, na, 4))
+        a = actions("f32" if t % 3 else "f64", rng, (n, na, 4), 0.4)
         if t == 10:
             a[::7, na - 1, 0] = np.nan
         r0, d0, i0 = envs[0].step(torch.from_numpy(a))
@@ -309,9 +265,9 @@ def test_observations_and_host_step(cuda, name, variant):
         else:
             r1, d1, i1, ring = envs[1].step(torch.from_numpy(a), return_obs="ring")
             o1 = ring.dense()
-        assert torch.equal(_bits(r0), _bits(r1)) and torch.equal(d0, d1), t
+        assert torch.equal(bits(r0), bits(r1)) and torch.equal(d0, d1), t
         assert torch.equal(o0, o1), t
-        assert torch.equal(envs[0].rec, envs[1].rec) and torch.equal(_bits(envs[0].voltages), _bits(envs[1].voltages)), t
+        assert torch.equal(envs[0].rec, envs[1].rec) and torch.equal(bits(envs[0].voltages), bits(envs[1].voltages)), t
         if a.dtype == np.float32:
             h = torch.from_numpy(a.reshape(n, -1)).pin_memory().numpy()    # zero-copy
         else:
@@ -321,16 +277,15 @@ def test_observations_and_host_step(cuda, name, variant):
         assert np.array_equal(r2, r0.cpu().numpy()) and np.array_equal(d2, d0.cpu().numpy()), t
         for k in i0:
             assert np.array_equal(i2[k], i0[k].cpu().numpy()), (t, k)
-        assert torch.equal(envs[0].rec, envs[2].rec) and torch.equal(_bits(envs[0].voltages), _bits(envs[2].voltages)), t
+        assert torch.equal(envs[0].rec, envs[2].rec) and torch.equal(bits(envs[0].voltages), bits(envs[2].voltages)), t
     for env in envs:
         env.close()
 
 
 def _safety_env(cuda, net, n, seed):
-    env = _make(cuda, net, "thread", n, _profiles(net))
+    env = make_env(cuda, feeder_profiles(net), n, "thread", net=net)
     na = env.n_agents
-    start, e0, a0 = _draws(env, n, na, seed)
-    env.reset(start, e0, a0, return_obs=False)
+    env.reset(*draws(seed, env), return_obs=False)
     g = torch.Generator(device=cuda).manual_seed(seed)
     for _ in range(3):
         env.step(torch.rand(n, na, 4, device=cuda, generator=g), want_info=False)
@@ -432,8 +387,8 @@ def test_thread_variant_rejects_feeders_beyond_its_limits(cuda, name):
     from flexgpu import FlexGpuError
     net = F.feeder(name)
     with pytest.raises(FlexGpuError, match="use FP_VARIANT_WARP"):
-        _make(cuda, net, "thread", 64, _profiles(net))
-    env = _make(cuda, net, "warp", 64, _profiles(net))               # the warp variant runs it (tests above: parity)
+        make_env(cuda, feeder_profiles(net), 64, "thread", net=net)
+    env = make_env(cuda, feeder_profiles(net), 64, "warp", net=net)    # the warp variant runs it (tests above: parity)
     env.close()
 
 
@@ -457,7 +412,7 @@ def test_create_rejects_invalid_feeders(cuda, variant):
     from flexgpu.network import Network
     for key, net in _bad_feeders().items():
         with pytest.raises((FlexGpuError, ValueError)):
-            _make(cuda, net, variant, 8, None if key == "34_buses" else _profiles(net))
+            make_env(cuda, None if key == "34_buses" else feeder_profiles(net), 8, variant, net=net)
     net = F.custom14()
     network = Network(net)
     lib = _lib.lib()

@@ -10,6 +10,8 @@ import numpy as np
 import pytest
 import torch
 
+from _env_check import make_env, reset_draws
+
 N = 300                  # not a multiple of the 32-env tile
 
 # (verb, launches on the thread variant, launches on the warp variant), in the order they run
@@ -51,13 +53,10 @@ EXPECTED = [
 
 @pytest.mark.gpu
 def test_launches_per_verb(cuda, profiles, variant):
-    from flexgpu import BatchedFlexProvisionEnv
-    env = BatchedFlexProvisionEnv({"kernel_variant": variant}, n_envs=N, device=cuda, profiles=profiles, seed=3)
+    env = make_env(cuda, profiles, N, variant, seed=3)
     na, nl, nb = env.n_agents, env.n_lines, env.n_bus
     rng = np.random.default_rng(0)
-    start = rng.integers(0, env.max_start(), N).astype(np.int32)
-    e0 = rng.uniform(0.9 * 0.0125, 1.1 * 0.0125, (N, na))
-    a0 = rng.uniform(0, 1, (N, na * 4))
+    start, e0, a0 = reset_draws(rng, N, na, env.max_start())
     mask = torch.from_numpy((np.arange(N) % 3 == 0).astype(np.uint8))
 
     def acts(*lead, dtype=torch.float32):

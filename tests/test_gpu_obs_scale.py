@@ -22,6 +22,8 @@ import numpy as np
 import pytest
 import torch
 
+from _env_check import actions, check_state, make_env, mirror_actions, reset_draws, same
+from _env_check import all_cores  # noqa: F401  (autouse fixture)
 from _obs_ref import ObsRef, clamp_tables
 from oracle import c_mirror
 
@@ -29,50 +31,6 @@ pytestmark = pytest.mark.gpu
 N = 131072 + 19
 H, NA = 24, 5
 SENT = -7.25e6
-
-
-@pytest.fixture(scope="module", autouse=True)
-def all_cores():
-    c_mirror.use_all_cores()
-
-
-def make(cuda, profiles, n, variant="thread", seed=1):
-    from flexgpu import BatchedFlexProvisionEnv
-    return BatchedFlexProvisionEnv({"kernel_variant": variant}, n_envs=n, device=cuda, profiles=profiles, seed=seed)
-
-
-def bits(t):
-    t = t.contiguous()
-    if t.dtype == torch.float64:
-        return t.view(torch.int64)
-    if t.dtype == torch.float32:
-        return t.view(torch.int32)
-    return t
-
-
-def same(got, want, what, where):
-    """got == want bit for bit (NaN and -0.0 included), or an error that names the first differing element."""
-    want = torch.as_tensor(want).to(got.device)
-    assert got.shape == want.shape and got.dtype == want.dtype, f"{where}: {what}: {got.shape} {got.dtype} vs {want.shape} {want.dtype}"
-    d = bits(got) != bits(want)
-    if bool(d.any()):
-        i = tuple(int(x) for x in torch.nonzero(d)[0])
-        raise AssertionError(f"{where}: {what} differs at {i} ({int(d.sum())} elements): {got[i].item()!r} vs {want[i].item()!r}")
-
-
-def u64(lo, hi):
-    return (np.asarray(lo).astype(np.uint32).astype(np.uint64) | (np.asarray(hi).astype(np.uint32).astype(np.uint64) << np.uint64(32))).view(np.int64)
-
-
-def check_state(env, mb, ref, where):
-    """Records (push count from the reference), voltages and setpoints of every env."""
-    rec = np.empty((mb.n, 16), dtype=np.int64)
-    rec[:, 0:5] = mb.E_init.view(np.int64); rec[:, 5:10] = mb.E_cur.view(np.int64); rec[:, 10] = mb.cum.view(np.int64)
-    rec[:, 11] = u64(mb.start, mb.steps); rec[:, 12] = u64(ref.cnt.cpu().numpy(), mb.episode)
-    rec[:, 13] = mb.vmask.view(np.int64); rec[:, 14] = u64(mb.vcount, mb.flags); rec[:, 15] = u64(mb.lmask, mb.iters)
-    same(env.rec, torch.from_numpy(rec), "record", where)
-    same(env.voltages, torch.from_numpy(mb.V), "voltages", where)
-    same(env.setpoints, torch.from_numpy(mb.setp), "setpoints", where)
 
 
 def check_outputs(env, r, d, rr, dd, ii, where, info=True, mask=None):
@@ -141,15 +99,13 @@ class Slot:
         return self.q
 
 
-def act_for(t, g, n, cuda):
-    """Actions cycling through fp32, fp64 and raw fp32 policy outputs (translate=True); what the mirror steps with."""
-    raw = torch.randn(n, NA, 4, device=cuda, generator=g) * 0.6 + 0.3
-    if t % 3 == 0:
-        return raw, {}, raw.cpu().numpy()
-    if t % 3 == 1:
-        a = raw.double()
-        return a, {}, a.cpu().numpy()
-    return raw, {"translate": True}, c_mirror.translate_action_f32(raw.cpu().numpy())
+def act_for(t, g, n):
+    """Actions cycling through fp32, fp64 (the fp32 draw widened) and raw fp32 policy outputs (translate=True); what the
+    mirror steps with."""
+    raw = actions("f32", g, (n, NA, 4), 0.3)
+    kind = ("f32", "f64", "policy")[t % 3]
+    a = raw.double() if kind == "f64" else raw
+    return a, {"translate": kind == "policy"}, mirror_actions(kind, a)
 
 
 def test_a_fused_ring_step_default_mode(cuda, profiles, fonets):
@@ -157,7 +113,7 @@ def test_a_fused_ring_step_default_mode(cuda, profiles, fonets):
     failures, one masked (unfused) step, one generic fp64 push; records, rewards, info, V, setpoints, the whole ring and
     the fp64 history every step, the dense gather, get_obs and get_state every few steps."""
     t0 = time.time()
-    env = make(cuda, profiles, N, seed=21)
+    env = make_env(cuda, profiles, N, seed=21)
     mb = c_mirror.MirrorBatch(fonets["thread"], profiles.as_dict(), N)
     ref = ObsRef(N, NA, H, cuda)
     slot = Slot()
@@ -167,7 +123,7 @@ def test_a_fused_ring_step_default_mode(cuda, profiles, fonets):
     rng = np.random.default_rng(6)
     for t in range(100):
         where = f"A step {t}"
-        a, kw, am = act_for(t, g, N, cuda)
+        a, kw, am = act_for(t, g, N)
         want_info = t % 4 != 1
         inj = mask = None
         if t == 37:
@@ -183,7 +139,7 @@ def test_a_fused_ring_step_default_mode(cuda, profiles, fonets):
             slot.generic_push()
         ref.push(mb.current_obs())
         check_outputs(env, r, d, rr, dd, ii, where, info=want_info, mask=mask)
-        check_state(env, mb, ref, where)
+        check_state(env, mb, where, pushes=ref.cnt)
         check_ring(ring, ref, slot.ring_op(True) if mask is None else slot.ring_op(False), where)
         check_history(env, ref, where)
         if t == 37:
@@ -199,7 +155,7 @@ def test_a_fused_ring_step_default_mode(cuda, profiles, fonets):
             ring = env.reset(mask=done, return_obs="ring", retries=0); mb.reset_random(21, mask=done)
             ref.reset(done); ref.push(mb.current_obs(), done)
             check_ring(ring, ref, slot.ring_op(False), where + " reset")
-    check_state(env, mb, ref, "A end")
+    check_state(env, mb, "A end", pushes=ref.cnt)
     check_reads(env, mb, ref, "A end", env.obs_ring())
     env.close()
     print(f"leg A: {time.time() - t0:.1f} s")
@@ -210,7 +166,7 @@ def test_b_ring_only_stepping(cuda, profiles, fonets):
     fp64 reads restore the history from the ring (k_hist_from_ring): history entries are the mirror values rounded to
     fp32 and widened, the newest entry exact fp64; then back to the default mode with a generic push."""
     t0 = time.time()
-    env = make(cuda, profiles, N, seed=31)
+    env = make_env(cuda, profiles, N, seed=31)
     mb = c_mirror.MirrorBatch(fonets["thread"], profiles.as_dict(), N)
     ref = ObsRef(N, NA, H, cuda)
     slot = Slot()
@@ -220,9 +176,9 @@ def test_b_ring_only_stepping(cuda, profiles, fonets):
     g = torch.Generator(device=cuda).manual_seed(7)
     for t in range(60):
         where = f"B step {t}"
-        raw = torch.randn(N, NA, 4, device=cuda, generator=g) * 0.6 + 0.3
+        raw = actions("f32", g, (N, NA, 4), 0.3)
         r, d, _, ring = env.step(raw, translate=True, return_obs="ring")
-        rr, dd, ii = mb.step(c_mirror.translate_action_f32(raw.cpu().numpy()))
+        rr, dd, ii = mb.step(mirror_actions("policy", raw))
         ref.push(mb.current_obs())
         check_outputs(env, r, d, rr, dd, ii, where)
         check_ring(ring, ref, slot.ring_op(True), where)
@@ -232,7 +188,7 @@ def test_b_ring_only_stepping(cuda, profiles, fonets):
             ref.round_f32()
             check_windows(lambda lo, hi: o[lo:hi], ref, f"{where} restored get_obs(push=False, float64)", cur, torch.float64)
             check_history(env, ref, where + " restored")
-            check_state(env, mb, ref, where)
+            check_state(env, mb, where, pushes=ref.cnt)
         done = (mb.flags & 1).astype(np.uint8)
         if done.any():
             ring = env.reset(mask=done, return_obs="ring", retries=0); mb.reset_random(31, mask=done)
@@ -242,7 +198,7 @@ def test_b_ring_only_stepping(cuda, profiles, fonets):
     o = env.get_obs(dtype=torch.float64)           # restore, then a generic push in fp64
     ref.round_f32(); ref.push(mb.current_obs())
     check_windows(lambda lo, hi: o[lo:hi], ref, "B generic push", dtype=torch.float64)
-    check_history(env, ref, "B end"); check_state(env, mb, ref, "B end")
+    check_history(env, ref, "B end"); check_state(env, mb, "B end", pushes=ref.cnt)
     env.close()
     print(f"leg B: {time.time() - t0:.1f} s")
 
@@ -254,7 +210,7 @@ def test_c_window_ring(cuda, profiles, fonets, variant):
     returned strided view and its strides against the reference every step.  The warp variant alternates with
     return_obs="ring" (step, window-ring push, env-minor ring rebuild), which pushes the window ring as well."""
     t0 = time.time()
-    env = make(cuda, profiles, N, variant, seed=41)
+    env = make_env(cuda, profiles, N, variant, seed=41)
     mb = c_mirror.MirrorBatch(fonets[variant], profiles.as_dict(), N)
     ref = ObsRef(N, NA, H, cuda)
     env.reset(return_obs=False, retries=0); mb.reset_random(41)
@@ -262,7 +218,7 @@ def test_c_window_ring(cuda, profiles, fonets, variant):
     rng = np.random.default_rng(9)
     for t in range(104):
         where = f"C[{variant}] step {t}"
-        a, kw, am = act_for(t, g, N, cuda)
+        a, kw, am = act_for(t, g, N)
         as_ring = variant == "warp" and t % 2 == 1
         r, d, _, o = env.step(a, return_obs="ring" if as_ring else True, **kw)
         rr, dd, ii = mb.step(am)
@@ -274,13 +230,13 @@ def test_c_window_ring(cuda, profiles, fonets, variant):
             assert o.stride() == (NA * 3 * H * 6, 3 * H * 6, 1) and o.shape == (N, NA, 6 * H), where
             check_windows(lambda lo, hi: o[lo:hi], ref, where)
         if t % 10 == 3:
-            check_state(env, mb, ref, where)
+            check_state(env, mb, where, pushes=ref.cnt)
         if t == 100:                               # generic push (after the second compaction): rebuilt at the next step
             env.get_obs(dtype=torch.float64); ref.push(mb.current_obs())
         if t % 4 == 2:
             m = ((mb.flags & 1) | (rng.uniform(size=N) < 0.1)).astype(np.uint8)
             env.reset(mask=m, return_obs=False, retries=0); mb.reset_random(41, mask=m); ref.reset(m)
-    check_state(env, mb, ref, f"C[{variant}] end"); check_history(env, ref, f"C[{variant}] end")
+    check_state(env, mb, f"C[{variant}] end", pushes=ref.cnt); check_history(env, ref, f"C[{variant}] end")
     env.close()
     print(f"leg C[{variant}]: {time.time() - t0:.1f} s")
 
@@ -292,7 +248,7 @@ def test_d_two_pow_20_envs(cuda, profiles, fonets):
     window ring, whose element offsets pass 2^31."""
     t0 = time.time()
     n = 2 ** 20 + 77
-    env = make(cuda, profiles, n, seed=51)
+    env = make_env(cuda, profiles, n, seed=51)
     mb = c_mirror.MirrorBatch(fonets["thread"], profiles.as_dict(), n)
     ref = ObsRef(n, NA, H, cuda)
     slot = Slot()
@@ -302,7 +258,7 @@ def test_d_two_pow_20_envs(cuda, profiles, fonets):
     rng = np.random.default_rng(11)
     for t in range(30):
         where = f"D step {t}"
-        a, kw, am = act_for(t, g, n, cuda)
+        a, kw, am = act_for(t, g, n)
         if t == 12:
             env.set_obs_history(False)
         if t < 24:
@@ -324,7 +280,7 @@ def test_d_two_pow_20_envs(cuda, profiles, fonets):
             check_windows(lambda lo, hi: o64[lo:hi], ref, f"{where} restored", cur, torch.float64)
             env.set_obs_history(True)
         if t in (5, 23):
-            check_state(env, mb, ref, where)
+            check_state(env, mb, where, pushes=ref.cnt)
             check_reads(env, mb, ref, where, ring)
         m = (mb.flags & 1).astype(np.uint8)
         if t == 8:
@@ -336,7 +292,7 @@ def test_d_two_pow_20_envs(cuda, profiles, fonets):
                 check_ring(ring, ref, slot.ring_op(False), where + " half reset")
             else:
                 slot.ring_op(False)
-    check_state(env, mb, ref, "D end"); check_history(env, ref, "D end")
+    check_state(env, mb, "D end", pushes=ref.cnt); check_history(env, ref, "D end")
     env.close()
     print(f"leg D: {time.time() - t0:.1f} s")
 
@@ -350,16 +306,17 @@ def test_f_row_clamp_past_the_episode_slice(cuda, profiles, fonets, variant):
     t0 = time.time()
     s0, n = 2000, 40000 + 7
     _, prof = clamp_tables(profiles, s0)
-    env = make(cuda, prof, n, variant)
+    env = make_env(cuda, prof, n, variant, seed=1)
     mb = c_mirror.MirrorBatch(fonets[variant], prof.as_dict(), n)
     ref = ObsRef(n, NA, H, cuda)
     slot = Slot()
     rng = np.random.default_rng(12)
 
     def draw():
-        st = (s0 - rng.integers(0, 41, n)).astype(np.int32)
+        back, e0, a0 = reset_draws(rng, n, NA, 41)
+        st = (s0 - back).astype(np.int32)
         st[::3] = s0                               # the never-reset subset starts on the last start
-        return st, rng.uniform(0.9 * 0.0125, 1.1 * 0.0125, (n, NA)), rng.uniform(0, 1, (n, NA * 4))
+        return st, e0, a0
 
     st, e0, a0 = draw()
     ring = env.reset(st, e0, a0, return_obs="ring"); mb.reset(st, e0, a0)
@@ -368,14 +325,14 @@ def test_f_row_clamp_past_the_episode_slice(cuda, profiles, fonets, variant):
     g = torch.Generator(device=cuda).manual_seed(13)
     for t in range(130):
         where = f"F[{variant}] step {t}"
-        a, kw, am = act_for(t, g, n, cuda)
+        a, kw, am = act_for(t, g, n)
         as_window = t % 5 == 4
         r, d, info, o = env.step(a, return_obs=True if as_window else "ring", **kw)
         rr, dd, ii = mb.step(am)
         ref.push(mb.current_obs())
         assert bool(torch.isfinite(r).all()) and bool(torch.isfinite(env._info).all()), where
         check_outputs(env, r, d, rr, dd, ii, where)
-        check_state(env, mb, ref, where)
+        check_state(env, mb, where, pushes=ref.cnt)
         if as_window:
             slot.generic_push()
             check_windows(lambda lo, hi: o[lo:hi], ref, where)

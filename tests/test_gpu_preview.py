@@ -13,37 +13,13 @@ import numpy as np
 import pytest
 import torch
 
+from _env_check import actions, bits, draws, make_env, ptr, scaled_profiles
 from _feeders import assert_same_bytes, snapshot
 from flexgpu import _lib
 
 
-def make(cuda, profiles, n, variant, **args):
-    from flexgpu import BatchedFlexProvisionEnv
-    a = dict(args)
-    a["kernel_variant"] = variant
-    return BatchedFlexProvisionEnv(a, n_envs=n, device=cuda, profiles=profiles)
-
-
-def reset(env, seed):
-    n = env.n_envs
-    rng = np.random.default_rng(seed)
-    start = rng.integers(0, env.max_start(), n).astype(np.int32)
-    e0 = rng.uniform(0.9 * 0.0125, 1.1 * 0.0125, (n, 5))
-    a0 = rng.uniform(0, 1, (n, 20))
-    env.reset(start, e0, a0, return_obs=False)
-
-
 def candidates(kind, rng, shape):
-    """Actions of one dtype kind: policy outputs for "policy", setpoints for the raw_actions ("raw") env."""
-    if kind == "raw":
-        a = rng.uniform(0, 1, shape) * np.array([0.5, 0.01, 0.01, 0.02])
-        return torch.from_numpy(a)
-    a = rng.normal(0.3, 0.6, shape)
-    return torch.from_numpy(a.astype(np.float64 if kind == "f64" else np.float32))
-
-
-def bits(t):
-    return t.view(torch.int64) if t.dtype == torch.float64 else t
+    return torch.from_numpy(actions(kind, rng, shape, 0.3))
 
 
 @pytest.mark.gpu
@@ -52,8 +28,8 @@ def bits(t):
 def test_preview_equals_the_following_step_over_an_episode(cuda, profiles, variant, kind, n):
     """At every step of a 95-step episode (the first step, the episode limit, done and the row in force included),
     preview_step(a) returns what step(a) then returns, and the voltages / mask that step leaves in the env."""
-    env = make(cuda, profiles, n, variant, **({"alg": "safemaddpg"} if kind == "raw" else {}))
-    reset(env, 1)
+    env = make_env(cuda, profiles, n, variant, **({"alg": "safemaddpg"} if kind == "raw" else {}))
+    env.reset(*draws(1, env), return_obs=False)
     rng = np.random.default_rng(2)
     translate = kind == "policy"
     n_failed = 0
@@ -89,14 +65,13 @@ def test_preview_equals_the_following_step_over_an_episode(cuda, profiles, varia
 def test_preview_touches_nothing(cuda, profiles, variant, k):
     """Heavy loading (thousands of violations), injected failures and NaN actions: the handle's state is
     byte-identical before and after previews, and the next step gives the bits of a twin env that never previewed."""
-    from flexgpu import Profiles
-    heavy = Profiles(profiles.P * 2.4, profiles.Q * 2.4, profiles.PV, profiles.price)
+    heavy = scaled_profiles(profiles, every_other_day=False)
     n = 1000
-    envs = [make(cuda, heavy, n, variant) for _ in range(2)]
+    envs = [make_env(cuda, heavy, n, variant) for _ in range(2)]
     rng = np.random.default_rng(5)
     for env in envs:
         env.keep_line_flows(True)
-        reset(env, 3)
+        env.reset(*draws(3, env), return_obs=False)
     for t in range(3):                                              # some history in both observation rings
         a = candidates("f32", np.random.default_rng(10 + t), (n, 5, 4))
         for env in envs:
@@ -136,8 +111,8 @@ def test_preview_touches_nothing(cuda, profiles, variant, k):
 @pytest.mark.parametrize("kind", ["f32", "f64"])
 def test_k_candidates_equal_k_single_calls(cuda, profiles, variant, kind, k):
     n = 777                                                         # not a multiple of 32
-    env = make(cuda, profiles, n, variant)
-    reset(env, 7)
+    env = make_env(cuda, profiles, n, variant)
+    env.reset(*draws(7, env), return_obs=False)
     rng = np.random.default_rng(8)
     env.step(candidates(kind, rng, (n, 5, 4)))                      # past the first step: the row in force moves
     cand = candidates(kind, rng, (k, n, 5, 4))
@@ -163,21 +138,20 @@ def test_preview_argument_and_state_checks(cuda, profiles, variant):
     from flexgpu import FlexGpuError
     from flexgpu.config import make_fp_config, normalize_args
     n = 40
-    env = make(cuda, profiles, n, variant)
-    reset(env, 1)
+    env = make_env(cuda, profiles, n, variant)
+    env.reset(*draws(1, env), return_obs=False)
     l, h = env._lib, env._h
     a = torch.rand(n, 5, 4, device=cuda)
     r = torch.empty(n, dtype=torch.float64, device=cuda)
     d = torch.empty(n, dtype=torch.uint8, device=cuda)
-    p = lambda t: C.c_void_p(t.data_ptr())
     s = _lib.stream(env.device)
-    assert l.fp_step_preview(h, 1, p(a), _lib.FP_F32, p(r), p(d), None, None, None, s) == 0
-    assert l.fp_step_preview(h, 1, None, _lib.FP_F32, p(r), p(d), None, None, None, s) == -1
-    assert l.fp_step_preview(h, 1, p(a), _lib.FP_F32, None, p(d), None, None, None, s) == -1
-    assert l.fp_step_preview(h, 1, p(a), _lib.FP_F32, p(r), None, None, None, None, s) == -1
-    assert l.fp_step_preview(h, 0, p(a), _lib.FP_F32, p(r), p(d), None, None, None, s) == -1
-    assert l.fp_step_preview(h, -3, p(a), _lib.FP_F32, p(r), p(d), None, None, None, s) == -1
-    assert l.fp_step_preview(h, 1, p(a), 7, p(r), p(d), None, None, None, s) == -1
+    assert l.fp_step_preview(h, 1, ptr(a), _lib.FP_F32, ptr(r), ptr(d), None, None, None, s) == 0
+    assert l.fp_step_preview(h, 1, None, _lib.FP_F32, ptr(r), ptr(d), None, None, None, s) == -1
+    assert l.fp_step_preview(h, 1, ptr(a), _lib.FP_F32, None, ptr(d), None, None, None, s) == -1
+    assert l.fp_step_preview(h, 1, ptr(a), _lib.FP_F32, ptr(r), None, None, None, None, s) == -1
+    assert l.fp_step_preview(h, 0, ptr(a), _lib.FP_F32, ptr(r), ptr(d), None, None, None, s) == -1
+    assert l.fp_step_preview(h, -3, ptr(a), _lib.FP_F32, ptr(r), ptr(d), None, None, None, s) == -1
+    assert l.fp_step_preview(h, 1, ptr(a), 7, ptr(r), ptr(d), None, None, None, s) == -1
     assert b"fp_step_preview" in l.fp_last_error(h)
     with pytest.raises(ValueError):
         env.preview_step(torch.rand(n + 1, 5, 4))
@@ -190,15 +164,15 @@ def test_preview_argument_and_state_checks(cuda, profiles, variant):
     hh = C.c_void_p()
     assert l.fp_create(C.byref(cfg), n, 0, C.byref(hh)) == 0
     try:
-        assert l.fp_step_preview(hh, 1, p(a), _lib.FP_F32, p(r), p(d), None, None, None, s) == -3
-        assert l.fp_step(hh, p(a), _lib.FP_F32, p(r), p(d), None, None, s) == -3
+        assert l.fp_step_preview(hh, 1, ptr(a), _lib.FP_F32, ptr(r), ptr(d), None, None, None, s) == -3
+        assert l.fp_step(hh, ptr(a), _lib.FP_F32, ptr(r), ptr(d), None, None, s) == -3
     finally:
         l.fp_destroy(hh)
-    env = make(cuda, profiles, n, variant)
+    env = make_env(cuda, profiles, n, variant)
     with pytest.raises(ValueError):
         env.preview_step(torch.rand(0, n, 5, 4))
     with pytest.raises(FlexGpuError):                                # failures of the entry point surface as FlexGpuError
-        env._check(l.fp_step_preview(env._h, 0, p(a), _lib.FP_F32, p(r), p(d), None, None, None, s), "fp_step_preview")
+        env._check(l.fp_step_preview(env._h, 0, ptr(a), _lib.FP_F32, ptr(r), ptr(d), None, None, None, s), "fp_step_preview")
     env.close()
 
 

@@ -19,7 +19,6 @@ the leg, the step, the candidate, the env and the first differing element.
   E  2^20 + 77 envs, K = 16: a 4.4 GB voltage output (byte offsets past 2^32), k N + e up to 1.7e7
   F  the C ABI into sentinel-filled buffers with guard bands, both variants, every combination of null outputs
 """
-import ctypes as C
 import itertools
 import time
 
@@ -28,8 +27,10 @@ import pytest
 import torch
 
 import _feeders as F
+from _env_check import actions, feeder_profiles, make_env, ptr, reset_both, same, same_outputs, scaled_profiles, step_both
+from _env_check import all_cores  # noqa: F401  (autouse fixture)
 from _feeders import assert_same_bytes, snapshot
-from _preview_ref import mirror_preview, same, same_outputs
+from _preview_ref import mirror_preview
 from flexgpu import _lib
 from oracle import c_mirror, ieee33
 
@@ -38,27 +39,10 @@ N = 131072 + 19
 NA = 5
 
 
-@pytest.fixture(scope="module", autouse=True)
-def all_cores():
-    c_mirror.use_all_cores()
-
-
-def heavy(p):
-    """Every other day's demand x 2.4 (an episode spans a normal and a heavily loaded day)."""
-    from flexgpu.profiles import Profiles
-    f = np.where((np.arange(p.P.shape[0]) // 96) % 2 == 1, 2.4, 1.0)[:, None]
-    return Profiles(p.P * f, p.Q * f, p.PV, p.price)
-
-
 @pytest.fixture(scope="module")
 def loaded(profiles):
-    return heavy(profiles)
-
-
-def make(cuda, prof, n, variant="thread", net=None, seed=1, **extra):
-    from flexgpu import BatchedFlexProvisionEnv
-    args = F.env_args(net, variant, **extra) if net is not None else dict(kernel_variant=variant, **extra)
-    return BatchedFlexProvisionEnv(args, n_envs=n, device=cuda, network=net, profiles=prof, seed=seed)
+    """Every other day's demand x 2.4 (an episode spans a normal and a heavily loaded day)."""
+    return scaled_profiles(profiles, every_other_day=True)
 
 
 def loops(cuda, k, n):
@@ -72,13 +56,7 @@ def loops(cuda, k, n):
 def candidates(g, kind, k, n, na=NA):
     """[K, N, na, 4] candidate actions on the device: fp32 / fp64 policy outputs, raw fp32 outputs to translate
     ("policy") or fp64 setpoints ("raw"); NaN at the candidate boundaries and at a tile edge."""
-    dev = g.device
-    if kind == "raw":
-        a = torch.rand(k, n, na, 4, dtype=torch.float64, device=dev, generator=g)
-        a *= torch.tensor([0.5, 0.01, 0.01, 0.02], dtype=torch.float64, device=dev)
-    else:
-        a = torch.randn(k, n, na, 4, dtype=torch.float64 if kind == "f64" else torch.float32, device=dev, generator=g)
-        a = a * 0.6 + 0.4
+    a = actions(kind, g, (k, n, na, 4), 0.4)
     for j in range(k):
         if j % 2 == 0:
             a[j, n - 1, j % na, j % 4] = float("nan")                          # last lane of the ragged tile
@@ -113,11 +91,6 @@ def check(out, want, where):
     return failed, violated
 
 
-def mirror_actions(a, translate):
-    a = a.cpu().numpy()
-    return c_mirror.translate_action_f32(a) if translate else a
-
-
 def check_commit(env, mb, out, step_out, where):
     """A step committing the preview's last candidate returned its bits and left its voltages and mask, the mirror's."""
     r, d, info = step_out
@@ -129,23 +102,6 @@ def check_commit(env, mb, out, step_out, where):
     same(env.setpoints, mb.setp, "setpoints", f"{where}: step vs mirror")
 
 
-def step_both(env, mb, a, where, translate=False, inject=None):
-    """One committed step of the env and the mirror; reward, done and info compared."""
-    r, d, info = env.step(a, translate=translate)
-    rr, dd, ii = mb.step(mirror_actions(a, translate), inject=inject)
-    same(r, rr, "reward", where); same(d, dd, "done", where)
-    same(env._info, ii, "info", where)
-    return r, d, info
-
-
-def reset_drawn(env, mb, rng, mask=None):
-    """An explicit reset of both batches from host draws (mask: the envs to reset)."""
-    n, na = env.n_envs, env.n_agents
-    start = rng.integers(0, env.max_start(), n).astype(np.int32)
-    e0, a0 = rng.uniform(0.9 * 0.0125, 1.1 * 0.0125, (n, na)), rng.uniform(0, 1, (n, 4 * na))
-    env.reset(start, e0, a0, mask=mask, return_obs=False); mb.reset(start, e0, a0, mask=mask)
-
-
 def test_a_thread_variant_over_an_episode(cuda, loaded, fonets):
     """Leg A: 30 steps, a reset of a random half (steps differ within a tile), then a 95-step episode whose done envs of
     even index are reset after every step while the odd ones step on past done into the row clamp.  Six steps preview
@@ -153,13 +109,13 @@ def test_a_thread_variant_over_an_episode(cuda, loaded, fonets):
     failures, K = 1, fp32 K = 16 again and fp64 K = 5 at the last step; the handle's bytes are unchanged by each, and
     the step committing candidate K - 1 returns its bits."""
     t0 = time.time()
-    env = make(cuda, loaded, N, seed=21)
+    env = make_env(cuda, loaded, N, seed=21)
     mb = c_mirror.MirrorBatch(fonets["thread"], loaded.as_dict(), N)
     env.reset(return_obs=False, retries=0); mb.reset_random(21)
     g = torch.Generator(device=cuda).manual_seed(22)
     rng = np.random.default_rng(23)
     for t in range(30):
-        step_both(env, mb, torch.randn(N, NA, 4, device=cuda, generator=g) * 0.6 + 0.4, f"A warm-up step {t}")
+        step_both(env, mb, actions("f32", g, (N, NA, 4), 0.4), f"A warm-up step {t}")
     m = (rng.uniform(size=N) < 0.5).astype(np.uint8)
     env.reset(mask=m, return_obs=False, retries=0); mb.reset_random(21, mask=m)
     plan = {0: ("f32", 16), 19: ("f64", 5), 45: ("policy", 8), 60: ("f32", 1), 77: ("f32", 16), 94: ("f64", 5)}
@@ -185,7 +141,7 @@ def test_a_thread_variant_over_an_episode(cuda, loaded, fonets):
             failed += f; violated += v
             a = cand[k - 1]
         else:
-            a = torch.randn(N, NA, 4, device=cuda, generator=g) * 0.6 + 0.4
+            a = actions("f32", g, (N, NA, 4), 0.4)
         step = step_both(env, mb, a, where, translate, inj)
         if k:
             check_commit(env, mb, out, step, where)
@@ -208,10 +164,10 @@ def test_b_raw_actions(cuda, loaded, tree, args):
     t0 = time.time()
     k = 5
     loops(cuda, k, N)
-    env = make(cuda, loaded, N, alg="safemaddpg")
+    env = make_env(cuda, loaded, N, seed=1, alg="safemaddpg")
     mb = c_mirror.MirrorBatch(c_mirror.make_net(tree, args, args["buildings"], raw_actions=True), loaded.as_dict(), N)
     rng = np.random.default_rng(31)
-    reset_drawn(env, mb, rng)
+    reset_both(env, mb, rng)
     g = torch.Generator(device=cuda).manual_seed(32)
     for t in range(3):
         step_both(env, mb, candidates(g, "raw", 1, N)[0], f"B step {t}")
@@ -230,7 +186,7 @@ def test_c_warp_variant(cuda, loaded, fonets):
     """Leg C: the warp kernel over K N virtual envs: fp32 K = 16, fp64 K = 4, then translated candidates with K = 1, 16
     (the FP_F32_POLICY scratch grows) and 4 (it is reused), then a translated step through the same scratch."""
     t0 = time.time()
-    env = make(cuda, loaded, N, "warp", seed=41)
+    env = make_env(cuda, loaded, N, "warp", seed=41)
     mb = c_mirror.MirrorBatch(fonets["warp"], loaded.as_dict(), N)
     env.reset(return_obs=False, retries=0); mb.reset_random(41)
     g = torch.Generator(device=cuda).manual_seed(42)
@@ -259,20 +215,18 @@ def test_c_warp_variant(cuda, loaded, fonets):
 def test_d_run_time_shape(cuda, name):
     """Leg D: k_env_t<MODE_PREVIEW, RtShape, ..> with na < 5 (the staged fp32 actions are n_left na 16-byte chunks),
     N = 100 000 + 13 (tpk = 3 126), fp32 and fp64 candidates, K = 7, two steps apart."""
-    from flexgpu.network import Network
-    from flexgpu.profiles import synthetic_profiles
     t0 = time.time()
     net = F.feeder(name)
-    prof = heavy(synthetic_profiles(Network(net), len(net['buildings']), T=1500, seed=3))
+    prof = scaled_profiles(feeder_profiles(net), every_other_day=True)
     n, k = 100000 + 13, 7
     loops(cuda, k, n)
-    env = make(cuda, prof, n, net=net)
+    env = make_env(cuda, prof, n, net=net, seed=1)
     na = env.n_agents
     assert na < 5
     fonet = c_mirror.make_net(ieee33.tree_arrays(net), F.env_args(net), net['buildings'])
     mb = c_mirror.MirrorBatch(fonet, prof.as_dict(), n)
     rng = np.random.default_rng(51)
-    reset_drawn(env, mb, rng)
+    reset_both(env, mb, rng)
     g = torch.Generator(device=cuda).manual_seed(52)
     failed = 0
     for t in range(5):
@@ -300,7 +254,7 @@ def test_e_two_pow_20_envs(cuda, loaded, fonets):
     t0 = time.time()
     n, k = 2 ** 20 + 77, 16
     loops(cuda, k, n)
-    env = make(cuda, loaded, n, seed=61)
+    env = make_env(cuda, loaded, n, seed=61)
     mb = c_mirror.MirrorBatch(fonets["thread"], loaded.as_dict(), n)
     env.reset(return_obs=False, retries=0); mb.reset_random(61)
     g = torch.Generator(device=cuda).manual_seed(62)
@@ -347,7 +301,7 @@ def test_f_outputs_through_the_c_abi(cuda, loaded, fonets, variant):
     k = 5
     if variant == "thread":
         loops(cuda, k, N)
-    env = make(cuda, loaded, N, variant, seed=71)
+    env = make_env(cuda, loaded, N, variant, seed=71)
     mb = c_mirror.MirrorBatch(fonets[variant], loaded.as_dict(), N)
     env.reset(return_obs=False, retries=0); mb.reset_random(71)
     g = torch.Generator(device=cuda).manual_seed(72)
@@ -357,14 +311,12 @@ def test_f_outputs_through_the_c_abi(cuda, loaded, fonets, variant):
     nb = env.n_bus
     shapes = {"reward": (k * N, torch.float64), "done": (k * N, torch.uint8), "info": (k * N * 8, torch.float64),
               "voltage": (k * N * nb, torch.float64), "mask": (k * N, torch.int64)}
-    p = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
-
     def call(want, where):
         bufs = {key: guarded(cnt, dt, SENTINELS[dt], cuda) for key, (cnt, dt) in shapes.items()
                 if key in ("reward", "done") or key in want}
         pay = {key: b[1] for key, b in bufs.items()}
-        rc = l.fp_step_preview(h, k, p(cand), _lib.FP_F32, p(pay["reward"]), p(pay["done"]), p(pay.get("info")),
-                               p(pay.get("voltage")), p(pay.get("mask")), s)
+        rc = l.fp_step_preview(h, k, ptr(cand), _lib.FP_F32, ptr(pay["reward"]), ptr(pay["done"]), ptr(pay.get("info")),
+                               ptr(pay.get("voltage")), ptr(pay.get("mask")), s)
         assert rc == 0, (where, l.fp_last_error(h))
         torch.cuda.synchronize()
         for key, (buf, _, pre) in bufs.items():

@@ -9,6 +9,7 @@ import torch
 
 import _feeders as F
 import _rollout_ref as R
+from _env_check import feeder_profiles, make_env
 
 pytestmark = pytest.mark.gpu
 AGENTS = [1, 2, 3, 4]
@@ -87,12 +88,8 @@ ROLLOUT_CASES = [("two_bus", "thread"), ("slack_star", "thread"), ("custom14", "
 
 
 def _feeder_env(cuda, name, variant, n, seed=1, **extra):
-    from flexgpu import BatchedFlexProvisionEnv
-    from flexgpu.network import Network
-    from flexgpu.profiles import synthetic_profiles
     net = F.feeder(name)
-    prof = synthetic_profiles(Network(net), len(net['buildings']), T=1500, seed=3)
-    return BatchedFlexProvisionEnv(F.env_args(net, variant, **extra), n_envs=n, device=cuda, network=net, profiles=prof, seed=seed)
+    return make_env(cuda, feeder_profiles(net), n, variant, net=net, seed=seed, **extra)
 
 
 @pytest.mark.parametrize("value_kind", ["native", "torch"])

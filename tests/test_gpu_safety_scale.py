@@ -35,6 +35,7 @@ import torch
 
 import _feeders as F
 import _safety_batch_ref as B
+from _env_check import feeder_profiles, make_env, ptr
 from oracle import ieee33, safety_ref
 
 pytestmark = pytest.mark.gpu
@@ -71,10 +72,6 @@ class _Out:
         assert not bool((bits[:self.n] == s).any()), f"{what}: an element was not written"
 
 
-def _ptr(t):
-    return C.c_void_p(t.data_ptr())
-
-
 @pytest.fixture(scope="module")
 def stream(cuda):
     return torch.cuda.Stream(device=cuda)
@@ -90,7 +87,7 @@ def _rowsum(env, actions, tm, stream, slack=True, moved=True):
     m = _Out(N * na, torch.uint8, dev) if moved else None
     torch.cuda.synchronize()
     with torch.cuda.stream(stream):
-        env._check(env._lib.fp_safety_project(env._h, _ptr(actions), 1 if actions.dtype == torch.float64 else 0, o.ptr(),
+        env._check(env._lib.fp_safety_project(env._h, ptr(actions), 1 if actions.dtype == torch.float64 else 0, o.ptr(),
                                               1 if tm else 0, s.ptr() if s else None, m.ptr() if m else None,
                                               C.c_void_p(stream.cuda_stream)), "fp_safety_project")
     stream.synchronize()
@@ -111,7 +108,7 @@ def _affine(env, actions, tm, stream, slack=True, moved=True, status=True):
     st = _Out(N, torch.int32, dev) if status else None
     torch.cuda.synchronize()
     with torch.cuda.stream(stream):
-        env._check(env._lib.fp_safety_project_affine(env._h, _ptr(actions), 1 if actions.dtype == torch.float64 else 0, o.ptr(),
+        env._check(env._lib.fp_safety_project_affine(env._h, ptr(actions), 1 if actions.dtype == torch.float64 else 0, o.ptr(),
                                                      1 if tm else 0, s.ptr() if s else None, m.ptr() if m else None,
                                                      st.ptr() if st else None, C.c_void_p(stream.cuda_stream)),
                    "fp_safety_project_affine")
@@ -211,15 +208,8 @@ _CACHE = {}
 def _batch(cuda, profiles, N, net=None, name=None):
     key = (name or "ieee33", N)
     if key not in _CACHE:
-        from flexgpu import BatchedFlexProvisionEnv
         seed = 1000 + N % 977
-        if net is None:
-            env = BatchedFlexProvisionEnv(None, n_envs=N, device=cuda, profiles=profiles, seed=seed)
-        else:
-            from flexgpu.network import Network
-            from flexgpu.profiles import synthetic_profiles
-            prof = synthetic_profiles(Network(net), len(net['buildings']), T=1500, seed=3)
-            env = BatchedFlexProvisionEnv(F.env_args(net, "thread"), n_envs=N, device=cuda, network=net, profiles=prof, seed=seed)
+        env = make_env(cuda, profiles if net is None else feeder_profiles(net), N, net=net, seed=seed)
         role = _drive(env, seed)
         _CACHE[key] = Batch(env, role, seed + 7)
     return _CACHE[key]

@@ -1,12 +1,16 @@
-"""CPU: tests/_preview_ref.py, the step preview's reference, on the C mirror alone.  mirror_preview() leaves the batch
-byte-identical, gives candidate j what a fresh batch in the same state gives for one step of candidate j (injected
-failures, NaN actions, translated actions and voltage violations included), and permutes with its candidates; same()
-compares bits and names the candidate and the env of a mismatch."""
+"""CPU: the step preview's reference (tests/_preview_ref.py) and the env-parity comparisons (tests/_env_check.py), on
+the C mirror alone.  mirror_preview() leaves the batch byte-identical, gives candidate j what a fresh batch in the same
+state gives for one step of candidate j (injected failures, NaN actions, translated actions and voltage violations
+included), and permutes with its candidates; same() compares bits and names the candidate and the env of a mismatch;
+check_state() names any one field of the state that differs from the mirror's."""
+from types import SimpleNamespace
+
 import numpy as np
 import pytest
 import torch
 
-from _preview_ref import mirror_copy, mirror_preview, same, same_outputs
+from _env_check import check_state, reset_draws, same, same_outputs, scaled_profiles
+from _preview_ref import mirror_copy, mirror_preview
 from oracle import c_mirror
 
 N, NA, K = 32 * 3 + 5, 5, 6
@@ -16,17 +20,14 @@ NAN_ENV = {1: N - 1, 2: 0, 4: 31}                                       # candid
 @pytest.fixture(scope="module")
 def heavy(profiles):
     """Every other day's demand x 2.4: voltage violations and some failed solves."""
-    from flexgpu.profiles import Profiles
-    f = np.where((np.arange(profiles.P.shape[0]) // 96) % 2 == 1, 2.4, 1.0)[:, None]
-    return Profiles(profiles.P * f, profiles.Q * f, profiles.PV, profiles.price).as_dict()
+    return scaled_profiles(profiles, every_other_day=True).as_dict()
 
 
 def batch(fonet, heavy):
     """A batch a few steps into an episode, the same every call: varied rows in force, energies and setpoints."""
     mb = c_mirror.MirrorBatch(fonet, heavy, N)
     rng = np.random.default_rng(1)
-    start = rng.integers(0, mb.start_range, N).astype(np.int32)
-    mb.reset(start, rng.uniform(0.9 * 0.0125, 1.1 * 0.0125, (N, NA)), rng.uniform(0, 1, (N, 4 * NA)))
+    mb.reset(*reset_draws(rng, N, NA, mb.start_range))
     for _ in range(3):
         mb.step(rng.normal(0.4, 0.6, (N, NA, 4)).astype(np.float32))
     return mb
@@ -144,3 +145,45 @@ def test_same_outputs_checks_every_part(fonet, heavy):
         with pytest.raises(AssertionError, match=f"{what} differs at env 7" if part == 2 else what):
             same_outputs(bad, want, "x")
         same_outputs(bad, want, "x", info=part != 2, voltage=part != 3, mask=part != 4)
+
+
+# ------------------------------------------------------------------ check_state
+FLIPS = [("E_init", 4, 0), ("E_cur", 5, 51), ("cumulative reward", 10, 62), ("start", 11, 2), ("steps", 11, 33),
+         ("push count", 12, 4), ("episode", 12, 40), ("violation mask", 13, 32), ("violation count", 14, 1),
+         ("flags", 14, 34), ("line-limit mask", 15, 31), ("power-flow passes", 15, 32)]    # (field, record word, bit)
+
+
+def test_check_state_names_every_field(fonet, heavy):
+    """check_state() passes on a stand-in env whose record, voltages and setpoints are the mirror's state, and names the
+    field and the env of any one flipped bit: each field of the 16 record words, the voltages and the setpoints.  The
+    push count is compared only when it is given."""
+    mb = batch(fonet, heavy)
+    mb.step(candidates()[0], inject=inject_mask())                      # failed envs: flags and rolled-back voltages
+    pushes = np.arange(N) % 25
+
+    def u64(lo, hi):
+        return (lo.astype(np.uint32).astype(np.uint64) | (hi.astype(np.uint32).astype(np.uint64) << np.uint64(32))).view(
+            np.int64)
+
+    def stand_in():
+        rec = np.empty((N, 16), dtype=np.int64)
+        rec[:, 0:5] = mb.E_init.view(np.int64); rec[:, 5:10] = mb.E_cur.view(np.int64); rec[:, 10] = mb.cum.view(np.int64)
+        rec[:, 11] = u64(mb.start, mb.steps); rec[:, 12] = u64(pushes, mb.episode); rec[:, 13] = mb.vmask.view(np.int64)
+        rec[:, 14] = u64(mb.vcount, mb.flags); rec[:, 15] = u64(mb.lmask, mb.iters)
+        return SimpleNamespace(rec=torch.from_numpy(rec), voltages=torch.from_numpy(mb.V.copy()),
+                               setpoints=torch.from_numpy(mb.setp.copy()))
+
+    assert (mb.flags != 0).any() and (mb.vmask != 0).any() and (mb.lmask != 0).any()
+    check_state(stand_in(), mb, "pin", pushes=pushes)
+    for k, (field, word, bit) in enumerate(FLIPS):
+        env, e = stand_in(), (37 * k + 5) % N
+        env.rec[e, word] ^= 1 << bit
+        with pytest.raises(AssertionError, match=f"pin: {field} differs at env {e},"):
+            check_state(env, mb, "pin", pushes=pushes)
+        if field == "push count":
+            check_state(env, mb, "pin")
+    for k, field in enumerate(("voltages", "setpoints")):
+        env, e = stand_in(), 3 + k
+        getattr(env, field).view(torch.int64).view(N, -1)[e, 7] ^= 1
+        with pytest.raises(AssertionError, match=f"pin: {field} differs at env {e},"):
+            check_state(env, mb, "pin")
